@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference algorithm on the host CPU (oracle port)
+    python bench.py --steps K --warmup W --dump-outputs DIR  # also write the outputs of the last timed step, to compare builds
 
 A "step" is one full training step (butterfly FIR -> soft demapper -> ELBO -> backward -> Adam on both
 parameter groups) over one minibatch of B = 2^22 synthetic DP 64-QAM PCS symbols (BASELINE configs[1]:
@@ -41,6 +42,7 @@ ALG_FLOP_PER_SYMBOL = 5 * 32 * M_EST + 1000                      # SURVEY.md §8
 FWD_DRAM_BYTES_PER_SYMBOL = (134.307e6 + 949.731e6) / (1 << 22)
 TRAFFIC_SOURCE = "ncu --set full dram__bytes_read.sum + dram__bytes_write.sum of k_dp_fwd_tc<8,12>, profiles/r02c_ncu_full_summary.json, scaled to this batch_len"
 CPU_SAMPLE_LOG2 = 17
+DUMP_SAMPLE_LOG2 = 18                                            # --dump-outputs: q / out columns kept (2^18 symbols = 36 MiB of float32)
 
 
 def load_peaks():
@@ -166,6 +168,19 @@ def reference_arm(args, rank, world):
     print(json.dumps(line), flush=True)
 
 
+def dump_outputs(eq, q, out, d):
+    """Write what the last train_step handed its caller to d/<name>.npy (float32): q and out on a fixed, seeded sample of
+    2^DUMP_SAMPLE_LOG2 symbol columns (all columns at smaller batch_len), loss, var_est, and the taps W and h after its Adam update."""
+    B = q.shape[-1]
+    n = min(B, 1 << DUMP_SAMPLE_LOG2)
+    cols = np.sort(np.random.default_rng(0).choice(B, n, replace=False))
+    idx = torch.from_numpy(cols).to(q.device)
+    arrays = {"q": q.index_select(2, idx), "out": out.index_select(2, idx), "loss": eq.loss, "var_est": eq.var_est, "W": eq.W, "h": eq.h}
+    os.makedirs(d, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), t.cpu().numpy())
+
+
 def ours_arm(args, rank, local_rank, world):
     import torch.distributed as dist
     from vae_equalizer_b200 import _lib
@@ -223,6 +238,8 @@ def ours_arm(args, rank, local_rank, world):
     ms = e0.elapsed_time(e1)
     clocks = sampler.finish()
     launches = launches_per_step * K
+    if args.dump_outputs and rank == 0:                # before the legs below overwrite q / out and step the taps further
+        dump_outputs(eq, q, out, args.dump_outputs)
     # ---- the same K steps as plain launches, and once more with the library's per-kernel event pairs on the launching stream
     # (12 event records per step: they cost ~30 us per step, so they stay out of the region `value` is taken from) ------------------
     p0, p1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -502,7 +519,11 @@ def main():
     ap.add_argument("--sustained-seconds", type=float, default=1.5)
     ap.add_argument("--m-est", type=int, default=M_EST, help="equalizer / channel-estimate taps (default 25 = the BASELINE config; "
                     "5, 9, 13 show the HBM-bound regime, SURVEY.md §8d)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy (rank 0; "
+                    "q and out on a fixed sample of 2^%d symbols)" % DUMP_SAMPLE_LOG2)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.m_est != M_EST:
         globals()["M_EST"] = args.m_est
         globals()["ALG_FLOP_PER_SYMBOL"] = 5 * 32 * args.m_est + 1000

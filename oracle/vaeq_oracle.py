@@ -519,12 +519,17 @@ def awgn_forward(x, w, amp, amp_mean, var, sps):
     oI = F.conv1d(lane_i, w, stride=sps, padding=pad)[0, 0]
     oQ = F.conv1d(lane_q, w, stride=sps, padding=pad)[0, 0]
     out = torch.stack((oI, oQ))
+    return awgn_demap(out, amp, amp_mean, var), out
+
+
+def awgn_demap(out, amp, amp_mean, var):
+    """The demapper of twoFIR.forward (awgn:228-231): out (2,N) -> q (2n,N)."""
     a = amp.view(-1, 1)
     q = []
     for c in range(2):
         yn = out[c] / torch.mean(torch.abs(out[c])) * amp_mean
         q.append(F.softmin((yn - a) ** 2 / var, dim=0))
-    return torch.cat(q, dim=0), out
+    return torch.cat(q, dim=0)
 
 
 def awgn_loss(q, rx, h, amp, P):
