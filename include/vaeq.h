@@ -372,6 +372,17 @@ int vaeq_gen_jones(float *X, const float *Pcd, const float *Picd, const float *t
                    void *stream);
 /* sf:83-88: rx (n_runs,2,2,L) float32 = Re/Im of sig[:, :, :L] + sigma[run] * N(0,1); sig (n_runs,2,n) complex64, L <= n */
 int vaeq_gen_noise(const float *sig, const float *sigma, uint64_t seed, int32_t n, int32_t L, float *rx, int32_t n_runs, void *stream);
+/* Single-polarisation signal of the AWGN module (generate_data, AWGN_channel/func_VAELE_MQAM_shaping.py:39-61), n_frames frames
+ * (frame indices frame0 ..) of N symbols for each of n_runs runs, all sps = 2:
+ *   lev (n_runs, n_frames, 2, n_conv) f32   levels drawn from P (n_runs, n_lev) by inverse CDF
+ *   sig (n_runs, n_frames, 2 n_conv - K) complex64   'valid' FIR of the zero-stuffed symbols with taps (K complex, re/im interleaved,
+ *       even K: rrcfir (*) h_channel), noise-free
+ *   rx  (n_runs, n_frames, 2, 2 N) f32   sig[:2N] + sigma_n (N(0,1) + j N(0,1)), sigma_n from the frame's mean |sig|^2 and snr[run] dB
+ *   tx  (n_runs, n_frames, 2, N) float16 bits   lev[:, tx_off : tx_off + N]
+ * Every draw is keyed by (seeds[run], frame index, row, position): a run's frames do not depend on the other runs of the call. */
+int vaeq_gen_awgn(const float *amps, const float *P, int32_t n_lev, const float *taps, int32_t K, int32_t N, int32_t tx_off, int32_t n_conv,
+                  const float *snr, const uint64_t *seeds, int32_t frame0, int32_t n_frames, int32_t n_runs, float *lev, float *sig, float *rx,
+                  uint16_t *tx, void *stream);
 
 /* ------------------------------------------------------------------------------------------------
  * AWGN single-polarisation VAE-LE step: twoFIR.forward (AWGN_channel/func_VAELE_MQAM_shaping.py:214-231)
@@ -398,6 +409,34 @@ size_t vaeq_adam_state_floats_awgn(int32_t M);
 int vaeq_awgn_forward(const vaeq_awgn_desc *d, void *stream);
 int vaeq_awgn_forward_backward(const vaeq_awgn_desc *d, void *stream);
 int vaeq_awgn_train_step(const vaeq_awgn_desc *d, float lr_w, float lr_h, void *stream);
+
+/* R independent runs in ONE launch, one CTA of the single-run step kernel per run (sweep engine): bit for bit a loop of
+ * vaeq_awgn_train_step / vaeq_awgn_forward per run.  `d` holds run 0's pointers (d->var and d->amp_mean are ignored: per-run
+ * values come from `r`); run k's arrays start at d->X + k * r->rs_X (elements).  workspace: vaeq_awgn_runs_workspace_bytes. */
+typedef struct vaeq_awgn_runs {
+    int32_t n_runs;
+    int64_t rs_rx, rs_W, rs_h, rs_adam, rs_P, rs_q, rs_out, rs_loss;
+    const float *lr;       /* (n_runs) Adam lr of both parameter groups (:305-306); train only */
+    const float *var;      /* (n_runs) 10^(-SNR/10) */
+    const float *amp_mean; /* (n_runs) */
+} vaeq_awgn_runs;
+size_t vaeq_awgn_runs_workspace_bytes(int32_t B, int32_t M, int32_t n_lev, int32_t n_runs);
+/* n_frames frames per run, each n_mb minibatches of B = d->B symbols (the epoch loop of :291-306; the frame's remaining symbols are
+ * unused): minibatch m of frame f is rx + f*fs_rx + m*sps*B, its Q row ld_rx after its I row.  d->q (2n,B) / d->out (2,B) per run are
+ * scratch; d->loss (n_runs, n_frames*n_mb) receives every step's loss (row stride r->rs_loss). */
+int vaeq_awgn_train_frames_runs(const vaeq_awgn_desc *d, const vaeq_awgn_runs *r, int64_t ld_rx, int64_t fs_rx, int32_t n_frames,
+                                int32_t n_mb, void *stream);
+/* forward of every run over B = d->B symbols (rx rows ld_rx apart): q (2n,B), out (2,B) and loss per run */
+int vaeq_awgn_forward_runs(const vaeq_awgn_desc *d, const vaeq_awgn_runs *r, int64_t ld_rx, void *stream);
+/* Validation scoring of the AWGN driver (processing.py awgn_find_shift + awgn_ser_q, :188-204, :97-124) for n_runs runs without a
+ * host sync.  q (n_runs, 2n, N): rows ld_q apart, runs rs_q apart; tx (n_runs, 2, N) float16 bits.  Shift search on the first
+ * n_corr symbols (circular), E from q's I rows, correlated with tx I and tx Q; then the counts of q[:, edge+shift : N-edge] against
+ * tx[:, edge : N-edge-shift] for the 4 rotations (no IQ flip).  Outputs: shift (n_runs), counts (n_runs, 4), ser (n_runs).
+ * scratch: vaeq_awgn_eval_scratch_bytes. */
+size_t vaeq_awgn_eval_scratch_bytes(int32_t n_runs, int32_t n_shift, int32_t n_corr);
+int vaeq_awgn_eval_runs(const float *q, int64_t ld_q, int64_t rs_q, const uint16_t *tx, int64_t ld_tx, int64_t rs_tx, const float *amp,
+                        int32_t n_lev, int32_t N, int32_t n_shift, int32_t n_corr, int32_t edge, int32_t n_runs, int32_t *shift_out,
+                        int32_t *counts_out, float *ser_out, void *scratch, void *stream);
 
 #ifdef __cplusplus
 }

@@ -53,6 +53,16 @@ class PeerComm(C.Structure):
     _fields_ = [("rank", C.c_int32), ("world", C.c_int32), ("slot", C.c_void_p * 8), ("epoch", C.c_void_p)]
 
 
+class AwgnRuns(C.Structure):
+    """Mirror of `struct vaeq_awgn_runs`: run strides (elements) and per-run values of the batched AWGN calls."""
+    _fields_ = [
+        ("n_runs", C.c_int32),
+        ("rs_rx", C.c_int64), ("rs_W", C.c_int64), ("rs_h", C.c_int64), ("rs_adam", C.c_int64), ("rs_P", C.c_int64),
+        ("rs_q", C.c_int64), ("rs_out", C.c_int64), ("rs_loss", C.c_int64),
+        ("lr", C.c_void_p), ("var", C.c_void_p), ("amp_mean", C.c_void_p),
+    ]
+
+
 class AwgnDesc(C.Structure):
     """Mirror of `struct vaeq_awgn_desc`."""
     _fields_ = [
@@ -132,6 +142,12 @@ PROTOTYPES = {
     "vaeq_awgn_forward": (C.c_int, [C.POINTER(AwgnDesc), _vp]),
     "vaeq_awgn_forward_backward": (C.c_int, [C.POINTER(AwgnDesc), _vp]),
     "vaeq_awgn_train_step": (C.c_int, [C.POINTER(AwgnDesc), _f, _f, _vp]),
+    "vaeq_awgn_runs_workspace_bytes": (_sz, [_i32, _i32, _i32, _i32]),
+    "vaeq_awgn_train_frames_runs": (C.c_int, [C.POINTER(AwgnDesc), C.POINTER(AwgnRuns), _i64, _i64, _i32, _i32, _vp]),
+    "vaeq_awgn_forward_runs": (C.c_int, [C.POINTER(AwgnDesc), C.POINTER(AwgnRuns), _i64, _vp]),
+    "vaeq_awgn_eval_scratch_bytes": (_sz, [_i32, _i32, _i32]),
+    "vaeq_awgn_eval_runs": (C.c_int, [_vp, _i64, _i64, _vp, _i64, _i64, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp]),
+    "vaeq_gen_awgn": (C.c_int, [_vp, _vp, _i32, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp]),
 }
 
 _lib = None

@@ -15,6 +15,7 @@ struct AwK {
     int B, L, M, mh, n_lev;
     float amp_mean, var;
     const float *rx, *amp, *P;
+    int64_t ld_rx;  // element stride between the I and Q rows of rx
     float *W, *h, *adam;
     float *q, *out, *loss, *gW_out, *gh_out;
     // scratch
@@ -45,8 +46,10 @@ __device__ __forceinline__ void adam_apply_awgn(float *param, float g, float *m,
     param[i] = __fadd_rn(param[i], __fmul_rn(step_size, __fdiv_rn(mi, __fadd_rn(__fdiv_rn(sqrtf(vv), bc2s), eps))));
 }
 
+// One step of one run by a whole CTA of AW_NT threads (the single-run kernel and the batched-runs kernel share it, so both give
+// the same bits).  Ends with a barrier: the caller may start the next step of the same run right away.
 template <int NL>
-__global__ void __launch_bounds__(AW_NT) k_awgn_step(AwK p) {
+__device__ __forceinline__ void awgn_step_body(const AwK p) {
     __shared__ DemapConst cst;
     __shared__ float Ws[2 * VAEQ_MAX_TAPS], hs[2 * VAEQ_MAX_TAPS], Ssh[VAEQ_MAX_TAPS], PSg[VAEQ_MAX_TAPS + 1];
     __shared__ double red[4 * 32];
@@ -75,7 +78,7 @@ __global__ void __launch_bounds__(AW_NT) k_awgn_step(AwK p) {
         for (int k = 0; k < M; ++k) {
             const int s = 2 * t + k - mh;
             if (s < 0 || s >= L) continue;
-            const float xI = p.rx[s], xQ = p.rx[L + s];
+            const float xI = p.rx[s], xQ = p.rx[p.ld_rx + s];
             oI += Ws[k] * xI + Ws[M + k] * xQ;
             oQ += Ws[k] * xQ - Ws[M + k] * xI;
         }
@@ -139,7 +142,7 @@ __global__ void __launch_bounds__(AW_NT) k_awgn_step(AwK p) {
                 di += hs[j] * eQ + hs[M + j] * eI;                                  // :87
             }
             er = dr - p.rx[s];
-            ei = di - p.rx[L + s];
+            ei = di - p.rx[p.ld_rx + s];
             accC[0] += (double)(er * er + ei * ei);
         }
         p.e[2 * s] = er;
@@ -226,7 +229,7 @@ __global__ void __launch_bounds__(AW_NT) k_awgn_step(AwK p) {
             for (int t = 0; t < B; ++t) {
                 const int s = 2 * t + k - mh;
                 if (s < 0 || s >= L) continue;
-                const float gI = p.gout[t], gQ = p.gout[B + t], xI = p.rx[s], xQ = p.rx[L + s];
+                const float gI = p.gout[t], gQ = p.gout[B + t], xI = p.rx[s], xQ = p.rx[p.ld_rx + s];
                 g += c ? (gI * xQ - gQ * xI) : (gI * xI + gQ * xQ);
             }
             if (p.gW_out) p.gW_out[idx] = g;
@@ -250,6 +253,11 @@ __global__ void __launch_bounds__(AW_NT) k_awgn_step(AwK p) {
     if (tid == 0 && p.mode == DP_MODE_TRAIN) *step_ptr = step_sh;
 }
 
+template <int NL>
+__global__ void __launch_bounds__(AW_NT) k_awgn_step(AwK p) {
+    awgn_step_body<NL>(p);
+}
+
 static size_t awgn_ws_floats(int B) { return (size_t)2 * B + B + 4 * (size_t)B + 2 * B + 2 * B + 64; }
 
 static int awgn_launch(const vaeq_awgn_desc *d, int mode, float lr_w, float lr_h, cudaStream_t st) {
@@ -266,7 +274,7 @@ static int awgn_launch(const vaeq_awgn_desc *d, int mode, float lr_w, float lr_h
     }
     AwK p;
     memset(&p, 0, sizeof(p));
-    p.B = d->B; p.L = d->B * 2; p.M = d->M; p.mh = d->M / 2; p.n_lev = d->n_lev;
+    p.B = d->B; p.L = d->B * 2; p.M = d->M; p.mh = d->M / 2; p.n_lev = d->n_lev; p.ld_rx = p.L;
     p.amp_mean = d->amp_mean; p.var = d->var;
     p.rx = d->rx; p.amp = d->amp; p.P = d->P; p.W = d->W; p.h = d->h; p.adam = d->adam;
     p.q = d->q; p.out = d->out; p.loss = d->loss; p.gW_out = d->gW; p.gh_out = d->gh;
@@ -288,9 +296,100 @@ static int awgn_launch(const vaeq_awgn_desc *d, int mode, float lr_w, float lr_h
     return VAEQ_OK;
 }
 
+// ---- R independent runs, one CTA each (sweep engine): the per-run values come from device arrays ----------------------------
+struct AwRunsK {
+    AwK base;                                   // run 0's pointers; per-run fields below
+    int64_t rs_rx, fs_rx, rs_W, rs_h, rs_adam, rs_P, rs_q, rs_out, rs_loss, rs_ws;
+    const float *lr, *var, *amp_mean;           // (R)
+    int n_frames, n_mb;                         // frames of n_mb minibatches of B symbols (train), or 1 x 1 (forward)
+};
+
+// blockIdx.x = run.  Train: the epoch loop of :291-306 over n_frames frames, minibatch m of frame f at rx + f*fs_rx + m*sps*B;
+// loss of step (f, m) at loss[run][f*n_mb + m].  Forward: one step over the whole rx row (validation, :311-313).
+template <int NL>
+__global__ void __launch_bounds__(AW_NT) k_awgn_runs(AwRunsK r) {
+    const int64_t run = blockIdx.x;
+    AwK p = r.base;
+    p.var = r.var[run];
+    p.amp_mean = r.amp_mean[run];
+    p.P = r.base.P + run * r.rs_P;
+    p.W = r.base.W + run * r.rs_W;
+    p.h = r.base.h + run * r.rs_h;
+    p.adam = r.base.adam ? r.base.adam + run * r.rs_adam : nullptr;
+    p.q = r.base.q + run * r.rs_q;
+    p.out = r.base.out + run * r.rs_out;
+    const int64_t wo = run * r.rs_ws;
+    p.m1 += wo; p.vs += wo; p.e += wo; p.gyp += wo; p.gout += wo;
+    if (p.mode == DP_MODE_TRAIN) p.lr_w = p.lr_h = r.lr[run];    // one lr for both parameter groups (:305-306)
+    const float *rx = r.base.rx + run * r.rs_rx;
+    float *loss = r.base.loss + run * r.rs_loss;
+    for (int f = 0; f < r.n_frames; ++f)
+        for (int m = 0; m < r.n_mb; ++m) {
+            p.rx = rx + f * r.fs_rx + (int64_t)m * p.L;
+            p.loss = loss + (int64_t)f * r.n_mb + m;
+            awgn_step_body<NL>(p);
+        }
+}
+
+static int awgn_runs_launch(const vaeq_awgn_desc *d, const vaeq_awgn_runs *rs, int mode, int64_t ld_rx, int64_t fs_rx, int n_frames,
+                            int n_mb, cudaStream_t st) {
+    VAEQ_CHECK_ARG(d != nullptr && rs != nullptr, "desc is NULL");
+    VAEQ_CHECK_ARG(d->sps == 2, "sps=%d: only sps=2 is implemented", d->sps);
+    VAEQ_CHECK_ARG(d->M >= 1 && d->M <= VAEQ_MAX_TAPS && (d->M & 1), "M_est=%d must be odd and <= %d", d->M, VAEQ_MAX_TAPS);
+    VAEQ_CHECK_ARG(d->n_lev == 2 || d->n_lev == 4 || d->n_lev == 8, "n_lev=%d must be 2, 4 or 8", d->n_lev);
+    VAEQ_CHECK_ARG(d->B > 2 * (d->M / 2), "batch_len=%d must exceed M_est-1", d->B);
+    VAEQ_CHECK_ARG(rs->n_runs > 0 && n_frames > 0 && n_mb > 0, "bad sizes (n_runs=%d n_frames=%d minibatches=%d)", rs->n_runs, n_frames, n_mb);
+    VAEQ_CHECK_ARG(ld_rx >= (int64_t)d->sps * d->B * n_mb, "ld_rx=%lld is shorter than %d minibatches", (long long)ld_rx, n_mb);
+    VAEQ_CHECK_ARG(d->rx && d->amp && d->P && d->W && d->h && d->q && d->out && d->loss && d->workspace && rs->var && rs->amp_mean, "NULL pointer");
+    VAEQ_CHECK_ARG(mode != DP_MODE_TRAIN || (d->adam && rs->lr), "adam state / lr is NULL");
+    const size_t per = awgn_ws_floats(d->B);
+    if (d->workspace_bytes < per * sizeof(float) * (size_t)rs->n_runs) {
+        set_error("workspace too small");
+        return VAEQ_EWORKSPACE;
+    }
+    AwRunsK r;
+    memset(&r, 0, sizeof(r));
+    AwK &p = r.base;
+    p.B = d->B; p.L = d->B * 2; p.M = d->M; p.mh = d->M / 2; p.n_lev = d->n_lev; p.ld_rx = ld_rx;
+    p.rx = d->rx; p.amp = d->amp; p.P = d->P; p.W = d->W; p.h = d->h; p.adam = d->adam;
+    p.q = d->q; p.out = d->out; p.loss = d->loss;
+    float *ws = static_cast<float *>(d->workspace);
+    p.m1 = ws; ws += 2 * (size_t)d->B;
+    p.vs = ws; ws += d->B;
+    p.e = ws; ws += 4 * (size_t)d->B;
+    p.gyp = ws; ws += 2 * (size_t)d->B;
+    p.gout = ws;
+    p.mode = mode; p.amsgrad = 1;
+    r.rs_rx = rs->rs_rx; r.fs_rx = fs_rx; r.rs_W = rs->rs_W; r.rs_h = rs->rs_h; r.rs_adam = rs->rs_adam; r.rs_P = rs->rs_P;
+    r.rs_q = rs->rs_q; r.rs_out = rs->rs_out; r.rs_loss = rs->rs_loss; r.rs_ws = (int64_t)per;
+    r.lr = rs->lr; r.var = rs->var; r.amp_mean = rs->amp_mean;
+    r.n_frames = n_frames; r.n_mb = n_mb;
+    ktime_begin(VAEQ_K_AWGN, st);
+    switch (d->n_lev) {
+        case 2: k_awgn_runs<2><<<rs->n_runs, AW_NT, 0, st>>>(r); break;
+        case 4: k_awgn_runs<4><<<rs->n_runs, AW_NT, 0, st>>>(r); break;
+        default: k_awgn_runs<8><<<rs->n_runs, AW_NT, 0, st>>>(r); break;
+    }
+    ktime_end(VAEQ_K_AWGN, st);
+    VAEQ_LAUNCH_CHECK("k_awgn_runs");
+    return VAEQ_OK;
+}
+
 }  // namespace vaeq
 
 using namespace vaeq;
+
+extern "C" size_t vaeq_awgn_runs_workspace_bytes(int32_t B, int32_t M, int32_t n_lev, int32_t n_runs) {
+    (void)M; (void)n_lev;
+    return (B > 0 && n_runs > 0) ? awgn_ws_floats(B) * sizeof(float) * (size_t)n_runs : 0;
+}
+extern "C" int vaeq_awgn_train_frames_runs(const vaeq_awgn_desc *d, const vaeq_awgn_runs *r, int64_t ld_rx, int64_t fs_rx, int32_t n_frames,
+                                           int32_t n_mb, void *stream) {
+    return awgn_runs_launch(d, r, DP_MODE_TRAIN, ld_rx, fs_rx, n_frames, n_mb, (cudaStream_t)stream);
+}
+extern "C" int vaeq_awgn_forward_runs(const vaeq_awgn_desc *d, const vaeq_awgn_runs *r, int64_t ld_rx, void *stream) {
+    return awgn_runs_launch(d, r, DP_MODE_FWD, ld_rx, 0, 1, 1, (cudaStream_t)stream);
+}
 
 extern "C" size_t vaeq_awgn_workspace_bytes(int32_t B, int32_t M, int32_t n_lev) {
     (void)M; (void)n_lev;

@@ -9,6 +9,11 @@
 //   vaeq_gen_pulse   sf:77-80   zero insertion (sps = 2) + 'valid' convolution with the RRC pulse = two polyphase FIRs on the symbol grid
 //   vaeq_gen_jones   sf:41-53   Y = R^T diag(e_pmd, 1/e_pmd) R X * e_cd per frequency bin, R from the run's rotation angle
 //   vaeq_gen_noise   sf:83-88   + sigma_n (N(0,1) + j N(0,1)), cut to sps*N samples, split into the (R,2,2,L) float32 layout
+//
+// vaeq_gen_awgn: the single-polarisation signal of the AWGN module (AWGN_channel/func_VAELE_MQAM_shaping.py generate_data :39-61) for
+// R runs x F frames with the same kernels: levels (two rows per frame), one complex 'valid' FIR with rrcfir (*) h_channel (two 'valid'
+// convolutions in a row are one with the full convolution of the filters), then sigma_n from the frame's realised power and the noise.
+// Draws are keyed by (the run's own seed, frame index, row, position), so a run's frames do not depend on the batch.
 #include <curand_kernel.h>
 #include "common.cuh"
 
@@ -17,16 +22,19 @@ namespace vaeq {
 constexpr int DG_NT = 256;
 constexpr int DG_MAXPULSE = 128;
 
-// grid (ceil(n_conv / (4 DG_NT)), 4 rows, R): a thread draws 4 consecutive levels of one row from one Philox output
+// grid (ceil(n_conv / (4 DG_NT)), nrows, R * frames): a thread draws 4 consecutive levels of one row from one Philox output.
+// seeds == NULL: one seed for the batch, draws keyed by (frame z = blockIdx.z, row, position), P row z.  Otherwise frame z is frame
+// frame0 + z % frames of run z / frames, keyed by (seeds[run], frame, row, position), P row run.
 __global__ void __launch_bounds__(DG_NT) k_gen_levels(const float *amps, const float *P, int n_lev, int n_conv, int N, int tx_off,
-                                                      unsigned long long seed, float *lev, uint16_t *tx) {
+                                                      unsigned long long seed, const unsigned long long *seeds, int nrows, int frames,
+                                                      int frame0, float *lev, uint16_t *tx) {
     __shared__ float cdf[VAEQ_MAX_LEVELS], a_s[VAEQ_MAX_LEVELS];
-    const int row = blockIdx.y, r = blockIdx.z;
+    const int row = blockIdx.y, r = blockIdx.z, run = r / frames;
     if (threadIdx.x == 0) {
         float tot = 0.f, acc = 0.f;
-        for (int l = 0; l < n_lev; ++l) tot += P[(int64_t)r * n_lev + l];
+        for (int l = 0; l < n_lev; ++l) tot += P[(int64_t)run * n_lev + l];
         for (int l = 0; l < n_lev; ++l) {
-            acc += P[(int64_t)r * n_lev + l];
+            acc += P[(int64_t)run * n_lev + l];
             cdf[l] = acc / tot;
             a_s[l] = amps[l];
         }
@@ -35,7 +43,8 @@ __global__ void __launch_bounds__(DG_NT) k_gen_levels(const float *amps, const f
     const int g = blockIdx.x * DG_NT + threadIdx.x, groups = (n_conv + 3) >> 2;
     if (g >= groups) return;
     curandStatePhilox4_32_10_t st;
-    curand_init(seed, ((unsigned long long)(r * 4 + row)) * (unsigned long long)groups + g, 0, &st);
+    const unsigned long long key = seeds ? (unsigned long long)(frame0 + r - run * frames) : (unsigned long long)r;
+    curand_init(seeds ? seeds[run] : seed, (key * nrows + row) * (unsigned long long)groups + g, 0, &st);
     const float4 u4 = curand_uniform4(&st);                                  // (0, 1]
     const float u[4] = {u4.x, u4.y, u4.z, u4.w};
 #pragma unroll
@@ -45,38 +54,47 @@ __global__ void __launch_bounds__(DG_NT) k_gen_levels(const float *amps, const f
         int idx = 0;
         for (int l = 0; l < n_lev - 1; ++l) idx += (u[k] > cdf[l]);
         const float a = a_s[idx];
-        lev[((int64_t)r * 4 + row) * n_conv + j] = a;
+        lev[((int64_t)r * nrows + row) * n_conv + j] = a;
         const int t = j - tx_off;                                            // data[:, T+M-1 : N+T+M-1]  (sf:89)
-        if (t >= 0 && t < N) tx[(((int64_t)r * 2 + (row >> 1)) * 2 + (row & 1)) * N + t] = __half_as_ushort(__float2half_rn(a));
+        if (t >= 0 && t < N) tx[((int64_t)r * nrows + row) * N + t] = __half_as_ushort(__float2half_rn(a));
     }
 }
 
-// grid (ceil(n_conv - K/2, DG_NT), 2 pols, R): thread u produces the even and the odd output sample 2u, 2u+1 (complex) of one pol:
+// grid (ceil(n_conv - K/2, DG_NT), nrows / 2 pols, R): thread u produces the even and the odd output sample 2u, 2u+1 (complex) of one pol:
 //   shaped[2u]   = sum_t h[K-1-2t] sym[u+t],   shaped[2u+1] = sum_t h[K-2-2t] sym[u+1+t],   t = 0 .. K/2-1
-// which is np.convolve(zero-stuffed symbols, h, 'valid') for sps = 2 and an even pulse length K (sf:57-61, 77-80)
-__global__ void __launch_bounds__(DG_NT) k_gen_pulse(const float *lev, const float *h, int K, int n_conv, float2 *shaped) {
-    __shared__ float we[DG_MAXPULSE / 2], wo[DG_MAXPULSE / 2];
+// which is np.convolve(zero-stuffed symbols, h, 'valid') for sps = 2 and an even pulse length K (sf:57-61, 77-80).
+// CPLX: h holds K complex taps (re, im interleaved), the composite pulse * channel filter of the AWGN module (:52-53).
+template <bool CPLX>
+__global__ void __launch_bounds__(DG_NT) k_gen_pulse(const float *lev, const float *h, int K, int n_conv, int nrows, float2 *shaped) {
+    __shared__ float2 we[DG_MAXPULSE / 2], wo[DG_MAXPULSE / 2];
     const int half = K >> 1, p = blockIdx.y, r = blockIdx.z, nu = n_conv - half;
     for (int t = threadIdx.x; t < half; t += DG_NT) {
-        we[t] = h[K - 1 - 2 * t];
-        wo[t] = h[K - 2 - 2 * t];
+        we[t] = CPLX ? make_float2(h[2 * (K - 1 - 2 * t)], h[2 * (K - 1 - 2 * t) + 1]) : make_float2(h[K - 1 - 2 * t], 0.f);
+        wo[t] = CPLX ? make_float2(h[2 * (K - 2 - 2 * t)], h[2 * (K - 2 - 2 * t) + 1]) : make_float2(h[K - 2 - 2 * t], 0.f);
     }
     __syncthreads();
     const int u = blockIdx.x * DG_NT + threadIdx.x;
     if (u >= nu) return;
-    const float *re = lev + ((int64_t)r * 4 + 2 * p) * n_conv + u, *im = re + n_conv;
+    const float *re = lev + ((int64_t)r * nrows + 2 * p) * n_conv + u, *im = re + n_conv;
     float er = 0.f, ei = 0.f, orr = 0.f, oi = 0.f;
     float xr = re[0], xi = im[0];
     for (int t = 0; t < half; ++t) {
         const float nr = re[t + 1], ni = im[t + 1];                          // u + half <= n_conv - 1
-        er = fmaf(we[t], xr, er);
-        ei = fmaf(we[t], xi, ei);
-        orr = fmaf(wo[t], nr, orr);
-        oi = fmaf(wo[t], ni, oi);
+        const float2 a = we[t], b = wo[t];
+        er = fmaf(a.x, xr, er);
+        ei = fmaf(a.x, xi, ei);
+        orr = fmaf(b.x, nr, orr);
+        oi = fmaf(b.x, ni, oi);
+        if (CPLX) {
+            er = fmaf(-a.y, xi, er);
+            ei = fmaf(a.y, xr, ei);
+            orr = fmaf(-b.y, ni, orr);
+            oi = fmaf(b.y, nr, oi);
+        }
         xr = nr;
         xi = ni;
     }
-    float4 *dst = reinterpret_cast<float4 *>(shaped + ((int64_t)r * 2 + p) * (2 * (int64_t)nu) + 2 * u);
+    float4 *dst = reinterpret_cast<float4 *>(shaped + ((int64_t)r * (nrows / 2) + p) * (2 * (int64_t)nu) + 2 * u);
     *dst = make_float4(er, ei, orr, oi);
 }
 
@@ -123,9 +141,73 @@ __global__ void __launch_bounds__(DG_NT) k_gen_noise(const float2 *sig, const fl
     }
 }
 
+// grid (R * frames): one CTA per single-polarisation frame.  sigma_n = sqrt(sps mean|sig|^2 / 2 / 10^(SNR/10)) over the whole 'valid'
+// signal of n samples (:55), then rx[z] = (Re, Im)(sig[:L] + sigma_n (N(0,1) + j N(0,1))) (:56-57), 2 samples per Philox output
+__global__ void __launch_bounds__(DG_NT) k_gen_awgn_noise(const float2 *sig, const float *snr, const unsigned long long *seeds, int frames,
+                                                          int frame0, int n, int L, float *rx) {
+    __shared__ double red[32];
+    __shared__ float sg_sh;
+    const int z = blockIdx.x, run = z / frames;
+    const float2 *s = sig + (int64_t)z * n;
+    double acc[1] = {0.0};
+    for (int m = threadIdx.x; m < n; m += DG_NT) {
+        const float2 a = s[m];
+        acc[0] += (double)a.x * a.x + (double)a.y * a.y;
+    }
+    block_sum<1>(acc, red);
+    if (threadIdx.x == 0) sg_sh = (float)sqrt(2.0 * (acc[0] / n) / 2.0 / pow(10.0, (double)snr[run] / 10.0));
+    __syncthreads();
+    const float sg = sg_sh;
+    const int groups = (L + 1) >> 1;
+    float *ri = rx + (int64_t)z * 2 * L, *rq = ri + L;
+    for (int g = threadIdx.x; g < groups; g += DG_NT) {
+        curandStatePhilox4_32_10_t st;
+        curand_init(seeds[run] ^ 0x9E3779B97F4A7C15ull, (unsigned long long)(frame0 + z - run * frames) * groups + g, 0, &st);
+        const float4 w = curand_normal4(&st);
+        const int m = 2 * g;
+        const float2 a = s[m];
+        ri[m] = fmaf(sg, w.x, a.x);
+        rq[m] = fmaf(sg, w.y, a.y);
+        if (m + 1 < L) {
+            const float2 b = s[m + 1];
+            ri[m + 1] = fmaf(sg, w.z, b.x);
+            rq[m + 1] = fmaf(sg, w.w, b.y);
+        }
+    }
+}
+
 }  // namespace vaeq
 
 using namespace vaeq;
+
+extern "C" int vaeq_gen_awgn(const float *amps, const float *P, int32_t n_lev, const float *taps, int32_t K, int32_t N, int32_t tx_off,
+                             int32_t n_conv, const float *snr, const uint64_t *seeds, int32_t frame0, int32_t n_frames, int32_t n_runs,
+                             float *lev, float *sig, float *rx, uint16_t *tx, void *stream) {
+    VAEQ_CHECK_ARG(amps && P && taps && snr && seeds && lev && sig && rx && tx, "NULL pointer");
+    VAEQ_CHECK_ARG(n_lev >= 2 && n_lev <= VAEQ_MAX_LEVELS && N > 0 && tx_off >= 0 && tx_off + N <= n_conv && frame0 >= 0 && n_frames > 0 &&
+                   n_runs > 0 && (int64_t)n_runs * n_frames <= 65535, "bad sizes (n_lev=%d N=%d tx_off=%d n_conv=%d frames=%d runs=%d)",
+                   n_lev, N, tx_off, n_conv, n_frames, n_runs);
+    VAEQ_CHECK_ARG(K >= 2 && K % 2 == 0 && K <= DG_MAXPULSE && n_conv > K / 2, "filter length K=%d must be even and <= %d", K, DG_MAXPULSE);
+    const int n = 2 * n_conv - K, L = 2 * N;
+    VAEQ_CHECK_ARG(L <= n, "sps*N=%d exceeds the %d filtered samples", L, n);
+    VAEQ_CHECK_ARG(reinterpret_cast<uintptr_t>(sig) % 16 == 0, "sig must be 16-byte aligned");
+    cudaStream_t st = (cudaStream_t)stream;
+    const int Z = n_runs * n_frames, groups = (n_conv + 3) / 4, nu = n_conv - K / 2;
+    const unsigned long long *sd = reinterpret_cast<const unsigned long long *>(seeds);
+    ktime_begin(VAEQ_K_OTHER, st);
+    k_gen_levels<<<dim3((groups + DG_NT - 1) / DG_NT, 2, Z), DG_NT, 0, st>>>(amps, P, n_lev, n_conv, N, tx_off, 0, sd, 2, n_frames, frame0, lev, tx);
+    ktime_end(VAEQ_K_OTHER, st);
+    VAEQ_LAUNCH_CHECK("k_gen_levels");
+    ktime_begin(VAEQ_K_OTHER, st);
+    k_gen_pulse<true><<<dim3((nu + DG_NT - 1) / DG_NT, 1, Z), DG_NT, 0, st>>>(lev, taps, K, n_conv, 2, reinterpret_cast<float2 *>(sig));
+    ktime_end(VAEQ_K_OTHER, st);
+    VAEQ_LAUNCH_CHECK("k_gen_pulse");
+    ktime_begin(VAEQ_K_OTHER, st);
+    k_gen_awgn_noise<<<Z, DG_NT, 0, st>>>(reinterpret_cast<const float2 *>(sig), snr, sd, n_frames, frame0, n, L, rx);
+    ktime_end(VAEQ_K_OTHER, st);
+    VAEQ_LAUNCH_CHECK("k_gen_awgn_noise");
+    return VAEQ_OK;
+}
 
 extern "C" int vaeq_gen_levels(const float *amps, const float *P, int32_t n_lev, int32_t n_conv, int32_t N, int32_t tx_off, uint64_t seed,
                                float *lev, uint16_t *tx, int32_t n_runs, void *stream) {
@@ -135,7 +217,8 @@ extern "C" int vaeq_gen_levels(const float *amps, const float *P, int32_t n_lev,
     cudaStream_t st = (cudaStream_t)stream;
     const int groups = (n_conv + 3) / 4;
     ktime_begin(VAEQ_K_OTHER, st);
-    k_gen_levels<<<dim3((groups + DG_NT - 1) / DG_NT, 4, n_runs), DG_NT, 0, st>>>(amps, P, n_lev, n_conv, N, tx_off, seed, lev, tx);
+    k_gen_levels<<<dim3((groups + DG_NT - 1) / DG_NT, 4, n_runs), DG_NT, 0, st>>>(amps, P, n_lev, n_conv, N, tx_off, seed, nullptr, 4, 1, 0, lev,
+                                                                                  tx);
     ktime_end(VAEQ_K_OTHER, st);
     VAEQ_LAUNCH_CHECK("k_gen_levels");
     return VAEQ_OK;
@@ -149,7 +232,7 @@ extern "C" int vaeq_gen_pulse(const float *lev, const float *h, int32_t n_pulse,
     cudaStream_t st = (cudaStream_t)stream;
     const int nu = n_conv - n_pulse / 2;
     ktime_begin(VAEQ_K_OTHER, st);
-    k_gen_pulse<<<dim3((nu + DG_NT - 1) / DG_NT, 2, n_runs), DG_NT, 0, st>>>(lev, h, n_pulse, n_conv, reinterpret_cast<float2 *>(shaped));
+    k_gen_pulse<false><<<dim3((nu + DG_NT - 1) / DG_NT, 2, n_runs), DG_NT, 0, st>>>(lev, h, n_pulse, n_conv, 4, reinterpret_cast<float2 *>(shaped));
     ktime_end(VAEQ_K_OTHER, st);
     VAEQ_LAUNCH_CHECK("k_gen_pulse");
     return VAEQ_OK;

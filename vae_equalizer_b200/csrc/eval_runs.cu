@@ -141,6 +141,40 @@ __device__ __forceinline__ void er_publish_counts(int (&cnt)[16], int *red, int 
     }
 }
 
+// hard decision of one symbol of one polarisation and its errors for the 4 rotations, straight and IQ-flipped (sf:188-222):
+// q = the pol's first posterior row at the symbol (rows ld_q apart), tx = its I row at the symbol (Q row ld_tx further);
+// cnt[(flip * 2 + pol) * 4 + rotation]
+template <int NL>
+__device__ __forceinline__ void er_count_q(const float *q, int64_t ld_q, const uint16_t *tx, int64_t ld_tx, int pol, int (&cnt)[16]) {
+    const float S = (float)(NL - 1), scale = (float)((NL - 1) / 2.0);
+    int d[2];
+#pragma unroll
+    for (int c = 0; c < 2; ++c) {                                         // torch.argmax: first maximal index
+        float best = q[(int64_t)(c * NL) * ld_q];
+        int bi = 0;
+#pragma unroll
+        for (int l = 1; l < NL; ++l) {
+            const float v = q[(int64_t)(c * NL + l) * ld_q];
+            if (v > best) {
+                best = v;
+                bi = l;
+            }
+        }
+        d[c] = bi;
+    }
+    const float dI = (float)d[0], dQ = (float)d[1];
+    const float hI[4] = {dI, S - dI, S - dQ, dQ};                         // 0, pi, pi/2, 3pi/2  (sf:201-219)
+    const float hQ[4] = {dQ, S - dQ, dI, S - dI};
+    const float DI = er_tx_level(tx[0], scale);
+    const float DQ = er_tx_level(tx[ld_tx], scale);
+    const float DQf = S - DQ;                                             // IQ-flipped reference data (sf:199)
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        cnt[(0 * 2 + pol) * 4 + k] += (DI != hI[k]) || (DQ != hQ[k]);
+        cnt[(1 * 2 + pol) * 4 + k] += (DI != hI[k]) || (DQf != hQ[k]);
+    }
+}
+
 // ---- SER from the posteriors (sf:188-222) on the aligned, cut region: grid (blocks, R) ----------------------------------------
 template <int NL>
 __global__ void __launch_bounds__(ER_NT) k_er_ser_iqflip(EvalRunsK p) {
@@ -150,7 +184,6 @@ __global__ void __launch_bounds__(ER_NT) k_er_ser_iqflip(EvalRunsK p) {
     const int sh[2] = {al[0], al[1]}, r = al[2], n_eval = al[3], keep = p.seg_len ? min(p.seg_len, p.seg_len - sh[0] - p.n_cut) : 0;
     const float *q = p.q + run * p.rs_q;
     const uint16_t *tx = p.tx + run * p.rs_tx;
-    const float S = (float)(NL - 1), scale = (float)((NL - 1) / 2.0);
     int cnt[16];
 #pragma unroll
     for (int k = 0; k < 16; ++k) cnt[k] = 0;
@@ -159,32 +192,7 @@ __global__ void __launch_bounds__(ER_NT) k_er_ser_iqflip(EvalRunsK p) {
 #pragma unroll
         for (int pol = 0; pol < 2; ++pol) {
             const int sp = (pol - r) & 1, ts = er_wrap(t + sh[pol], N);   // out.roll(r, 0)[pol].roll(-shift[pol], -1)  (VAELE_DP:71-72)
-            int d[2];
-#pragma unroll
-            for (int c = 0; c < 2; ++c) {                                 // torch.argmax: first maximal index
-                float best = q[(int64_t)(sp * 2 * NL + c * NL) * p.ld_q + ts];
-                int bi = 0;
-#pragma unroll
-                for (int l = 1; l < NL; ++l) {
-                    const float v = q[(int64_t)(sp * 2 * NL + c * NL + l) * p.ld_q + ts];
-                    if (v > best) {
-                        best = v;
-                        bi = l;
-                    }
-                }
-                d[c] = bi;
-            }
-            const float dI = (float)d[0], dQ = (float)d[1];
-            const float hI[4] = {dI, S - dI, S - dQ, dQ};                 // 0, pi, pi/2, 3pi/2  (sf:201-219)
-            const float hQ[4] = {dQ, S - dQ, dI, S - dI};
-            const float DI = er_tx_level(tx[(int64_t)(pol * 2 + 0) * p.ld_tx + t], scale);
-            const float DQ = er_tx_level(tx[(int64_t)(pol * 2 + 1) * p.ld_tx + t], scale);
-            const float DQf = S - DQ;                                     // IQ-flipped reference data (sf:199)
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                cnt[(0 * 2 + pol) * 4 + k] += (DI != hI[k]) || (DQ != hQ[k]);
-                cnt[(1 * 2 + pol) * 4 + k] += (DI != hI[k]) || (DQf != hQ[k]);
-            }
+            er_count_q<NL>(q + (int64_t)(sp * 2 * NL) * p.ld_q + ts, p.ld_q, tx + (int64_t)(pol * 2) * p.ld_tx + t, p.ld_tx, pol, cnt);
         }
     }
     er_publish_counts(cnt, red, p.counts + ((int64_t)run * 2 + 0) * 16);
@@ -321,9 +329,126 @@ __global__ void __launch_bounds__(ER_NT) k_er_align_rescale(const float *out, in
     }
 }
 
+// ---- AWGN single-polarisation driver (processing.py awgn_find_shift + awgn_ser_q, AWGN :188-204, :97-124), R runs ----------------
+struct AwgnEvalK {
+    const float *q; int64_t ld_q, rs_q;          // (R, 2n, N)
+    const uint16_t *tx; int64_t ld_tx, rs_tx;    // (R, 2, N) float16 bits
+    const float *amp;
+    int n_lev, N, n_shift, n_corr, edge, n_runs, chunks;
+    double *part;                                // [R][chunks][n_shift][8]
+    int *shift;                                  // [R]
+    int *cnt;                                    // [R][16] scratch counters
+    int *counts;                                 // [R][4]
+    float *ser;                                  // [R]
+};
+
+// grid (chunks, R): the correlation of the first n_corr symbols, one SC_T tile per CTA like vaeq_find_shift cuts it, so the partial
+// sums and their fixed-order total are those of the single-run search.  q's I rows against itself as both "polarisations"
+__global__ void __launch_bounds__(SC_NT, 4) k_aw_shift_corr(AwgnEvalK p) {
+    __shared__ ShiftSmem sm;
+    const int64_t run = blockIdx.y, t_lo = (int64_t)blockIdx.x * SC_T, t_hi = min((int64_t)p.n_corr, t_lo + SC_T);
+    shift_corr_range<true, 0, true>(sm, p.q + run * p.rs_q, p.ld_q, nullptr, 0, p.tx + run * p.rs_tx, p.ld_tx, p.amp, p.n_lev, p.n_corr, p.n_shift,
+                                    t_lo, t_hi, p.part + (run * p.chunks + blockIdx.x) * p.n_shift * 8);
+}
+
+// thread = run: |corr| with tx I (k = 0) and tx Q (k = 4), summed over the chunks in order as k_shift_decide does, then the rule of
+// awgn_find_shift in fp32 like the torch expressions (first index wins ties; 0.02 * N is a Python float compared with a float32 tensor)
+__global__ void k_aw_shift_decide(AwgnEvalK p) {
+    const int run = blockIdx.x * blockDim.x + threadIdx.x;
+    if (run >= p.n_runs) return;
+    const int nidx = p.n_shift * 8, half = p.n_shift / 2;
+    const double *part = p.part + (int64_t)run * p.chunks * nidx;
+    float mI = -1.f, mQ = -1.f;
+    int iI = 0, iQ = 0;
+    for (int i = 0; i < p.n_shift; ++i) {
+        double sI = 0.0, sQ = 0.0;
+        for (int c = 0; c < p.chunks; ++c) {
+            sI += part[(int64_t)c * nidx + i * 8 + 0];
+            sQ += part[(int64_t)c * nidx + i * 8 + 4];
+        }
+        const float vI = fabsf((float)sI), vQ = fabsf((float)sQ);
+        if (vI > mI) { mI = vI; iI = i; }
+        if (vQ > mQ) { mQ = vQ; iQ = i; }
+    }
+    const float thr = (float)(0.02 * (double)p.N);
+    const int idx = (mI >= thr) ? iI : ((mQ >= mI) ? iQ : iI);
+    p.shift[run] = half - idx;
+}
+
+// grid (blocks, R): error counts of q[:, edge + shift : N - edge] against tx[:, edge : N - edge - shift]
+template <int NL>
+__global__ void __launch_bounds__(ER_NT) k_aw_ser(AwgnEvalK p) {
+    __shared__ int red[16 * 32];
+    const int64_t run = blockIdx.y;
+    const int sh = p.shift[run], n_eval = p.N - 2 * p.edge - sh;
+    const float *q = p.q + run * p.rs_q + p.edge + sh;
+    const uint16_t *tx = p.tx + run * p.rs_tx + p.edge;
+    int cnt[16];
+#pragma unroll
+    for (int k = 0; k < 16; ++k) cnt[k] = 0;
+    for (int f = blockIdx.x * ER_NT + threadIdx.x; f < n_eval; f += gridDim.x * ER_NT) er_count_q<NL>(q + f, p.ld_q, tx + f, p.ld_tx, 0, cnt);
+    er_publish_counts(cnt, red, p.cnt + run * 16);
+}
+
+// thread = run: the 4 rotation counts (no IQ flip) and min count / symbols in fp32 as torch divides a float32 tensor by a Python int on
+// the GPU: times the fp32 reciprocal of the divisor (awgn_ser_q)
+__global__ void k_aw_ser_min(AwgnEvalK p) {
+    const int run = blockIdx.x * blockDim.x + threadIdx.x;
+    if (run >= p.n_runs) return;
+    const int n_eval = p.N - 2 * p.edge - p.shift[run];
+    int m = INT_MAX;
+    for (int k = 0; k < 4; ++k) {
+        const int c = p.cnt[run * 16 + k];
+        p.counts[run * 4 + k] = c;
+        m = min(m, c);
+    }
+    p.ser[run] = __fmul_rn((float)m, __fdiv_rn(1.f, (float)n_eval));
+}
+
 }  // namespace vaeq
 
 using namespace vaeq;
+
+extern "C" size_t vaeq_awgn_eval_scratch_bytes(int32_t n_runs, int32_t n_shift, int32_t n_corr) {
+    if (n_runs <= 0 || n_shift <= 0 || n_corr <= 0) return 0;
+    const size_t chunks = ((size_t)n_corr + SC_T - 1) / SC_T;
+    return align_up((size_t)n_runs * chunks * n_shift * 8 * sizeof(double), 256) + (size_t)n_runs * 16 * sizeof(int);
+}
+
+extern "C" int vaeq_awgn_eval_runs(const float *q, int64_t ld_q, int64_t rs_q, const uint16_t *tx, int64_t ld_tx, int64_t rs_tx, const float *amp,
+                                   int32_t n_lev, int32_t N, int32_t n_shift, int32_t n_corr, int32_t edge, int32_t n_runs, int32_t *shift_out,
+                                   int32_t *counts_out, float *ser_out, void *scratch, void *stream) {
+    VAEQ_CHECK_ARG(q && tx && amp && shift_out && counts_out && ser_out && scratch, "NULL pointer");
+    VAEQ_CHECK_ARG(n_lev == 2 || n_lev == 4 || n_lev == 8, "n_lev=%d must be 2, 4 or 8", n_lev);
+    VAEQ_CHECK_ARG(n_shift > 0 && n_shift <= 8 * SC_J && edge >= 0 && n_corr > 0 && n_corr <= N, "bad sizes (n_shift=%d <= %d, n_corr=%d <= N=%d)",
+                   n_shift, 8 * SC_J, n_corr, N);
+    VAEQ_CHECK_ARG(N - 2 * edge - n_shift / 2 > 0, "N=%d leaves no symbol to evaluate", N);
+    VAEQ_CHECK_ARG(n_runs > 0 && n_runs <= 65535, "n_runs=%d must be in 1..65535", n_runs);
+    cudaStream_t st = (cudaStream_t)stream;
+    AwgnEvalK p;
+    p.q = q; p.ld_q = ld_q; p.rs_q = rs_q; p.tx = tx; p.ld_tx = ld_tx; p.rs_tx = rs_tx; p.amp = amp;
+    p.n_lev = n_lev; p.N = N; p.n_shift = n_shift; p.n_corr = n_corr; p.edge = edge; p.n_runs = n_runs;
+    p.chunks = (n_corr + SC_T - 1) / SC_T;
+    const size_t part_b = align_up((size_t)n_runs * p.chunks * n_shift * 8 * sizeof(double), 256);
+    p.part = static_cast<double *>(scratch);
+    p.cnt = reinterpret_cast<int *>(static_cast<char *>(scratch) + part_b);
+    p.shift = shift_out; p.counts = counts_out; p.ser = ser_out;
+    VAEQ_CUDA(cudaMemsetAsync(p.cnt, 0, (size_t)n_runs * 16 * sizeof(int), st));
+    const int blocks = max(1, min((N + ER_NT - 1) / ER_NT, max(1, sm_count() * 8 / n_runs)));
+#define AW_LAUNCH(name, ...)                    \
+    ktime_begin(VAEQ_K_EVAL, st);               \
+    __VA_ARGS__;                                \
+    ktime_end(VAEQ_K_EVAL, st);                 \
+    VAEQ_LAUNCH_CHECK(name);
+    AW_LAUNCH("k_aw_shift_corr", k_aw_shift_corr<<<dim3(p.chunks, n_runs), SC_NT, 0, st>>>(p))
+    AW_LAUNCH("k_aw_shift_decide", k_aw_shift_decide<<<(n_runs + 127) / 128, 128, 0, st>>>(p))
+    if (n_lev == 2) { AW_LAUNCH("k_aw_ser", k_aw_ser<2><<<dim3(blocks, n_runs), ER_NT, 0, st>>>(p)) }
+    else if (n_lev == 4) { AW_LAUNCH("k_aw_ser", k_aw_ser<4><<<dim3(blocks, n_runs), ER_NT, 0, st>>>(p)) }
+    else { AW_LAUNCH("k_aw_ser", k_aw_ser<8><<<dim3(blocks, n_runs), ER_NT, 0, st>>>(p)) }
+    AW_LAUNCH("k_aw_ser_min", k_aw_ser_min<<<(n_runs + 127) / 128, 128, 0, st>>>(p))
+#undef AW_LAUNCH
+    return VAEQ_OK;
+}
 
 extern "C" size_t vaeq_frame_eval_scratch_bytes(int32_t n_runs, int32_t n_shift) {
     if (n_runs <= 0 || n_shift <= 0) return 0;

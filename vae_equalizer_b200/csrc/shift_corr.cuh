@@ -82,7 +82,9 @@ __device__ __forceinline__ void shift_corr_blocked_tile(const ShiftSmem &sm, int
 
 // Accumulates symbols [t_lo, t_hi) and writes dst[i * 8 + k], k = comp*4 + b*2 + a, for i < n_shift.  All threads of the CTA call it.
 // t_lo must be a multiple of 4 for the vector paths to engage (the callers cut their ranges at multiples of 64).
-template <bool FROM_Q, int NPASS_>            // 1: n_shift <= 32, 2: n_shift <= 64 (a lane owns shifts lane, lane + 32), 0: n_shift <= 24, blocked correlation
+// ONE_POL: both "polarisations" of E and of tx are polarisation 0 (rows 0 .. 2n-1 of q, rows I / Q of tx): the single-polarisation
+// AWGN driver correlates stack((q, q)) with stack((tx, tx)) (AWGN :188-204), so a run needs only its own rows.
+template <bool FROM_Q, int NPASS_, bool ONE_POL = false>   // 1: n_shift <= 32, 2: n_shift <= 64 (a lane owns shifts lane, lane + 32), 0: n_shift <= 24, blocked correlation
 __device__ __forceinline__ void shift_corr_range(ShiftSmem &sm, const float *__restrict__ q, int64_t ld_q, const float *__restrict__ out,
                                                  int64_t ld_out, const uint16_t *__restrict__ tx, int64_t ld_tx, const float *amp,
                                                  int n_lev, int N, int n_shift, int64_t t_lo, int64_t t_hi, double *dst) {
@@ -126,12 +128,12 @@ __device__ __forceinline__ void shift_corr_range(ShiftSmem &sm, const float *__r
 #pragma unroll
                         for (int l = 0; l < VAEQ_MAX_LEVELS; ++l)   // unrolled: the compiler keeps as many loads in flight as registers allow
                             if (l < n_lev) {
-                                const float4 v = ld4(q + (int64_t)(b * 2 * n_lev + l) * ld_q + p0);
+                                const float4 v = ld4(q + (int64_t)((ONE_POL ? 0 : b * 2 * n_lev) + l) * ld_q + p0);
                                 e[b][0] += a_l[l] * v.x; e[b][1] += a_l[l] * v.y;
                                 e[b][2] += a_l[l] * v.z; e[b][3] += a_l[l] * v.w;
                             }
                     } else {
-                        const float4 v = ld4(out + (int64_t)(b * 2) * ld_out + p0);      // rx[:,0,:]  (sf:321)
+                        const float4 v = ld4(out + (int64_t)(ONE_POL ? 0 : b * 2) * ld_out + p0);      // rx[:,0,:]  (sf:321)
                         e[b][0] = v.x; e[b][1] = v.y; e[b][2] = v.z; e[b][3] = v.w;
                     }
                 }
@@ -147,9 +149,9 @@ __device__ __forceinline__ void shift_corr_range(ShiftSmem &sm, const float *__r
                             acc = 0.f;
 #pragma unroll
                             for (int l = 0; l < VAEQ_MAX_LEVELS; ++l)
-                                if (l < n_lev) acc += a_l[l] * q[(int64_t)(b * 2 * n_lev + l) * ld_q + pos];
+                                if (l < n_lev) acc += a_l[l] * q[(int64_t)((ONE_POL ? 0 : b * 2 * n_lev) + l) * ld_q + pos];
                         } else {
-                            acc = out[(int64_t)(b * 2) * ld_out + pos];
+                            acc = out[(int64_t)(ONE_POL ? 0 : b * 2) * ld_out + pos];
                         }
                         e[b][k] = acc;
                     }
@@ -165,7 +167,7 @@ __device__ __forceinline__ void shift_corr_range(ShiftSmem &sm, const float *__r
             if (vec_x && j + 3 < tn) {
 #pragma unroll
                 for (int r = 0; r < 4; ++r) {
-                    const uint2 u = __ldg(reinterpret_cast<const uint2 *>(tx + (int64_t)r * ld_tx + t0 + j));
+                    const uint2 u = __ldg(reinterpret_cast<const uint2 *>(tx + (int64_t)(ONE_POL ? r & 1 : r) * ld_tx + t0 + j));
                     x[r][0] = half_bits_to_float((uint16_t)(u.x & 0xffffu)); x[r][1] = half_bits_to_float((uint16_t)(u.x >> 16));
                     x[r][2] = half_bits_to_float((uint16_t)(u.y & 0xffffu)); x[r][3] = half_bits_to_float((uint16_t)(u.y >> 16));
                 }
@@ -173,7 +175,7 @@ __device__ __forceinline__ void shift_corr_range(ShiftSmem &sm, const float *__r
 #pragma unroll
                 for (int r = 0; r < 4; ++r)
 #pragma unroll
-                    for (int k = 0; k < 4; ++k) x[r][k] = (j + k < tn) ? half_bits_to_float(tx[(int64_t)r * ld_tx + t0 + j + k]) : 0.f;
+                    for (int k = 0; k < 4; ++k) x[r][k] = (j + k < tn) ? half_bits_to_float(tx[(int64_t)(ONE_POL ? r & 1 : r) * ld_tx + t0 + j + k]) : 0.f;
             }
 #pragma unroll
             for (int k = 0; k < 4; ++k) sm.X[j + k] = make_float4(x[0][k], x[2][k], x[1][k], x[3][k]);

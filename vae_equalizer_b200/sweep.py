@@ -8,6 +8,10 @@ cell), then each cell is aligned and scored with the same evaluation kernels as 
 cells are dealt round-robin (parallel.shard_cells), no data-path collective.
 
 `sweep_vae_dp` returns the same three result tensors as `processing()` with a leading cell dimension.
+
+The AWGN single-polarisation VAE-LE (AWGN_channel/func_VAELE_MQAM_shaping.py, driven by Eval_run_shaping_vaele.py) has the same
+structure: `sweep_vae_awgn` steps all cells of a set together (one launch trains every cell's epochs of a validation period,
+one launch runs the validation forward, four score it, no host sync), `run_awgn_sweep` walks the reference's loops.
 """
 from __future__ import annotations
 
@@ -422,3 +426,155 @@ def save_mat(path, SER, Var_est, var_real, *, SNR_vec, nu_vec, theta_diff_vec, t
                                "SNR": list(SNR_vec), "nu": list(nu_vec), "theta_diff": list(theta_diff_vec), "theta": list(theta_vec),
                                "M": list(M_vec), "lr": list(lr_optim_vec), "batch_len": list(batch_len_vec),
                                "symb_rate": list(symb_rate_vec), "symb_step": list(flex_step_vec)}})
+
+
+# -------------------------------------------------------------------------------------------------
+# AWGN single-polarisation VAE-LE (AWGN_channel/func_VAELE_MQAM_shaping.py:235-324, Eval_run_shaping_vaele.py)
+# -------------------------------------------------------------------------------------------------
+AWGN_VALID_FRAME0 = 1 << 20          # device generator: frame indices of the validation frames (training frames are the epoch index)
+
+
+def _awgn_check(num_epochs, epe, channel, device):
+    if channel not in ("h1", "h2"):
+        raise KeyError(f"AWGN driver knows channels h1/h2, got {channel!r}")       # :239-242
+    if epe < 1 or num_epochs % epe != 0:
+        raise ValueError(f"num_epochs={num_epochs} must be a multiple of epe={epe} (the single-run driver fails on its last validation)")
+    dev = _cuda_device(device)
+    if dev.type != "cuda":
+        raise sfun._lib.VaeqError(f"device {dev}: the AWGN sweep runs on CUDA devices only, there is no CPU path")
+    return dev
+
+
+def sweep_vae_awgn(cells, mod, sps, M_est, batch_len, N_valid, N_train, num_epochs, epe, channel, *, device=None, datagen="gpu", verbose=False):
+    """processing_vaele_awgn (:235-324) for R = len(cells) independent cells in lockstep.
+
+    cells: dicts with SNR, nu, lr_optim and optionally seed (default: the cell's index).  Returns SER_valid (R, num_epochs // epe), row k
+    being what the single-run driver returns for cell k.  The driver validates after epoch e when e % epe == 0, so a validation period
+    is ONE launch training every cell's epochs since the last validation, the validation forward of all cells, and the batched scoring.
+    The epe - 1 epochs after the last validation do not change the result and are not trained.
+    datagen="gpu": every cell's frames from the device generator, keyed by the cell's seed (a cell gives the same SER alone or in any
+    batch); "numpy": each cell's frames from np.random.default_rng(seed) in exactly the order processing_vaele_awgn(rng=...) draws them."""
+    from .awgn import AWGNEqualizerRuns, awgn_eval_runs, generate_data, generate_frames_awgn_gpu
+    from .constants import awgn_constants, upsampled_channel
+    dev = _awgn_check(num_epochs, epe, channel, device)
+    if datagen not in ("gpu", "numpy"):
+        raise ValueError(f"datagen={datagen!r}: 'gpu' or 'numpy'")
+    R = len(cells)
+    if R == 0:
+        raise ValueError("no cells")
+    if N_train // batch_len < 1:
+        raise ValueError(f"N_train={N_train} holds no minibatch of batch_len={batch_len}")
+    h_channel = upsampled_channel(channel, sps)
+    M = (len(h_channel) - 1) // sps + 1
+    consts = [awgn_constants(mod, float(_cell(c, "nu")), float(_cell(c, "SNR"))) for c in cells]
+    amps = consts[0][0]
+    amp_levels = torch.tensor(amps, device=dev, dtype=torch.float32)
+    P = torch.tensor(np.stack([k[1] for k in consts]), dtype=torch.float32)
+    eqr = AWGNEqualizerRuns(R, M_est, sps, amp_levels, P, [k[2] for k in consts], [k[3] for k in consts], device=dev)
+    lr = torch.tensor([float(_cell(c, "lr_optim")) for c in cells], dtype=torch.float32, device=dev)
+    seeds = [int(c.get("seed", i)) for i, c in enumerate(cells)]
+    rngs = [np.random.default_rng(s) for s in seeds]
+    snr = [float(c["SNR"]) for c in cells]
+    n_val = num_epochs // epe
+    SER_valid = torch.empty(R, n_val, device=dev, dtype=torch.float32)
+
+    def host_frames(N, F):
+        rx = torch.empty(R, F, 2, sps * N, dtype=torch.float32, device=dev)
+        tx = torch.empty(R, F, 2, N, dtype=torch.float16, device=dev)
+        for r in range(R):
+            for f in range(F):
+                rx[r, f], tx[r, f] = generate_data(N, M, amps, snr[r], h_channel, sps, dev, consts[r][1], rng=rngs[r])
+        return rx, tx
+
+    epoch = 0
+    for k in range(n_val):
+        n_ep = 1 if k == 0 else epe                                  # epochs epoch .. epoch + n_ep - 1, then validate (epoch % epe == 0)
+        if datagen == "gpu":
+            rx, _ = generate_frames_awgn_gpu(N_train, amps, snr, P, h_channel, sps, dev, seeds, frame0=epoch, n_frames=n_ep)
+            rx_v, tx_v = generate_frames_awgn_gpu(N_valid, amps, snr, P, h_channel, sps, dev, seeds, frame0=AWGN_VALID_FRAME0 + k)
+        else:
+            rx, _ = host_frames(N_train, n_ep)
+            rx_v, tx_v = host_frames(N_valid, 1)
+        loss = eqr.train_frames(rx, lr, batch_len, N_train)
+        epoch += n_ep
+        q_v, _, _ = eqr.forward(rx_v[:, 0])
+        shift, _, ser = awgn_eval_runs(q_v, tx_v[:, 0], amp_levels)
+        SER_valid[:, k] = ser
+        if verbose:
+            print(epoch - 1, "loss", loss[:, -1].tolist(), "shift", shift.tolist(), "SER", ser.tolist())
+    return SER_valid
+
+
+def sweep_vae_awgn_sharded(cells, *args, rank=0, world=1, group=None, **kw):
+    """sweep_vae_awgn over a round-robin share of the cells per rank (one process per GPU); SER_valid of ALL cells on rank 0 (None
+    elsewhere).  No data-path collective."""
+    from .parallel import gather_cell_results, shard_cells
+    mine = shard_cells(cells, rank, world)
+    num_epochs, epe = (args[6], args[7]) if len(args) > 7 else (kw["num_epochs"], kw["epe"])
+    dev = _cuda_device(kw.get("device"))
+    loc = {}
+    if mine:
+        ser = sweep_vae_awgn([c for _, c in mine], *args, **kw)
+        loc = {i: ser[k] for k, (i, _) in enumerate(mine)}
+    return gather_cell_results(loc, len(cells), (num_epochs // epe,), rank, world, group, dev)
+
+
+AWGN_AXES = ("batch_len", "lr_optim", "M", "SNR", "nu")           # loop order of Eval_run_shaping_vaele.py (RUN_AWGN:42-58), then iter
+
+
+def run_awgn_sweep(mod="64-QAM", sps=2, channel="h1", N_train_vec=(350,), lr_optim_vec=(2e-3,), M_vec=(25,), SNR_vec=(12,), nu_vec=(0.0,),
+                   iter=1, N_valid=15000, train_len=1200, num_epochs=500, epe=20, *, device=None, datagen="gpu", rank=0, world=1, group=None,
+                   runner=None, verbose=False, checkpoint_dir=None):
+    """Eval_run_shaping_vaele.py's loops (RUN_AWGN:42-58) as batched run sets.  As in the reference, the N_train_vec entries are the
+    drivers' batch_len and train_len is their N_train (RUN_AWGN:53).  Cells that share (M, batch_len) train in the same launch; with
+    world > 1 every rank takes a round-robin share of each set.  Returns on rank 0 (None elsewhere)
+        SER (len(N_train_vec), len(lr_optim_vec), len(M_vec), len(SNR_vec), len(nu_vec), iter, num_epochs // epe) and the validation
+        epochs (num_epochs // epe,).
+    Cell (.., i) is seeded with its flat index.  checkpoint_dir: rank 0 stores every finished set (one .npz, keyed by the set's full
+    parameters); a restarted sweep loads what it finds instead of recomputing."""
+    import os
+    if channel not in ("h1", "h2"):
+        raise KeyError(f"AWGN driver knows channels h1/h2, got {channel!r}")
+    if epe < 1 or num_epochs % epe != 0:
+        raise ValueError(f"num_epochs={num_epochs} must be a multiple of epe={epe}")
+    vecs = dict(batch_len=list(N_train_vec), lr_optim=list(lr_optim_vec), M=list(M_vec), SNR=list(SNR_vec), nu=list(nu_vec))
+    shape = tuple(len(vecs[a]) for a in AWGN_AXES) + (iter,)
+    n_val = num_epochs // epe
+    dev = torch.device("cpu") if runner is not None and device is None else _cuda_device(device)
+    SER = torch.full(shape + (n_val,), float("nan"), dtype=torch.float32, device=dev)
+    groups = {}
+    for idx in np.ndindex(*shape):
+        c = {a: vecs[a][i] for a, i in zip(AWGN_AXES, idx[:-1])}
+        c["seed"] = int(np.ravel_multi_index(idx, shape))
+        groups.setdefault((c["M"], c["batch_len"]), []).append((idx, c))
+    for (M, batch_len), members in groups.items():
+        cells = [{k: c[k] for k in ("SNR", "nu", "lr_optim", "seed")} for _, c in members]
+        args = (cells, mod, sps, M, batch_len, N_valid, train_len, num_epochs, epe, channel)
+        ck, sig = None, None
+        if checkpoint_dir is not None:
+            os.makedirs(checkpoint_dir, exist_ok=True)
+            sig = _set_signature(driver="VAELE_AWGN", mod=mod, sps=sps, channel=channel, M=M, batch_len=batch_len, N_valid=N_valid,
+                                 train_len=train_len, num_epochs=num_epochs, epe=epe, datagen=datagen, cells=[sorted(c.items()) for c in cells])
+            ck = os.path.join(checkpoint_dir, f"AWGN_{mod}_M{M}_B{batch_len}_n{len(cells)}_e{num_epochs}_{sig[:12]}.npz")
+            have = 0
+            if rank == 0 and os.path.exists(ck):
+                z = np.load(ck)
+                if "signature" in z.files and str(z["signature"]) == sig:
+                    have = 1
+                    for k, (idx, _) in enumerate(members):
+                        SER[idx] = torch.from_numpy(z["ser"][k]).to(dev)
+            if _bcast_flag(have, rank, world, group, dev):
+                continue
+        if runner is not None:                                       # test hook: stands for sweep_vae_awgn_sharded
+            ser = runner(*args)
+        else:
+            ser = sweep_vae_awgn_sharded(*args, device=dev, datagen=datagen, verbose=verbose, rank=rank, world=world, group=group)
+        if ser is None:
+            continue
+        if ck is not None and rank == 0:
+            np.savez(ck, ser=ser.cpu().numpy(), signature=np.array(sig))
+        for k, (idx, _) in enumerate(members):
+            SER[idx] = ser[k].to(dev)
+    if rank != 0:
+        return None
+    return SER, np.arange(0, num_epochs, epe)
