@@ -124,14 +124,11 @@ int vaeq_dp_force_generic(int32_t on);
  * loss / gradients (summation order of the per-CTA partials); 0 = static striding, bitwise reproducible. */
 int vaeq_dp_dynamic_tiles(int32_t on);
 
-/* Backward pass of the fast path: != 0 runs it as ONE warp-specialised launch (dp_bwd_fused.cu: TMA bulk loads, dL/dout
- * never leaves the SM), 0 (default) = the three kernels of dp_fast.cu (dL/dout rows, dW, dh). */
-int vaeq_dp_fused_backward(int32_t on);
-
-/* Tap gradients of the fast path: != 0 (default) computes both correlations (dW, dh) on tcgen05 tensor cores as block outer products
+/* Tap gradients of the fast path: 1 (default) computes both correlations (dW, dh) on tcgen05 tensor cores as block outer products
  * with a 3 x tf32 split and fp32 accumulation in TMEM (dp_taps_tc.cu: 116 us instead of 168 us per 2^22 symbols, agreement with the
  * CUDA-core kernels 3e-7 ... 6e-6 relative, bitwise reproducible); 0 = the two CUDA-core correlation kernels of dp_fast.cu.  This
- * departs from the hot path's stated "no tensor cores" design and was adopted on measurement (DESIGN.md 4a, profiles/r02_tc_taps.txt). */
+ * departs from the hot path's stated "no tensor cores" design and was adopted on measurement (DESIGN.md 4a, profiles/r02_tc_taps.txt).
+ * Any other value returns VAEQ_EINVAL and leaves the setting unchanged. */
 int vaeq_dp_tc_taps(int32_t on);
 
 /* Forward kernel of the fast path: != 0 (default since r02c) runs the 2x2 butterfly FIR and the channel convolution D = h * E_q on

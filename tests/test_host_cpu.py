@@ -34,6 +34,20 @@ def test_library_exports_every_declared_symbol():
     assert bound.vaeq_dp_workspace_bytes(100, 25, 8) > 0 and bound.vaeq_adam_state_floats(25) == 48 * 25 + 4
 
 
+def test_tc_taps_switch_rejects_values_other_than_0_and_1():
+    """vaeq_dp_tc_taps selects the tap-gradient kernels (1 = tcgen05, 0 = CUDA cores); any other value is an error, never a
+    third mode, and the call only sets a flag, so it runs without a GPU."""
+    from vae_equalizer_b200 import _lib
+    lib = _lib.load()
+    try:
+        for bad in (2, 3, 4, 6, -1):
+            assert lib.vaeq_dp_tc_taps(bad) == -1                    # VAEQ_EINVAL
+            assert b"vaeq_dp_tc_taps" in lib.vaeq_last_error()
+        assert lib.vaeq_dp_tc_taps(0) == 0 and lib.vaeq_dp_tc_taps(1) == 0
+    finally:
+        lib.vaeq_dp_tc_taps(1)
+
+
 def test_struct_layout_matches_header_field_order():
     from vae_equalizer_b200 import _lib
     src = open(os.path.join(ROOT, "include", "vaeq.h")).read()

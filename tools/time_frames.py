@@ -40,16 +40,6 @@ for persistent in (0, 2, 1):
     ms = timeit(lambda: eq.train_frame(rx, B, B, n_steps, lr, lr, ot, oc, 0, B, keep_lo_in_dst=True))
     print(f"1 run, persistent mode {persistent}: {ms:.3f} ms per frame of {n_steps} steps x {B} symbols = {ms * 1e3 / n_steps:.2f} us/step, {N / ms / 1e3:.3f} M symbols/s")
 _lib.check(lib.vaeq_dp_persistent_frames(1))
-import ctypes as C
-raw = C.CDLL(_lib.LIB_PATH)
-if hasattr(raw, "vaeq_debug_small_cycles"):
-    eq.train_frame(rx, B, B, n_steps, lr, lr, ot, oc, 0, B, keep_lo_in_dst=True)
-    torch.cuda.synchronize()
-    cyc = (C.c_ulonglong * 16)()
-    raw.vaeq_debug_small_cycles(cyc)
-    names = ["P0 taps+x load", "P1 FIR", "P2 demap", "P3 D+resid", "P4 scalars", "P5 dEq+gy", "P6 tap grads", "P7 adam"]
-    print("dp_small cycles per step:", {n: int(c) // n_steps for n, c in zip(names, cyc)}, "total", sum(int(c) for c in cyc[:8]) // n_steps)
-
 _lib.check(lib.vaeq_dp_frame_runs_per_sm(int(os.environ.get('PER_SM', 0))))       # 0 = automatic, 3 / 4 = force the kernel variant
 for R in [int(v) for v in os.environ.get('RUNS', '1,37,148,296,592,888,1184,2368').split(',')]:
     rxs = torch.stack([generate_data_gpu(N, amps, 23, P, 2, np.pi / 10 + 0.01 * r, dev, 10 + r)[0] for r in range(R)])

@@ -1,4 +1,5 @@
-"""Per-kernel CUDA-event times of the DP step at batch_len 2^22 with the fused backward on and off (vaeq_kernel_timing)."""
+"""Per-kernel CUDA-event times of the DP step at batch_len 2^22 with the tap gradients on the tensor cores and on the CUDA cores
+(vaeq_kernel_timing)."""
 import ctypes as C, os, sys
 import numpy as np, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -13,9 +14,8 @@ h_est, h_ch, P, amp, amps, pol, nu_sc, var, pow_mean = init("h0", "64-QAM", "cpu
 rxs = [generate_data_gpu(B, amps, 23, P, 2, np.pi / 10, "cuda", 1 + i)[0] for i in range(3)]
 q = torch.empty(2, 16, B, device="cuda"); out = torch.empty(2, 2, B, device="cuda")
 NK = 11
-for fused in [int(a) for a in (sys.argv[1:] or ["2", "1", "0"])]:      # 2: tensor-core tap gradients, 1: fused CUDA-core backward, 0: three kernels
-    lib.vaeq_dp_fused_backward(1 if fused == 1 else 0)
-    lib.vaeq_dp_tc_taps(1 | int(os.environ.get('TC_DEBUG', 0)) if fused == 2 else 0)
+for tc in [int(a) for a in (sys.argv[1:] or ["1", "0"])]:             # 1: tensor-core tap gradients, 0: the two CUDA-core kernels
+    _lib.check(lib.vaeq_dp_tc_taps(tc))
     lib.vaeq_dp_tc_forward(int(os.environ.get('TC_FWD', 1)))
     eq = DPEqualizer(M, 2, amp, P, var, nu_sc)
     for i in range(4):
@@ -36,8 +36,7 @@ for fused in [int(a) for a in (sys.argv[1:] or ["2", "1", "0"])]:      # 2: tens
     lib.vaeq_kernel_timing_read(ms, cnt)
     lib.vaeq_kernel_timing(0)
     per = {k: ms[k] / cnt[k] * 1e3 for k in range(NK) if cnt[k]}
-    print(f"backward mode {fused}: step {plain * 1e3:.1f} us plain launches ({B / plain / 1e6:.2f} G symbols/s); kernels (us, by kind id): "
+    print(f"tensor-core taps {tc}: step {plain * 1e3:.1f} us plain launches ({B / plain / 1e6:.2f} G symbols/s); kernels (us, by kind id): "
           + ", ".join(f"{k}: {v:.1f}" for k, v in per.items()) + f"; loss {float(eq.loss):.6g}")
-lib.vaeq_dp_fused_backward(0)
 lib.vaeq_dp_tc_taps(1)
 lib.vaeq_dp_tc_forward(1)

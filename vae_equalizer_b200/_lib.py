@@ -89,7 +89,6 @@ PROTOTYPES = {
     "vaeq_adam_state_floats": (_sz, [_i32]),
     "vaeq_dp_force_generic": (C.c_int, [_i32]),
     "vaeq_dp_dynamic_tiles": (C.c_int, [_i32]),
-    "vaeq_dp_fused_backward": (C.c_int, [_i32]),
     "vaeq_dp_tc_taps": (C.c_int, [_i32]),
     "vaeq_dp_tc_forward": (C.c_int, [_i32]),
     "vaeq_dp_forward": (C.c_int, [C.POINTER(DpDesc), _vp]),

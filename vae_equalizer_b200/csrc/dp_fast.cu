@@ -22,22 +22,6 @@
 
 namespace vaeq {
 
-#ifdef VAEQ_PHASE_TIMING
-__device__ unsigned long long g_phase_cycles[8];
-__device__ __forceinline__ unsigned long long gtime_ns() { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); return t; }
-__device__ unsigned long long g_phase_wall[4];
-__device__ unsigned long long g_cta_t0[2048], g_cta_t1[2048];
-__device__ unsigned int g_cta_sm[2048];
-#define PT_DECL long long _pt = clock64(); const long long _c0 = _pt; const unsigned long long _g0 = gtime_ns(); unsigned long long _acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-#define PT(i) { long long _n = clock64(); _acc[i] += (unsigned long long)(_n - _pt); _pt = _n; }
-#define PT_FLUSH if (threadIdx.x == 64) { g_cta_t0[blockIdx.x] = _g0; g_cta_t1[blockIdx.x] = gtime_ns(); unsigned int _sm; asm("mov.u32 %0, %%smid;" : "=r"(_sm)); g_cta_sm[blockIdx.x] = _sm; } if (threadIdx.x == 64 && blockIdx.x == 3) { for (int i = 0; i < 8; ++i) g_phase_cycles[i] = _acc[i]; g_phase_wall[0] = (unsigned long long)(clock64() - _c0); g_phase_wall[1] = gtime_ns() - _g0; }
-#else
-#define PT_DECL
-#define PT(i)
-#define PT_FLUSH
-#endif
-
-
 // load the even/odd phase arrays of rx for the tile starting at symbol t0 (logical position 0 <-> symbol t0-HP-XOFF)
 // SWZ = false: {I0,Q0,I1,Q1} per position (FIR windows); SWZ = true: {I0,I1,Q0,Q1} (tap-gradient windows, see corr4)
 template <bool SWZ = false>
@@ -111,21 +95,6 @@ __device__ __forceinline__ void transpose_x_raw(const float4 *raw, float4 *xe, f
         xo[pidx(2 * j)] = make_float4(v[0].y, v[r1].y, v[r2].y, v[3].y);
         xe[pidx(2 * j + 1)] = make_float4(v[0].z, v[r1].z, v[r2].z, v[3].z);
         xo[pidx(2 * j + 1)] = make_float4(v[0].w, v[r1].w, v[r2].w, v[3].w);
-    }
-}
-
-#ifndef VAEQ_PREFETCH_OP
-#define VAEQ_PREFETCH_OP "prefetch.global.L2"
-#endif
-// L2 prefetch of `nrows` rows x [first, first+count) floats (128-byte lines), spread over the CTA: issued right after a
-// tile is staged so that the NEXT tile of this persistent CTA is L2-resident when its loads are issued.
-__device__ __forceinline__ void prefetch_rows(const float *base, int64_t ld, int nrows, int64_t first, int count, int64_t limit) {
-    const int lines = (count + 31) / 32;
-#pragma unroll 1
-    for (int idx = threadIdx.x; idx < nrows * lines; idx += FT_NT) {
-        const int r = idx / lines, ln = idx - r * lines;
-        const int64_t off = first + 32 * (int64_t)ln;
-        if (off >= 0 && off < limit) asm volatile(VAEQ_PREFETCH_OP " [%0];" ::"l"(base + (int64_t)r * ld + off));
     }
 }
 
@@ -278,18 +247,14 @@ __global__ void __launch_bounds__(FT_NT, FT_MINB_PW) k_dp_fwd_fast(DpK p) {
 
     float accC[2] = {0.f, 0.f}, accEnt = 0.f, accV0 = 0.f, accV1 = 0.f;   // scalars: accV[pol] in the rolled pol loop lived in local memory
     const int i0 = FT_R * tid;                               // local index of this thread's first symbol
-    PT_DECL
     __shared__ int s_next;
 
 #pragma unroll 1
     for (int tile = blockIdx.x; tile < p.ntiles;) {
         const int t0 = p.clo + tile * FT_T;
-        PT(7)
         tile_fetch_next(p, 0, tile, &s_next);
         transpose_x_raw(raw, xe, xo);                        // this tile's rows were staged while the previous one was computed
-        PT(0)
         __syncthreads();
-        PT(1)
         const int tile_next = s_next;
         if (tile_next < p.ntiles) issue_x_raw(p, p.clo + tile_next * FT_T, raw);      // lands during this tile's compute
 
@@ -310,15 +275,12 @@ __global__ void __launch_bounds__(FT_NT, FT_MINB_PW) k_dp_fwd_fast(DpK p) {
 #pragma unroll 1
             for (int ph = 0; ph < 2; ++ph)
                 fir4(ph ? xo : xe, i0 + FT_XOFF - HF, tapF + (ph ? FT_TAPV * NE : 0), ph ? NO : NE, y);
-            PT(2)
             // point-wise stage: moment form when the prior is of the Maxwell-Boltzmann family (every reference constellation), else the
             // per-level sums (CTA-uniform branch: one of the two code paths runs for the whole launch)
             if (c.quad) fwd_pointwise<NL, MH, true>(p, c, y, m1s, tid, u0, owned, counted, accEnt, accV0, accV1);
             else fwd_pointwise<NL, MH, false>(p, c, y, m1s, tid, u0, owned, counted, accEnt, accV0, accV1);
         }
-        PT(3)
         __syncthreads();
-        PT(4)
 
         // ---- D = h * E_q for the owned samples, residual e = D - rx ------------------------------------
         if (owned) {
@@ -351,13 +313,10 @@ __global__ void __launch_bounds__(FT_NT, FT_MINB_PW) k_dp_fwd_fast(DpK p) {
                 for (int k = 0; k < 4; ++k) st_row4(p.erows, p.B, 4 * ph + k, u0, make_float4(ev[k][0], ev[k][1], ev[k][2], ev[k][3]));
             }
         }
-        PT(5)
         cp_async_wait_all();
         __syncthreads();
-        PT(6)
         tile = tile_next;
     }
-    PT_FLUSH
 
     float v[5] = {accC[0], accC[1], accEnt, accV0, accV1};
     block_sum<5>(v, red);
@@ -372,11 +331,8 @@ __global__ void __launch_bounds__(FT_NT, FT_MINB_PW) k_dp_fwd_fast(DpK p) {
 // backward 1: dL/dE_q (FIR-like over gD = 2 kappa e), then dL/dout = dL/dE_q*S1 + dL/dVar*T2 + w*S3 (coefficients from
 // the forward pass) -> dL/dout rows.  No q, no transcendental: 400 FFMA + ~30 other instructions per symbol.
 // ---------------------------------------------------------------------------------------------
-#ifndef FT_MINB_BWD1
-#define FT_MINB_BWD1 FT_MINB_PW
-#endif
 template <int NL, int MH>
-__global__ void __launch_bounds__(FT_NT, FT_MINB_BWD1) k_dp_bwd1_fast(DpK p) {
+__global__ void __launch_bounds__(FT_NT, FT_MINB_PW) k_dp_bwd1_fast(DpK p) {
     constexpr int M = 2 * MH + 1, HF = MH / 2, NE = MH + 1, NO = MH;
     extern __shared__ __align__(16) float4 smem4[];
     float4 *ge = smem4, *go = ge + FT_ES;
@@ -664,7 +620,7 @@ static int fast_prepare(K kern, size_t smem, int *grid) {
     return VAEQ_OK;
 }
 
-extern bool g_fused_bwd, g_tc_taps, g_tc_fwd;
+extern bool g_tc_taps, g_tc_fwd;
 template <int NL, int MH>
 static int dp_run_fast_t(DpK p, int mode, cudaStream_t st, int *grid_bwd_out) {
     static int grids[VAEQ_MAX_DEVICES][4] = {{0}};           // occupancy-derived grids and the shared-memory attribute are per device
@@ -700,10 +656,6 @@ static int dp_run_fast_t(DpK p, int mode, cudaStream_t st, int *grid_bwd_out) {
         if (rc) return rc;
     }
     if (mode == DP_MODE_FWD) return VAEQ_OK;
-    if (g_fused_bwd) {
-        int rc = VAEQ_OK;
-        if (dp_bwd_fused_launch(p, st, grid_bwd_out, &rc)) return rc;
-    }
     p.ntiles = nt_b;
     ktime_begin(VAEQ_K_DP_BWD, st);
     k_dp_bwd1_fast<NL, MH><<<gb1, FT_NT, s1, st>>>(p);
@@ -724,8 +676,6 @@ static int dp_run_fast_t(DpK p, int mode, cudaStream_t st, int *grid_bwd_out) {
     *grid_bwd_out = gt;
     return VAEQ_OK;
 }
-
-bool g_fused_bwd = false;   // until the fused launch beats the three kernels (profiles/r02_fused_backward.txt)
 
 bool g_tc_fwd = true;       // forward kernel with the FIR and the channel convolution on tcgen05 (dp_fwd_tc.cu), default since r02c: with the moment-form
                             // demapper and the magnitude-ordered MMAs it is faster than k_dp_fwd_fast (244 vs 257 us) at a smaller output error
@@ -759,29 +709,16 @@ int dp_try_fast(const DpK &p, int n_lev, int mode, cudaStream_t st, int *grid_bw
 
 }  // namespace vaeq
 
-extern "C" int vaeq_dp_fused_backward(int32_t on) {
-    vaeq::g_fused_bwd = on != 0;
-    return VAEQ_OK;
-}
-
 extern "C" int vaeq_dp_tc_forward(int32_t on) {
     vaeq::g_tc_fwd = on != 0;
     return VAEQ_OK;
 }
 
-namespace vaeq { extern int g_tc_debug; }
 extern "C" int vaeq_dp_tc_taps(int32_t on) {
+    if (on != 0 && on != 1) {
+        vaeq::set_error("vaeq_dp_tc_taps: %d is not 0 (CUDA-core kernels) or 1 (tensor cores)", on);
+        return VAEQ_EINVAL;
+    }
     vaeq::g_tc_taps = on != 0;
-    vaeq::g_tc_debug = on & ~1;
     return VAEQ_OK;
 }
-
-#ifdef VAEQ_PHASE_TIMING
-extern "C" int vaeq_debug_phase_cycles(unsigned long long *out8) {
-    cudaMemcpyFromSymbol(out8 + 8, vaeq::g_phase_wall, 4 * sizeof(unsigned long long));
-    cudaMemcpyFromSymbol(out8 + 12, vaeq::g_cta_t0, 296 * sizeof(unsigned long long));
-    cudaMemcpyFromSymbol(out8 + 12 + 296, vaeq::g_cta_t1, 296 * sizeof(unsigned long long));
-    { unsigned int sm[296]; cudaMemcpyFromSymbol(sm, vaeq::g_cta_sm, 296 * sizeof(unsigned int)); for (int i = 0; i < 296; ++i) out8[12 + 592 + i] = sm[i]; }
-    return (int)cudaMemcpyFromSymbol(out8, vaeq::g_phase_cycles, 8 * sizeof(unsigned long long));
-}
-#endif

@@ -1,4 +1,4 @@
-// Building blocks of the register-blocked DP kernels (dp_fast.cu, dp_bwd_fused.cu): tile geometry, padded float4 window
+// Building blocks of the register-blocked DP kernels (dp_fast.cu, dp_fwd_tc.cu): tile geometry, padded float4 window
 // indexing, the 3-multiplication FIR-like contraction and the packed tap-gradient correlation.
 #pragma once
 #include "dp_math.cuh"
@@ -6,10 +6,7 @@
 
 namespace vaeq {
 
-#ifndef FT_NT_DEF
-#define FT_NT_DEF 128
-#endif
-constexpr int FT_NT = FT_NT_DEF;           // threads per CTA.  Every tile is load -> barrier -> FIR -> point-wise -> barrier -> ...,
+constexpr int FT_NT = 128;                 // threads per CTA.  Every tile is load -> barrier -> FIR -> point-wise -> barrier -> ...,
                                            // so what hides one CTA's load / barrier phases is the OTHER CTAs of the SM: four
                                            // 128-thread CTAs per SM interleave better than two of 256 (0.664 -> 0.627 ms per step,
                                            // profiles/r01c_*), one of 512 is worst (0.782 vs 0.744, profiles/r01_cta_imbalance.txt).
@@ -22,10 +19,8 @@ constexpr int FT_HP = 8;                   // halo per side in symbols (>= MH/2,
 constexpr int FT_T = FT_TE - 2 * FT_HP;    // owned symbols per tile (1008)
 constexpr int FT_XOFF = 8;                 // extra margin of the x phase arrays (FIR reaches MH/2 further)
 constexpr int FT_XN = FT_TE + 2 * FT_XOFF; // logical length of xe / xo
-#ifndef FT_MINB_PW
-#define FT_MINB_PW FT_CTAS_PER_SM           // min CTAs per SM for the point-wise heavy kernels (fwd, bwd1)
-#endif
-#define FT_MINB FT_CTAS_PER_SM              // ... and for the tap-gradient kernels (56 live accumulators)
+constexpr int FT_MINB_PW = FT_CTAS_PER_SM; // min CTAs per SM for the point-wise heavy kernels (fwd, bwd1)
+constexpr int FT_MINB = FT_CTAS_PER_SM;    // ... and for the tap-gradient kernels (56 live accumulators)
 
 __host__ __device__ constexpr int fdiv4(int c) { return c >= 0 ? c / 4 : -((3 - c) / 4); }
 // padded float4 index of logical position 4*l + c (c compile-time, may be negative)

@@ -31,11 +31,6 @@
 
 namespace vaeq {
 
-#ifndef FWDTC_CENTER
-#define FWDTC_CENTER 1                            // number of centre taps of W and of h kept on the CUDA cores in fp32: 0 (all taps on tcgen05), 1 or 3 (precision, see the kernel)
-#endif
-static_assert(FWDTC_CENTER == 0 || FWDTC_CENTER == 1 || FWDTC_CENTER == 3, "FWDTC_CENTER");
-constexpr int FC_CH = (FWDTC_CENTER - 1) / 2;     // half width of the CUDA-core tap range (meaningful for FWDTC_CENTER > 0)
 constexpr int FC_NG = 4;                          // groups per CTA
 constexpr int FC_GT = 128;                        // threads per group = TMEM lanes = 4-symbol blocks per tile
 constexpr int FC_NT = FC_NG * FC_GT;
@@ -171,7 +166,7 @@ __global__ void __launch_bounds__(FC_NT, 1) k_dp_fwd_tc(DpK p) {
     int *s_next = reinterpret_cast<int *>(smem + 80);                    // [4]
     float *red = reinterpret_cast<float *>(smem + 128);                  // [4 groups][4 warps][8]
     FastConst *cst = reinterpret_cast<FastConst *>(smem + 640);
-    float4 *ctrF = reinterpret_cast<float4 *>(smem + 1024), *ctrD = ctrF + 12;   // centre taps [d = -1, 0, 1][input component] -> 4 outputs
+    float4 *ctrF = reinterpret_cast<float4 *>(smem + 1024), *ctrD = ctrF + 12;   // taps k = MH - 1 + d of W, h: [d][input component] -> 4 outputs
     float *tapF = reinterpret_cast<float *>(smem + 2048);
     float *tapD = tapF + G::TAPF_FLOATS;
     const int tid = threadIdx.x, gt = tid & 127, lane = tid & 31;
@@ -186,7 +181,7 @@ __global__ void __launch_bounds__(FC_NT, 1) k_dp_fwd_tc(DpK p) {
         const int c = step / NKF, s = step - c * NKF, j = 8 * s + k8;
         const int half = n >> 4, i = (n >> 2) & 3, o = n & 3, k = j - 2 * i - SH;
         float v = 0.f;
-        if (k >= 0 && k < M && (!FWDTC_CENTER || k < MH - FC_CH || k > MH + FC_CH)) {      // the centre taps stay on the CUDA cores (see below)
+        if (k >= 0 && k < M && (k < MH || k > MH)) {         // the centre tap stays on the CUDA cores (see below)
             const int op = o >> 1, oc = o & 1, ip = c >> 1, ic = c & 1;
             const float tr = p.W[(op * 4 + ip) * M + k], ti = p.W[(op * 4 + 2 + ip) * M + k];
             v = oc == ic ? tr : (oc ? ti : -ti);             // Re = tr xr - ti xi, Im = ti xr + tr xi
@@ -199,14 +194,16 @@ __global__ void __launch_bounds__(FC_NT, 1) k_dp_fwd_tc(DpK p) {
         const int half = n >> 5, ph = (n >> 4) & 1, i = (n >> 2) & 3, o = n & 3, a = j - i - ph;
         float v = 0.f;
         const int jj = ph ? 2 * MH - 1 - 2 * a : 2 * MH - 2 * a;
-        if (a >= 0 && a < (ph ? MH : MH + 1) && (!FWDTC_CENTER || jj < MH - FC_CH || jj > MH + FC_CH)) {   // even samples: h[2MH - 2a] E_q[u + a - HF];  odd: h[2MH - 1 - 2b] E_q[u + b - HF + 1]
+        if (a >= 0 && a < (ph ? MH : MH + 1) && (jj < MH || jj > MH)) {  // even samples: h[2MH - 2a] E_q[u + a - HF];  odd: h[2MH - 1 - 2b] E_q[u + b - HF + 1]
             const int chi = o >> 1, oc = o & 1, nu = c >> 1, ic = c & 1;
             const float hr = p.h[((chi * 2 + nu) * 2 + 0) * M + jj], hi_ = p.h[((chi * 2 + nu) * 2 + 1) * M + jj];
             v = oc == ic ? hr : (oc ? hi_ : -hi_);
         }
         tapD[idx] = half ? tf32_lo_part(v) : v;
     }
-    if (tid < 96) {                                          // centre taps k = MH - 1 + d of W and h, real-expanded: [d][input component].{4 outputs}
+    // real-expanded taps k = MH - 1 + d of W and h, [d][input component].{4 outputs}; only the centre tap (d = 1) is read.  The table keeps
+    // its three entries: with one, ptxas allocates k_dp_fwd_tc<8, 12> differently and spills 4 bytes
+    if (tid < 96) {
         const int fam = tid / 48, e = tid % 48, d = e / 16, ci = (e >> 2) & 3, o = e & 3, k = MH - 1 + d;
         const int op = o >> 1, oc = o & 1, ip = ci >> 1, ic = ci & 1;
         const float tr = fam ? p.h[((op * 2 + ip) * 2 + 0) * M + k] : p.W[(op * 4 + ip) * M + k];
@@ -339,7 +336,7 @@ __global__ void __launch_bounds__(FC_NT, 1) k_dp_fwd_tc(DpK p) {
         const bool in_seq = (u0 >= 0) && (u0 < p.B);         // B % 4 == 0: all four symbols in or out together
         const bool owned = in_seq && (i0 >= FT_HP) && (i0 < FT_HP + FT_T) && (u0 < p.chi);
         const bool counted = owned && (u0 >= p.sym_lo) && (u0 < p.sym_hi);   // sums only over this rank's symbols
-        // the three centre taps (k = MH - 1, MH, MH + 1: samples 2u - 1, 2u, 2u + 1) on the CUDA cores, in fp32, while the MMAs run: the
+        // the centre tap (k = MH: sample 2u) on the CUDA cores, in fp32, while the MMAs run: the
         // tensor core TRUNCATES every group of four products at the accumulator's ulp (tools/tc_accum_bench.cu), so the terms of
         // magnitude ~1 must not pass through it; what remains there is ~0.1 and its truncation error below the fp32 rounding noise
         float y[FT_R][4];
@@ -355,18 +352,12 @@ __global__ void __launch_bounds__(FC_NT, 1) k_dp_fwd_tc(DpK p) {
                 const float4 xa = *reinterpret_cast<const float4 *>(row + swz32(16u * ch)), xb = *reinterpret_cast<const float4 *>(row + swz32(16u * (ch + 1)));
                 rxs[0][4 * ci + 0] = xa.x; rxs[0][4 * ci + 1] = xa.z; rxs[0][4 * ci + 2] = xb.x; rxs[0][4 * ci + 3] = xb.z;
                 rxs[1][4 * ci + 0] = xa.y; rxs[1][4 * ci + 1] = xa.w; rxs[1][4 * ci + 2] = xb.y; rxs[1][4 * ci + 3] = xb.w;
-                if (FWDTC_CENTER) {
-                    const float xs[9] = {FWDTC_CENTER == 3 ? *reinterpret_cast<const float *>(row + swz32(16u * (ch - 1)) + 12) : 0.f, xa.x, xa.y, xa.z, xa.w, xb.x, xb.y, xb.z, xb.w};
+                const float4 w = ctrF[4 + ci];
 #pragma unroll
-                    for (int d = 1 - FC_CH; d <= 1 + FC_CH; ++d) {
-                        const float4 w = ctrF[d * 4 + ci];
-#pragma unroll
-                        for (int r = 0; r < FT_R; ++r) {
-                            const float2 xx = make_float2(xs[2 * r + d], xs[2 * r + d]);
-                            yc[r][0] = __ffma2_rn(make_float2(w.x, w.y), xx, yc[r][0]);
-                            yc[r][1] = __ffma2_rn(make_float2(w.z, w.w), xx, yc[r][1]);
-                        }
-                    }
+                for (int r = 0; r < FT_R; ++r) {
+                    const float2 xx = make_float2(rxs[0][4 * ci + r], rxs[0][4 * ci + r]);
+                    yc[r][0] = __ffma2_rn(make_float2(w.x, w.y), xx, yc[r][0]);
+                    yc[r][1] = __ffma2_rn(make_float2(w.z, w.w), xx, yc[r][1]);
                 }
             }
             // x_hi is not read again after this point (the FIR MMAs are waited for just below): the samples the residual e = D - rx needs go to
@@ -523,28 +514,22 @@ __global__ void __launch_bounds__(FC_NT, 1) k_dp_fwd_tc(DpK p) {
         }
         __syncwarp();
         if (tile_next < p.ntiles) stage_rx(tile_next);       // every thread of the group is past its last read of x_hi (barrier above): the rows land during the D MMAs and the next tile's top
-        // centre taps of h (j = MH - 1, MH, MH + 1) on the CUDA cores while the MMAs run: even sample h[MH] E_q[u], odd h[MH+1] E_q[u] + h[MH-1] E_q[u+1]
+        // centre tap of h (j = MH) on the CUDA cores while the MMAs run: even sample h[MH] E_q[u]; the odd samples have no centre-tap term
         {
-            float4 eq[FT_R + 1];
+            float4 eq[FT_R];
 #pragma unroll
-            for (int r = 0; r < FT_R + 1; ++r) eq[r] = *reinterpret_cast<const float4 *>(qhi + swz64(qoff0 + 16u * r));
+            for (int r = 0; r < FT_R; ++r) eq[r] = *reinterpret_cast<const float4 *>(qhi + swz64(qoff0 + 16u * r));
 #pragma unroll
             for (int r = 0; r < FT_R; ++r) {
-                float2 a0 = make_float2(0.f, 0.f), a1 = a0, b0 = a0, b1 = a0;
+                float2 a0 = make_float2(0.f, 0.f), a1 = a0;
 #pragma unroll
-                for (int ci = 0; ci < (FWDTC_CENTER ? 4 : 0); ++ci) {
-                    const float4 wm = ctrD[ci], w0 = ctrD[4 + ci], wp = ctrD[8 + ci];
-                    const float q0 = f4c(eq[r], ci), q1 = f4c(eq[r + 1], ci);
-                    a0 = __ffma2_rn(make_float2(w0.x, w0.y), make_float2(q0, q0), a0);
-                    a1 = __ffma2_rn(make_float2(w0.z, w0.w), make_float2(q0, q0), a1);
-                    if (FWDTC_CENTER == 3) {
-                        b0 = __ffma2_rn(make_float2(wp.x, wp.y), make_float2(q0, q0), b0);
-                        b1 = __ffma2_rn(make_float2(wp.z, wp.w), make_float2(q0, q0), b1);
-                        b0 = __ffma2_rn(make_float2(wm.x, wm.y), make_float2(q1, q1), b0);
-                        b1 = __ffma2_rn(make_float2(wm.z, wm.w), make_float2(q1, q1), b1);
-                    }
+                for (int ci = 0; ci < 4; ++ci) {
+                    const float4 w = ctrD[4 + ci];
+                    const float q0 = f4c(eq[r], ci);
+                    a0 = __ffma2_rn(make_float2(w.x, w.y), make_float2(q0, q0), a0);
+                    a1 = __ffma2_rn(make_float2(w.z, w.w), make_float2(q0, q0), a1);
                 }
-                dc[0][r][0] = a0; dc[0][r][1] = a1; dc[1][r][0] = b0; dc[1][r][1] = b1;
+                dc[0][r][0] = a0; dc[0][r][1] = a1; dc[1][r][0] = dc[1][r][1] = make_float2(0.f, 0.f);
             }
         }
         mbar_wait(bar_d, par);

@@ -70,8 +70,6 @@ int dp_launch_fin(const DpK &p, int nparts, cudaStream_t st);
 // dp_fast.cu: returns 1 if the register-blocked path ran (then *rc is its status, *grid_bwd_out the number of
 // gradient partials), 0 if the problem does not qualify (alignment, M_est, size) and the generic kernels must run
 int dp_try_fast(const DpK &p, int n_lev, int mode, cudaStream_t st, int *grid_bwd_out, int *rc);
-// dp_bwd_fused.cu: the fast path's backward pass as one launch; returns 0 if M_est does not qualify
-int dp_bwd_fused_launch(const DpK &p, cudaStream_t st, int *nparts, int *rc);
 // dp_taps_tc.cu: dW and dh on tcgen05 (after k_dp_bwd1_fast); returns 0 if M_est does not qualify
 int dp_taps_tc_launch(const DpK &p, cudaStream_t st, int *nparts, int *rc);
 // dp_fwd_tc.cu: the fast path's forward kernel with the FIR and the channel convolution on tcgen05; returns 0 if (n_lev, M_est) is not built

@@ -41,17 +41,6 @@ __device__ __forceinline__ void block_sum_last(float (&v)[NV], float *scratch) {
 
 __device__ __forceinline__ float fneg(float v) { return __uint_as_float(__float_as_uint(v) ^ 0x80000000u); }   // sign flip as an integer op
 
-#ifdef VAEQ_SMALL_TIMING
-__device__ unsigned long long g_small_cyc[16];
-#define ST_DECL long long _st = clock64(); unsigned long long _sa[16] = {0};
-#define ST(i) { __syncthreads(); long long _n = clock64(); _sa[i] += (unsigned long long)(_n - _st); _st = _n; }
-#define ST_END if (threadIdx.x == 0 && blockIdx.x == 0) for (int i = 0; i < 16; ++i) g_small_cyc[i] = _sa[i];
-#else
-#define ST_DECL
-#define ST(i)
-#define ST_END
-#endif
-
 constexpr int SM_NT = 256;
 
 // shared-memory plan (offsets in floats); doubles first (8-byte aligned), then float4 arrays, then floats
@@ -103,9 +92,7 @@ __device__ __forceinline__ void cp_async4(void *dst_smem, const void *src_gmem) 
     asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(d), "l"(src_gmem) : "memory");
 }
 
-#ifndef SM_MINB
-#define SM_MINB 3          // 85 registers: 3 CTAs (runs) per SM; 98 registers uncapped = 2 CTAs, 64 = 4 CTAs with spills (profiles/r01b_experiments.txt)
-#endif
+constexpr int SM_MINB = 3;   // 3 CTAs (runs) per SM; 98 registers uncapped = 2 CTAs, 64 = 4 CTAs with spills (profiles/r01b_experiments.txt)
 // MINB = 3 (80 registers) is the faster kernel per run; MINB = 4 (64 registers, a few spills) is launched when a fourth run per SM saves a
 // whole wave of CTAs (e.g. 592 runs on 148 SMs: 444 + a tail of 148 at 3 per SM, one wave at 4 per SM), see dp_small_launch
 // MT: M_est at compile time (0 = run time): the tap loops then have constant trip counts and immediate offsets (the kernel is issue-bound:
@@ -177,7 +164,6 @@ __global__ void __launch_bounds__(SM_NT, MINB) k_dp_frame_fast(DpK p, DpRunsK rs
     if (n_steps > 0) issue_window(0);
     const FastConst &c = *cst;
 
-    ST_DECL
     for (int m = 0; m < n_steps; ++m) {
         const int64_t keep_base = (int64_t)m * stride_sym + (keep_lo_in_dst ? p.keep_lo : 0);
         const bool last = m == n_steps - 1;
@@ -227,7 +213,6 @@ __global__ void __launch_bounds__(SM_NT, MINB) k_dp_frame_fast(DpK p, DpRunsK rs
             if (lane == 0) Asum[cn] = carry;
         }
 
-        ST(0)
         // ---- P1: butterfly FIR (sf:500-518) + soft demapper, moments, entropy, backward coefficients (sf:511-523, 101-113):
         //      one (symbol, output pol) item per thread, its two components demapped right away ------------------------------
         float accEnt = 0.f, accV0 = 0.f, accV1 = 0.f;
@@ -285,8 +270,6 @@ __global__ void __launch_bounds__(SM_NT, MINB) k_dp_frame_fast(DpK p, DpRunsK rs
         }
         __syncthreads();
 
-        ST(1)
-        ST(2)
         // ---- P3: D = h * E_q on the valid samples, residual e = D - rx (sf:115-134), one (sample, rx pol) item per thread;
         //      then the edge sums of S_nu(j) = V_nu - edge_nu(j) (Var over source symbols outside Mh <= 2u+j < L, sf:128) --------
         float accC0 = 0.f, accC1 = 0.f;
@@ -331,7 +314,6 @@ __global__ void __launch_bounds__(SM_NT, MINB) k_dp_frame_fast(DpK p, DpRunsK rs
             accB1 += hsq[2 * M + idx] * ed;
         }
 
-        ST(3)
         // ---- P4: ELBO scalars (sf:131-137): C = sum|e|^2 + sum_nu V_nu A_chi,nu - B_chi, loss, var_est, kappa = (L-Mh)/C ---------
         {
             float v[7] = {accC0, accC1, accEnt, accV0, accV1, accB0, accB1};
@@ -386,7 +368,6 @@ __global__ void __launch_bounds__(SM_NT, MINB) k_dp_frame_fast(DpK p, DpRunsK rs
         __syncthreads();
         const float kap0 = scal[0], kap1 = scal[1];
 
-        ST(4)
         for (int u = tid; u < B; u += SM_NT) {
             if (!one_item) contract(u);
             const int jlo = max(0, Mh - 2 * u), jhi = min(M, L - 2 * u);
@@ -406,7 +387,6 @@ __global__ void __launch_bounds__(SM_NT, MINB) k_dp_frame_fast(DpK p, DpRunsK rs
         }
         __syncthreads();
 
-        ST(5)
         // ---- P6: tap gradients.  Warps 0-3: dW[o=0,1][in][k] = sum_u gy_o(u) conj(x_in[2u+k-mh]); warps 4-7:
         //      dh[chi=0,1][nu][j] = 2 kappa_chi sum_v e_chi(2v+j-mh) conj(E_q,nu[v]) (warp-uniform roles).  A thread owns a PAIR of
         //      neighbouring taps of one sample phase (k, k+2): their windows are one position apart, so one LDS.128 of the window
@@ -502,7 +482,6 @@ __global__ void __launch_bounds__(SM_NT, MINB) k_dp_frame_fast(DpK p, DpRunsK rs
             __syncthreads();
         }
 
-        ST(6)
         // ---- P7: E-term of dh (2 kappa_chi h S_nu(j), S = V_nu - edge), Adam on both parameter groups (VAELE_DP:28-31,66) -----
         {
             const double bc1 = dsc[0];
@@ -526,9 +505,7 @@ __global__ void __launch_bounds__(SM_NT, MINB) k_dp_frame_fast(DpK p, DpRunsK rs
             }
         }
         __syncthreads();
-        ST(7)
     }
-    ST_END
 
     // ---- write the trained state back -------------------------------------------------------------------------------
     for (int i = tid; i < 8 * M; i += SM_NT) {
@@ -538,12 +515,6 @@ __global__ void __launch_bounds__(SM_NT, MINB) k_dp_frame_fast(DpK p, DpRunsK rs
     for (int i = tid; i < 48 * M; i += SM_NT) adg[i] = ad[i];
     if (tid == 0) *reinterpret_cast<int *>(adg + 48 * M) = step0 + n_steps;
 }
-
-#ifdef VAEQ_SMALL_TIMING
-}
-extern "C" int vaeq_debug_small_cycles(unsigned long long *out16) { return (int)cudaMemcpyFromSymbol(out16, vaeq::g_small_cyc, 16 * sizeof(unsigned long long)); }
-namespace vaeq {
-#endif
 
 static int g_small_per_sm = 0;       // vaeq_dp_frame_runs_per_sm: 0 = choose by waves, 3 / 4 = force that kernel (tests, A/B timing)
 size_t dp_small_smem(int B, int M) { return (size_t)small_layout(B, M).total * sizeof(float); }

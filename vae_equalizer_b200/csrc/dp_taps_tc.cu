@@ -1,7 +1,8 @@
 // DP VAE step: BOTH tap-gradient correlations (dW and dh) on the 5th-generation tensor cores (tcgen05, accumulators in TMEM).
 //
-// EXPERIMENT OUTSIDE north_star's STATED DESIGN ("tensor cores are not used because the path is not a dense contraction"), asked for by
-// the round-1 review with the 1e-4 gradient gate as the accept / reject criterion; opt-in through vaeq_dp_tc_taps(1).
+// OUTSIDE north_star's STATED DESIGN ("tensor cores are not used because the path is not a dense contraction"), accepted against the
+// 1e-4 gradient tolerance and adopted on measurement (profiles/r02_tc_taps.txt); the default since r02, vaeq_dp_tc_taps(0) selects the
+// CUDA-core kernels of dp_fast.cu.
 //
 // The correlations ARE a dense contraction once the symbol axis is cut into blocks of 16: for a per-symbol operand a(.) and a
 // window operand w(.),
@@ -63,7 +64,7 @@ __device__ __forceinline__ void split_store(unsigned char *hi, unsigned char *lo
 }
 
 template <int MH>
-__global__ void __launch_bounds__(TC_NT, 1) k_dp_taps_tc(DpK p, int t_lo, int dbg) {
+__global__ void __launch_bounds__(TC_NT, 1) k_dp_taps_tc(DpK p, int t_lo) {
     constexpr int M = 2 * MH + 1, HF = MH / 2;
     static_assert(MH % 2 == 0 && HF <= TC_SH, "tensor-core tap gradients need M_est = 1 (mod 4), M_est <= 33");
     extern __shared__ __align__(1024) unsigned char smem[];
@@ -102,7 +103,7 @@ __global__ void __launch_bounds__(TC_NT, 1) k_dp_taps_tc(DpK p, int t_lo, int db
                 asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                 const uint32_t ob = smem_u32(ops + s * 8 * TC_OPB);
 #pragma unroll
-                for (int ks = 0; ks < ((dbg & 2) ? 0 : TC_NK / 8); ++ks) {
+                for (int ks = 0; ks < TC_NK / 8; ++ks) {
 #pragma unroll
                     for (int corr = 0; corr < 2; ++corr) {
                         const uint32_t a_hi = ob + (2 * corr) * TC_OPB + ks * 1024, b_hi = ob + (4 + 2 * corr) * TC_OPB + ks * 1024;
@@ -156,12 +157,10 @@ __global__ void __launch_bounds__(TC_NT, 1) k_dp_taps_tc(DpK p, int t_lo, int db
             cur = nxt;
             if (tile + (int)gridDim.x < nt) fetch(tile + gridDim.x, nxt);
             mbar_wait(mma_done + s, ((it / TC_OS) & 1) ^ 1);                 // the MMAs of tile it - TC_OS have read this stage's operand arrays
-            if (!(dbg & 4)) {
-                split_store(op, op + TC_OPB, off, cur.x);
-                split_store(op + 2 * TC_OPB, op + 3 * TC_OPB, off, make_float4(cur.ea.x, cur.eb.x, cur.ea.y, cur.eb.y));
-                split_store(op + 4 * TC_OPB, op + 5 * TC_OPB, off, cur.g);
-                split_store(op + 6 * TC_OPB, op + 7 * TC_OPB, off, cur.q);
-            }
+            split_store(op, op + TC_OPB, off, cur.x);
+            split_store(op + 2 * TC_OPB, op + 3 * TC_OPB, off, make_float4(cur.ea.x, cur.eb.x, cur.ea.y, cur.eb.y));
+            split_store(op + 4 * TC_OPB, op + 5 * TC_OPB, off, cur.g);
+            split_store(op + 6 * TC_OPB, op + 7 * TC_OPB, off, cur.q);
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");     // generic-proxy stores -> visible to the tensor core's reads
             mbar_arrive(conv_done + s);
         }
@@ -227,7 +226,6 @@ __global__ void __launch_bounds__(TC_NT, 1) k_dp_taps_tc(DpK p, int t_lo, int db
     }
 }
 
-int g_tc_debug = 0;   // timing experiments only (results are wrong): 2 = no MMAs, 4 = no conversion stores
 template <int MH>
 static int taps_tc_launch_t(DpK p, cudaStream_t st, int *nparts) {
     static SmemAttrCache set;
@@ -238,7 +236,7 @@ static int taps_tc_launch_t(DpK p, cudaStream_t st, int *nparts) {
     p.ntiles = (t_hi - t_lo + TC_TS - 1) / TC_TS;
     const int grid = min(sm_count(), p.ntiles);
     ktime_begin(VAEQ_K_DP_BWD2, st);
-    k_dp_taps_tc<MH><<<grid, TC_NT, sm, st>>>(p, t_lo, g_tc_debug);
+    k_dp_taps_tc<MH><<<grid, TC_NT, sm, st>>>(p, t_lo);
     ktime_end(VAEQ_K_DP_BWD2, st);
     VAEQ_LAUNCH_CHECK("k_dp_taps_tc");
     *nparts = grid;

@@ -24,10 +24,7 @@ constexpr int SC_NT = 128, SC_NW = SC_NT / 32;
 constexpr int SC_T = 384;                      // symbols per tile
 constexpr int SC_SLICE = SC_T / SC_NW;         // symbols per warp and tile
 constexpr int SC_MAXSHIFT = 64;
-#ifndef SC_MINB_DEF
-#define SC_MINB_DEF 6
-#endif
-constexpr int SC_MINB = SC_MINB_DEF;            // CTAs per SM: the tile loop is load -> barrier -> correlate -> barrier, other CTAs hide the waits
+constexpr int SC_MINB = 6;                     // CTAs per SM: the tile loop is load -> barrier -> correlate -> barrier, other CTAs hide the waits
 
 struct ShiftSmem {
     float E[2][SC_T + 2 * SC_MAXSHIFT];        // window of E, starting SC back4 positions before the tile

@@ -1,19 +1,15 @@
-// mbarrier / TMA bulk-copy / tcgen05 helpers (PTX) shared by the warp-specialised kernels (dp_bwd_fused.cu, dp_taps_tc.cu).
+// mbarrier and named-barrier helpers (PTX) shared by the tcgen05 kernels (dp_fwd_tc.cu, dp_taps_tc.cu).
 #pragma once
 #include "common.cuh"
 
 namespace vaeq {
 
-// ---- mbarrier / TMA bulk copy (PTX) -----------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(uint64_t *b, int count) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(b)), "r"(count) : "memory");
 }
 __device__ __forceinline__ void mbar_arrive(uint64_t *b) {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(b)) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t *b, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(b)), "r"(bytes) : "memory");
 }
 __device__ __forceinline__ void mbar_wait(uint64_t *b, uint32_t parity) {
     asm volatile(
@@ -27,36 +23,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t *b, uint32_t parity) {
         "}" ::"r"(smem_u32(b)), "r"(parity)
         : "memory");
 }
-__device__ __forceinline__ void bulk_g2s(void *dst_smem, const void *src_gmem, uint32_t bytes, uint64_t *bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst_smem)),
-                 "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar))
-                 : "memory");
-}
 __device__ __forceinline__ void named_bar_sync(int id, int nthreads) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory"); }
-
-// ---- staging of row segments by one warp ------------------------------------------------------------------------------
-// `nrows` segments [start, start+len) of the rows `src + r*ld` go to dst + r*len; only the part inside [lo, hi) is copied
-// (cp.async.bulk, 16-byte granules: start, lo, hi are multiples of 4 floats), the rest is zero-filled by the warp.
-__device__ __forceinline__ uint32_t rows_bytes(int nrows, int64_t start, int len, int64_t lo, int64_t hi) {
-    const int64_t c0 = start < lo ? lo : start, c1 = start + len > hi ? hi : start + len;
-    return c1 > c0 ? (uint32_t)(nrows * (c1 - c0) * 4) : 0u;
-}
-__device__ __forceinline__ void rows_zero_fill(float *dst, int nrows, int64_t start, int len, int64_t lo, int64_t hi, int lane) {
-    const int64_t c0 = start < lo ? lo : start, c1 = start + len > hi ? hi : start + len;
-    if (c0 == start && c1 == start + len) return;
-    const int n0 = c1 > c0 ? (int)(c0 - start) : len, n1 = c1 > c0 ? (int)(c1 - start) : len;   // keep [n0, n1)
-    for (int r = 0; r < nrows; ++r) {
-        for (int i = lane; i < n0; i += 32) dst[r * len + i] = 0.f;
-        for (int i = n1 + lane; i < len; i += 32) dst[r * len + i] = 0.f;
-    }
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-}
-__device__ __forceinline__ void rows_issue(float *dst, const float *src, int64_t ld, int nrows, int64_t start, int len, int64_t lo, int64_t hi,
-                                           uint64_t *bar) {
-    const int64_t c0 = start < lo ? lo : start, c1 = start + len > hi ? hi : start + len;
-    if (c1 <= c0) return;
-    const uint32_t bytes = (uint32_t)((c1 - c0) * 4);
-    for (int r = 0; r < nrows; ++r) bulk_g2s(dst + r * len + (c0 - start), src + (int64_t)r * ld + c0, bytes, bar);
-}
 
 }  // namespace vaeq
