@@ -348,6 +348,25 @@ int vaeq_ser_cma(float *rx, int64_t ld_rx, const uint16_t *tx, int64_t ld_tx, co
  * max|corr_I| < 0.02 n_rx and max|corr_Q| >= max|corr_I| */
 int vaeq_find_shift_symb(const float *rx, int32_t n_rx, const uint16_t *tx, int64_t ld_tx, int32_t n_tx, int32_t n_shift, float *corr_out,
                          int32_t *shift_out, void *stream);
+/* A validation period of the AWGN CMA driver for n_runs runs in ONE launch (one warp per run): n_frames training frames in sequence
+ * (cm:142-168 with updates, no per-symbol output), then the pass without updates over the validation frame.  Bit for bit a loop of
+ * vaeq_cma_awgn calls per run (n_frames with train = 1, then one with train = 0).
+ *   rx_train: frame f of run k at rx_train + k*rs_t + f*fs_t, I row of N_train samples, Q row ld_t further
+ *   rx_valid: run k at rx_valid + k*rs_v, I row of N_valid samples, Q row ld_v further
+ *   h (n_runs,2,M) taps, updated in place; lr (n_runs) float per run; out_v (n_runs,2,N_valid/sps) */
+int vaeq_cma_awgn_runs(const float *rx_train, int64_t ld_t, int64_t fs_t, int64_t rs_t, int32_t n_frames, int32_t N_train,
+                       const float *rx_valid, int64_t ld_v, int64_t rs_v, int32_t N_valid, float *h, int32_t M, const float *lr, float R,
+                       int32_t sps, float *out_v, int32_t n_runs, void *stream);
+/* Validation scoring of the AWGN CMA driver (cm:227-229) for n_runs runs without a host sync: per run
+ *   shift = find_shift_symb(y, tx, n_shift), then SER_CMA(y[:, edge+shift : N-edge], tx[:, edge : N-edge-shift]),
+ * bit for bit as vaeq_find_shift_symb + vaeq_ser_cma, except that the rescaled values are NOT written back to y (the driver never
+ * reads them).  y (n_runs,2,N) float: rows ld_y apart, runs rs_y apart; tx (n_runs,2,N) float16 bits.  Needs N >= 1000 + n_shift/2
+ * and edge >= n_shift/2.  Outputs on the device: shift (n_runs) int32, counts (n_runs,4) int32, ser (n_runs) float.
+ * scratch: vaeq_awgn_cma_eval_scratch_bytes. */
+size_t vaeq_awgn_cma_eval_scratch_bytes(int32_t n_runs, int32_t N, int32_t n_shift, int32_t edge);
+int vaeq_awgn_cma_eval_runs(const float *y, int64_t ld_y, int64_t rs_y, const uint16_t *tx, int64_t ld_tx, int64_t rs_tx, const float *amp,
+                            int32_t n_lev, int32_t N, int32_t n_shift, int32_t edge, int32_t n_runs, int32_t *shift_out, int32_t *counts_out,
+                            float *ser_out, void *scratch, void *stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Synthetic test signal on the device, n_runs independent runs per call (generate_data_shaping sf:65-90, channel 'h0'; the

@@ -136,6 +136,9 @@ PROTOTYPES = {
     "vaeq_cpe_awgn": (C.c_int, [_vp, _i32, _i32, _vp, _vp, _vp]),
     "vaeq_ser_cma": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _i32, _i32, _vp, _vp, _vp, _vp]),
     "vaeq_find_shift_symb": (C.c_int, [_vp, _i32, _vp, _i64, _i32, _i32, _vp, _vp, _vp]),
+    "vaeq_cma_awgn_runs": (C.c_int, [_vp, _i64, _i64, _i64, _i32, _i32, _vp, _i64, _i64, _i32, _vp, _i32, _vp, _f, _i32, _vp, _i32, _vp]),
+    "vaeq_awgn_cma_eval_scratch_bytes": (_sz, [_i32, _i32, _i32, _i32]),
+    "vaeq_awgn_cma_eval_runs": (C.c_int, [_vp, _i64, _i64, _vp, _i64, _i64, _vp, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp]),
     "vaeq_awgn_workspace_bytes": (_sz, [_i32, _i32, _i32]),
     "vaeq_adam_state_floats_awgn": (_sz, [_i32]),
     "vaeq_awgn_forward": (C.c_int, [C.POINTER(AwgnDesc), _vp]),

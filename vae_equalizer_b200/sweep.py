@@ -445,6 +445,18 @@ def _awgn_check(num_epochs, epe, channel, device):
     return dev
 
 
+def _awgn_host_frames(N, F, M, amps, snr, h_channel, sps, dev, P, rngs):
+    """F frames of N symbols per run from the host generator, run r drawing from rngs[r] in frame order: rx (R, F, 2, sps*N), tx (R, F, 2, N)."""
+    from .awgn import generate_data
+    R = len(rngs)
+    rx = torch.empty(R, F, 2, sps * N, dtype=torch.float32, device=dev)
+    tx = torch.empty(R, F, 2, N, dtype=torch.float16, device=dev)
+    for r in range(R):
+        for f in range(F):
+            rx[r, f], tx[r, f] = generate_data(N, M, amps, snr[r], h_channel, sps, dev, P[r], rng=rngs[r])
+    return rx, tx
+
+
 def sweep_vae_awgn(cells, mod, sps, M_est, batch_len, N_valid, N_train, num_epochs, epe, channel, *, device=None, datagen="gpu", verbose=False):
     """processing_vaele_awgn (:235-324) for R = len(cells) independent cells in lockstep.
 
@@ -454,7 +466,7 @@ def sweep_vae_awgn(cells, mod, sps, M_est, batch_len, N_valid, N_train, num_epoc
     The epe - 1 epochs after the last validation do not change the result and are not trained.
     datagen="gpu": every cell's frames from the device generator, keyed by the cell's seed (a cell gives the same SER alone or in any
     batch); "numpy": each cell's frames from np.random.default_rng(seed) in exactly the order processing_vaele_awgn(rng=...) draws them."""
-    from .awgn import AWGNEqualizerRuns, awgn_eval_runs, generate_data, generate_frames_awgn_gpu
+    from .awgn import AWGNEqualizerRuns, awgn_eval_runs, generate_frames_awgn_gpu
     from .constants import awgn_constants, upsampled_channel
     dev = _awgn_check(num_epochs, epe, channel, device)
     if datagen not in ("gpu", "numpy"):
@@ -479,12 +491,7 @@ def sweep_vae_awgn(cells, mod, sps, M_est, batch_len, N_valid, N_train, num_epoc
     SER_valid = torch.empty(R, n_val, device=dev, dtype=torch.float32)
 
     def host_frames(N, F):
-        rx = torch.empty(R, F, 2, sps * N, dtype=torch.float32, device=dev)
-        tx = torch.empty(R, F, 2, N, dtype=torch.float16, device=dev)
-        for r in range(R):
-            for f in range(F):
-                rx[r, f], tx[r, f] = generate_data(N, M, amps, snr[r], h_channel, sps, dev, consts[r][1], rng=rngs[r])
-        return rx, tx
+        return _awgn_host_frames(N, F, M, amps, snr, h_channel, sps, dev, [k[1] for k in consts], rngs)
 
     epoch = 0
     for k in range(n_val):
@@ -532,30 +539,56 @@ def run_awgn_sweep(mod="64-QAM", sps=2, channel="h1", N_train_vec=(350,), lr_opt
         epochs (num_epochs // epe,).
     Cell (.., i) is seeded with its flat index.  checkpoint_dir: rank 0 stores every finished set (one .npz, keyed by the set's full
     parameters); a restarted sweep loads what it finds instead of recomputing."""
-    import os
     if channel not in ("h1", "h2"):
         raise KeyError(f"AWGN driver knows channels h1/h2, got {channel!r}")
     if epe < 1 or num_epochs % epe != 0:
         raise ValueError(f"num_epochs={num_epochs} must be a multiple of epe={epe}")
     vecs = dict(batch_len=list(N_train_vec), lr_optim=list(lr_optim_vec), M=list(M_vec), SNR=list(SNR_vec), nu=list(nu_vec))
-    shape = tuple(len(vecs[a]) for a in AWGN_AXES) + (iter,)
-    n_val = num_epochs // epe
     dev = torch.device("cpu") if runner is not None and device is None else _cuda_device(device)
+
+    def signature(key, cells):
+        M, batch_len = key
+        return _set_signature(driver="VAELE_AWGN", mod=mod, sps=sps, channel=channel, M=M, batch_len=batch_len, N_valid=N_valid,
+                              train_len=train_len, num_epochs=num_epochs, epe=epe, datagen=datagen, cells=[sorted(c.items()) for c in cells])
+
+    def file_name(key, cells, sig):
+        M, batch_len = key
+        return f"AWGN_{mod}_M{M}_B{batch_len}_n{len(cells)}_e{num_epochs}_{sig[:12]}.npz"
+
+    def run_set(key, cells):
+        M, batch_len = key
+        args = (cells, mod, sps, M, batch_len, N_valid, train_len, num_epochs, epe, channel)
+        if runner is not None:                                       # test hook: stands for sweep_vae_awgn_sharded
+            return runner(*args)
+        return sweep_vae_awgn_sharded(*args, device=dev, datagen=datagen, verbose=verbose, rank=rank, world=world, group=group)
+
+    SER = _walk_awgn_sets(AWGN_AXES, vecs, ("M", "batch_len"), iter, num_epochs // epe, dev, checkpoint_dir, rank, world, group, signature,
+                          file_name, run_set)
+    if rank != 0:
+        return None
+    return SER, np.arange(0, num_epochs, epe)
+
+
+def _walk_awgn_sets(axes, vecs, group_by, iter, n_val, dev, checkpoint_dir, rank, world, group, signature, file_name, run_set):
+    """The cells of vecs[axes[0]] x ... x iter, seeded by their flat index, grouped into one run set per value of the `group_by` axes.
+    Per set: with checkpoint_dir, rank 0 loads the set's file if its stored signature(key, cells) matches (all ranks then skip it);
+    otherwise run_set(key, cells) gives SER_valid (n, n_val) on rank 0 (None elsewhere), which rank 0 stores under
+    file_name(key, cells, sig).  Returns SER (shape of the cells, n_val)."""
+    import os
+    shape = tuple(len(vecs[a]) for a in axes) + (iter,)
     SER = torch.full(shape + (n_val,), float("nan"), dtype=torch.float32, device=dev)
     groups = {}
     for idx in np.ndindex(*shape):
-        c = {a: vecs[a][i] for a, i in zip(AWGN_AXES, idx[:-1])}
+        c = {a: vecs[a][i] for a, i in zip(axes, idx[:-1])}
         c["seed"] = int(np.ravel_multi_index(idx, shape))
-        groups.setdefault((c["M"], c["batch_len"]), []).append((idx, c))
-    for (M, batch_len), members in groups.items():
+        groups.setdefault(tuple(c[a] for a in group_by), []).append((idx, c))
+    for key, members in groups.items():
         cells = [{k: c[k] for k in ("SNR", "nu", "lr_optim", "seed")} for _, c in members]
-        args = (cells, mod, sps, M, batch_len, N_valid, train_len, num_epochs, epe, channel)
         ck, sig = None, None
         if checkpoint_dir is not None:
             os.makedirs(checkpoint_dir, exist_ok=True)
-            sig = _set_signature(driver="VAELE_AWGN", mod=mod, sps=sps, channel=channel, M=M, batch_len=batch_len, N_valid=N_valid,
-                                 train_len=train_len, num_epochs=num_epochs, epe=epe, datagen=datagen, cells=[sorted(c.items()) for c in cells])
-            ck = os.path.join(checkpoint_dir, f"AWGN_{mod}_M{M}_B{batch_len}_n{len(cells)}_e{num_epochs}_{sig[:12]}.npz")
+            sig = signature(key, cells)
+            ck = os.path.join(checkpoint_dir, file_name(key, cells, sig))
             have = 0
             if rank == 0 and os.path.exists(ck):
                 z = np.load(ck)
@@ -565,16 +598,122 @@ def run_awgn_sweep(mod="64-QAM", sps=2, channel="h1", N_train_vec=(350,), lr_opt
                         SER[idx] = torch.from_numpy(z["ser"][k]).to(dev)
             if _bcast_flag(have, rank, world, group, dev):
                 continue
-        if runner is not None:                                       # test hook: stands for sweep_vae_awgn_sharded
-            ser = runner(*args)
-        else:
-            ser = sweep_vae_awgn_sharded(*args, device=dev, datagen=datagen, verbose=verbose, rank=rank, world=world, group=group)
+        ser = run_set(key, cells)
         if ser is None:
             continue
         if ck is not None and rank == 0:
             np.savez(ck, ser=ser.cpu().numpy(), signature=np.array(sig))
         for k, (idx, _) in enumerate(members):
             SER[idx] = ser[k].to(dev)
+    return SER
+
+
+# -------------------------------------------------------------------------------------------------
+# AWGN single-polarisation CMA baseline (AWGN_channel/func_CMA_MQAM_shaping.py:201-256, `cm:`)
+# -------------------------------------------------------------------------------------------------
+def sweep_cma_awgn(cells, mod, sps, M_est, N_valid, N_train, num_epochs, epe, channel, *, device=None, datagen="gpu", verbose=False):
+    """processing_cma_awgn (cm:201-256) for R = len(cells) independent cells in lockstep.
+
+    cells: dicts with SNR, nu, lr_optim and optionally seed (default: the cell's index).  Returns SER_valid (R, num_epochs // epe), row k
+    being what processing_cma_awgn returns for cell k, bit for bit.  A validation period is generation, ONE launch that runs every cell's
+    CMA over its training frames since the last validation and then over its validation frame (awgn_cma.CMA_runs), one batched CPE and
+    the batched scoring (awgn_cma.awgn_cma_eval_runs): no host sync.  The epe - 1 epochs after the last validation do not change the
+    result and are not trained.
+    datagen="gpu": frames from the device generator with the frame keys of sweep_vae_awgn (training frame = epoch index, validation
+    frame k = AWGN_VALID_FRAME0 + k), so a cell with the same seed, N_train and N_valid sees the same frames in both sweeps and the two
+    baselines are compared on identical data; a cell gives the same SER alone or in any batch.  "numpy": each cell's frames from
+    np.random.default_rng(seed) in exactly the order processing_cma_awgn(rng=...) draws them."""
+    from . import awgn_cma as cm
+    from .awgn import generate_frames_awgn_gpu
+    from .constants import awgn_constants, upsampled_channel
+    dev = _awgn_check(num_epochs, epe, channel, device)
+    if datagen not in ("gpu", "numpy"):
+        raise ValueError(f"datagen={datagen!r}: 'gpu' or 'numpy'")
+    R = len(cells)
+    if R == 0:
+        raise ValueError("no cells")
+    h_channel = upsampled_channel(channel, sps)
+    M = (len(h_channel) - 1) // sps + 1
+    consts = [awgn_constants(mod, float(_cell(c, "nu")), float(_cell(c, "SNR"))) for c in cells]
+    amps = consts[0][0]
+    amp_levels = torch.tensor(amps, device=dev, dtype=torch.float32)
+    P = torch.tensor(np.stack([k[1] for k in consts]), dtype=torch.float32)
+    lr = torch.tensor([float(_cell(c, "lr_optim")) for c in cells], dtype=torch.float32, device=dev)     # the fp32 value CMA() passes
+    seeds = [int(c.get("seed", i)) for i, c in enumerate(cells)]
+    rngs = [np.random.default_rng(s) for s in seeds]
+    snr = [float(c["SNR"]) for c in cells]
+    h = torch.zeros(R, 2, M_est, device=dev, dtype=torch.float32)         # cm:233-235
+    h[:, 0, M_est // 2] = 1.0
+    n_val = num_epochs // epe
+    SER_valid = torch.empty(R, n_val, device=dev, dtype=torch.float32)
+    epoch = 0
+    for k in range(n_val):
+        n_ep = 1 if k == 0 else epe                                  # epochs epoch .. epoch + n_ep - 1, then validate (epoch % epe == 0)
+        if datagen == "gpu":
+            rx, _ = generate_frames_awgn_gpu(N_train, amps, snr, P, h_channel, sps, dev, seeds, frame0=epoch, n_frames=n_ep)
+            rx_v, tx_v = generate_frames_awgn_gpu(N_valid, amps, snr, P, h_channel, sps, dev, seeds, frame0=AWGN_VALID_FRAME0 + k)
+        else:
+            rx, _ = _awgn_host_frames(N_train, n_ep, M, amps, snr, h_channel, sps, dev, [c[1] for c in consts], rngs)
+            rx_v, tx_v = _awgn_host_frames(N_valid, 1, M, amps, snr, h_channel, sps, dev, [c[1] for c in consts], rngs)
+        out_v = cm.CMA_runs(rx, rx_v[:, 0], h, lr, sps)
+        epoch += n_ep
+        shift, _, ser = cm.awgn_cma_eval_runs(cm.CPE(out_v), tx_v[:, 0], amp_levels)
+        SER_valid[:, k] = ser
+        if verbose:
+            print(epoch - 1, "shift", shift.tolist(), "SER", ser.tolist())
+    return SER_valid
+
+
+def sweep_cma_awgn_sharded(cells, *args, rank=0, world=1, group=None, **kw):
+    """sweep_cma_awgn over a round-robin share of the cells per rank (one process per GPU); SER_valid of ALL cells on rank 0 (None
+    elsewhere).  No data-path collective."""
+    from .parallel import gather_cell_results, shard_cells
+    mine = shard_cells(cells, rank, world)
+    num_epochs, epe = (args[5], args[6]) if len(args) > 6 else (kw["num_epochs"], kw["epe"])
+    dev = _cuda_device(kw.get("device"))
+    loc = {}
+    if mine:
+        ser = sweep_cma_awgn([c for _, c in mine], *args, **kw)
+        loc = {i: ser[k] for k, (i, _) in enumerate(mine)}
+    return gather_cell_results(loc, len(cells), (num_epochs // epe,), rank, world, group, dev)
+
+
+AWGN_CMA_AXES = ("lr_optim", "M", "SNR", "nu")                     # index order of run_awgn_cma_sweep's SER, then iter
+
+
+def run_awgn_cma_sweep(mod="64-QAM", sps=2, channel="h1", lr_optim_vec=(5e-4,), M_vec=(25,), SNR_vec=(12,), nu_vec=(0.0,), iter=1, N_valid=15000,
+                       N_train=1200, num_epochs=500, epe=20, *, device=None, datagen="gpu", rank=0, world=1, group=None, runner=None,
+                       verbose=False, checkpoint_dir=None):
+    """A sweep of the AWGN CMA baseline over lr_optim x M x SNR x nu x iter as batched run sets (sweep_cma_awgn_sharded), one set per M.
+    The reference's sweep script for this driver is not part of this package: the axis order (that of run_awgn_sweep without its
+    batch_len axis) and the defaults (N_valid, N_train, num_epochs and epe as run_awgn_sweep's) are this package's choice.  With
+    world > 1 every rank takes a round-robin share of each set.  Returns on rank 0 (None elsewhere)
+        SER (len(lr_optim_vec), len(M_vec), len(SNR_vec), len(nu_vec), iter, num_epochs // epe) and the validation epochs (num_epochs // epe,).
+    Cell (.., i) is seeded with its flat index, as in run_awgn_sweep.  checkpoint_dir: rank 0 stores every finished set (one .npz named
+    AWGNCMA_..., keyed by the set's full parameters; never mistaken for a VAE-LE set of the same directory); a restarted sweep loads what
+    it finds instead of recomputing.  runner: stands for sweep_cma_awgn_sharded (called with its positional arguments)."""
+    if channel not in ("h1", "h2"):
+        raise KeyError(f"AWGN driver knows channels h1/h2, got {channel!r}")
+    if epe < 1 or num_epochs % epe != 0:
+        raise ValueError(f"num_epochs={num_epochs} must be a multiple of epe={epe}")
+    vecs = dict(lr_optim=list(lr_optim_vec), M=list(M_vec), SNR=list(SNR_vec), nu=list(nu_vec))
+    dev = torch.device("cpu") if runner is not None and device is None else _cuda_device(device)
+
+    def signature(key, cells):
+        return _set_signature(driver="CMA_AWGN", mod=mod, sps=sps, channel=channel, M=key[0], N_valid=N_valid, N_train=N_train,
+                              num_epochs=num_epochs, epe=epe, datagen=datagen, cells=[sorted(c.items()) for c in cells])
+
+    def file_name(key, cells, sig):
+        return f"AWGNCMA_{mod}_M{key[0]}_n{len(cells)}_e{num_epochs}_{sig[:12]}.npz"
+
+    def run_set(key, cells):
+        args = (cells, mod, sps, key[0], N_valid, N_train, num_epochs, epe, channel)
+        if runner is not None:
+            return runner(*args)
+        return sweep_cma_awgn_sharded(*args, device=dev, datagen=datagen, verbose=verbose, rank=rank, world=world, group=group)
+
+    SER = _walk_awgn_sets(AWGN_CMA_AXES, vecs, ("M",), iter, num_epochs // epe, dev, checkpoint_dir, rank, world, group, signature, file_name,
+                          run_set)
     if rank != 0:
         return None
     return SER, np.arange(0, num_epochs, epe)
