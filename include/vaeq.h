@@ -304,6 +304,19 @@ int vaeq_frame_eval_runs_ex(const float *q, int64_t ld_q, int64_t rs_q, const fl
 int vaeq_cma_align_rescale(const float *out, int64_t ld_out, int64_t rs_out, const int32_t *align, const float *scale, int32_t N,
                            int32_t edge, int32_t n_runs, float *oc, void *stream);
 
+/* extension, not in the reference: GMI of the soft-demapper SER's region and hypothesis for n_runs runs, without a host sync.
+ *   GMI = H(X) + mean over the evaluated symbols of log2 q(x_tx | y), per pol, bit per 2-D symbol; H(X) = -2 sum_l P_l log2 P_l of
+ *   the run's pmf; q clamped at 1e-30 before the log; logs and sums in double, one cast to float at the end.
+ * The symbols are exactly those the SER counts: estimator 0 (from q) of vaeq_frame_eval_runs_ex, i.e. align (R,2,4) row [run][0] =
+ * {shift_x, shift_y, r, n_eval}, cut per minibatch with seg_len (0: no cut).  Per pol the (IQ flip, rotation) with the smallest error
+ * count of counts (R,2,2,2,4) [est][flip][pol][rotation] is scored (counter order, the first wins ties), so GMI is invariant under the
+ * symmetries the SER forgives.  q (R,2,2n,N), tx (R,2,2,N) float16 bits, P (R,n) with run stride rs_P; gmi_out (R,2); n_eval == 0
+ * gives NaN.  A run's result depends on its own inputs only (not on n_runs).  scratch: vaeq_frame_gmi_scratch_bytes. */
+size_t vaeq_frame_gmi_scratch_bytes(int32_t n_runs, int32_t N);
+int vaeq_frame_gmi_runs(const float *q, int64_t ld_q, int64_t rs_q, const uint16_t *tx, int64_t ld_tx, int64_t rs_tx, const float *P,
+                        int64_t rs_P, const int32_t *align, const int32_t *counts, int32_t n_lev, int32_t N, int32_t n_runs, int32_t seg_len,
+                        int32_t edge, int32_t n_cut, float *gmi_out, void *scratch, void *stream);
+
 /* extension, not in the reference: achievable-rate estimate H(X)+E[log2 q(x_tx|y)] per pol (bit/2D symbol);
  * scratch: VAEQ_EVAL_SCRATCH_BYTES */
 int vaeq_gmi(const float *q, int64_t ld_q, const uint16_t *tx, int64_t ld_tx, const float *P, int32_t n_lev, int32_t N,
@@ -453,6 +466,14 @@ size_t vaeq_awgn_eval_scratch_bytes(int32_t n_runs, int32_t n_shift, int32_t n_c
 int vaeq_awgn_eval_runs(const float *q, int64_t ld_q, int64_t rs_q, const uint16_t *tx, int64_t ld_tx, int64_t rs_tx, const float *amp,
                         int32_t n_lev, int32_t N, int32_t n_shift, int32_t n_corr, int32_t edge, int32_t n_runs, int32_t *shift_out,
                         int32_t *counts_out, float *ser_out, void *scratch, void *stream);
+/* The GMI of vaeq_frame_gmi_runs for the AWGN driver: one polarisation, no IQ flip.  q[:, edge + shift : N - edge] against
+ * tx[:, edge : N - edge - shift] with shift (R) and counts (R,4) [rotation] of vaeq_awgn_eval_runs; gmi_out (R).  Needs
+ * edge >= n_shift/2 of that call (the default 11 >= 10), so edge + shift >= 0; a run whose shift is below -edge gives NaN.
+ * scratch: vaeq_awgn_gmi_scratch_bytes. */
+size_t vaeq_awgn_gmi_scratch_bytes(int32_t n_runs, int32_t N);
+int vaeq_awgn_gmi_runs(const float *q, int64_t ld_q, int64_t rs_q, const uint16_t *tx, int64_t ld_tx, int64_t rs_tx, const float *P, int64_t rs_P,
+                       const int32_t *shift, const int32_t *counts, int32_t n_lev, int32_t N, int32_t n_runs, int32_t edge, float *gmi_out,
+                       void *scratch, void *stream);
 
 #ifdef __cplusplus
 }

@@ -120,6 +120,10 @@ PROTOTYPES = {
     "vaeq_frame_eval_runs_ex": (C.c_int, [_vp, _i64, _i64, _vp, _i64, _i64, _vp, _i64, _i64, _vp, _vp, _i64, _vp, _i32, _i32, _i32, _i32, _i32,
                                          _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
     "vaeq_cma_align_rescale": (C.c_int, [_vp, _i64, _i64, _vp, _vp, _i32, _i32, _i32, _vp, _vp]),
+    "vaeq_frame_gmi_scratch_bytes": (_sz, [_i32, _i32]),
+    "vaeq_frame_gmi_runs": (C.c_int, [_vp, _i64, _i64, _vp, _i64, _i64, _vp, _i64, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp]),
+    "vaeq_awgn_gmi_scratch_bytes": (_sz, [_i32, _i32]),
+    "vaeq_awgn_gmi_runs": (C.c_int, [_vp, _i64, _i64, _vp, _i64, _i64, _vp, _i64, _vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp]),
     "vaeq_soft_dec_runs": (C.c_int, [_vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp, _vp]),
     "vaeq_gmi": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _i32, _i32, _vp, _vp, _vp]),
     "vaeq_cma_scratch_bytes": (_sz, [_i32, _i32, _i32]),

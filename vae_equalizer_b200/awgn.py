@@ -207,6 +207,35 @@ def awgn_eval_runs(q, tx, amp_levels, n_shift=21, n_corr=1000, edge=11):
     return shift, counts, ser
 
 
+@_lib.device_guard
+def awgn_gmi_runs(q, tx, P, shift, counts, edge=11):
+    """EXTENSION (not in the reference): GMI = H(X) + mean log2 q(x_tx|y) (bit/2D-symbol) of R runs on exactly the symbols awgn_eval_runs
+    scores (q[:, edge+shift : N-edge] against tx[:, edge : N-edge-shift]) under its best rotation: q (R,2n,N), tx (R,2,N) float16, P (R,n)
+    or (n,) pmf, shift (R,) and counts (R,4) int32 from awgn_eval_runs with the same edge.  Returns (R,) float32 on the device; no host sync."""
+    from .dp import _require_cuda
+    from .shared_funcs import _run_pmf
+    _need_cuda(q, "q")
+    _require_cuda(q, "q")                                          # float32 posteriors, on the call's device
+    _need_cuda(tx, "tx")
+    if tx.dtype != torch.float16:
+        raise _lib.VaeqError(f"tx must be float16, got {tx.dtype}")
+    if q.dim() != 3 or tx.dim() != 3 or tx.shape[0] != q.shape[0] or tx.shape[1] != 2 or tx.shape[-1] != q.shape[-1] or q.stride(2) != 1 or tx.stride(2) != 1:
+        raise _lib.VaeqError(f"need q (R,2n,N) and tx (R,2,N) with unit time stride, got {tuple(q.shape)} {tuple(tx.shape)}")
+    lib = _lib.load()
+    R, N, n = int(q.shape[0]), int(q.shape[-1]), int(q.shape[1]) // 2
+    dev = q.device
+    for t, name, shape in ((shift, "shift", (R,)), (counts, "counts", (R, 4))):
+        if not torch.is_tensor(t) or t.dtype != torch.int32 or tuple(t.shape) != shape or not t.is_contiguous() or t.device != dev:
+            raise _lib.VaeqError(f"{name}: need a contiguous int32 {shape} tensor on {dev} (awgn_eval_runs)")
+    Pt, rs_P = _run_pmf(P, R, n, dev)
+    gmi = torch.empty(R, dtype=_F32, device=dev)
+    scr = torch.empty(max(1, int(lib.vaeq_awgn_gmi_scratch_bytes(R, N))), dtype=torch.uint8, device=dev)
+    _lib.check(lib.vaeq_awgn_gmi_runs(q.data_ptr(), int(q.stride(1)), int(q.stride(0)), tx.data_ptr(), int(tx.stride(1)), int(tx.stride(0)),
+                                      Pt.data_ptr(), rs_P, shift.data_ptr(), counts.data_ptr(), n, N, R, int(edge), gmi.data_ptr(), scr.data_ptr(),
+                                      _lib.current_stream()), "vaeq_awgn_gmi_runs")
+    return gmi
+
+
 _TAPS_CACHE: dict = {}
 
 

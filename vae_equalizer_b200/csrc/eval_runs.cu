@@ -405,9 +405,177 @@ __global__ void k_aw_ser_min(AwgnEvalK p) {
     p.ser[run] = __fmul_rn((float)m, __fdiv_rn(1.f, (float)n_eval));
 }
 
+// ---- GMI of the SER's region under the SER's hypothesis (extension, not in the reference) -----------------------------------------
+// GMI = H(X) + mean over the evaluated symbols of log2 q(x_tx | y) per polarisation, bit per 2-D symbol, on exactly the symbols the
+// soft-demapper SER counts and with the (IQ flip, rotation) whose error count is smallest, so it is invariant under the symmetries the
+// SER forgives.  Symbols are split into fixed chunks of GMI_CHUNK: the partial sums of a run depend on its own n_eval only, never on
+// the number of runs of the call, so a run's GMI is bit-identical alone or in any batch.
+constexpr int GMI_CHUNK = 2048;
+
+struct GmiRunsK {
+    const float *q; int64_t ld_q, rs_q;          // DP (R,2,2n,N), AWGN (R,2n,N)
+    const uint16_t *tx; int64_t ld_tx, rs_tx;    // DP (R,2,2,N), AWGN (R,2,N) float16 bits
+    const float *P; int64_t rs_P;                // (R,n) pmf of each run
+    const int *align;                            // DP: (R,2,4) of vaeq_frame_eval_runs_ex (estimator 0 row); AWGN: shift (R)
+    const int *counts;                           // DP: (R,2,2,2,4) [est][flip][pol][rotation]; AWGN: (R,4) [rotation]
+    int N, seg_len, edge, n_cut, n_runs, max_chunks;
+    double *part;                                // [R][max_chunks][2]
+    float *gmi;                                  // DP (R,2), AWGN (R)
+};
+
+// the hypothesis h = flip * 4 + rotation with the smallest error count, in counter order (flip 0 rotations 0..3, then flip 1);
+// the first wins ties.  cnt = the pol's rotation 0 counter, the flip-1 counters flip_stride further
+__device__ __forceinline__ int gmi_hypothesis(const int *cnt, int n_flip, int flip_stride) {
+    int best = cnt[0], h = 0;
+    for (int f = 0; f < n_flip; ++f)
+        for (int k = 0; k < 4; ++k) {
+            const int c = cnt[f * flip_stride + k];
+            if (c < best) {
+                best = c;
+                h = f * 4 + k;
+            }
+        }
+    return h;
+}
+
+// evaluated-region geometry of one run: shifts, polarisation swap and symbol count (DP: estimator 0 of the frame evaluation;
+// AWGN: q[:, edge + shift : N - edge] against tx[:, edge : N - edge - shift], as k_aw_ser)
+template <int NPOL>
+__device__ __forceinline__ void gmi_geometry(const GmiRunsK &p, int run, int (&sh)[2], int &r, int &n_eval, int &keep) {
+    if (NPOL == 2) {
+        const int *al = p.align + (int64_t)run * 8;
+        sh[0] = al[0]; sh[1] = al[1]; r = al[2]; n_eval = al[3];
+        keep = p.seg_len ? min(p.seg_len, p.seg_len - sh[0] - p.n_cut) : 0;
+    } else {
+        sh[0] = sh[1] = p.align[run];
+        r = 0; keep = 0;
+        // q starts at edge + shift: a shift below -edge (impossible for shifts of awgn_eval_runs with edge >= n_shift / 2) scores
+        // nothing rather than reading before the row.  Otherwise n_eval <= N - edge, inside the chunks the grid covers.
+        n_eval = p.edge + sh[0] < 0 ? 0 : p.N - 2 * p.edge - sh[0];
+    }
+}
+
+// grid (max_chunks, R): CTA c sums log2 q of the chosen hypothesis over evaluated symbols [c GMI_CHUNK, (c + 1) GMI_CHUNK) per pol.
+// NPOL = 2: the DP drivers (pol swap, circular shift, minibatch cut); NPOL = 1: the AWGN driver (one pol, no flip, no wrap)
+template <int NL, int NPOL>
+__global__ void __launch_bounds__(ER_NT) k_gmi_runs(GmiRunsK p) {
+    __shared__ double red[2 * 32];
+    const int run = blockIdx.y, N = p.N;
+    int sh[2], r, n_eval, keep;
+    gmi_geometry<NPOL>(p, run, sh, r, n_eval, keep);
+    const int f0 = blockIdx.x * GMI_CHUNK, f1 = min(n_eval, f0 + GMI_CHUNK);
+    if (f0 >= f1) return;                                    // beyond this run's symbols: the finish reads no partial of this CTA
+    int hyp[2];
+#pragma unroll
+    for (int pol = 0; pol < NPOL; ++pol)
+        hyp[pol] = NPOL == 2 ? gmi_hypothesis(p.counts + (int64_t)run * 32 + pol * 4, 2, 8) : gmi_hypothesis(p.counts + (int64_t)run * 4, 1, 0);
+    const float *q = p.q + run * p.rs_q;
+    const uint16_t *tx = p.tx + run * p.rs_tx;
+    const float scale = (float)((NL - 1) / 2.0);
+    constexpr int S = NL - 1;
+    double acc[2] = {0.0, 0.0};
+    for (int f = f0 + threadIdx.x; f < f1; f += ER_NT) {
+        const int t = er_map(f, p.edge, p.seg_len, keep);
+#pragma unroll
+        for (int pol = 0; pol < NPOL; ++pol) {
+            const int sp = (pol - r) & 1, ts = NPOL == 2 ? er_wrap(t + sh[pol], N) : t + sh[0];
+            const int DI = min(max((int)er_tx_level(tx[(int64_t)(pol * 2) * p.ld_tx + t], scale), 0), S);
+            const int DQ = min(max((int)er_tx_level(tx[(int64_t)(pol * 2 + 1) * p.ld_tx + t], scale), 0), S);
+            const int k = hyp[pol] & 3, DQp = (hyp[pol] >> 2) ? S - DQ : DQ;     // IQ-flipped reference data (sf:199)
+            // inverse of er_count_q's hI / hQ: the q levels that rotation k maps onto the tx levels
+            const int iI = k == 0 ? DI : k == 1 ? S - DI : k == 2 ? DQp : S - DQp;
+            const int iQ = k == 0 ? DQp : k == 1 ? S - DQp : k == 2 ? S - DI : DI;
+            const float *qp = q + (int64_t)(sp * 2 * NL) * p.ld_q + ts;
+            const float qI = qp[(int64_t)iI * p.ld_q], qQ = qp[(int64_t)(NL + iQ) * p.ld_q];
+            acc[pol] += log2((double)fmaxf(qI, 1e-30f)) + log2((double)fmaxf(qQ, 1e-30f));
+        }
+    }
+    block_sum<2>(acc, red);
+    if (threadIdx.x == 0) {
+        double *dst = p.part + ((int64_t)run * p.max_chunks + blockIdx.x) * 2;
+        dst[0] = acc[0];
+        dst[1] = acc[1];
+    }
+}
+
+// thread = (run, pol): the run's chunk partials in chunk order, plus H(X) = -2 sum_l P_l log2 P_l of the run's pmf (as k_gmi_fin)
+template <int NPOL>
+__global__ void k_gmi_runs_fin(GmiRunsK p, int n_lev) {
+    const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= NPOL * p.n_runs) return;
+    const int run = idx / NPOL, pol = idx % NPOL;
+    int sh[2], r, n_eval, keep;
+    gmi_geometry<NPOL>(p, run, sh, r, n_eval, keep);
+    const int nch = min(p.max_chunks, (max(n_eval, 0) + GMI_CHUNK - 1) / GMI_CHUNK);
+    const double *part = p.part + (int64_t)run * p.max_chunks * 2 + pol;
+    double s = 0.0;
+    for (int c = 0; c < nch; ++c) s += part[2 * c];
+    const float *P = p.P + run * p.rs_P;
+    double H = 0.0;
+    for (int l = 0; l < n_lev; ++l) H -= 2.0 * (double)P[l] * log2((double)P[l]);
+    p.gmi[idx] = n_eval > 0 ? (float)(H + s / (double)n_eval) : __int_as_float(0x7fc00000);
+}
+
+static int gmi_runs_launch(GmiRunsK &p, int n_lev, int npol, cudaStream_t st) {
+    const dim3 grid(p.max_chunks, p.n_runs);
+    ktime_begin(VAEQ_K_EVAL, st);
+#define GMI_CASE(NL_)                                                                                  \
+    if (npol == 2) k_gmi_runs<NL_, 2><<<grid, ER_NT, 0, st>>>(p);                                      \
+    else k_gmi_runs<NL_, 1><<<grid, ER_NT, 0, st>>>(p);
+    if (n_lev == 2) { GMI_CASE(2) } else if (n_lev == 4) { GMI_CASE(4) } else { GMI_CASE(8) }
+#undef GMI_CASE
+    ktime_end(VAEQ_K_EVAL, st);
+    VAEQ_LAUNCH_CHECK("k_gmi_runs");
+    const int n = npol * p.n_runs;
+    ktime_begin(VAEQ_K_EVAL, st);
+    if (npol == 2) k_gmi_runs_fin<2><<<(n + 127) / 128, 128, 0, st>>>(p, n_lev);
+    else k_gmi_runs_fin<1><<<(n + 127) / 128, 128, 0, st>>>(p, n_lev);
+    ktime_end(VAEQ_K_EVAL, st);
+    VAEQ_LAUNCH_CHECK("k_gmi_runs_fin");
+    return VAEQ_OK;
+}
+
+static int gmi_max_chunks(int N) { return (N + GMI_CHUNK - 1) / GMI_CHUNK; }
+
 }  // namespace vaeq
 
 using namespace vaeq;
+
+extern "C" size_t vaeq_frame_gmi_scratch_bytes(int32_t n_runs, int32_t N) {
+    if (n_runs <= 0 || N <= 0) return 0;
+    return (size_t)n_runs * gmi_max_chunks(N) * 2 * sizeof(double);
+}
+
+extern "C" size_t vaeq_awgn_gmi_scratch_bytes(int32_t n_runs, int32_t N) { return vaeq_frame_gmi_scratch_bytes(n_runs, N); }
+
+extern "C" int vaeq_frame_gmi_runs(const float *q, int64_t ld_q, int64_t rs_q, const uint16_t *tx, int64_t ld_tx, int64_t rs_tx, const float *P,
+                                   int64_t rs_P, const int32_t *align, const int32_t *counts, int32_t n_lev, int32_t N, int32_t n_runs,
+                                   int32_t seg_len, int32_t edge, int32_t n_cut, float *gmi_out, void *scratch, void *stream) {
+    VAEQ_CHECK_ARG(q && tx && P && align && counts && gmi_out && scratch, "NULL pointer");
+    VAEQ_CHECK_ARG(n_lev == 2 || n_lev == 4 || n_lev == 8, "n_lev=%d must be 2, 4 or 8", n_lev);
+    VAEQ_CHECK_ARG(N > 0 && edge >= 0 && n_cut >= 0, "bad sizes (N=%d, edge=%d, n_cut=%d)", N, edge, n_cut);
+    VAEQ_CHECK_ARG(seg_len == 0 || (seg_len > 0 && N % seg_len == 0), "N=%d must be a multiple of seg_len=%d", N, seg_len);
+    VAEQ_CHECK_ARG(n_runs > 0 && n_runs <= 65535, "n_runs=%d must be in 1..65535", n_runs);
+    GmiRunsK p;
+    p.q = q; p.ld_q = ld_q; p.rs_q = rs_q; p.tx = tx; p.ld_tx = ld_tx; p.rs_tx = rs_tx; p.P = P; p.rs_P = rs_P;
+    p.align = align; p.counts = counts; p.N = N; p.seg_len = seg_len; p.edge = edge; p.n_cut = n_cut; p.n_runs = n_runs;
+    p.max_chunks = gmi_max_chunks(N); p.part = static_cast<double *>(scratch); p.gmi = gmi_out;
+    return gmi_runs_launch(p, n_lev, 2, (cudaStream_t)stream);
+}
+
+extern "C" int vaeq_awgn_gmi_runs(const float *q, int64_t ld_q, int64_t rs_q, const uint16_t *tx, int64_t ld_tx, int64_t rs_tx, const float *P,
+                                  int64_t rs_P, const int32_t *shift, const int32_t *counts, int32_t n_lev, int32_t N, int32_t n_runs, int32_t edge,
+                                  float *gmi_out, void *scratch, void *stream) {
+    VAEQ_CHECK_ARG(q && tx && P && shift && counts && gmi_out && scratch, "NULL pointer");
+    VAEQ_CHECK_ARG(n_lev == 2 || n_lev == 4 || n_lev == 8, "n_lev=%d must be 2, 4 or 8", n_lev);
+    VAEQ_CHECK_ARG(N > 0 && edge >= 0 && N - 2 * edge > 0, "N=%d leaves no symbol to evaluate with edge=%d", N, edge);
+    VAEQ_CHECK_ARG(n_runs > 0 && n_runs <= 65535, "n_runs=%d must be in 1..65535", n_runs);
+    GmiRunsK p;
+    p.q = q; p.ld_q = ld_q; p.rs_q = rs_q; p.tx = tx; p.ld_tx = ld_tx; p.rs_tx = rs_tx; p.P = P; p.rs_P = rs_P;
+    p.align = shift; p.counts = counts; p.N = N; p.seg_len = 0; p.edge = edge; p.n_cut = 0; p.n_runs = n_runs;
+    p.max_chunks = gmi_max_chunks(N); p.part = static_cast<double *>(scratch); p.gmi = gmi_out;
+    return gmi_runs_launch(p, n_lev, 1, (cudaStream_t)stream);
+}
 
 extern "C" size_t vaeq_awgn_eval_scratch_bytes(int32_t n_runs, int32_t n_shift, int32_t n_corr) {
     if (n_runs <= 0 || n_shift <= 0 || n_corr <= 0) return 0;

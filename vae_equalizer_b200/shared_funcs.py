@@ -346,6 +346,44 @@ def frame_eval_runs(out_train, out_const, tx, amp_levels, var, nu_sc, seg_len, n
     return (ser, align, counts) if return_counts else (ser, align)
 
 
+def _run_pmf(P, R, n, dev):
+    """(R, n) float32 pmf rows on `dev` (one shared row is repeated) and the run stride the C ABI takes."""
+    Pt = torch.as_tensor(P, dtype=_F32, device=dev)
+    if Pt.dim() == 1:
+        Pt = Pt.unsqueeze(0).expand(R, n)
+    if tuple(Pt.shape) != (R, n):
+        raise _lib.VaeqError(f"P: need (R={R}, n={n}) or (n,), got {tuple(Pt.shape)}")
+    Pt = Pt.contiguous()
+    return Pt, int(Pt.stride(0))
+
+
+@_lib.device_guard
+def gmi_runs(q, tx, P, align, counts, seg_len, edge=11, n_cut=10):
+    """EXTENSION (not in the reference): GMI = H(X) + mean log2 q(x_tx|y) per pol (bit/2D-symbol) of R runs, scored on exactly the symbols
+    and under the (IQ flip, rotation) hypothesis of the soft-demapper SER of frame_eval_runs: q (R,2,2n,N) and tx (R,2,2,N) float16 as
+    given to frame_eval_runs, P (R,n) or (n,) pmf, align (R,2,4) and counts (R,2,2,2,4) from frame_eval_runs(..., return_counts=True)
+    with the same seg_len / edge / n_cut.  Returns (R,2) float32 on the device, NaN where no symbol was evaluated; no host sync."""
+    _require_cuda(q, "q")
+    tx = _tx_bits(tx)
+    lib = _lib.load()
+    R, N, n = int(q.shape[0]), int(q.shape[-1]), int(q.shape[2]) // 2 if q.dim() == 4 else 0
+    dev = q.device
+    for t, name, rows in ((q, "q", 2 * n), (tx, "tx", 2)):
+        if t.dim() != 4 or t.shape[0] != R or t.shape[1] != 2 or t.shape[2] != rows or t.shape[-1] != N or t.stride(3) != 1 \
+                or t.stride(1) != t.shape[2] * t.stride(2):
+            raise _lib.VaeqError(f"{name}: need (R,2,rows,N) with unit time stride and evenly strided rows, got {tuple(t.shape)} {t.stride()}")
+    for t, name, shape in ((align, "align", (R, 2, 4)), (counts, "counts", (R, 2, 2, 2, 4))):
+        if not torch.is_tensor(t) or t.dtype != torch.int32 or tuple(t.shape) != shape or not t.is_contiguous() or t.device != dev:
+            raise _lib.VaeqError(f"{name}: need a contiguous int32 {shape} tensor on {dev} (frame_eval_runs(..., return_counts=True))")
+    Pt, rs_P = _run_pmf(P, R, n, dev)
+    gmi = torch.empty(R, 2, dtype=_F32, device=dev)
+    scr = _scratch(dev, max(1, int(lib.vaeq_frame_gmi_scratch_bytes(R, N))))
+    _lib.check(lib.vaeq_frame_gmi_runs(q.data_ptr(), int(q.stride(2)), int(q.stride(0)), tx.data_ptr(), int(tx.stride(2)), int(tx.stride(0)),
+                                       Pt.data_ptr(), rs_P, align.data_ptr(), counts.data_ptr(), n, N, R, int(seg_len), int(edge), int(n_cut),
+                                       gmi.data_ptr(), scr.data_ptr(), _lib.current_stream()), "vaeq_frame_gmi_runs")
+    return gmi
+
+
 @_lib.device_guard
 def soft_dec_runs(out, var, amp_levels, nu_sc):
     """soft_dec (sf:529-542) for R independent runs in one launch: out (R,2,2,N), var (R,2), nu_sc (R,) -> q (R,2,2n,N)."""

@@ -32,7 +32,7 @@ def _cell(c, key):
 
 def sweep_vae_dp(cells, mod, sps, M_est, batch_len, N_frame_max, num_frames, flex_step=None, channel="h0", symb_rate=90e9,
                  tau_cd=-26e-24, tau_pmd=0.1e-12 * np.sqrt(1000), phiIQ=(0.0314, 0.0314), N_lrhalf=None, *, kind="VAE",
-                 device=None, datagen="gpu", eval_every=1, eval_mode="batched", verbose=False):
+                 device=None, datagen="gpu", eval_every=1, eval_mode="batched", verbose=False, gmi=False):
     """Train and score R = len(cells) independent runs in lockstep.
 
     cells: list of dicts with per-cell values: SNR, nu, lr_optim, theta, theta_diff, and optionally seed.
@@ -43,7 +43,10 @@ def sweep_vae_dp(cells, mod, sps, M_est, batch_len, N_frame_max, num_frames, fle
     drivers' own sequence of calls per cell: find_shift -> roll -> cut -> SER; the two agree to the last error count).
     kind: "VAE" (func_VAELE_DP_MQAM_shaping.py: non-overlapping minibatches) or "VAEflex" (func_VAEflex_DP_MQAM_shaping.py:
     window batch_len advanced by flex_step).  eval_every: score every k-th frame (and the last); unscored frames hold NaN.
-    Returns (SER_valid (R,4,num_frames), Var_est (R,2,num_frames), var (R,2))."""
+    gmi: also score GMI (shared_funcs.gmi_runs: the soft-demapper SER's symbols and hypothesis; eval_mode="batched" only).
+    Returns (SER_valid (R,4,num_frames), Var_est (R,2,num_frames), var (R,2)), and GMI (R,2,num_frames) as a 4th tensor with gmi=True
+    (NaN on unscored frames)."""
+    _gmi_batched_only(gmi, eval_mode)
     device = _cuda_device(device)
     R = len(cells)
     if R == 0:
@@ -88,6 +91,8 @@ def sweep_vae_dp(cells, mod, sps, M_est, batch_len, N_frame_max, num_frames, fle
 
     SER_valid = torch.full((R, 4, num_frames), float("nan"), device=device, dtype=torch.float32)
     Var_est = torch.empty(R, pol, num_frames, device=device, dtype=torch.float32)
+    GMI = torch.full((R, pol, num_frames), float("nan"), device=device, dtype=torch.float32) if gmi else None
+    P_gmi = P_all.to(device) if gmi else None
     rx_all = None if datagen == "gpu_batched" else torch.empty(R, 2, 2, sps * N_frame, device=device, dtype=torch.float32)
     out_train = torch.empty(R, pol, 2 * num_lev, N_keep, device=device, dtype=torch.float32)
     out_const = torch.empty(R, pol, 2, N_keep, device=device, dtype=torch.float32)
@@ -127,9 +132,12 @@ def sweep_vae_dp(cells, mod, sps, M_est, batch_len, N_frame_max, num_frames, fle
                 tx_b4 = tx_b if kind == "VAE" else tx_b[:, :, :, batch_len // 2:m_max + batch_len // 2]
             else:
                 tx_b4 = torch.stack(tx_all)
-            ser, _ = sfun.frame_eval_runs(out_train, out_const, tx_b4, amp_dev, var_dev, nu_dev, batch_len if kind == "VAE" else 0,
-                                          n_cut=N_CUT)
+            seg_len = batch_len if kind == "VAE" else 0
+            ser, al, counts = sfun.frame_eval_runs(out_train, out_const, tx_b4, amp_dev, var_dev, nu_dev, seg_len, n_cut=N_CUT,
+                                                   return_counts=True)
             SER_valid[:, :, frame] = ser
+            if gmi:
+                GMI[:, :, frame] = sfun.gmi_runs(out_train, tx_b4, P_gmi, al, counts, seg_len, n_cut=N_CUT)
             if verbose:
                 print(frame, "loss", loss_steps[:, -1].tolist(), "SER", SER_valid[:, :, frame].tolist())
             continue
@@ -147,12 +155,20 @@ def sweep_vae_dp(cells, mod, sps, M_est, batch_len, N_frame_max, num_frames, fle
         if verbose:
             snr_db = 10 * torch.log10(torch.tensor(pow_mean, device=device) / var_steps.mean(dim=(1, 2)))
             print(frame, "loss", loss_steps[:, -1].tolist(), "SNR_est", snr_db.tolist(), "SER", SER_valid[:, :, frame].tolist())
+    if gmi:
+        return SER_valid, Var_est, var_all.to(device), GMI
     return SER_valid, Var_est, var_all.to(device)
+
+
+def _gmi_batched_only(gmi, eval_mode):
+    if gmi and eval_mode != "batched":
+        raise ValueError(f"gmi=True needs eval_mode='batched' (GMI is scored from the batched evaluation's alignment and counts), got "
+                         f"{eval_mode!r}")
 
 
 def sweep_cma_dp(cells, mod, sps, M_est, batch_len, N_train_max, num_frames, flex_step=None, channel="h0", symb_rate=90e9,
                  tau_cd=-26e-24, tau_pmd=0.1e-12 * np.sqrt(1000), phiIQ=(0.0314, 0.0314), N_lrhalf=None, *, kind="CMA", device=None,
-                 datagen="gpu", eval_mode="batched", verbose=False):
+                 datagen="gpu", eval_mode="batched", verbose=False, gmi=False):
     """The CMA / CMAbatch / CMAflex drivers (func_CMA_DP_MQAM_shaping.py:16-56 and siblings) for R = len(cells) independent cells
     in lockstep.  The tap recurrence of a cell is sequential in the symbols, but cells are independent: per frame ONE equalizer
     launch sequence covers all cells that share lr_optim (vaeq_cma n_runs: one warp / one CTA per cell) and ONE batched CPE
@@ -160,8 +176,10 @@ def sweep_cma_dp(cells, mod, sps, M_est, batch_len, N_train_max, num_frames, fle
     aligned, partially rescaled copy -> soft_dec -> estimator from q, 4 calls and no host sync for all cells) or replays the single-run
     drivers' call sequence per cell (eval_mode="per_cell", two host syncs per frame); both give the same error counts.  A cell gives the same SER alone (processing_cma*_dp) or in any batch when
     datagen="gpu" (its data depends on its own seed only); datagen="gpu_batched" generates all cells in one call (fastest).
-    Returns (SER_valid (R,4,num_frames), Var_est zeros (R,2,num_frames), var (R,2))."""
+    gmi: also score GMI of the soft-demapper posteriors q the SER is taken from (shared_funcs.gmi_runs; eval_mode="batched" only).
+    Returns (SER_valid (R,4,num_frames), Var_est zeros (R,2,num_frames), var (R,2)), and GMI (R,2,num_frames) as a 4th tensor with gmi=True."""
     from .processing import _make_frame
+    _gmi_batched_only(gmi, eval_mode)
     device = _cuda_device(device)
     R = len(cells)
     if R == 0:
@@ -189,6 +207,8 @@ def sweep_cma_dp(cells, mod, sps, M_est, batch_len, N_train_max, num_frames, fle
     Var_est = torch.zeros(R, pol, num_frames, device=device, dtype=torch.float32)
     var_all = torch.stack([k[7].to(device, torch.float32) for k in consts])
     nu_all = torch.tensor([float(k[6]) for k in consts], dtype=torch.float32, device=device)
+    GMI = torch.full((R, pol, num_frames), float("nan"), device=device, dtype=torch.float32) if gmi else None
+    P_gmi = torch.stack([torch.as_tensor(k[2], dtype=torch.float32) for k in consts]).to(device) if gmi else None
     lr_scale = 1.0
     for frame in range(num_frames):
         if frame % N_lrhalf == 0 and frame != 0:
@@ -227,9 +247,11 @@ def sweep_cma_dp(cells, mod, sps, M_est, batch_len, N_train_max, num_frames, fle
             ser_c, al, g = sfun.frame_eval_runs(None, out_c, tx_c, amp_levels, var_all, nu_all, 0, which=2, return_scale=True)
             # CMA_DP:44-48: soft_dec sees the aligned copy with the evaluated slice rescaled in place
             q_all = sfun.soft_dec_runs(sfun.cma_align_rescale(out_c, al, g), var_all, amp_levels, nu_all)
-            ser_q, _ = sfun.frame_eval_runs(q_all, None, tx_c, amp_levels, var_all, nu_all, 0, which=1)      # CMA_DP:49-52
+            ser_q, al_q, counts_q = sfun.frame_eval_runs(q_all, None, tx_c, amp_levels, var_all, nu_all, 0, which=1, return_counts=True)  # CMA_DP:49-52
             SER_valid[:, :2, frame] = ser_c[:, :2]
             SER_valid[:, 2:, frame] = ser_q[:, 2:]
+            if gmi:
+                GMI[:, :, frame] = sfun.gmi_runs(q_all, tx_c, P_gmi, al_q, counts_q, 0)
             if verbose:
                 print(frame, "SER", SER_valid[:, :, frame].tolist())
             continue
@@ -254,6 +276,8 @@ def sweep_cma_dp(cells, mod, sps, M_est, batch_len, N_train_max, num_frames, fle
             SER_valid[r, 2:, frame] = sfun.SER_IQflip(qa[:, :, 11:-tail], tx_c[r][:, :, 11:-tail])
         if verbose:
             print(frame, "SER", SER_valid[:, :, frame].tolist())
+    if gmi:
+        return SER_valid, Var_est, var_all, GMI
     return SER_valid, Var_est, var_all
 
 
@@ -275,13 +299,15 @@ def _score(kind, what, aligned, tx, sh, batch_len, m_max, pol, num_lev, amp_leve
 
 def sweep_vae_dp_sharded(cells, *args, rank=0, world=1, group=None, **kw):
     """Round-robin the cells over the ranks (one process per GPU), run each share as one batched run set, and reassemble
-    (SER_valid, Var_est, var) for ALL cells on rank 0 (None elsewhere).  No data-path collective."""
+    (SER_valid, Var_est, var) -- plus GMI with gmi=True -- for ALL cells on rank 0 (None elsewhere).  No data-path collective."""
     from .parallel import gather_cell_results, shard_cells
     mine = shard_cells(cells, rank, world)
     num_frames = args[5] if len(args) > 5 else kw["num_frames"]
     dev = _cuda_device(kw.get("device"))
+    gmi = kw.get("gmi", False)
     if mine:
-        ser, ve, var = sweep_vae_dp([c for _, c in mine], *args, **kw)
+        res = sweep_vae_dp([c for _, c in mine], *args, **kw)
+        ser, ve, var = res[:3]
     loc_ser = {i: ser[k] for k, (i, _) in enumerate(mine)} if mine else {}
     loc_ve = {i: ve[k] for k, (i, _) in enumerate(mine)} if mine else {}
     loc_var = {i: var[k] for k, (i, _) in enumerate(mine)} if mine else {}
@@ -290,10 +316,26 @@ def sweep_vae_dp_sharded(cells, *args, rank=0, world=1, group=None, **kw):
     ser_g = gather_cell_results({i: torch.nan_to_num(t, nan=-1.0) for i, t in loc_ser.items()}, n, (4, num_frames), rank, world, group, dev)
     ve_g = gather_cell_results(loc_ve, n, (2, num_frames), rank, world, group, dev)
     var_g = gather_cell_results(loc_var, n, (2,), rank, world, group, dev)
+    if gmi:                                                          # a collective: every rank takes part, before any rank returns
+        loc_g = {i: res[3][k] for k, (i, _) in enumerate(mine)} if mine else {}
+        gmi_g = _gather_with_nan(loc_g, n, (2, num_frames), rank, world, group, dev)
     if rank != 0:
         return None
     ser_g = torch.where(ser_g < 0, torch.full_like(ser_g, float("nan")), ser_g)
+    if gmi:
+        return ser_g, ve_g, var_g, gmi_g
     return ser_g, ve_g, var_g
+
+
+def _gather_with_nan(local, n_cells, shape, rank, world, group, dev):
+    """parallel.gather_cell_results for values of any sign with NaN entries (GMI can be negative, so NaN cannot be carried as a negative
+    sentinel): the values with NaN as 0 and a NaN mask travel in one block.  (n_cells, *shape) on rank 0, None elsewhere."""
+    from .parallel import gather_cell_results
+    packed = {i: torch.stack((torch.where(torch.isnan(t), torch.zeros_like(t), t), torch.isnan(t).to(t.dtype))) for i, t in local.items()}
+    g = gather_cell_results(packed, n_cells, (2,) + tuple(shape), rank, world, group, dev)
+    if g is None:
+        return None
+    return torch.where(g[:, 1] > 0, torch.full_like(g[:, 0], float("nan")), g[:, 0])
 
 
 # -------------------------------------------------------------------------------------------------
@@ -306,7 +348,7 @@ def run_dp_sweep(mod="64-QAM", sps=2, loss_type="VAE", channel="h0", nu_vec=(0,)
                  theta_diff_vec=(0.06 * np.pi,), SNR_vec=(23,), M_vec=(25,), batch_len_vec=(100,), flex_step_vec=(10,),
                  lr_optim_vec=(2.5e-3, 2e-3, 3e-3), iter=5, N_lrhalf=170, num_frames=170, N_frame_max=10000,
                  tau_pmd=0.1e-12 * np.sqrt(1000), tau_cd=-26e-24, phiIQ=(0.0314, 0.0314), *, device=None, datagen="gpu_batched",
-                 eval_every=1, rank=0, world=1, group=None, runner=None, verbose=False, checkpoint_dir=None):
+                 eval_every=1, rank=0, world=1, group=None, runner=None, verbose=False, checkpoint_dir=None, gmi=False):
     """Eval_run_DP.py's ten nested loops (RUN_DP:68-95) as batched run sets.  Cells that share (M, batch_len, flex_step, symb_rate)
     train in the same persistent launch; with world > 1 every rank takes a round-robin share of each set.  Returns the
     reference's result arrays on rank 0 (None elsewhere):
@@ -314,7 +356,9 @@ def run_dp_sweep(mod="64-QAM", sps=2, loss_type="VAE", channel="h0", nu_vec=(0,)
     loss_type 'VAE' / 'VAEflex' use the batched VAE engine (sweep_vae_dp), the CMA variants the batched CMA engine (sweep_cma_dp: a cell's tap
     recurrence is sequential in the symbols, the cells of a set run side by side).
     checkpoint_dir: rank 0 writes each finished run set there (one .npz per set, keyed by the set's parameters); a restarted sweep
-    loads what it finds instead of recomputing (the reference only saves once, at the very end: RUN_DP:99-114)."""
+    loads what it finds instead of recomputing (the reference only saves once, at the very end: RUN_DP:99-114).
+    gmi=True: also GMI (2, SNR, ..., iter, num_frames), shaped like Var_est, as a 4th result (sweep_vae_dp / sweep_cma_dp with gmi=True;
+    the runner hook is then called with gmi=True).  Its checkpoints hold the GMI and are never mixed up with those of gmi=False."""
     vecs = dict(SNR=list(SNR_vec), symb_rate=list(symb_rate_vec), nu=list(nu_vec), theta_diff=list(theta_diff_vec), M=list(M_vec),
                 lr_optim=list(lr_optim_vec), batch_len=list(batch_len_vec), flex_step=list(flex_step_vec), theta=list(theta_vec))
     shape = tuple(len(vecs[a]) for a in AXES) + (iter,)
@@ -322,6 +366,8 @@ def run_dp_sweep(mod="64-QAM", sps=2, loss_type="VAE", channel="h0", nu_vec=(0,)
     SER = torch.full((4,) + shape + (num_frames,), float("nan"), dtype=torch.float32, device=dev)
     Var_est = torch.zeros((2,) + shape + (num_frames,), dtype=torch.float32, device=dev)
     var_real = torch.zeros((2,) + shape + (1,), dtype=torch.float32, device=dev)
+    GMI = torch.full((2,) + shape + (num_frames,), float("nan"), dtype=torch.float32, device=dev) if gmi else None
+    gkw = dict(gmi=True) if gmi else {}                              # gmi=False: every call, name and signature exactly as without GMI
     groups = {}
     for idx in np.ndindex(*shape):
         c = {a: vecs[a][i] for a, i in zip(AXES, idx[:-1])}
@@ -338,39 +384,46 @@ def run_dp_sweep(mod="64-QAM", sps=2, loss_type="VAE", channel="h0", nu_vec=(0,)
             sig = _set_signature(loss_type=loss_type, mod=mod, sps=sps, channel=channel, M=M, batch_len=batch_len, flex_step=flex_step,
                                  symb_rate=symb_rate, N_frame_max=N_frame_max, num_frames=num_frames, N_lrhalf=N_lrhalf, tau_cd=tau_cd,
                                  tau_pmd=tau_pmd, phiIQ=list(phiIQ), datagen=datagen, eval_every=eval_every,
-                                 cells=[sorted(c.items()) for c in cells])
+                                 cells=[sorted(c.items()) for c in cells], **gkw)
             ck = os.path.join(checkpoint_dir, f"{loss_type}_{mod}_M{M}_B{batch_len}_F{flex_step}_R{symb_rate:g}_n{len(cells)}_f{num_frames}"
                                               f"_{sig[:12]}.npz")
             have = 0
             if rank == 0 and os.path.exists(ck):
                 z = np.load(ck)
-                if "signature" in z.files and str(z["signature"]) == sig:
+                if "signature" in z.files and str(z["signature"]) == sig and (not gmi or "gmi" in z.files):
                     have = 1
                     for k, (idx, _) in enumerate(members):
                         SER[(slice(None),) + idx] = torch.from_numpy(z["ser"][k]).to(dev)
                         Var_est[(slice(None),) + idx] = torch.from_numpy(z["ve"][k]).to(dev)
                         var_real[(slice(None),) + idx + (0,)] = torch.from_numpy(z["var"][k]).to(dev)
+                        if gmi:
+                            GMI[(slice(None),) + idx] = torch.from_numpy(z["gmi"][k]).to(dev)
             if _bcast_flag(have, rank, world, group, dev):           # rank 0 decides (the directory need not be shared); all ranks follow
                 continue
         kw = dict(flex_step=flex_step, channel=channel, symb_rate=symb_rate, tau_cd=tau_cd, tau_pmd=tau_pmd, phiIQ=phiIQ, N_lrhalf=N_lrhalf)
         if runner is not None:                                       # test hook: stands for sweep_vae_dp_sharded
-            res = runner(cells, *common, **kw)
+            res = runner(cells, *common, **kw, **gkw)
         elif loss_type in ("VAE", "VAEflex"):
             res = sweep_vae_dp_sharded(cells, *common, kind=loss_type, device=dev, datagen=datagen, eval_every=eval_every,
-                                       verbose=verbose, rank=rank, world=world, group=group, **kw)
+                                       verbose=verbose, rank=rank, world=world, group=group, **kw, **gkw)
         else:
-            res = _cma_cells(loss_type, cells, common, kw, dev, rank, world, group, num_frames, datagen=datagen)
+            res = _cma_cells(loss_type, cells, common, kw, dev, rank, world, group, num_frames, datagen=datagen, gmi=gmi)
         if res is None:
             continue
-        ser, ve, var = res
+        ser, ve, var = res[:3]
         if ck is not None and rank == 0:
-            np.savez(ck, ser=ser.cpu().numpy(), ve=ve.cpu().numpy(), var=var.cpu().numpy(), signature=np.array(sig))
+            extra = dict(gmi=res[3].cpu().numpy()) if gmi else {}
+            np.savez(ck, ser=ser.cpu().numpy(), ve=ve.cpu().numpy(), var=var.cpu().numpy(), signature=np.array(sig), **extra)
         for k, (idx, _) in enumerate(members):
             SER[(slice(None),) + idx] = ser[k].to(dev)
             Var_est[(slice(None),) + idx] = ve[k].to(dev)
             var_real[(slice(None),) + idx + (0,)] = var[k].to(dev)
+            if gmi:
+                GMI[(slice(None),) + idx] = res[3][k].to(dev)
     if rank != 0:
         return None
+    if gmi:
+        return SER, Var_est, var_real, GMI
     return SER, Var_est, var_real
 
 
@@ -401,31 +454,41 @@ def _bcast_flag(flag, rank, world, group, dev):
     return bool(int(t.item()))
 
 
-def _cma_cells(loss_type, cells, common, kw, dev, rank, world, group, num_frames, datagen="gpu"):
+def _cma_cells(loss_type, cells, common, kw, dev, rank, world, group, num_frames, datagen="gpu", gmi=False):
     """This rank's share of the cells of a CMA-family run set through the batched engine (sweep_cma_dp), gathered on rank 0."""
     from .parallel import gather_cell_results, shard_cells
     mod, sps, M, batch_len, N_frame_max, nf = common
     mine = shard_cells(cells, rank, world)
-    loc_s, loc_v, loc_r = {}, {}, {}
+    loc_s, loc_v, loc_r, loc_g = {}, {}, {}, {}
     if mine:
-        s, v, r = sweep_cma_dp([c for _, c in mine], mod, sps, M, batch_len, N_frame_max, nf, kw["flex_step"], kw["channel"], kw["symb_rate"],
-                               kw["tau_cd"], kw["tau_pmd"], kw["phiIQ"], kw["N_lrhalf"], kind=loss_type, device=dev, datagen=datagen)
+        res = sweep_cma_dp([c for _, c in mine], mod, sps, M, batch_len, N_frame_max, nf, kw["flex_step"], kw["channel"], kw["symb_rate"],
+                           kw["tau_cd"], kw["tau_pmd"], kw["phiIQ"], kw["N_lrhalf"], kind=loss_type, device=dev, datagen=datagen,
+                           **(dict(gmi=True) if gmi else {}))
+        s, v, r = res[:3]
         for k, (i, _) in enumerate(mine):
             loc_s[i], loc_v[i], loc_r[i] = s[k], v[k], r[k]
+            if gmi:
+                loc_g[i] = res[3][k]
     n = len(cells)
     out = (gather_cell_results(loc_s, n, (4, num_frames), rank, world, group, dev), gather_cell_results(loc_v, n, (2, num_frames), rank, world, group, dev),
            gather_cell_results(loc_r, n, (2,), rank, world, group, dev))
+    if gmi:
+        out = out + (_gather_with_nan(loc_g, n, (2, num_frames), rank, world, group, dev),)
     return out if rank == 0 else None
 
 
 def save_mat(path, SER, Var_est, var_real, *, SNR_vec, nu_vec, theta_diff_vec, theta_vec, M_vec, lr_optim_vec, batch_len_vec, symb_rate_vec,
-             flex_step_vec):
-    """The .mat file of Eval_run_DP.py:99-114: one struct 'dict' with the result arrays and the parameter lists under the same keys."""
+             flex_step_vec, GMI=None):
+    """The .mat file of Eval_run_DP.py:99-114: one struct 'dict' with the result arrays and the parameter lists under the same keys.
+    GMI (run_dp_sweep(..., gmi=True)), when given, is stored under the extra key 'GMI'; without it the file is exactly the reference's."""
     from scipy import io
-    io.savemat(path, {"dict": {"SER": SER.cpu().numpy(), "Var_est": Var_est.cpu().numpy(), "var_real": var_real.cpu().numpy(),
-                               "SNR": list(SNR_vec), "nu": list(nu_vec), "theta_diff": list(theta_diff_vec), "theta": list(theta_vec),
-                               "M": list(M_vec), "lr": list(lr_optim_vec), "batch_len": list(batch_len_vec),
-                               "symb_rate": list(symb_rate_vec), "symb_step": list(flex_step_vec)}})
+    d = {"SER": SER.cpu().numpy(), "Var_est": Var_est.cpu().numpy(), "var_real": var_real.cpu().numpy(),
+         "SNR": list(SNR_vec), "nu": list(nu_vec), "theta_diff": list(theta_diff_vec), "theta": list(theta_vec),
+         "M": list(M_vec), "lr": list(lr_optim_vec), "batch_len": list(batch_len_vec),
+         "symb_rate": list(symb_rate_vec), "symb_step": list(flex_step_vec)}
+    if GMI is not None:
+        d["GMI"] = GMI.cpu().numpy()
+    io.savemat(path, {"dict": d})
 
 
 # -------------------------------------------------------------------------------------------------
@@ -457,7 +520,8 @@ def _awgn_host_frames(N, F, M, amps, snr, h_channel, sps, dev, P, rngs):
     return rx, tx
 
 
-def sweep_vae_awgn(cells, mod, sps, M_est, batch_len, N_valid, N_train, num_epochs, epe, channel, *, device=None, datagen="gpu", verbose=False):
+def sweep_vae_awgn(cells, mod, sps, M_est, batch_len, N_valid, N_train, num_epochs, epe, channel, *, device=None, datagen="gpu", verbose=False,
+                   gmi=False):
     """processing_vaele_awgn (:235-324) for R = len(cells) independent cells in lockstep.
 
     cells: dicts with SNR, nu, lr_optim and optionally seed (default: the cell's index).  Returns SER_valid (R, num_epochs // epe), row k
@@ -465,8 +529,10 @@ def sweep_vae_awgn(cells, mod, sps, M_est, batch_len, N_valid, N_train, num_epoc
     is ONE launch training every cell's epochs since the last validation, the validation forward of all cells, and the batched scoring.
     The epe - 1 epochs after the last validation do not change the result and are not trained.
     datagen="gpu": every cell's frames from the device generator, keyed by the cell's seed (a cell gives the same SER alone or in any
-    batch); "numpy": each cell's frames from np.random.default_rng(seed) in exactly the order processing_vaele_awgn(rng=...) draws them."""
-    from .awgn import AWGNEqualizerRuns, awgn_eval_runs, generate_frames_awgn_gpu
+    batch); "numpy": each cell's frames from np.random.default_rng(seed) in exactly the order processing_vaele_awgn(rng=...) draws them.
+    gmi=True: returns (SER_valid, GMI_valid (R, num_epochs // epe)), GMI scored on the SER's symbols under its best rotation
+    (awgn.awgn_gmi_runs)."""
+    from .awgn import AWGNEqualizerRuns, awgn_eval_runs, awgn_gmi_runs, generate_frames_awgn_gpu
     from .constants import awgn_constants, upsampled_channel
     dev = _awgn_check(num_epochs, epe, channel, device)
     if datagen not in ("gpu", "numpy"):
@@ -489,6 +555,8 @@ def sweep_vae_awgn(cells, mod, sps, M_est, batch_len, N_valid, N_train, num_epoc
     snr = [float(c["SNR"]) for c in cells]
     n_val = num_epochs // epe
     SER_valid = torch.empty(R, n_val, device=dev, dtype=torch.float32)
+    GMI_valid = torch.empty(R, n_val, device=dev, dtype=torch.float32) if gmi else None
+    P_gmi = P.to(dev) if gmi else None
 
     def host_frames(N, F):
         return _awgn_host_frames(N, F, M, amps, snr, h_channel, sps, dev, [k[1] for k in consts], rngs)
@@ -505,25 +573,37 @@ def sweep_vae_awgn(cells, mod, sps, M_est, batch_len, N_valid, N_train, num_epoc
         loss = eqr.train_frames(rx, lr, batch_len, N_train)
         epoch += n_ep
         q_v, _, _ = eqr.forward(rx_v[:, 0])
-        shift, _, ser = awgn_eval_runs(q_v, tx_v[:, 0], amp_levels)
+        shift, counts, ser = awgn_eval_runs(q_v, tx_v[:, 0], amp_levels)
         SER_valid[:, k] = ser
+        if gmi:
+            GMI_valid[:, k] = awgn_gmi_runs(q_v, tx_v[:, 0], P_gmi, shift, counts)
         if verbose:
             print(epoch - 1, "loss", loss[:, -1].tolist(), "shift", shift.tolist(), "SER", ser.tolist())
+    if gmi:
+        return SER_valid, GMI_valid
     return SER_valid
 
 
 def sweep_vae_awgn_sharded(cells, *args, rank=0, world=1, group=None, **kw):
     """sweep_vae_awgn over a round-robin share of the cells per rank (one process per GPU); SER_valid of ALL cells on rank 0 (None
-    elsewhere).  No data-path collective."""
+    elsewhere), with gmi=True the pair (SER_valid, GMI_valid).  No data-path collective."""
     from .parallel import gather_cell_results, shard_cells
     mine = shard_cells(cells, rank, world)
     num_epochs, epe = (args[6], args[7]) if len(args) > 7 else (kw["num_epochs"], kw["epe"])
     dev = _cuda_device(kw.get("device"))
-    loc = {}
+    gmi = kw.get("gmi", False)
+    loc, loc_g = {}, {}
     if mine:
-        ser = sweep_vae_awgn([c for _, c in mine], *args, **kw)
+        res = sweep_vae_awgn([c for _, c in mine], *args, **kw)
+        ser = res[0] if gmi else res
         loc = {i: ser[k] for k, (i, _) in enumerate(mine)}
-    return gather_cell_results(loc, len(cells), (num_epochs // epe,), rank, world, group, dev)
+        if gmi:
+            loc_g = {i: res[1][k] for k, (i, _) in enumerate(mine)}
+    ser_g = gather_cell_results(loc, len(cells), (num_epochs // epe,), rank, world, group, dev)
+    if not gmi:
+        return ser_g
+    gmi_g = _gather_with_nan(loc_g, len(cells), (num_epochs // epe,), rank, world, group, dev)
+    return None if rank != 0 else (ser_g, gmi_g)
 
 
 AWGN_AXES = ("batch_len", "lr_optim", "M", "SNR", "nu")           # loop order of Eval_run_shaping_vaele.py (RUN_AWGN:42-58), then iter
@@ -531,25 +611,28 @@ AWGN_AXES = ("batch_len", "lr_optim", "M", "SNR", "nu")           # loop order o
 
 def run_awgn_sweep(mod="64-QAM", sps=2, channel="h1", N_train_vec=(350,), lr_optim_vec=(2e-3,), M_vec=(25,), SNR_vec=(12,), nu_vec=(0.0,),
                    iter=1, N_valid=15000, train_len=1200, num_epochs=500, epe=20, *, device=None, datagen="gpu", rank=0, world=1, group=None,
-                   runner=None, verbose=False, checkpoint_dir=None):
+                   runner=None, verbose=False, checkpoint_dir=None, gmi=False):
     """Eval_run_shaping_vaele.py's loops (RUN_AWGN:42-58) as batched run sets.  As in the reference, the N_train_vec entries are the
     drivers' batch_len and train_len is their N_train (RUN_AWGN:53).  Cells that share (M, batch_len) train in the same launch; with
     world > 1 every rank takes a round-robin share of each set.  Returns on rank 0 (None elsewhere)
         SER (len(N_train_vec), len(lr_optim_vec), len(M_vec), len(SNR_vec), len(nu_vec), iter, num_epochs // epe) and the validation
         epochs (num_epochs // epe,).
     Cell (.., i) is seeded with its flat index.  checkpoint_dir: rank 0 stores every finished set (one .npz, keyed by the set's full
-    parameters); a restarted sweep loads what it finds instead of recomputing."""
+    parameters); a restarted sweep loads what it finds instead of recomputing.
+    gmi=True: also GMI shaped like SER as a 3rd result (sweep_vae_awgn(..., gmi=True); the runner hook is then called with gmi=True and
+    returns (SER_valid, GMI_valid)).  Its checkpoints hold the GMI and are never mixed up with those of gmi=False."""
     if channel not in ("h1", "h2"):
         raise KeyError(f"AWGN driver knows channels h1/h2, got {channel!r}")
     if epe < 1 or num_epochs % epe != 0:
         raise ValueError(f"num_epochs={num_epochs} must be a multiple of epe={epe}")
+    gkw = dict(gmi=True) if gmi else {}                              # gmi=False: every call, name and signature exactly as without GMI
     vecs = dict(batch_len=list(N_train_vec), lr_optim=list(lr_optim_vec), M=list(M_vec), SNR=list(SNR_vec), nu=list(nu_vec))
     dev = torch.device("cpu") if runner is not None and device is None else _cuda_device(device)
 
     def signature(key, cells):
         M, batch_len = key
         return _set_signature(driver="VAELE_AWGN", mod=mod, sps=sps, channel=channel, M=M, batch_len=batch_len, N_valid=N_valid,
-                              train_len=train_len, num_epochs=num_epochs, epe=epe, datagen=datagen, cells=[sorted(c.items()) for c in cells])
+                              train_len=train_len, num_epochs=num_epochs, epe=epe, datagen=datagen, cells=[sorted(c.items()) for c in cells], **gkw)
 
     def file_name(key, cells, sig):
         M, batch_len = key
@@ -559,24 +642,28 @@ def run_awgn_sweep(mod="64-QAM", sps=2, channel="h1", N_train_vec=(350,), lr_opt
         M, batch_len = key
         args = (cells, mod, sps, M, batch_len, N_valid, train_len, num_epochs, epe, channel)
         if runner is not None:                                       # test hook: stands for sweep_vae_awgn_sharded
-            return runner(*args)
-        return sweep_vae_awgn_sharded(*args, device=dev, datagen=datagen, verbose=verbose, rank=rank, world=world, group=group)
+            return runner(*args, **gkw)
+        return sweep_vae_awgn_sharded(*args, device=dev, datagen=datagen, verbose=verbose, rank=rank, world=world, group=group, **gkw)
 
-    SER = _walk_awgn_sets(AWGN_AXES, vecs, ("M", "batch_len"), iter, num_epochs // epe, dev, checkpoint_dir, rank, world, group, signature,
-                          file_name, run_set)
+    res = _walk_awgn_sets(AWGN_AXES, vecs, ("M", "batch_len"), iter, num_epochs // epe, dev, checkpoint_dir, rank, world, group, signature,
+                          file_name, run_set, gmi=gmi)
     if rank != 0:
         return None
-    return SER, np.arange(0, num_epochs, epe)
+    if gmi:
+        return res[0], np.arange(0, num_epochs, epe), res[1]
+    return res, np.arange(0, num_epochs, epe)
 
 
-def _walk_awgn_sets(axes, vecs, group_by, iter, n_val, dev, checkpoint_dir, rank, world, group, signature, file_name, run_set):
+def _walk_awgn_sets(axes, vecs, group_by, iter, n_val, dev, checkpoint_dir, rank, world, group, signature, file_name, run_set, gmi=False):
     """The cells of vecs[axes[0]] x ... x iter, seeded by their flat index, grouped into one run set per value of the `group_by` axes.
     Per set: with checkpoint_dir, rank 0 loads the set's file if its stored signature(key, cells) matches (all ranks then skip it);
     otherwise run_set(key, cells) gives SER_valid (n, n_val) on rank 0 (None elsewhere), which rank 0 stores under
-    file_name(key, cells, sig).  Returns SER (shape of the cells, n_val)."""
+    file_name(key, cells, sig).  Returns SER (shape of the cells, n_val).  gmi=True: run_set gives (SER_valid, GMI_valid), the files
+    hold both and (SER, GMI) is returned."""
     import os
     shape = tuple(len(vecs[a]) for a in axes) + (iter,)
     SER = torch.full(shape + (n_val,), float("nan"), dtype=torch.float32, device=dev)
+    GMI = torch.full(shape + (n_val,), float("nan"), dtype=torch.float32, device=dev) if gmi else None
     groups = {}
     for idx in np.ndindex(*shape):
         c = {a: vecs[a][i] for a, i in zip(axes, idx[:-1])}
@@ -592,20 +679,26 @@ def _walk_awgn_sets(axes, vecs, group_by, iter, n_val, dev, checkpoint_dir, rank
             have = 0
             if rank == 0 and os.path.exists(ck):
                 z = np.load(ck)
-                if "signature" in z.files and str(z["signature"]) == sig:
+                if "signature" in z.files and str(z["signature"]) == sig and (not gmi or "gmi" in z.files):
                     have = 1
                     for k, (idx, _) in enumerate(members):
                         SER[idx] = torch.from_numpy(z["ser"][k]).to(dev)
+                        if gmi:
+                            GMI[idx] = torch.from_numpy(z["gmi"][k]).to(dev)
             if _bcast_flag(have, rank, world, group, dev):
                 continue
-        ser = run_set(key, cells)
-        if ser is None:
+        res = run_set(key, cells)
+        if res is None:
             continue
+        ser, g = res if gmi else (res, None)
         if ck is not None and rank == 0:
-            np.savez(ck, ser=ser.cpu().numpy(), signature=np.array(sig))
+            extra = dict(gmi=g.cpu().numpy()) if gmi else {}
+            np.savez(ck, ser=ser.cpu().numpy(), signature=np.array(sig), **extra)
         for k, (idx, _) in enumerate(members):
             SER[idx] = ser[k].to(dev)
-    return SER
+            if gmi:
+                GMI[idx] = g[k].to(dev)
+    return (SER, GMI) if gmi else SER
 
 
 # -------------------------------------------------------------------------------------------------
@@ -622,7 +715,8 @@ def sweep_cma_awgn(cells, mod, sps, M_est, N_valid, N_train, num_epochs, epe, ch
     datagen="gpu": frames from the device generator with the frame keys of sweep_vae_awgn (training frame = epoch index, validation
     frame k = AWGN_VALID_FRAME0 + k), so a cell with the same seed, N_train and N_valid sees the same frames in both sweeps and the two
     baselines are compared on identical data; a cell gives the same SER alone or in any batch.  "numpy": each cell's frames from
-    np.random.default_rng(seed) in exactly the order processing_cma_awgn(rng=...) draws them."""
+    np.random.default_rng(seed) in exactly the order processing_cma_awgn(rng=...) draws them.
+    No GMI: the AWGN CMA driver makes no posteriors (it decides on the nearest level), so there is no q to score."""
     from . import awgn_cma as cm
     from .awgn import generate_frames_awgn_gpu
     from .constants import awgn_constants, upsampled_channel
@@ -691,7 +785,8 @@ def run_awgn_cma_sweep(mod="64-QAM", sps=2, channel="h1", lr_optim_vec=(5e-4,), 
         SER (len(lr_optim_vec), len(M_vec), len(SNR_vec), len(nu_vec), iter, num_epochs // epe) and the validation epochs (num_epochs // epe,).
     Cell (.., i) is seeded with its flat index, as in run_awgn_sweep.  checkpoint_dir: rank 0 stores every finished set (one .npz named
     AWGNCMA_..., keyed by the set's full parameters; never mistaken for a VAE-LE set of the same directory); a restarted sweep loads what
-    it finds instead of recomputing.  runner: stands for sweep_cma_awgn_sharded (called with its positional arguments)."""
+    it finds instead of recomputing.  runner: stands for sweep_cma_awgn_sharded (called with its positional arguments).
+    No GMI (unlike run_awgn_sweep): the AWGN CMA driver makes no posteriors to score."""
     if channel not in ("h1", "h2"):
         raise KeyError(f"AWGN driver knows channels h1/h2, got {channel!r}")
     if epe < 1 or num_epochs % epe != 0:
