@@ -127,7 +127,9 @@ class AdamState:
         f4 = np.float32
         g = g.astype(f4)
         self.t += 1
-        self.m = (self.m + (g - self.m) * f4(1 - self.b1)).astype(f4)           # exp_avg.lerp_(grad, 1-beta1)
+        # exp_avg.lerp_(grad, 1-beta1): torch computes it as ONE fused multiply-add, m + w * (g - m); the float64 product of two floats
+        # is exact, so only the float64 sum rounds before the float32 result
+        self.m = (self.m.astype(np.float64) + (g - self.m).astype(f4).astype(np.float64) * np.float64(f4(1 - self.b1))).astype(f4)
         self.v = (self.v * f4(self.b2) + f4(1 - self.b2) * g * g).astype(f4)    # mul_(beta2).addcmul_(g,g,1-beta2)
         bc1 = 1 - self.b1 ** self.t
         bc2 = 1 - self.b2 ** self.t

@@ -543,14 +543,15 @@ def awgn_loss(q, rx, h, amp, P):
     qv = q.reshape(2, n, B)
     m1 = (amp.view(1, n, 1) * qv).sum(1)
     m2 = ((amp ** 2).view(1, n, 1) * qv).sum(1)
-    Eq = torch.zeros(2, L, dtype=F32)
-    Ex2 = torch.zeros(2, L, dtype=F32)
+    dt = q.dtype                                              # float32 as the reference; float64 as the yardstick of the tests
+    Eq = torch.zeros(2, L, dtype=dt)
+    Ex2 = torch.zeros(2, L, dtype=dt)
     Eq[:, ::sps] = m1
     Ex2[:, ::sps] = m2
     width = L - Mh
-    D_re = torch.zeros(width, dtype=F32)
-    D_im = torch.zeros(width, dtype=F32)
-    E = torch.zeros(width, dtype=F32)
+    D_re = torch.zeros(width, dtype=dt)
+    D_im = torch.zeros(width, dtype=dt)
+    E = torch.zeros(width, dtype=dt)
     for j in range(Mh + 1):                                   # awgn:85-88
         lo, hi = Mh - j, L - j
         D_re = D_re + (h[0, j] * Eq[0, lo:hi] - h[1, j] * Eq[1, lo:hi])
@@ -562,6 +563,23 @@ def awgn_loss(q, rx, h, amp, P):
     C = torch.sum(rx[:, mh:L - mh] ** 2)
     C = C + (-2 * torch.sum(rx[0, mh:L - mh] * D_re + rx[1, mh:L - mh] * D_im) + torch.sum(D_re ** 2 + D_im ** 2 + E))
     return width * torch.log(C) - entropy
+
+
+def awgn_step(rx, W, h, amp, P, amp_mean, var, dtype=F32, want_grads=True):
+    """awgn_forward + awgn_loss (+ autograd) in dtype on the CPU: dict of out (2,N), q (2n,N), loss and, with want_grads, gW (1,2,M)
+    and gh (2,M).  float32 is the reference's own arithmetic; float64 is the yardstick the float32 paths are measured against."""
+    cv = lambda a: torch.as_tensor(np.asarray(a.detach().cpu() if torch.is_tensor(a) else a)).to(dtype)
+    x, a = cv(rx), cv(amp)
+    Wt = cv(W).reshape(1, 2, -1).requires_grad_(want_grads)
+    ht = cv(h).requires_grad_(want_grads)
+    with torch.set_grad_enabled(want_grads):
+        q, out = awgn_forward(x, Wt, a, amp_mean, var, 2)
+        loss = awgn_loss(q, x, ht, a, cv(P))
+    res = dict(out=out.detach(), q=q.detach(), loss=loss.detach())
+    if want_grads:
+        gW, gh = torch.autograd.grad(loss, (Wt, ht))
+        res.update(gW=gW, gh=gh)
+    return res
 
 
 def awgn_constants(mod, nu, SNR):

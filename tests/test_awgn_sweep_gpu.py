@@ -211,15 +211,21 @@ def test_sweep_numpy_datagen_equals_driver(channel):
 
 
 def test_sweep_gpu_datagen_batch_independent_and_converges():
+    """Blind VAE-LE training from the Dirac start does not converge for every seed: at this setting about 4 cells in 10 stay near SER
+    0.8 (the reference algorithm's own behaviour, measured on B200 with the device generator), and WHICH seeds converge moves with any
+    last-bit change of the step.  So convergence is asserted over 41 cells: at least a third must end below SER 1e-2 (23 of 41 do; 14
+    is about 3 standard deviations below that)."""
     from vae_equalizer_b200.sweep import sweep_vae_awgn
     cells = [dict(SNR=20.0, nu=0.0, lr_optim=5e-3, seed=s) for s in (1, 2, 3, 4)] + _cells(5)
+    cells += [dict(SNR=20.0, nu=0.0, lr_optim=5e-3, seed=s) for s in range(100, 132)]
     args = ("16-QAM", 2, 25, 350, 5000, 1200, 200, 50, "h1")       # the setting of test_dropin_awgn_runs, trained longer
     ser = sweep_vae_awgn(cells, *args, datagen="gpu")
     alone = sweep_vae_awgn([cells[2]], *args, datagen="gpu")
     assert torch.equal(alone[0], ser[2])
     assert torch.isfinite(ser).all()
-    for r in range(4):
-        assert float(ser[r, -1]) < float(ser[r, 0]), ser[r].tolist()
+    assert bool((ser[:, 0] > 0.5).all()), ser[:, 0].tolist()        # the validation after the first epoch is far from converged
+    converged = int((ser[:, -1] < 0.01).sum())
+    assert 3 * converged >= len(cells), ser[:, -1].tolist()
 
 
 def test_sweep_gpu_datagen_tx_alignment():

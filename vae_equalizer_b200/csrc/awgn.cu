@@ -31,10 +31,13 @@ struct AwK {
 
 __device__ __forceinline__ void adam_apply_awgn(float *param, float g, float *m, float *v, float *vmax, int i, float lr,
                                                 bool amsgrad, double bc1, float bc2s) {
-    const float b1 = 0.9f, b2 = 0.999f, eps = 1e-8f;
+    const float b2 = 0.999f, eps = 1e-8f;
+    // torch passes 1 - beta as a double and rounds it to float: 0.1f and 0.001f.  1.f - 0.999f would be 1.3e-5 below 0.001f, about
+    // 200 ulp in every exp_avg_sq.
+    const float w1 = (float)(1.0 - 0.9), w2 = (float)(1.0 - 0.999);
     float mi = m[i], vi = v[i];
-    mi = mi + (g - mi) * (1.f - b1);
-    vi = vi * b2 + (1.f - b2) * g * g;
+    mi = __fmaf_rn(g - mi, w1, mi);                      // exp_avg.lerp_(grad, 1 - beta1), one fused multiply-add as in torch
+    vi = vi * b2 + w2 * g * g;                           // exp_avg_sq.mul_(beta2).addcmul_(grad, grad, value=1 - beta2)
     m[i] = mi;
     v[i] = vi;
     const float step_size = (float)(-(double)lr / bc1);    // bias corrections: two double-precision pow, computed ONCE per step by thread 0
