@@ -181,8 +181,16 @@ int vaeq_dp_persistent_frames(int32_t mode);
  * is found rs_* ELEMENTS further (0 = shared by all runs).  d->loss (n_runs), d->var_est (n_runs,2), d->gW (n_runs,2,4,M),
  * d->gh (n_runs,2,2,2,M) get a leading run dimension; d->workspace holds vaeq_dp_runs_workspace_bytes(B,M,n_lev,n_runs) (the
  * default kernel keeps all scratch in shared memory: 256 bytes; testing mode 2 needs a full workspace per run);
- * loss_steps (n_runs,n_steps), var_est_steps (n_runs,2,n_steps).  nu_sc / lr_w / lr_h: optional per-run device arrays. */
+ * loss_steps (n_runs,n_steps), var_est_steps (n_runs,2,n_steps).  nu_sc / lr_w / lr_h: optional per-run device arrays.
+ * Minibatches that one CTA's shared memory cannot hold (batch_len > 1000, or a plan > 220 KB at large M_est) run on ONE
+ * THREAD-BLOCK CLUSTER per run instead (dp_cluster.cu, DESIGN.md §4c): K = 2, 4 or 8 CTAs, each owning a slice of the window, K chosen
+ * from (batch_len, M_est) only, so a run's result is bit-identical alone or in any batch; it agrees with vaeq_dp_train_frame (which
+ * steps such a run launch by launch) within the step tolerances, not bitwise.  Up to vaeq_dp_runs_max_batch_len(M, n_lev) symbols
+ * (about 8900 at M_est 25); above it the call returns VAEQ_EINVAL naming that limit.  Every call needs the same 256-byte workspace. */
 size_t vaeq_dp_runs_workspace_bytes(int32_t B, int32_t M, int32_t n_lev, int32_t n_runs);
+/* Largest batch_len vaeq_dp_train_frame_runs accepts at (M_est, n_lev) (testing mode 2 of vaeq_dp_persistent_frames aside); 0 for an
+ * invalid M_est / n_lev. */
+int32_t vaeq_dp_runs_max_batch_len(int32_t M, int32_t n_lev);
 typedef struct vaeq_dp_runs {
     int32_t n_runs;
     int64_t rs_rx, rs_amp, rs_P, rs_var, rs_W, rs_h, rs_adam, rs_q, rs_out, rs_q_keep, rs_out_keep;

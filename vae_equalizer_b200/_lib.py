@@ -101,6 +101,7 @@ PROTOTYPES = {
     "vaeq_dp_persistent_frames": (C.c_int, [_i32]),
     "vaeq_dp_frame_runs_per_sm": (C.c_int, [_i32]),
     "vaeq_dp_runs_workspace_bytes": (_sz, [_i32, _i32, _i32, _i32]),
+    "vaeq_dp_runs_max_batch_len": (_i32, [_i32, _i32]),
     "vaeq_dp_train_frame_runs": (C.c_int, [C.POINTER(DpDesc), C.POINTER(DpRuns), _i32, _i32, _i32, _f, _f, _vp, _vp, _vp]),
     "vaeq_dp_split_stats_doubles": (_sz, [_i32]),
     "vaeq_dp_split_forward": (C.c_int, [C.POINTER(DpDesc), _i32, _i32, _vp, _vp]),

@@ -91,5 +91,12 @@ constexpr int DP_SMALL_MAX_B = 1000;   // ~200 KB of shared memory at M_est = 25
 size_t dp_small_smem(int B, int M);
 int dp_small_launch(const DpK &p, const DpRunsK &rs, int n_lev, int n_runs, int n_steps, int stride_sym, int keep_lo_in_dst,
                     float lr_w, float lr_h, int amsgrad, cudaStream_t st);
+inline bool dp_small_fits(int B, int M) { return B <= DP_SMALL_MAX_B && dp_small_smem(B, M) <= 220 * 1024; }
+
+// dp_cluster.cu: batched runs that dp_small.cu cannot hold, one thread-block cluster of 2, 4 or 8 CTAs per run
+int dp_cluster_max_b(int M);             // largest batch_len with a cluster plan at this M_est
+int dp_cluster_check(int B, int M);      // VAEQ_OK, or VAEQ_EINVAL with a message naming dp_cluster_max_b(M)
+int dp_cluster_launch(const DpK &p, const DpRunsK &rs, int n_lev, int n_runs, int n_steps, int stride_sym, int keep_lo_in_dst,
+                      float lr_w, float lr_h, int amsgrad, cudaStream_t st);
 
 }  // namespace vaeq

@@ -857,6 +857,11 @@ extern "C" size_t vaeq_dp_runs_workspace_bytes(int32_t B, int32_t M, int32_t n_l
     return g_persistent_frames_mode() == 2 ? (size_t)n_runs * vaeq_dp_workspace_bytes(B, M, n_lev) : 256;
 }
 
+extern "C" int32_t vaeq_dp_runs_max_batch_len(int32_t M, int32_t n_lev) {
+    if (M < 1 || M > VAEQ_MAX_TAPS || !(M & 1) || (n_lev != 2 && n_lev != 4 && n_lev != 8)) return 0;
+    return max(vaeq::dp_cluster_max_b(M), vaeq::dp_small_fits(DP_SMALL_MAX_B, M) ? DP_SMALL_MAX_B : 0);
+}
+
 extern "C" int vaeq_dp_dynamic_tiles(int32_t on) {
     g_dynamic_tiles = on != 0;
     return VAEQ_OK;
@@ -945,8 +950,11 @@ static int dp_frame_persistent(const vaeq_dp_desc *d, const vaeq_dp_runs *runs, 
     rs.loss_last = d->loss; rs.var_last = d->var_est; rs.gW_last = d->gW; rs.gh_last = d->gh;
     const size_t smem = max(dp_fwd_smem(p.M, p.T, p.H, p.mh), dp_bwd_smem(p.M, p.T, p.H, p.mh));
     const int amsgrad = (d->flags & VAEQ_F_AMSGRAD) ? 1 : 0;
-    if (g_persistent_frames != 2)
+    if (g_persistent_frames != 2) {
+        if (runs && !dp_small_fits(d->B, d->M))
+            return dp_cluster_launch(p, rs, d->n_lev, n_runs, n_steps, stride_sym, keep_lo_in_dst, lr_w, lr_h, amsgrad, st);
         return dp_small_launch(p, rs, d->n_lev, n_runs, n_steps, stride_sym, keep_lo_in_dst, lr_w, lr_h, amsgrad, st);
+    }
     static SmemAttrCache set_smem[3];
 #define FRAME_CASE(NL_, IDX_)                                                                                             \
     {                                                                                                                     \
@@ -973,7 +981,7 @@ extern "C" int vaeq_dp_train_frame(const vaeq_dp_desc *d, int32_t n_steps, int32
     if (n_steps == 0) return VAEQ_OK;
     // mode 1 (dp_small.cu) covers batch_len up to DP_SMALL_MAX_B, i.e. up to where the register-blocked fast path takes over for
     // single steps; mode 2 (generic bodies in one launch) needs the minibatch to be one tile
-    if ((g_persistent_frames == 1 && d->B <= DP_SMALL_MAX_B && dp_small_smem(d->B, d->M) <= 220 * 1024) ||
+    if ((g_persistent_frames == 1 && dp_small_fits(d->B, d->M)) ||
         (g_persistent_frames == 2 && d->B <= DP_TILE))
         return dp_frame_persistent(d, nullptr, n_steps, stride_sym, keep_lo_in_dst, lr_w, lr_h, loss_steps, var_est_steps,
                                    (cudaStream_t)stream);
@@ -995,8 +1003,11 @@ extern "C" int vaeq_dp_train_frame_runs(const vaeq_dp_desc *d, const vaeq_dp_run
                                         int32_t keep_lo_in_dst, float lr_w, float lr_h, float *loss_steps, float *var_est_steps,
                                         void *stream) {
     VAEQ_CHECK_ARG(d != nullptr && runs != nullptr && runs->n_runs >= 1, "desc / runs is NULL or n_runs < 1");
-    VAEQ_CHECK_ARG(d->B <= (g_persistent_frames == 2 ? DP_TILE : DP_SMALL_MAX_B) && dp_small_smem(d->B, d->M) <= 220 * 1024,
-                   "batched runs need batch_len <= %d and a shared-memory plan <= 220 KB (one CTA per run), got batch_len %d", DP_SMALL_MAX_B, d->B);
+    if (g_persistent_frames == 2)
+        VAEQ_CHECK_ARG(d->B <= DP_TILE && dp_small_smem(d->B, d->M) <= 220 * 1024,
+                       "batched runs need batch_len <= %d and a shared-memory plan <= 220 KB (one CTA per run), got batch_len %d", DP_SMALL_MAX_B, d->B);
+    else if (!dp_small_fits(d->B, d->M) && d->M >= 1 && d->M <= VAEQ_MAX_TAPS)   // above dp_small.cu's range: one cluster per run
+        if (int rc = dp_cluster_check(d->B, d->M)) return rc;
     vaeq_dp_desc one = *d;
     static char dummy_ws;                                    // dp_small.cu keeps everything in shared memory: no workspace
     if (g_persistent_frames == 2) {

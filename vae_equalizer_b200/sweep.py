@@ -47,6 +47,7 @@ def sweep_vae_dp(cells, mod, sps, M_est, batch_len, N_frame_max, num_frames, fle
     Returns (SER_valid (R,4,num_frames), Var_est (R,2,num_frames), var (R,2)), and GMI (R,2,num_frames) as a 4th tensor with gmi=True
     (NaN on unscored frames)."""
     _gmi_batched_only(gmi, eval_mode)
+    _check_dp_batch_len(mod, M_est, batch_len)
     device = _cuda_device(device)
     R = len(cells)
     if R == 0:
@@ -158,6 +159,16 @@ def sweep_vae_dp(cells, mod, sps, M_est, batch_len, N_frame_max, num_frames, fle
     if gmi:
         return SER_valid, Var_est, var_all.to(device), GMI
     return SER_valid, Var_est, var_all.to(device)
+
+
+def _check_dp_batch_len(mod, M_est, batch_len):
+    """Raise VaeqError, before any data is generated, if the batched DP kernels cannot train a minibatch of batch_len symbols at M_est
+    (one CTA per run up to 1000 symbols, one thread-block cluster per run above; vaeq_dp_runs_max_batch_len)."""
+    n_lev = int(round(np.sqrt(int(str(mod).split("-")[0]))))
+    lim = int(sfun._lib.load().vaeq_dp_runs_max_batch_len(int(M_est), n_lev))
+    if int(batch_len) > lim:
+        raise sfun._lib.VaeqError(f"batch_len={batch_len} exceeds the largest batch_len the batched DP engine supports at M_est={M_est}, "
+                                  f"{mod}: {lim}")
 
 
 def _gmi_batched_only(gmi, eval_mode):
@@ -359,6 +370,10 @@ def run_dp_sweep(mod="64-QAM", sps=2, loss_type="VAE", channel="h0", nu_vec=(0,)
     loads what it finds instead of recomputing (the reference only saves once, at the very end: RUN_DP:99-114).
     gmi=True: also GMI (2, SNR, ..., iter, num_frames), shaped like Var_est, as a 4th result (sweep_vae_dp / sweep_cma_dp with gmi=True;
     the runner hook is then called with gmi=True).  Its checkpoints hold the GMI and are never mixed up with those of gmi=False."""
+    if runner is None and loss_type in ("VAE", "VAEflex"):
+        for M in M_vec:                                              # every set's minibatch, before the first set generates data
+            for batch_len in batch_len_vec:
+                _check_dp_batch_len(mod, M, batch_len)
     vecs = dict(SNR=list(SNR_vec), symb_rate=list(symb_rate_vec), nu=list(nu_vec), theta_diff=list(theta_diff_vec), M=list(M_vec),
                 lr_optim=list(lr_optim_vec), batch_len=list(batch_len_vec), flex_step=list(flex_step_vec), theta=list(theta_vec))
     shape = tuple(len(vecs[a]) for a in AXES) + (iter,)
