@@ -330,6 +330,26 @@ int vaeq_frame_gmi_runs(const float *q, int64_t ld_q, int64_t rs_q, const uint16
 int vaeq_gmi(const float *q, int64_t ld_q, const uint16_t *tx, int64_t ld_tx, const float *P, int32_t n_lev, int32_t N,
              float *gmi_out, void *scratch, void *stream);
 
+/* extension, not in the reference: the bit-metric decoding rate (BMI) of a receiver that feeds Gray-labelled bit LLRs to a binary
+ * decoder.  Labels: per ASK component the binary reflected Gray code g(l) = l ^ (l >> 1) over the ascending level index, m = log2(n)
+ * bits MSB first; bit posteriors q_c(b_i = v | y) = sum of q_c[l] over the levels whose label has bit i = v (q as given, no
+ * renormalisation).  BMI = H(X) + mean over the evaluated symbols of sum over c in {I, Q}, i < m of log2 max(q_c(b_i = bit i of
+ * g(lev_c) | y), 1e-30), per pol, bit per 2-D symbol; in double, one cast to float at the end.  n = 2: BMI = GMI.
+ * vaeq_frame_bmi_runs: argument for argument vaeq_frame_gmi_runs (same symbols, hypothesis -- lev_c is the q level the hypothesis maps
+ * the tx level onto -- and scratch, vaeq_frame_gmi_scratch_bytes); bmi_out (R,2). */
+int vaeq_frame_bmi_runs(const float *q, int64_t ld_q, int64_t rs_q, const uint16_t *tx, int64_t ld_tx, int64_t rs_tx, const float *P,
+                        int64_t rs_P, const int32_t *align, const int32_t *counts, int32_t n_lev, int32_t N, int32_t n_runs, int32_t seg_len,
+                        int32_t edge, int32_t n_cut, float *bmi_out, void *scratch, void *stream);
+/* the BMI of vaeq_gmi's symbols (all N, tx levels as given); scratch: VAEQ_EVAL_SCRATCH_BYTES */
+int vaeq_bmi(const float *q, int64_t ld_q, const uint16_t *tx, int64_t ld_tx, const float *P, int32_t n_lev, int32_t N,
+             float *bmi_out, void *scratch, void *stream);
+/* Gray-labelled bit LLRs of n_runs runs: q (n_runs,2,2n,N) with row stride ld_q and run stride rs_q -> llr (n_runs,2,2m,N) with row
+ * stride ld_llr and run stride rs_llr, rows [I bits MSB..LSB | Q bits MSB..LSB] per pol, time innermost;
+ * L = ln max(q_c(b_i = 0 | y), 1e-30) - ln max(q_c(b_i = 1 | y), 1e-30) (positive: bit 0), the bit posteriors of vaeq_frame_bmi_runs.
+ * One launch, no scratch. */
+int vaeq_bit_llr_runs(const float *q, int64_t ld_q, int64_t rs_q, int32_t n_lev, int32_t N, int32_t n_runs, float *llr, int64_t ld_llr,
+                      int64_t rs_llr, void *stream);
+
 /* ------------------------------------------------------------------------------------------------
  * CMA baselines (sf:341-488) and carrier phase estimation (sf:140-186)
  * ---------------------------------------------------------------------------------------------- */
@@ -481,6 +501,11 @@ int vaeq_awgn_eval_runs(const float *q, int64_t ld_q, int64_t rs_q, const uint16
 size_t vaeq_awgn_gmi_scratch_bytes(int32_t n_runs, int32_t N);
 int vaeq_awgn_gmi_runs(const float *q, int64_t ld_q, int64_t rs_q, const uint16_t *tx, int64_t ld_tx, int64_t rs_tx, const float *P, int64_t rs_P,
                        const int32_t *shift, const int32_t *counts, int32_t n_lev, int32_t N, int32_t n_runs, int32_t edge, float *gmi_out,
+                       void *scratch, void *stream);
+/* The BMI (vaeq_frame_bmi_runs) of the same symbols and rotation, argument for argument; bmi_out (R); scratch:
+ * vaeq_awgn_gmi_scratch_bytes. */
+int vaeq_awgn_bmi_runs(const float *q, int64_t ld_q, int64_t rs_q, const uint16_t *tx, int64_t ld_tx, int64_t rs_tx, const float *P, int64_t rs_P,
+                       const int32_t *shift, const int32_t *counts, int32_t n_lev, int32_t N, int32_t n_runs, int32_t edge, float *bmi_out,
                        void *scratch, void *stream);
 
 #ifdef __cplusplus

@@ -125,8 +125,12 @@ PROTOTYPES = {
     "vaeq_frame_gmi_runs": (C.c_int, [_vp, _i64, _i64, _vp, _i64, _i64, _vp, _i64, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp]),
     "vaeq_awgn_gmi_scratch_bytes": (_sz, [_i32, _i32]),
     "vaeq_awgn_gmi_runs": (C.c_int, [_vp, _i64, _i64, _vp, _i64, _i64, _vp, _i64, _vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp]),
+    "vaeq_frame_bmi_runs": (C.c_int, [_vp, _i64, _i64, _vp, _i64, _i64, _vp, _i64, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp]),
+    "vaeq_awgn_bmi_runs": (C.c_int, [_vp, _i64, _i64, _vp, _i64, _i64, _vp, _i64, _vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp]),
     "vaeq_soft_dec_runs": (C.c_int, [_vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp, _vp]),
     "vaeq_gmi": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _i32, _i32, _vp, _vp, _vp]),
+    "vaeq_bmi": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _i32, _i32, _vp, _vp, _vp]),
+    "vaeq_bit_llr_runs": (C.c_int, [_vp, _i64, _i64, _i32, _i32, _i32, _vp, _i64, _i64, _vp]),
     "vaeq_cma_scratch_bytes": (_sz, [_i32, _i32, _i32]),
     "vaeq_cma": (C.c_int, [_i32, _vp, _i32, _f, _vp, _i32, _f, _i32, _i32, _i32, _i32, _vp, _vp, _i32, _vp, _vp]),
     "vaeq_cpe_scratch_bytes": (_sz, [_i32]),

@@ -207,11 +207,22 @@ def awgn_eval_runs(q, tx, amp_levels, n_shift=21, n_corr=1000, edge=11):
     return shift, counts, ser
 
 
-@_lib.device_guard
 def awgn_gmi_runs(q, tx, P, shift, counts, edge=11):
     """EXTENSION (not in the reference): GMI = H(X) + mean log2 q(x_tx|y) (bit/2D-symbol) of R runs on exactly the symbols awgn_eval_runs
     scores (q[:, edge+shift : N-edge] against tx[:, edge : N-edge-shift]) under its best rotation: q (R,2n,N), tx (R,2,N) float16, P (R,n)
     or (n,) pmf, shift (R,) and counts (R,4) int32 from awgn_eval_runs with the same edge.  Returns (R,) float32 on the device; no host sync."""
+    return _awgn_rate_runs("vaeq_awgn_gmi_runs", q, tx, P, shift, counts, edge)
+
+
+def awgn_bmi_runs(q, tx, P, shift, counts, edge=11):
+    """EXTENSION (not in the reference): the bit-metric decoding rate of Gray-labelled bits (BMI, DESIGN.md §2) of R runs, bit/2D-symbol.
+    Arguments, symbols, rotation and result exactly as awgn_gmi_runs."""
+    return _awgn_rate_runs("vaeq_awgn_bmi_runs", q, tx, P, shift, counts, edge)
+
+
+@_lib.device_guard
+def _awgn_rate_runs(fn, q, tx, P, shift, counts, edge):
+    """awgn_gmi_runs / awgn_bmi_runs through the C entry `fn` (vaeq_awgn_gmi_runs or vaeq_awgn_bmi_runs: same arguments)."""
     from .dp import _require_cuda
     from .shared_funcs import _run_pmf
     _need_cuda(q, "q")
@@ -228,12 +239,12 @@ def awgn_gmi_runs(q, tx, P, shift, counts, edge=11):
         if not torch.is_tensor(t) or t.dtype != torch.int32 or tuple(t.shape) != shape or not t.is_contiguous() or t.device != dev:
             raise _lib.VaeqError(f"{name}: need a contiguous int32 {shape} tensor on {dev} (awgn_eval_runs)")
     Pt, rs_P = _run_pmf(P, R, n, dev)
-    gmi = torch.empty(R, dtype=_F32, device=dev)
+    rate = torch.empty(R, dtype=_F32, device=dev)
     scr = torch.empty(max(1, int(lib.vaeq_awgn_gmi_scratch_bytes(R, N))), dtype=torch.uint8, device=dev)
-    _lib.check(lib.vaeq_awgn_gmi_runs(q.data_ptr(), int(q.stride(1)), int(q.stride(0)), tx.data_ptr(), int(tx.stride(1)), int(tx.stride(0)),
-                                      Pt.data_ptr(), rs_P, shift.data_ptr(), counts.data_ptr(), n, N, R, int(edge), gmi.data_ptr(), scr.data_ptr(),
-                                      _lib.current_stream()), "vaeq_awgn_gmi_runs")
-    return gmi
+    _lib.check(getattr(lib, fn)(q.data_ptr(), int(q.stride(1)), int(q.stride(0)), tx.data_ptr(), int(tx.stride(1)), int(tx.stride(0)),
+                                Pt.data_ptr(), rs_P, shift.data_ptr(), counts.data_ptr(), n, N, R, int(edge), rate.data_ptr(), scr.data_ptr(),
+                                _lib.current_stream()), fn)
+    return rate
 
 
 _TAPS_CACHE: dict = {}

@@ -3,6 +3,7 @@
 // error COUNTS returned next to the float SER so that "bit-exact SER counts" is checkable.
 #include "common.cuh"
 #include "shift_corr.cuh"
+#include "bits.cuh"
 
 namespace vaeq {
 
@@ -341,7 +342,9 @@ __global__ void __launch_bounds__(EV_NT) k_ser_constell(float *rx, int64_t ld_rx
 // ---------------------------------------------------------------------------------------------
 // extension (not in the reference): GMI-style achievable rate from the posteriors
 // ---------------------------------------------------------------------------------------------
-template <int NL, int V>
+// BITS: the bit-metric rate (BMI) instead, H(X) + the mean of sum_i log2 q(b_i = bit i of g(x_tx) | y) over the I and Q components
+// (bits.cuh); it reads every row of q at the thread's symbols, V at a time
+template <int NL, int V, bool BITS>
 __global__ void __launch_bounds__(EV_NT) k_gmi(const float *q, int64_t ld_q, const uint16_t *tx, int64_t ld_tx, int N, double *sums) {
     __shared__ double red[2 * 32];
     const float scale = (float)((NL - 1) / 2.0);
@@ -352,12 +355,33 @@ __global__ void __launch_bounds__(EV_NT) k_gmi(const float *q, int64_t ld_q, con
             float xI[V], xQ[V];
             ld_f16<V>(tx + (int64_t)(p * 2) * ld_tx + t, xI);
             ld_f16<V>(tx + (int64_t)(p * 2 + 1) * ld_tx + t, xQ);
+            if constexpr (BITS) {
+                float qI[NL][V], qQ[NL][V];
 #pragma unroll
-            for (int k = 0; k < V; ++k) {
-                const int iI = min(max((int)tx_level_f(xI[k], scale), 0), NL - 1);
-                const int iQ = min(max((int)tx_level_f(xQ[k], scale), 0), NL - 1);
-                const float qi = q[(int64_t)(p * 2 * NL + iI) * ld_q + t + k], qq = q[(int64_t)(p * 2 * NL + NL + iQ) * ld_q + t + k];
-                acc[p] += log2((double)fmaxf(qi, 1e-30f)) + log2((double)fmaxf(qq, 1e-30f));
+                for (int l = 0; l < NL; ++l) {
+                    ld_f32<V>(q + (int64_t)(p * 2 * NL + l) * ld_q + t, qI[l]);
+                    ld_f32<V>(q + (int64_t)(p * 2 * NL + NL + l) * ld_q + t, qQ[l]);
+                }
+#pragma unroll
+                for (int k = 0; k < V; ++k) {
+                    const int iI = min(max((int)tx_level_f(xI[k], scale), 0), NL - 1);
+                    const int iQ = min(max((int)tx_level_f(xQ[k], scale), 0), NL - 1);
+                    float vI[NL], vQ[NL];
+#pragma unroll
+                    for (int l = 0; l < NL; ++l) {
+                        vI[l] = qI[l][k];
+                        vQ[l] = qQ[l][k];
+                    }
+                    acc[p] += bmi_log2_component<NL>(vI, iI) + bmi_log2_component<NL>(vQ, iQ);
+                }
+            } else {
+#pragma unroll
+                for (int k = 0; k < V; ++k) {
+                    const int iI = min(max((int)tx_level_f(xI[k], scale), 0), NL - 1);
+                    const int iQ = min(max((int)tx_level_f(xQ[k], scale), 0), NL - 1);
+                    const float qi = q[(int64_t)(p * 2 * NL + iI) * ld_q + t + k], qq = q[(int64_t)(p * 2 * NL + NL + iQ) * ld_q + t + k];
+                    acc[p] += log2((double)fmaxf(qi, 1e-30f)) + log2((double)fmaxf(qq, 1e-30f));
+                }
             }
         }
     }
@@ -375,6 +399,40 @@ __global__ void k_gmi_fin(const double *sums, int nparts, const float *P, int n_
         double H = 0.0;
         for (int l = 0; l < n_lev; ++l) H -= 2.0 * (double)P[l] * log2((double)P[l]);
         gmi_out[threadIdx.x] = (float)(H + s[threadIdx.x] / (double)N);
+    }
+}
+
+// Bit LLRs of R runs: q (R, 2, 2n, N) -> llr (R, 2, 2m, N), rows [I bits MSB..LSB | Q bits MSB..LSB] per pol,
+// L = ln max(q(b = 0 | y), 1e-30) - ln max(q(b = 1 | y), 1e-30) (positive: bit 0), the bit posteriors of bits.cuh.  grid (blocks, R);
+// a thread owns V consecutive symbols (V = 4: 16-byte loads and streaming stores, as k_soft_dec_vec)
+template <int NL, int V>
+__global__ void __launch_bounds__(EV_NT) k_bit_llr(const float *__restrict__ q, int64_t ld_q, int64_t rs_q, int N, float *__restrict__ llr,
+                                                   int64_t ld_llr, int64_t rs_llr) {
+    constexpr int m = gray_bits<NL>();
+    q += (int64_t)blockIdx.y * rs_q;
+    llr += (int64_t)blockIdx.y * rs_llr;
+    for (int64_t t = ((int64_t)blockIdx.x * EV_NT + threadIdx.x) * V; t < N; t += (int64_t)gridDim.x * EV_NT * V) {
+#pragma unroll
+        for (int c = 0; c < 4; ++c) {                          // (pol, component): q rows c NL .., llr rows c m ..
+            float qv[NL][V], L[m][V];
+#pragma unroll
+            for (int l = 0; l < NL; ++l) ld_f32<V>(q + (int64_t)(c * NL + l) * ld_q + t, qv[l]);
+#pragma unroll
+            for (int k = 0; k < V; ++k) {
+                float v[NL], pb[m][2];
+#pragma unroll
+                for (int l = 0; l < NL; ++l) v[l] = qv[l][k];
+                bit_marginals<NL>(v, pb);
+#pragma unroll
+                for (int i = 0; i < m; ++i) L[i][k] = logf(fmaxf(pb[i][0], 1e-30f)) - logf(fmaxf(pb[i][1], 1e-30f));
+            }
+#pragma unroll
+            for (int i = 0; i < m; ++i) {
+                float *dst = llr + (int64_t)(c * m + i) * ld_llr + t;
+                if constexpr (V == 4) stg_stream(reinterpret_cast<float4 *>(dst), make_float4(L[i][0], L[i][1], L[i][2], L[i][3]));
+                else *dst = L[i][0];
+            }
+        }
     }
 }
 
@@ -470,8 +528,8 @@ extern "C" int vaeq_ser_constell(float *rx, int64_t ld_rx, const uint16_t *tx, i
     return VAEQ_OK;
 }
 
-extern "C" int vaeq_gmi(const float *q, int64_t ld_q, const uint16_t *tx, int64_t ld_tx, const float *P, int32_t n_lev,
-                        int32_t N, float *gmi_out, void *scratch, void *stream) {
+static int rate(const float *q, int64_t ld_q, const uint16_t *tx, int64_t ld_tx, const float *P, int32_t n_lev, int32_t N, float *gmi_out,
+                void *scratch, void *stream, bool bits) {
     VAEQ_CHECK_ARG(q && tx && P && gmi_out && scratch && N > 0, "bad gmi arguments");
     VAEQ_CHECK_ARG(n_lev == 2 || n_lev == 4 || n_lev == 8, "n_lev=%d must be 2, 4 or 8", n_lev);
     cudaStream_t st = (cudaStream_t)stream;
@@ -479,10 +537,13 @@ extern "C" int vaeq_gmi(const float *q, int64_t ld_q, const uint16_t *tx, int64_
     const bool vec = ev_vec_ok(q, ld_q, tx, ld_tx, N);
     const int grid = ev_grid(N, vec ? 4 : 1);
     ktime_begin(VAEQ_K_EVAL, st);
-#define EV_CASE(NL_)                                                                        \
-    if (vec) k_gmi<NL_, 4><<<grid, EV_NT, 0, st>>>(q, ld_q, tx, ld_tx, N, sums);            \
-    else k_gmi<NL_, 1><<<grid, EV_NT, 0, st>>>(q, ld_q, tx, ld_tx, N, sums);
-    if (n_lev == 2) { EV_CASE(2) } else if (n_lev == 4) { EV_CASE(4) } else { EV_CASE(8) }
+#define EV_CASE(NL_, B_)                                                                    \
+    if (vec) k_gmi<NL_, 4, B_><<<grid, EV_NT, 0, st>>>(q, ld_q, tx, ld_tx, N, sums);        \
+    else k_gmi<NL_, 1, B_><<<grid, EV_NT, 0, st>>>(q, ld_q, tx, ld_tx, N, sums);
+#define EV_LEV(B_)                                                                          \
+    if (n_lev == 2) { EV_CASE(2, B_) } else if (n_lev == 4) { EV_CASE(4, B_) } else { EV_CASE(8, B_) }
+    if (bits) { EV_LEV(true) } else { EV_LEV(false) }
+#undef EV_LEV
 #undef EV_CASE
     ktime_end(VAEQ_K_EVAL, st);
     VAEQ_LAUNCH_CHECK("k_gmi");
@@ -490,5 +551,40 @@ extern "C" int vaeq_gmi(const float *q, int64_t ld_q, const uint16_t *tx, int64_
     k_gmi_fin<<<1, 32, 0, st>>>(sums, grid, P, n_lev, N, gmi_out);
     ktime_end(VAEQ_K_EVAL, st);
     VAEQ_LAUNCH_CHECK("k_gmi_fin");
+    return VAEQ_OK;
+}
+
+extern "C" int vaeq_gmi(const float *q, int64_t ld_q, const uint16_t *tx, int64_t ld_tx, const float *P, int32_t n_lev,
+                        int32_t N, float *gmi_out, void *scratch, void *stream) {
+    return rate(q, ld_q, tx, ld_tx, P, n_lev, N, gmi_out, scratch, stream, false);
+}
+
+extern "C" int vaeq_bmi(const float *q, int64_t ld_q, const uint16_t *tx, int64_t ld_tx, const float *P, int32_t n_lev,
+                        int32_t N, float *bmi_out, void *scratch, void *stream) {
+    return rate(q, ld_q, tx, ld_tx, P, n_lev, N, bmi_out, scratch, stream, true);
+}
+
+extern "C" int vaeq_bit_llr_runs(const float *q, int64_t ld_q, int64_t rs_q, int32_t n_lev, int32_t N, int32_t n_runs, float *llr,
+                                 int64_t ld_llr, int64_t rs_llr, void *stream) {
+    VAEQ_CHECK_ARG(q && llr, "NULL pointer");
+    VAEQ_CHECK_ARG(n_lev == 2 || n_lev == 4 || n_lev == 8, "n_lev=%d must be 2, 4 or 8", n_lev);
+    VAEQ_CHECK_ARG(N > 0, "N=%d must be positive", N);
+    VAEQ_CHECK_ARG(n_runs > 0 && n_runs <= 65535, "n_runs=%d must be in 1..65535", n_runs);
+    const int m = n_lev == 2 ? 1 : n_lev == 4 ? 2 : 3;
+    VAEQ_CHECK_ARG(ld_llr >= N && (n_runs == 1 || rs_llr >= 4 * m * ld_llr), "llr strides (ld_llr=%lld, rs_llr=%lld) overlap rows of N=%d",
+                   (long long)ld_llr, (long long)rs_llr, N);
+    cudaStream_t st = (cudaStream_t)stream;
+    const bool vec = (N % 4 == 0) && (ld_q % 4 == 0) && (rs_q % 4 == 0) && (ld_llr % 4 == 0) && (rs_llr % 4 == 0) &&
+                     ((reinterpret_cast<uintptr_t>(q) | reinterpret_cast<uintptr_t>(llr)) % 16 == 0);
+    const int V = vec ? 4 : 1;
+    const dim3 grid(max(1, min((N / V + EV_NT - 1) / EV_NT, max(1, sm_count() * 8 / n_runs))), n_runs);
+    ktime_begin(VAEQ_K_EVAL, st);
+#define EV_CASE(NL_)                                                                                              \
+    if (vec) k_bit_llr<NL_, 4><<<grid, EV_NT, 0, st>>>(q, ld_q, rs_q, N, llr, ld_llr, rs_llr);                    \
+    else k_bit_llr<NL_, 1><<<grid, EV_NT, 0, st>>>(q, ld_q, rs_q, N, llr, ld_llr, rs_llr);
+    if (n_lev == 2) { EV_CASE(2) } else if (n_lev == 4) { EV_CASE(4) } else { EV_CASE(8) }
+#undef EV_CASE
+    ktime_end(VAEQ_K_EVAL, st);
+    VAEQ_LAUNCH_CHECK("k_bit_llr");
     return VAEQ_OK;
 }

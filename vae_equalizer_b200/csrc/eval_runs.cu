@@ -9,6 +9,7 @@
 // launches and two syncs per run.  The arithmetic per element is that of eval.cu (same decisions, same counts).
 #include "common.cuh"
 #include "shift_corr.cuh"
+#include "bits.cuh"
 
 namespace vaeq {
 
@@ -456,8 +457,10 @@ __device__ __forceinline__ void gmi_geometry(const GmiRunsK &p, int run, int (&s
 }
 
 // grid (max_chunks, R): CTA c sums log2 q of the chosen hypothesis over evaluated symbols [c GMI_CHUNK, (c + 1) GMI_CHUNK) per pol.
-// NPOL = 2: the DP drivers (pol swap, circular shift, minibatch cut); NPOL = 1: the AWGN driver (one pol, no flip, no wrap)
-template <int NL, int NPOL>
+// NPOL = 2: the DP drivers (pol swap, circular shift, minibatch cut); NPOL = 1: the AWGN driver (one pol, no flip, no wrap).
+// BITS: the bit-metric rate (BMI) instead: per component the m bit posteriors of the q level the hypothesis maps the tx level onto
+// (bits.cuh), from all NL rows of that component, which every thread reads at its own symbol (coalesced, unlike GMI's level-indexed rows)
+template <int NL, int NPOL, bool BITS>
 __global__ void __launch_bounds__(ER_NT) k_gmi_runs(GmiRunsK p) {
     __shared__ double red[2 * 32];
     const int run = blockIdx.y, N = p.N;
@@ -486,8 +489,18 @@ __global__ void __launch_bounds__(ER_NT) k_gmi_runs(GmiRunsK p) {
             const int iI = k == 0 ? DI : k == 1 ? S - DI : k == 2 ? DQp : S - DQp;
             const int iQ = k == 0 ? DQp : k == 1 ? S - DQp : k == 2 ? S - DI : DI;
             const float *qp = q + (int64_t)(sp * 2 * NL) * p.ld_q + ts;
-            const float qI = qp[(int64_t)iI * p.ld_q], qQ = qp[(int64_t)(NL + iQ) * p.ld_q];
-            acc[pol] += log2((double)fmaxf(qI, 1e-30f)) + log2((double)fmaxf(qQ, 1e-30f));
+            if constexpr (BITS) {
+                float qI[NL], qQ[NL];
+#pragma unroll
+                for (int l = 0; l < NL; ++l) {
+                    qI[l] = qp[(int64_t)l * p.ld_q];
+                    qQ[l] = qp[(int64_t)(NL + l) * p.ld_q];
+                }
+                acc[pol] += bmi_log2_component<NL>(qI, iI) + bmi_log2_component<NL>(qQ, iQ);
+            } else {
+                const float qI = qp[(int64_t)iI * p.ld_q], qQ = qp[(int64_t)(NL + iQ) * p.ld_q];
+                acc[pol] += log2((double)fmaxf(qI, 1e-30f)) + log2((double)fmaxf(qQ, 1e-30f));
+            }
         }
     }
     block_sum<2>(acc, red);
@@ -516,13 +529,17 @@ __global__ void k_gmi_runs_fin(GmiRunsK p, int n_lev) {
     p.gmi[idx] = n_eval > 0 ? (float)(H + s / (double)n_eval) : __int_as_float(0x7fc00000);
 }
 
-static int gmi_runs_launch(GmiRunsK &p, int n_lev, int npol, cudaStream_t st) {
+// bits: BMI instead of GMI (same geometry, hypothesis, chunks and finish)
+static int gmi_runs_launch(GmiRunsK &p, int n_lev, int npol, bool bits, cudaStream_t st) {
     const dim3 grid(p.max_chunks, p.n_runs);
     ktime_begin(VAEQ_K_EVAL, st);
-#define GMI_CASE(NL_)                                                                                  \
-    if (npol == 2) k_gmi_runs<NL_, 2><<<grid, ER_NT, 0, st>>>(p);                                      \
-    else k_gmi_runs<NL_, 1><<<grid, ER_NT, 0, st>>>(p);
-    if (n_lev == 2) { GMI_CASE(2) } else if (n_lev == 4) { GMI_CASE(4) } else { GMI_CASE(8) }
+#define GMI_CASE(NL_, B_)                                                                              \
+    if (npol == 2) k_gmi_runs<NL_, 2, B_><<<grid, ER_NT, 0, st>>>(p);                                  \
+    else k_gmi_runs<NL_, 1, B_><<<grid, ER_NT, 0, st>>>(p);
+#define GMI_LEV(B_)                                                                                    \
+    if (n_lev == 2) { GMI_CASE(2, B_) } else if (n_lev == 4) { GMI_CASE(4, B_) } else { GMI_CASE(8, B_) }
+    if (bits) { GMI_LEV(true) } else { GMI_LEV(false) }
+#undef GMI_LEV
 #undef GMI_CASE
     ktime_end(VAEQ_K_EVAL, st);
     VAEQ_LAUNCH_CHECK("k_gmi_runs");
@@ -548,9 +565,9 @@ extern "C" size_t vaeq_frame_gmi_scratch_bytes(int32_t n_runs, int32_t N) {
 
 extern "C" size_t vaeq_awgn_gmi_scratch_bytes(int32_t n_runs, int32_t N) { return vaeq_frame_gmi_scratch_bytes(n_runs, N); }
 
-extern "C" int vaeq_frame_gmi_runs(const float *q, int64_t ld_q, int64_t rs_q, const uint16_t *tx, int64_t ld_tx, int64_t rs_tx, const float *P,
-                                   int64_t rs_P, const int32_t *align, const int32_t *counts, int32_t n_lev, int32_t N, int32_t n_runs,
-                                   int32_t seg_len, int32_t edge, int32_t n_cut, float *gmi_out, void *scratch, void *stream) {
+static int frame_rate_runs(const float *q, int64_t ld_q, int64_t rs_q, const uint16_t *tx, int64_t ld_tx, int64_t rs_tx, const float *P,
+                           int64_t rs_P, const int32_t *align, const int32_t *counts, int32_t n_lev, int32_t N, int32_t n_runs, int32_t seg_len,
+                           int32_t edge, int32_t n_cut, float *gmi_out, void *scratch, void *stream, bool bits) {
     VAEQ_CHECK_ARG(q && tx && P && align && counts && gmi_out && scratch, "NULL pointer");
     VAEQ_CHECK_ARG(n_lev == 2 || n_lev == 4 || n_lev == 8, "n_lev=%d must be 2, 4 or 8", n_lev);
     VAEQ_CHECK_ARG(N > 0 && edge >= 0 && n_cut >= 0, "bad sizes (N=%d, edge=%d, n_cut=%d)", N, edge, n_cut);
@@ -560,12 +577,26 @@ extern "C" int vaeq_frame_gmi_runs(const float *q, int64_t ld_q, int64_t rs_q, c
     p.q = q; p.ld_q = ld_q; p.rs_q = rs_q; p.tx = tx; p.ld_tx = ld_tx; p.rs_tx = rs_tx; p.P = P; p.rs_P = rs_P;
     p.align = align; p.counts = counts; p.N = N; p.seg_len = seg_len; p.edge = edge; p.n_cut = n_cut; p.n_runs = n_runs;
     p.max_chunks = gmi_max_chunks(N); p.part = static_cast<double *>(scratch); p.gmi = gmi_out;
-    return gmi_runs_launch(p, n_lev, 2, (cudaStream_t)stream);
+    return gmi_runs_launch(p, n_lev, 2, bits, (cudaStream_t)stream);
 }
 
-extern "C" int vaeq_awgn_gmi_runs(const float *q, int64_t ld_q, int64_t rs_q, const uint16_t *tx, int64_t ld_tx, int64_t rs_tx, const float *P,
-                                  int64_t rs_P, const int32_t *shift, const int32_t *counts, int32_t n_lev, int32_t N, int32_t n_runs, int32_t edge,
-                                  float *gmi_out, void *scratch, void *stream) {
+extern "C" int vaeq_frame_gmi_runs(const float *q, int64_t ld_q, int64_t rs_q, const uint16_t *tx, int64_t ld_tx, int64_t rs_tx, const float *P,
+                                   int64_t rs_P, const int32_t *align, const int32_t *counts, int32_t n_lev, int32_t N, int32_t n_runs,
+                                   int32_t seg_len, int32_t edge, int32_t n_cut, float *gmi_out, void *scratch, void *stream) {
+    return frame_rate_runs(q, ld_q, rs_q, tx, ld_tx, rs_tx, P, rs_P, align, counts, n_lev, N, n_runs, seg_len, edge, n_cut, gmi_out, scratch,
+                           stream, false);
+}
+
+extern "C" int vaeq_frame_bmi_runs(const float *q, int64_t ld_q, int64_t rs_q, const uint16_t *tx, int64_t ld_tx, int64_t rs_tx, const float *P,
+                                   int64_t rs_P, const int32_t *align, const int32_t *counts, int32_t n_lev, int32_t N, int32_t n_runs,
+                                   int32_t seg_len, int32_t edge, int32_t n_cut, float *bmi_out, void *scratch, void *stream) {
+    return frame_rate_runs(q, ld_q, rs_q, tx, ld_tx, rs_tx, P, rs_P, align, counts, n_lev, N, n_runs, seg_len, edge, n_cut, bmi_out, scratch,
+                           stream, true);
+}
+
+static int awgn_rate_runs(const float *q, int64_t ld_q, int64_t rs_q, const uint16_t *tx, int64_t ld_tx, int64_t rs_tx, const float *P,
+                          int64_t rs_P, const int32_t *shift, const int32_t *counts, int32_t n_lev, int32_t N, int32_t n_runs, int32_t edge,
+                          float *gmi_out, void *scratch, void *stream, bool bits) {
     VAEQ_CHECK_ARG(q && tx && P && shift && counts && gmi_out && scratch, "NULL pointer");
     VAEQ_CHECK_ARG(n_lev == 2 || n_lev == 4 || n_lev == 8, "n_lev=%d must be 2, 4 or 8", n_lev);
     VAEQ_CHECK_ARG(N > 0 && edge >= 0 && N - 2 * edge > 0, "N=%d leaves no symbol to evaluate with edge=%d", N, edge);
@@ -574,7 +605,19 @@ extern "C" int vaeq_awgn_gmi_runs(const float *q, int64_t ld_q, int64_t rs_q, co
     p.q = q; p.ld_q = ld_q; p.rs_q = rs_q; p.tx = tx; p.ld_tx = ld_tx; p.rs_tx = rs_tx; p.P = P; p.rs_P = rs_P;
     p.align = shift; p.counts = counts; p.N = N; p.seg_len = 0; p.edge = edge; p.n_cut = 0; p.n_runs = n_runs;
     p.max_chunks = gmi_max_chunks(N); p.part = static_cast<double *>(scratch); p.gmi = gmi_out;
-    return gmi_runs_launch(p, n_lev, 1, (cudaStream_t)stream);
+    return gmi_runs_launch(p, n_lev, 1, bits, (cudaStream_t)stream);
+}
+
+extern "C" int vaeq_awgn_gmi_runs(const float *q, int64_t ld_q, int64_t rs_q, const uint16_t *tx, int64_t ld_tx, int64_t rs_tx, const float *P,
+                                  int64_t rs_P, const int32_t *shift, const int32_t *counts, int32_t n_lev, int32_t N, int32_t n_runs, int32_t edge,
+                                  float *gmi_out, void *scratch, void *stream) {
+    return awgn_rate_runs(q, ld_q, rs_q, tx, ld_tx, rs_tx, P, rs_P, shift, counts, n_lev, N, n_runs, edge, gmi_out, scratch, stream, false);
+}
+
+extern "C" int vaeq_awgn_bmi_runs(const float *q, int64_t ld_q, int64_t rs_q, const uint16_t *tx, int64_t ld_tx, int64_t rs_tx, const float *P,
+                                  int64_t rs_P, const int32_t *shift, const int32_t *counts, int32_t n_lev, int32_t N, int32_t n_runs, int32_t edge,
+                                  float *bmi_out, void *scratch, void *stream) {
+    return awgn_rate_runs(q, ld_q, rs_q, tx, ld_tx, rs_tx, P, rs_P, shift, counts, n_lev, N, n_runs, edge, bmi_out, scratch, stream, true);
 }
 
 extern "C" size_t vaeq_awgn_eval_scratch_bytes(int32_t n_runs, int32_t n_shift, int32_t n_corr) {

@@ -357,12 +357,24 @@ def _run_pmf(P, R, n, dev):
     return Pt, int(Pt.stride(0))
 
 
-@_lib.device_guard
 def gmi_runs(q, tx, P, align, counts, seg_len, edge=11, n_cut=10):
     """EXTENSION (not in the reference): GMI = H(X) + mean log2 q(x_tx|y) per pol (bit/2D-symbol) of R runs, scored on exactly the symbols
     and under the (IQ flip, rotation) hypothesis of the soft-demapper SER of frame_eval_runs: q (R,2,2n,N) and tx (R,2,2,N) float16 as
     given to frame_eval_runs, P (R,n) or (n,) pmf, align (R,2,4) and counts (R,2,2,2,4) from frame_eval_runs(..., return_counts=True)
     with the same seg_len / edge / n_cut.  Returns (R,2) float32 on the device, NaN where no symbol was evaluated; no host sync."""
+    return _rate_runs("vaeq_frame_gmi_runs", q, tx, P, align, counts, seg_len, edge, n_cut)
+
+
+def bmi_runs(q, tx, P, align, counts, seg_len, edge=11, n_cut=10):
+    """EXTENSION (not in the reference): the bit-metric decoding rate of Gray-labelled bits (BMI, DESIGN.md §2) per pol (bit/2D-symbol)
+    of R runs: H(X) + mean over the symbols of sum over the I and Q bits of log2 q(b_i = tx's bit | y), with the bit posteriors summed
+    from q.  Arguments, symbols, hypothesis and result exactly as gmi_runs."""
+    return _rate_runs("vaeq_frame_bmi_runs", q, tx, P, align, counts, seg_len, edge, n_cut)
+
+
+@_lib.device_guard
+def _rate_runs(fn, q, tx, P, align, counts, seg_len, edge, n_cut):
+    """gmi_runs / bmi_runs through the C entry `fn` (vaeq_frame_gmi_runs or vaeq_frame_bmi_runs: same arguments)."""
     _require_cuda(q, "q")
     tx = _tx_bits(tx)
     lib = _lib.load()
@@ -376,12 +388,12 @@ def gmi_runs(q, tx, P, align, counts, seg_len, edge=11, n_cut=10):
         if not torch.is_tensor(t) or t.dtype != torch.int32 or tuple(t.shape) != shape or not t.is_contiguous() or t.device != dev:
             raise _lib.VaeqError(f"{name}: need a contiguous int32 {shape} tensor on {dev} (frame_eval_runs(..., return_counts=True))")
     Pt, rs_P = _run_pmf(P, R, n, dev)
-    gmi = torch.empty(R, 2, dtype=_F32, device=dev)
+    rate = torch.empty(R, 2, dtype=_F32, device=dev)
     scr = _scratch(dev, max(1, int(lib.vaeq_frame_gmi_scratch_bytes(R, N))))
-    _lib.check(lib.vaeq_frame_gmi_runs(q.data_ptr(), int(q.stride(2)), int(q.stride(0)), tx.data_ptr(), int(tx.stride(2)), int(tx.stride(0)),
-                                       Pt.data_ptr(), rs_P, align.data_ptr(), counts.data_ptr(), n, N, R, int(seg_len), int(edge), int(n_cut),
-                                       gmi.data_ptr(), scr.data_ptr(), _lib.current_stream()), "vaeq_frame_gmi_runs")
-    return gmi
+    _lib.check(getattr(lib, fn)(q.data_ptr(), int(q.stride(2)), int(q.stride(0)), tx.data_ptr(), int(tx.stride(2)), int(tx.stride(0)),
+                                Pt.data_ptr(), rs_P, align.data_ptr(), counts.data_ptr(), n, N, R, int(seg_len), int(edge), int(n_cut),
+                                rate.data_ptr(), scr.data_ptr(), _lib.current_stream()), fn)
+    return rate
 
 
 @_lib.device_guard
@@ -415,18 +427,49 @@ def cma_align_rescale(out, align, scale, edge=11):
     return oc
 
 
-@_lib.device_guard
 def GMI(q, tx, P):
     """EXTENSION (not in the reference, SURVEY.md fact 3): H(X) + E[log2 q(x_tx|y)] per pol, bit/2D-symbol."""
+    return _rate("vaeq_gmi", q, tx, P)
+
+
+def BMI(q, tx, P):
+    """EXTENSION (not in the reference): the bit-metric decoding rate of Gray-labelled bits (DESIGN.md §2) per pol, bit/2D-symbol:
+    H(X) + E[sum over the I and Q bits of log2 q(b_i = tx's bit | y)].  Arguments and result as GMI."""
+    return _rate("vaeq_bmi", q, tx, P)
+
+
+@_lib.device_guard
+def _rate(fn, q, tx, P):
     _require_cuda(q, "q")
     lib = _lib.load()
     n, N = q.shape[1] // 2, int(q.shape[-1])
     Pt = torch.as_tensor(P, dtype=_F32, device=q.device).contiguous()
     out = torch.empty(2, dtype=_F32, device=q.device)
     scr = _scratch(q.device)
-    _lib.check(lib.vaeq_gmi(q.data_ptr(), _rows(q, "q"), _tx_bits(tx).data_ptr(), _rows(tx, "tx"), Pt.data_ptr(), n, N,
-                            out.data_ptr(), scr.data_ptr(), _lib.current_stream()), "vaeq_gmi")
+    _lib.check(getattr(lib, fn)(q.data_ptr(), _rows(q, "q"), _tx_bits(tx).data_ptr(), _rows(tx, "tx"), Pt.data_ptr(), n, N,
+                                out.data_ptr(), scr.data_ptr(), _lib.current_stream()), fn)
     return out
+
+
+@_lib.device_guard
+def bit_llr(q):
+    """EXTENSION (not in the reference): Gray-labelled bit LLRs of the posteriors (DESIGN.md §2), the soft input of a binary decoder.
+    q (2,2n,N) or (R,2,2n,N) float32 with unit time stride and evenly strided rows (views allowed) -> (2,2m,N) or (R,2,2m,N) float32,
+    m = log2(n), rows [I bits MSB..LSB | Q bits MSB..LSB] per pol; L = ln q(b=0|y) - ln q(b=1|y), each clamped at 1e-30 (positive: bit 0).
+    One launch, no host sync."""
+    _require_cuda(q, "q")
+    single = q.dim() == 3
+    q4 = q.unsqueeze(0) if single else q
+    if q4.dim() != 4 or q4.shape[1] != 2 or q4.shape[2] not in (4, 8, 16) or q4.stride(3) != 1 or q4.stride(1) != q4.shape[2] * q4.stride(2):
+        raise _lib.VaeqError(f"q: need (2,2n,N) or (R,2,2n,N), n in 2/4/8, with unit time stride and evenly strided rows, got "
+                             f"{tuple(q.shape)} {q.stride()}")
+    lib = _lib.load()
+    R, n, N = int(q4.shape[0]), int(q4.shape[2]) // 2, int(q4.shape[3])
+    m = n.bit_length() - 1
+    llr = torch.empty(R, 2, 2 * m, N, dtype=_F32, device=q.device)
+    _lib.check(lib.vaeq_bit_llr_runs(q4.data_ptr(), int(q4.stride(2)), int(q4.stride(0)) if R > 1 else 4 * n * int(q4.stride(2)), n, N, R,
+                                     llr.data_ptr(), N, 4 * m * N, _lib.current_stream()), "vaeq_bit_llr_runs")
+    return llr[0] if single else llr
 
 
 # -------------------------------------------------------------------------------------------------

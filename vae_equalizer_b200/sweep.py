@@ -32,7 +32,7 @@ def _cell(c, key):
 
 def sweep_vae_dp(cells, mod, sps, M_est, batch_len, N_frame_max, num_frames, flex_step=None, channel="h0", symb_rate=90e9,
                  tau_cd=-26e-24, tau_pmd=0.1e-12 * np.sqrt(1000), phiIQ=(0.0314, 0.0314), N_lrhalf=None, *, kind="VAE",
-                 device=None, datagen="gpu", eval_every=1, eval_mode="batched", verbose=False, gmi=False):
+                 device=None, datagen="gpu", eval_every=1, eval_mode="batched", verbose=False, gmi=False, bmi=False):
     """Train and score R = len(cells) independent runs in lockstep.
 
     cells: list of dicts with per-cell values: SNR, nu, lr_optim, theta, theta_diff, and optionally seed.
@@ -44,9 +44,11 @@ def sweep_vae_dp(cells, mod, sps, M_est, batch_len, N_frame_max, num_frames, fle
     kind: "VAE" (func_VAELE_DP_MQAM_shaping.py: non-overlapping minibatches) or "VAEflex" (func_VAEflex_DP_MQAM_shaping.py:
     window batch_len advanced by flex_step).  eval_every: score every k-th frame (and the last); unscored frames hold NaN.
     gmi: also score GMI (shared_funcs.gmi_runs: the soft-demapper SER's symbols and hypothesis; eval_mode="batched" only).
-    Returns (SER_valid (R,4,num_frames), Var_est (R,2,num_frames), var (R,2)), and GMI (R,2,num_frames) as a 4th tensor with gmi=True
-    (NaN on unscored frames)."""
-    _gmi_batched_only(gmi, eval_mode)
+    bmi: also score the bit-metric rate of Gray-labelled bits (shared_funcs.bmi_runs: the same symbols and hypothesis; batched only).
+    Returns (SER_valid (R,4,num_frames), Var_est (R,2,num_frames), var (R,2)), then GMI with gmi=True and BMI with bmi=True, each
+    (R,2,num_frames) with NaN on unscored frames, in that order."""
+    metrics = _metrics(gmi, bmi)
+    _rates_batched_only(metrics, eval_mode)
     _check_dp_batch_len(mod, M_est, batch_len)
     device = _cuda_device(device)
     R = len(cells)
@@ -92,8 +94,8 @@ def sweep_vae_dp(cells, mod, sps, M_est, batch_len, N_frame_max, num_frames, fle
 
     SER_valid = torch.full((R, 4, num_frames), float("nan"), device=device, dtype=torch.float32)
     Var_est = torch.empty(R, pol, num_frames, device=device, dtype=torch.float32)
-    GMI = torch.full((R, pol, num_frames), float("nan"), device=device, dtype=torch.float32) if gmi else None
-    P_gmi = P_all.to(device) if gmi else None
+    rates = {m: torch.full((R, pol, num_frames), float("nan"), device=device, dtype=torch.float32) for m in metrics}
+    P_rate = P_all.to(device) if metrics else None
     rx_all = None if datagen == "gpu_batched" else torch.empty(R, 2, 2, sps * N_frame, device=device, dtype=torch.float32)
     out_train = torch.empty(R, pol, 2 * num_lev, N_keep, device=device, dtype=torch.float32)
     out_const = torch.empty(R, pol, 2, N_keep, device=device, dtype=torch.float32)
@@ -137,8 +139,8 @@ def sweep_vae_dp(cells, mod, sps, M_est, batch_len, N_frame_max, num_frames, fle
             ser, al, counts = sfun.frame_eval_runs(out_train, out_const, tx_b4, amp_dev, var_dev, nu_dev, seg_len, n_cut=N_CUT,
                                                    return_counts=True)
             SER_valid[:, :, frame] = ser
-            if gmi:
-                GMI[:, :, frame] = sfun.gmi_runs(out_train, tx_b4, P_gmi, al, counts, seg_len, n_cut=N_CUT)
+            for m in metrics:                                            # shared_funcs.gmi_runs / bmi_runs
+                rates[m][:, :, frame] = getattr(sfun, f"{m}_runs")(out_train, tx_b4, P_rate, al, counts, seg_len, n_cut=N_CUT)
             if verbose:
                 print(frame, "loss", loss_steps[:, -1].tolist(), "SER", SER_valid[:, :, frame].tolist())
             continue
@@ -156,9 +158,7 @@ def sweep_vae_dp(cells, mod, sps, M_est, batch_len, N_frame_max, num_frames, fle
         if verbose:
             snr_db = 10 * torch.log10(torch.tensor(pow_mean, device=device) / var_steps.mean(dim=(1, 2)))
             print(frame, "loss", loss_steps[:, -1].tolist(), "SNR_est", snr_db.tolist(), "SER", SER_valid[:, :, frame].tolist())
-    if gmi:
-        return SER_valid, Var_est, var_all.to(device), GMI
-    return SER_valid, Var_est, var_all.to(device)
+    return (SER_valid, Var_est, var_all.to(device)) + tuple(rates[m] for m in metrics)
 
 
 def _check_dp_batch_len(mod, M_est, batch_len):
@@ -171,15 +171,24 @@ def _check_dp_batch_len(mod, M_est, batch_len):
                                   f"{mod}: {lim}")
 
 
-def _gmi_batched_only(gmi, eval_mode):
-    if gmi and eval_mode != "batched":
-        raise ValueError(f"gmi=True needs eval_mode='batched' (GMI is scored from the batched evaluation's alignment and counts), got "
-                         f"{eval_mode!r}")
+RATE_METRICS = ("gmi", "bmi")          # the engines' optional rate results, appended after their base results in this order
+
+
+def _metrics(gmi=False, bmi=False, **_):
+    """The rate metrics switched on, in RATE_METRICS order (also takes an engine's keyword dict)."""
+    on = dict(gmi=gmi, bmi=bmi)
+    return [m for m in RATE_METRICS if on[m]]
+
+
+def _rates_batched_only(metrics, eval_mode):
+    if metrics and eval_mode != "batched":
+        raise ValueError(f"{metrics[0]}=True needs eval_mode='batched' (rates are scored from the batched evaluation's alignment and counts), "
+                         f"got {eval_mode!r}")
 
 
 def sweep_cma_dp(cells, mod, sps, M_est, batch_len, N_train_max, num_frames, flex_step=None, channel="h0", symb_rate=90e9,
                  tau_cd=-26e-24, tau_pmd=0.1e-12 * np.sqrt(1000), phiIQ=(0.0314, 0.0314), N_lrhalf=None, *, kind="CMA", device=None,
-                 datagen="gpu", eval_mode="batched", verbose=False, gmi=False):
+                 datagen="gpu", eval_mode="batched", verbose=False, gmi=False, bmi=False):
     """The CMA / CMAbatch / CMAflex drivers (func_CMA_DP_MQAM_shaping.py:16-56 and siblings) for R = len(cells) independent cells
     in lockstep.  The tap recurrence of a cell is sequential in the symbols, but cells are independent: per frame ONE equalizer
     launch sequence covers all cells that share lr_optim (vaeq_cma n_runs: one warp / one CTA per cell) and ONE batched CPE
@@ -187,10 +196,13 @@ def sweep_cma_dp(cells, mod, sps, M_est, batch_len, N_train_max, num_frames, fle
     aligned, partially rescaled copy -> soft_dec -> estimator from q, 4 calls and no host sync for all cells) or replays the single-run
     drivers' call sequence per cell (eval_mode="per_cell", two host syncs per frame); both give the same error counts.  A cell gives the same SER alone (processing_cma*_dp) or in any batch when
     datagen="gpu" (its data depends on its own seed only); datagen="gpu_batched" generates all cells in one call (fastest).
-    gmi: also score GMI of the soft-demapper posteriors q the SER is taken from (shared_funcs.gmi_runs; eval_mode="batched" only).
-    Returns (SER_valid (R,4,num_frames), Var_est zeros (R,2,num_frames), var (R,2)), and GMI (R,2,num_frames) as a 4th tensor with gmi=True."""
+    gmi / bmi: also score GMI / the bit-metric rate of the soft-demapper posteriors q the SER is taken from (shared_funcs.gmi_runs /
+    bmi_runs; eval_mode="batched" only).
+    Returns (SER_valid (R,4,num_frames), Var_est zeros (R,2,num_frames), var (R,2)), then GMI with gmi=True and BMI with bmi=True, each
+    (R,2,num_frames), in that order."""
     from .processing import _make_frame
-    _gmi_batched_only(gmi, eval_mode)
+    metrics = _metrics(gmi, bmi)
+    _rates_batched_only(metrics, eval_mode)
     device = _cuda_device(device)
     R = len(cells)
     if R == 0:
@@ -218,8 +230,8 @@ def sweep_cma_dp(cells, mod, sps, M_est, batch_len, N_train_max, num_frames, fle
     Var_est = torch.zeros(R, pol, num_frames, device=device, dtype=torch.float32)
     var_all = torch.stack([k[7].to(device, torch.float32) for k in consts])
     nu_all = torch.tensor([float(k[6]) for k in consts], dtype=torch.float32, device=device)
-    GMI = torch.full((R, pol, num_frames), float("nan"), device=device, dtype=torch.float32) if gmi else None
-    P_gmi = torch.stack([torch.as_tensor(k[2], dtype=torch.float32) for k in consts]).to(device) if gmi else None
+    rates = {m: torch.full((R, pol, num_frames), float("nan"), device=device, dtype=torch.float32) for m in metrics}
+    P_rate = torch.stack([torch.as_tensor(k[2], dtype=torch.float32) for k in consts]).to(device) if metrics else None
     lr_scale = 1.0
     for frame in range(num_frames):
         if frame % N_lrhalf == 0 and frame != 0:
@@ -261,8 +273,8 @@ def sweep_cma_dp(cells, mod, sps, M_est, batch_len, N_train_max, num_frames, fle
             ser_q, al_q, counts_q = sfun.frame_eval_runs(q_all, None, tx_c, amp_levels, var_all, nu_all, 0, which=1, return_counts=True)  # CMA_DP:49-52
             SER_valid[:, :2, frame] = ser_c[:, :2]
             SER_valid[:, 2:, frame] = ser_q[:, 2:]
-            if gmi:
-                GMI[:, :, frame] = sfun.gmi_runs(q_all, tx_c, P_gmi, al_q, counts_q, 0)
+            for m in metrics:                                            # shared_funcs.gmi_runs / bmi_runs
+                rates[m][:, :, frame] = getattr(sfun, f"{m}_runs")(q_all, tx_c, P_rate, al_q, counts_q, 0)
             if verbose:
                 print(frame, "SER", SER_valid[:, :, frame].tolist())
             continue
@@ -287,9 +299,7 @@ def sweep_cma_dp(cells, mod, sps, M_est, batch_len, N_train_max, num_frames, fle
             SER_valid[r, 2:, frame] = sfun.SER_IQflip(qa[:, :, 11:-tail], tx_c[r][:, :, 11:-tail])
         if verbose:
             print(frame, "SER", SER_valid[:, :, frame].tolist())
-    if gmi:
-        return SER_valid, Var_est, var_all, GMI
-    return SER_valid, Var_est, var_all
+    return (SER_valid, Var_est, var_all) + tuple(rates[m] for m in metrics)
 
 
 def _score(kind, what, aligned, tx, sh, batch_len, m_max, pol, num_lev, amp_levels, const):
@@ -310,12 +320,13 @@ def _score(kind, what, aligned, tx, sh, batch_len, m_max, pol, num_lev, amp_leve
 
 def sweep_vae_dp_sharded(cells, *args, rank=0, world=1, group=None, **kw):
     """Round-robin the cells over the ranks (one process per GPU), run each share as one batched run set, and reassemble
-    (SER_valid, Var_est, var) -- plus GMI with gmi=True -- for ALL cells on rank 0 (None elsewhere).  No data-path collective."""
+    (SER_valid, Var_est, var) -- plus GMI with gmi=True, then BMI with bmi=True -- for ALL cells on rank 0 (None elsewhere).  No data-path
+    collective."""
     from .parallel import gather_cell_results, shard_cells
     mine = shard_cells(cells, rank, world)
     num_frames = args[5] if len(args) > 5 else kw["num_frames"]
     dev = _cuda_device(kw.get("device"))
-    gmi = kw.get("gmi", False)
+    metrics = _metrics(**kw)
     if mine:
         res = sweep_vae_dp([c for _, c in mine], *args, **kw)
         ser, ve, var = res[:3]
@@ -327,19 +338,18 @@ def sweep_vae_dp_sharded(cells, *args, rank=0, world=1, group=None, **kw):
     ser_g = gather_cell_results({i: torch.nan_to_num(t, nan=-1.0) for i, t in loc_ser.items()}, n, (4, num_frames), rank, world, group, dev)
     ve_g = gather_cell_results(loc_ve, n, (2, num_frames), rank, world, group, dev)
     var_g = gather_cell_results(loc_var, n, (2,), rank, world, group, dev)
-    if gmi:                                                          # a collective: every rank takes part, before any rank returns
-        loc_g = {i: res[3][k] for k, (i, _) in enumerate(mine)} if mine else {}
-        gmi_g = _gather_with_nan(loc_g, n, (2, num_frames), rank, world, group, dev)
+    rates = []
+    for j, m in enumerate(metrics):                                  # collectives: every rank takes part, before any rank returns
+        loc_m = {i: res[3 + j][k] for k, (i, _) in enumerate(mine)} if mine else {}
+        rates.append(_gather_with_nan(loc_m, n, (2, num_frames), rank, world, group, dev))
     if rank != 0:
         return None
     ser_g = torch.where(ser_g < 0, torch.full_like(ser_g, float("nan")), ser_g)
-    if gmi:
-        return ser_g, ve_g, var_g, gmi_g
-    return ser_g, ve_g, var_g
+    return (ser_g, ve_g, var_g) + tuple(rates)
 
 
 def _gather_with_nan(local, n_cells, shape, rank, world, group, dev):
-    """parallel.gather_cell_results for values of any sign with NaN entries (GMI can be negative, so NaN cannot be carried as a negative
+    """parallel.gather_cell_results for values of any sign with NaN entries (GMI and BMI can be negative, so NaN cannot be carried as a negative
     sentinel): the values with NaN as 0 and a NaN mask travel in one block.  (n_cells, *shape) on rank 0, None elsewhere."""
     from .parallel import gather_cell_results
     packed = {i: torch.stack((torch.where(torch.isnan(t), torch.zeros_like(t), t), torch.isnan(t).to(t.dtype))) for i, t in local.items()}
@@ -359,7 +369,7 @@ def run_dp_sweep(mod="64-QAM", sps=2, loss_type="VAE", channel="h0", nu_vec=(0,)
                  theta_diff_vec=(0.06 * np.pi,), SNR_vec=(23,), M_vec=(25,), batch_len_vec=(100,), flex_step_vec=(10,),
                  lr_optim_vec=(2.5e-3, 2e-3, 3e-3), iter=5, N_lrhalf=170, num_frames=170, N_frame_max=10000,
                  tau_pmd=0.1e-12 * np.sqrt(1000), tau_cd=-26e-24, phiIQ=(0.0314, 0.0314), *, device=None, datagen="gpu_batched",
-                 eval_every=1, rank=0, world=1, group=None, runner=None, verbose=False, checkpoint_dir=None, gmi=False):
+                 eval_every=1, rank=0, world=1, group=None, runner=None, verbose=False, checkpoint_dir=None, gmi=False, bmi=False):
     """Eval_run_DP.py's ten nested loops (RUN_DP:68-95) as batched run sets.  Cells that share (M, batch_len, flex_step, symb_rate)
     train in the same persistent launch; with world > 1 every rank takes a round-robin share of each set.  Returns the
     reference's result arrays on rank 0 (None elsewhere):
@@ -369,7 +379,9 @@ def run_dp_sweep(mod="64-QAM", sps=2, loss_type="VAE", channel="h0", nu_vec=(0,)
     checkpoint_dir: rank 0 writes each finished run set there (one .npz per set, keyed by the set's parameters); a restarted sweep
     loads what it finds instead of recomputing (the reference only saves once, at the very end: RUN_DP:99-114).
     gmi=True: also GMI (2, SNR, ..., iter, num_frames), shaped like Var_est, as a 4th result (sweep_vae_dp / sweep_cma_dp with gmi=True;
-    the runner hook is then called with gmi=True).  Its checkpoints hold the GMI and are never mixed up with those of gmi=False."""
+    the runner hook is then called with gmi=True).  Its checkpoints hold the GMI and are never mixed up with those of gmi=False.
+    bmi=True: likewise the bit-metric rate of Gray-labelled bits (BMI, shaped like GMI), after GMI when both are on; the runner hook gets
+    bmi=True, the checkpoints a 'bmi' array and a signature entry of their own."""
     if runner is None and loss_type in ("VAE", "VAEflex"):
         for M in M_vec:                                              # every set's minibatch, before the first set generates data
             for batch_len in batch_len_vec:
@@ -381,8 +393,9 @@ def run_dp_sweep(mod="64-QAM", sps=2, loss_type="VAE", channel="h0", nu_vec=(0,)
     SER = torch.full((4,) + shape + (num_frames,), float("nan"), dtype=torch.float32, device=dev)
     Var_est = torch.zeros((2,) + shape + (num_frames,), dtype=torch.float32, device=dev)
     var_real = torch.zeros((2,) + shape + (1,), dtype=torch.float32, device=dev)
-    GMI = torch.full((2,) + shape + (num_frames,), float("nan"), dtype=torch.float32, device=dev) if gmi else None
-    gkw = dict(gmi=True) if gmi else {}                              # gmi=False: every call, name and signature exactly as without GMI
+    metrics = _metrics(gmi, bmi)
+    rates = {m: torch.full((2,) + shape + (num_frames,), float("nan"), dtype=torch.float32, device=dev) for m in metrics}
+    mkw = {m: True for m in metrics}                                 # a metric off: every call, name and signature exactly as without it
     groups = {}
     for idx in np.ndindex(*shape):
         c = {a: vecs[a][i] for a, i in zip(AXES, idx[:-1])}
@@ -399,47 +412,45 @@ def run_dp_sweep(mod="64-QAM", sps=2, loss_type="VAE", channel="h0", nu_vec=(0,)
             sig = _set_signature(loss_type=loss_type, mod=mod, sps=sps, channel=channel, M=M, batch_len=batch_len, flex_step=flex_step,
                                  symb_rate=symb_rate, N_frame_max=N_frame_max, num_frames=num_frames, N_lrhalf=N_lrhalf, tau_cd=tau_cd,
                                  tau_pmd=tau_pmd, phiIQ=list(phiIQ), datagen=datagen, eval_every=eval_every,
-                                 cells=[sorted(c.items()) for c in cells], **gkw)
+                                 cells=[sorted(c.items()) for c in cells], **mkw)
             ck = os.path.join(checkpoint_dir, f"{loss_type}_{mod}_M{M}_B{batch_len}_F{flex_step}_R{symb_rate:g}_n{len(cells)}_f{num_frames}"
                                               f"_{sig[:12]}.npz")
             have = 0
             if rank == 0 and os.path.exists(ck):
                 z = np.load(ck)
-                if "signature" in z.files and str(z["signature"]) == sig and (not gmi or "gmi" in z.files):
+                if "signature" in z.files and str(z["signature"]) == sig and all(m in z.files for m in metrics):
                     have = 1
                     for k, (idx, _) in enumerate(members):
                         SER[(slice(None),) + idx] = torch.from_numpy(z["ser"][k]).to(dev)
                         Var_est[(slice(None),) + idx] = torch.from_numpy(z["ve"][k]).to(dev)
                         var_real[(slice(None),) + idx + (0,)] = torch.from_numpy(z["var"][k]).to(dev)
-                        if gmi:
-                            GMI[(slice(None),) + idx] = torch.from_numpy(z["gmi"][k]).to(dev)
+                        for m in metrics:
+                            rates[m][(slice(None),) + idx] = torch.from_numpy(z[m][k]).to(dev)
             if _bcast_flag(have, rank, world, group, dev):           # rank 0 decides (the directory need not be shared); all ranks follow
                 continue
         kw = dict(flex_step=flex_step, channel=channel, symb_rate=symb_rate, tau_cd=tau_cd, tau_pmd=tau_pmd, phiIQ=phiIQ, N_lrhalf=N_lrhalf)
         if runner is not None:                                       # test hook: stands for sweep_vae_dp_sharded
-            res = runner(cells, *common, **kw, **gkw)
+            res = runner(cells, *common, **kw, **mkw)
         elif loss_type in ("VAE", "VAEflex"):
             res = sweep_vae_dp_sharded(cells, *common, kind=loss_type, device=dev, datagen=datagen, eval_every=eval_every,
-                                       verbose=verbose, rank=rank, world=world, group=group, **kw, **gkw)
+                                       verbose=verbose, rank=rank, world=world, group=group, **kw, **mkw)
         else:
-            res = _cma_cells(loss_type, cells, common, kw, dev, rank, world, group, num_frames, datagen=datagen, gmi=gmi)
+            res = _cma_cells(loss_type, cells, common, kw, dev, rank, world, group, num_frames, datagen=datagen, **mkw)
         if res is None:
             continue
         ser, ve, var = res[:3]
         if ck is not None and rank == 0:
-            extra = dict(gmi=res[3].cpu().numpy()) if gmi else {}
+            extra = {m: res[3 + j].cpu().numpy() for j, m in enumerate(metrics)}
             np.savez(ck, ser=ser.cpu().numpy(), ve=ve.cpu().numpy(), var=var.cpu().numpy(), signature=np.array(sig), **extra)
         for k, (idx, _) in enumerate(members):
             SER[(slice(None),) + idx] = ser[k].to(dev)
             Var_est[(slice(None),) + idx] = ve[k].to(dev)
             var_real[(slice(None),) + idx + (0,)] = var[k].to(dev)
-            if gmi:
-                GMI[(slice(None),) + idx] = res[3][k].to(dev)
+            for j, m in enumerate(metrics):
+                rates[m][(slice(None),) + idx] = res[3 + j][k].to(dev)
     if rank != 0:
         return None
-    if gmi:
-        return SER, Var_est, var_real, GMI
-    return SER, Var_est, var_real
+    return (SER, Var_est, var_real) + tuple(rates[m] for m in metrics)
 
 
 def _set_signature(**params):
@@ -469,33 +480,34 @@ def _bcast_flag(flag, rank, world, group, dev):
     return bool(int(t.item()))
 
 
-def _cma_cells(loss_type, cells, common, kw, dev, rank, world, group, num_frames, datagen="gpu", gmi=False):
+def _cma_cells(loss_type, cells, common, kw, dev, rank, world, group, num_frames, datagen="gpu", gmi=False, bmi=False):
     """This rank's share of the cells of a CMA-family run set through the batched engine (sweep_cma_dp), gathered on rank 0."""
     from .parallel import gather_cell_results, shard_cells
     mod, sps, M, batch_len, N_frame_max, nf = common
     mine = shard_cells(cells, rank, world)
-    loc_s, loc_v, loc_r, loc_g = {}, {}, {}, {}
+    metrics = _metrics(gmi, bmi)
+    loc_s, loc_v, loc_r, loc_m = {}, {}, {}, {m: {} for m in metrics}
     if mine:
         res = sweep_cma_dp([c for _, c in mine], mod, sps, M, batch_len, N_frame_max, nf, kw["flex_step"], kw["channel"], kw["symb_rate"],
                            kw["tau_cd"], kw["tau_pmd"], kw["phiIQ"], kw["N_lrhalf"], kind=loss_type, device=dev, datagen=datagen,
-                           **(dict(gmi=True) if gmi else {}))
+                           **{m: True for m in metrics})
         s, v, r = res[:3]
         for k, (i, _) in enumerate(mine):
             loc_s[i], loc_v[i], loc_r[i] = s[k], v[k], r[k]
-            if gmi:
-                loc_g[i] = res[3][k]
+            for j, m in enumerate(metrics):
+                loc_m[m][i] = res[3 + j][k]
     n = len(cells)
     out = (gather_cell_results(loc_s, n, (4, num_frames), rank, world, group, dev), gather_cell_results(loc_v, n, (2, num_frames), rank, world, group, dev),
            gather_cell_results(loc_r, n, (2,), rank, world, group, dev))
-    if gmi:
-        out = out + (_gather_with_nan(loc_g, n, (2, num_frames), rank, world, group, dev),)
+    out = out + tuple(_gather_with_nan(loc_m[m], n, (2, num_frames), rank, world, group, dev) for m in metrics)
     return out if rank == 0 else None
 
 
 def save_mat(path, SER, Var_est, var_real, *, SNR_vec, nu_vec, theta_diff_vec, theta_vec, M_vec, lr_optim_vec, batch_len_vec, symb_rate_vec,
-             flex_step_vec, GMI=None):
+             flex_step_vec, GMI=None, BMI=None):
     """The .mat file of Eval_run_DP.py:99-114: one struct 'dict' with the result arrays and the parameter lists under the same keys.
-    GMI (run_dp_sweep(..., gmi=True)), when given, is stored under the extra key 'GMI'; without it the file is exactly the reference's."""
+    GMI (run_dp_sweep(..., gmi=True)) and BMI (bmi=True), when given, are stored under the extra keys 'GMI' and 'BMI'; without them the
+    file is exactly the reference's."""
     from scipy import io
     d = {"SER": SER.cpu().numpy(), "Var_est": Var_est.cpu().numpy(), "var_real": var_real.cpu().numpy(),
          "SNR": list(SNR_vec), "nu": list(nu_vec), "theta_diff": list(theta_diff_vec), "theta": list(theta_vec),
@@ -503,6 +515,8 @@ def save_mat(path, SER, Var_est, var_real, *, SNR_vec, nu_vec, theta_diff_vec, t
          "symb_rate": list(symb_rate_vec), "symb_step": list(flex_step_vec)}
     if GMI is not None:
         d["GMI"] = GMI.cpu().numpy()
+    if BMI is not None:
+        d["BMI"] = BMI.cpu().numpy()
     io.savemat(path, {"dict": d})
 
 
@@ -536,7 +550,7 @@ def _awgn_host_frames(N, F, M, amps, snr, h_channel, sps, dev, P, rngs):
 
 
 def sweep_vae_awgn(cells, mod, sps, M_est, batch_len, N_valid, N_train, num_epochs, epe, channel, *, device=None, datagen="gpu", verbose=False,
-                   gmi=False):
+                   gmi=False, bmi=False):
     """processing_vaele_awgn (:235-324) for R = len(cells) independent cells in lockstep.
 
     cells: dicts with SNR, nu, lr_optim and optionally seed (default: the cell's index).  Returns SER_valid (R, num_epochs // epe), row k
@@ -546,8 +560,10 @@ def sweep_vae_awgn(cells, mod, sps, M_est, batch_len, N_valid, N_train, num_epoc
     datagen="gpu": every cell's frames from the device generator, keyed by the cell's seed (a cell gives the same SER alone or in any
     batch); "numpy": each cell's frames from np.random.default_rng(seed) in exactly the order processing_vaele_awgn(rng=...) draws them.
     gmi=True: returns (SER_valid, GMI_valid (R, num_epochs // epe)), GMI scored on the SER's symbols under its best rotation
-    (awgn.awgn_gmi_runs)."""
-    from .awgn import AWGNEqualizerRuns, awgn_eval_runs, awgn_gmi_runs, generate_frames_awgn_gpu
+    (awgn.awgn_gmi_runs).  bmi=True: the bit-metric rate of Gray-labelled bits likewise (awgn.awgn_bmi_runs), after GMI when both are on:
+    (SER_valid, GMI_valid, BMI_valid)."""
+    from . import awgn
+    from .awgn import AWGNEqualizerRuns, awgn_eval_runs, generate_frames_awgn_gpu
     from .constants import awgn_constants, upsampled_channel
     dev = _awgn_check(num_epochs, epe, channel, device)
     if datagen not in ("gpu", "numpy"):
@@ -570,8 +586,9 @@ def sweep_vae_awgn(cells, mod, sps, M_est, batch_len, N_valid, N_train, num_epoc
     snr = [float(c["SNR"]) for c in cells]
     n_val = num_epochs // epe
     SER_valid = torch.empty(R, n_val, device=dev, dtype=torch.float32)
-    GMI_valid = torch.empty(R, n_val, device=dev, dtype=torch.float32) if gmi else None
-    P_gmi = P.to(dev) if gmi else None
+    metrics = _metrics(gmi, bmi)
+    rates = {m: torch.empty(R, n_val, device=dev, dtype=torch.float32) for m in metrics}
+    P_rate = P.to(dev) if metrics else None
 
     def host_frames(N, F):
         return _awgn_host_frames(N, F, M, amps, snr, h_channel, sps, dev, [k[1] for k in consts], rngs)
@@ -590,35 +607,33 @@ def sweep_vae_awgn(cells, mod, sps, M_est, batch_len, N_valid, N_train, num_epoc
         q_v, _, _ = eqr.forward(rx_v[:, 0])
         shift, counts, ser = awgn_eval_runs(q_v, tx_v[:, 0], amp_levels)
         SER_valid[:, k] = ser
-        if gmi:
-            GMI_valid[:, k] = awgn_gmi_runs(q_v, tx_v[:, 0], P_gmi, shift, counts)
+        for m in metrics:                                            # awgn.awgn_gmi_runs / awgn_bmi_runs
+            rates[m][:, k] = getattr(awgn, f"awgn_{m}_runs")(q_v, tx_v[:, 0], P_rate, shift, counts)
         if verbose:
             print(epoch - 1, "loss", loss[:, -1].tolist(), "shift", shift.tolist(), "SER", ser.tolist())
-    if gmi:
-        return SER_valid, GMI_valid
-    return SER_valid
+    return (SER_valid,) + tuple(rates[m] for m in metrics) if metrics else SER_valid
 
 
 def sweep_vae_awgn_sharded(cells, *args, rank=0, world=1, group=None, **kw):
     """sweep_vae_awgn over a round-robin share of the cells per rank (one process per GPU); SER_valid of ALL cells on rank 0 (None
-    elsewhere), with gmi=True the pair (SER_valid, GMI_valid).  No data-path collective."""
+    elsewhere), with gmi=True / bmi=True the tuple (SER_valid, GMI_valid, BMI_valid) of those switched on.  No data-path collective."""
     from .parallel import gather_cell_results, shard_cells
     mine = shard_cells(cells, rank, world)
     num_epochs, epe = (args[6], args[7]) if len(args) > 7 else (kw["num_epochs"], kw["epe"])
     dev = _cuda_device(kw.get("device"))
-    gmi = kw.get("gmi", False)
-    loc, loc_g = {}, {}
+    metrics = _metrics(**kw)
+    loc, loc_m = {}, {m: {} for m in metrics}
     if mine:
         res = sweep_vae_awgn([c for _, c in mine], *args, **kw)
-        ser = res[0] if gmi else res
+        ser = res[0] if metrics else res
         loc = {i: ser[k] for k, (i, _) in enumerate(mine)}
-        if gmi:
-            loc_g = {i: res[1][k] for k, (i, _) in enumerate(mine)}
+        for j, m in enumerate(metrics):
+            loc_m[m] = {i: res[1 + j][k] for k, (i, _) in enumerate(mine)}
     ser_g = gather_cell_results(loc, len(cells), (num_epochs // epe,), rank, world, group, dev)
-    if not gmi:
+    if not metrics:
         return ser_g
-    gmi_g = _gather_with_nan(loc_g, len(cells), (num_epochs // epe,), rank, world, group, dev)
-    return None if rank != 0 else (ser_g, gmi_g)
+    rates = tuple(_gather_with_nan(loc_m[m], len(cells), (num_epochs // epe,), rank, world, group, dev) for m in metrics)
+    return None if rank != 0 else (ser_g,) + rates
 
 
 AWGN_AXES = ("batch_len", "lr_optim", "M", "SNR", "nu")           # loop order of Eval_run_shaping_vaele.py (RUN_AWGN:42-58), then iter
@@ -626,7 +641,7 @@ AWGN_AXES = ("batch_len", "lr_optim", "M", "SNR", "nu")           # loop order o
 
 def run_awgn_sweep(mod="64-QAM", sps=2, channel="h1", N_train_vec=(350,), lr_optim_vec=(2e-3,), M_vec=(25,), SNR_vec=(12,), nu_vec=(0.0,),
                    iter=1, N_valid=15000, train_len=1200, num_epochs=500, epe=20, *, device=None, datagen="gpu", rank=0, world=1, group=None,
-                   runner=None, verbose=False, checkpoint_dir=None, gmi=False):
+                   runner=None, verbose=False, checkpoint_dir=None, gmi=False, bmi=False):
     """Eval_run_shaping_vaele.py's loops (RUN_AWGN:42-58) as batched run sets.  As in the reference, the N_train_vec entries are the
     drivers' batch_len and train_len is their N_train (RUN_AWGN:53).  Cells that share (M, batch_len) train in the same launch; with
     world > 1 every rank takes a round-robin share of each set.  Returns on rank 0 (None elsewhere)
@@ -635,19 +650,22 @@ def run_awgn_sweep(mod="64-QAM", sps=2, channel="h1", N_train_vec=(350,), lr_opt
     Cell (.., i) is seeded with its flat index.  checkpoint_dir: rank 0 stores every finished set (one .npz, keyed by the set's full
     parameters); a restarted sweep loads what it finds instead of recomputing.
     gmi=True: also GMI shaped like SER as a 3rd result (sweep_vae_awgn(..., gmi=True); the runner hook is then called with gmi=True and
-    returns (SER_valid, GMI_valid)).  Its checkpoints hold the GMI and are never mixed up with those of gmi=False."""
+    returns (SER_valid, GMI_valid)).  Its checkpoints hold the GMI and are never mixed up with those of gmi=False.
+    bmi=True: likewise the bit-metric rate of Gray-labelled bits (BMI), after GMI when both are on: (SER, epochs, GMI, BMI); the runner
+    hook gets bmi=True and returns (SER_valid, [GMI_valid,] BMI_valid)."""
     if channel not in ("h1", "h2"):
         raise KeyError(f"AWGN driver knows channels h1/h2, got {channel!r}")
     if epe < 1 or num_epochs % epe != 0:
         raise ValueError(f"num_epochs={num_epochs} must be a multiple of epe={epe}")
-    gkw = dict(gmi=True) if gmi else {}                              # gmi=False: every call, name and signature exactly as without GMI
+    metrics = _metrics(gmi, bmi)
+    mkw = {m: True for m in metrics}                                 # a metric off: every call, name and signature exactly as without it
     vecs = dict(batch_len=list(N_train_vec), lr_optim=list(lr_optim_vec), M=list(M_vec), SNR=list(SNR_vec), nu=list(nu_vec))
     dev = torch.device("cpu") if runner is not None and device is None else _cuda_device(device)
 
     def signature(key, cells):
         M, batch_len = key
         return _set_signature(driver="VAELE_AWGN", mod=mod, sps=sps, channel=channel, M=M, batch_len=batch_len, N_valid=N_valid,
-                              train_len=train_len, num_epochs=num_epochs, epe=epe, datagen=datagen, cells=[sorted(c.items()) for c in cells], **gkw)
+                              train_len=train_len, num_epochs=num_epochs, epe=epe, datagen=datagen, cells=[sorted(c.items()) for c in cells], **mkw)
 
     def file_name(key, cells, sig):
         M, batch_len = key
@@ -657,28 +675,28 @@ def run_awgn_sweep(mod="64-QAM", sps=2, channel="h1", N_train_vec=(350,), lr_opt
         M, batch_len = key
         args = (cells, mod, sps, M, batch_len, N_valid, train_len, num_epochs, epe, channel)
         if runner is not None:                                       # test hook: stands for sweep_vae_awgn_sharded
-            return runner(*args, **gkw)
-        return sweep_vae_awgn_sharded(*args, device=dev, datagen=datagen, verbose=verbose, rank=rank, world=world, group=group, **gkw)
+            return runner(*args, **mkw)
+        return sweep_vae_awgn_sharded(*args, device=dev, datagen=datagen, verbose=verbose, rank=rank, world=world, group=group, **mkw)
 
     res = _walk_awgn_sets(AWGN_AXES, vecs, ("M", "batch_len"), iter, num_epochs // epe, dev, checkpoint_dir, rank, world, group, signature,
-                          file_name, run_set, gmi=gmi)
+                          file_name, run_set, metrics=metrics)
     if rank != 0:
         return None
-    if gmi:
-        return res[0], np.arange(0, num_epochs, epe), res[1]
+    if metrics:
+        return (res[0], np.arange(0, num_epochs, epe)) + res[1:]
     return res, np.arange(0, num_epochs, epe)
 
 
-def _walk_awgn_sets(axes, vecs, group_by, iter, n_val, dev, checkpoint_dir, rank, world, group, signature, file_name, run_set, gmi=False):
+def _walk_awgn_sets(axes, vecs, group_by, iter, n_val, dev, checkpoint_dir, rank, world, group, signature, file_name, run_set, metrics=()):
     """The cells of vecs[axes[0]] x ... x iter, seeded by their flat index, grouped into one run set per value of the `group_by` axes.
     Per set: with checkpoint_dir, rank 0 loads the set's file if its stored signature(key, cells) matches (all ranks then skip it);
     otherwise run_set(key, cells) gives SER_valid (n, n_val) on rank 0 (None elsewhere), which rank 0 stores under
-    file_name(key, cells, sig).  Returns SER (shape of the cells, n_val).  gmi=True: run_set gives (SER_valid, GMI_valid), the files
-    hold both and (SER, GMI) is returned."""
+    file_name(key, cells, sig).  Returns SER (shape of the cells, n_val).  metrics (names of RATE_METRICS, in that order): run_set gives
+    (SER_valid, one array per metric), the files hold them under the metrics' names and (SER, one array per metric) is returned."""
     import os
     shape = tuple(len(vecs[a]) for a in axes) + (iter,)
     SER = torch.full(shape + (n_val,), float("nan"), dtype=torch.float32, device=dev)
-    GMI = torch.full(shape + (n_val,), float("nan"), dtype=torch.float32, device=dev) if gmi else None
+    rates = {m: torch.full(shape + (n_val,), float("nan"), dtype=torch.float32, device=dev) for m in metrics}
     groups = {}
     for idx in np.ndindex(*shape):
         c = {a: vecs[a][i] for a, i in zip(axes, idx[:-1])}
@@ -694,26 +712,26 @@ def _walk_awgn_sets(axes, vecs, group_by, iter, n_val, dev, checkpoint_dir, rank
             have = 0
             if rank == 0 and os.path.exists(ck):
                 z = np.load(ck)
-                if "signature" in z.files and str(z["signature"]) == sig and (not gmi or "gmi" in z.files):
+                if "signature" in z.files and str(z["signature"]) == sig and all(m in z.files for m in metrics):
                     have = 1
                     for k, (idx, _) in enumerate(members):
                         SER[idx] = torch.from_numpy(z["ser"][k]).to(dev)
-                        if gmi:
-                            GMI[idx] = torch.from_numpy(z["gmi"][k]).to(dev)
+                        for m in metrics:
+                            rates[m][idx] = torch.from_numpy(z[m][k]).to(dev)
             if _bcast_flag(have, rank, world, group, dev):
                 continue
         res = run_set(key, cells)
         if res is None:
             continue
-        ser, g = res if gmi else (res, None)
+        ser, got = (res[0], res[1:]) if metrics else (res, ())
         if ck is not None and rank == 0:
-            extra = dict(gmi=g.cpu().numpy()) if gmi else {}
+            extra = {m: t.cpu().numpy() for m, t in zip(metrics, got)}
             np.savez(ck, ser=ser.cpu().numpy(), signature=np.array(sig), **extra)
         for k, (idx, _) in enumerate(members):
             SER[idx] = ser[k].to(dev)
-            if gmi:
-                GMI[idx] = g[k].to(dev)
-    return (SER, GMI) if gmi else SER
+            for m, t in zip(metrics, got):
+                rates[m][idx] = t[k].to(dev)
+    return (SER,) + tuple(rates[m] for m in metrics) if metrics else SER
 
 
 # -------------------------------------------------------------------------------------------------
@@ -731,7 +749,7 @@ def sweep_cma_awgn(cells, mod, sps, M_est, N_valid, N_train, num_epochs, epe, ch
     frame k = AWGN_VALID_FRAME0 + k), so a cell with the same seed, N_train and N_valid sees the same frames in both sweeps and the two
     baselines are compared on identical data; a cell gives the same SER alone or in any batch.  "numpy": each cell's frames from
     np.random.default_rng(seed) in exactly the order processing_cma_awgn(rng=...) draws them.
-    No GMI: the AWGN CMA driver makes no posteriors (it decides on the nearest level), so there is no q to score."""
+    No GMI or BMI: the AWGN CMA driver makes no posteriors (it decides on the nearest level), so there is no q to score."""
     from . import awgn_cma as cm
     from .awgn import generate_frames_awgn_gpu
     from .constants import awgn_constants, upsampled_channel
@@ -801,7 +819,7 @@ def run_awgn_cma_sweep(mod="64-QAM", sps=2, channel="h1", lr_optim_vec=(5e-4,), 
     Cell (.., i) is seeded with its flat index, as in run_awgn_sweep.  checkpoint_dir: rank 0 stores every finished set (one .npz named
     AWGNCMA_..., keyed by the set's full parameters; never mistaken for a VAE-LE set of the same directory); a restarted sweep loads what
     it finds instead of recomputing.  runner: stands for sweep_cma_awgn_sharded (called with its positional arguments).
-    No GMI (unlike run_awgn_sweep): the AWGN CMA driver makes no posteriors to score."""
+    No GMI or BMI (unlike run_awgn_sweep): the AWGN CMA driver makes no posteriors to score."""
     if channel not in ("h1", "h2"):
         raise KeyError(f"AWGN driver knows channels h1/h2, got {channel!r}")
     if epe < 1 or num_epochs % epe != 0:
