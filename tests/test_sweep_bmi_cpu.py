@@ -321,7 +321,7 @@ def test_sharded_order_gmi_then_bmi(monkeypatch):
     kw = dict(flex_step=10, channel="h0", symb_rate=90e9, tau_cd=0.0, tau_pmd=0.0, phiIQ=(0.0, 0.0), N_lrhalf=3)
     for mk in (dict(bmi=True), dict(gmi=True, bmi=True)):
         outs = [sweep.sweep_vae_dp_sharded(cells, "64-QAM", 2, 25, 100, 1000, 3, device=dev, **mk),
-                sweep._cma_cells("CMA", cells, ("64-QAM", 2, 25, 100, 1000, 3), kw, dev, 0, 1, None, 3, **mk)]
+                sweep.sweep_cma_dp_sharded(cells, "64-QAM", 2, 25, 100, 1000, 3, kind="CMA", device=dev, **kw, **mk)]
         for out in outs:
             assert len(out) == 3 + len(mk)
             assert float(out[-1][2, 0, 0]) == -22.0 and (len(mk) == 1 or float(out[3][2, 0, 0]) == -8.0)

@@ -81,7 +81,28 @@ def _files(ck):
     return {f: str(np.load(os.path.join(ck, f))["signature"]) for f in sorted(os.listdir(ck))}
 
 
+# the same with the rate metrics on, the CMA loss types and the AWGN CMA sweep
+PINNED_DP_GMI_BMI = {
+    "VAE_64-QAM_M25_B100_F10_R9e+10_n2_f2_88aa446b7735.npz": "88aa446b7735bec60e28bf417cdd1e065f1ed7342de173327b0b8d6de31f2d75",
+    "VAE_64-QAM_M9_B100_F10_R9e+10_n2_f2_6afa2df0556c.npz": "6afa2df0556cc92a611f5371376b3cfb98253b11b11f55076ea7def9237c6c77",
+}
+PINNED_CMA_GMI = {
+    "CMAbatch_64-QAM_M25_B100_F10_R9e+10_n2_f2_c2c8b0b156ba.npz": "c2c8b0b156ba8626c73c88ad734a9b20c1ae8d0a78b5b90e3ddb99af9d409be9",
+    "CMAbatch_64-QAM_M9_B100_F10_R9e+10_n2_f2_46b2c5813710.npz": "46b2c5813710fe651b88f344f0a43d4e3d4219b9ce75b9a53c376c6b2bd2a1d7",
+}
+PINNED_AWGN_BMI = {
+    "AWGN_16-QAM_M25_B200_n2_e4_217ab2bb2855.npz": "217ab2bb28556b28757c75e0fc1e5ecb3e4965742274a8e68be9966c6129406a",
+    "AWGN_16-QAM_M9_B200_n2_e4_24dd245e9443.npz": "24dd245e94433d13eef4bf9b2037ca92aa83ec3c74e4c8ba71a8dac5735a75a8",
+}
+PINNED_AWGN_CMA = {
+    "AWGNCMA_16-QAM_M25_n24_e6_1e7efde9d60f.npz": "1e7efde9d60fd12e36d5b5e38038c519711b16bf7f699bdef8ab9b2ea0b666d0",
+    "AWGNCMA_16-QAM_M9_n24_e6_55137de1e97b.npz": "55137de1e97b1f66544ef6695f8dc5836aef00f20dad33189e117929fa7e14b4",
+}
+
+
 def test_checkpoint_names_and_signatures_pinned_without_gmi(tmp_path):
+    import test_awgn_cma_sweep_cpu as tc
+    import test_sweep_bmi_cpu as tb
     from vae_equalizer_b200 import sweep
     ck_dp, ck_aw = str(tmp_path / "dp"), str(tmp_path / "aw")
     sweep.run_dp_sweep(iter=1, num_frames=2, runner=_dp_runner([]), checkpoint_dir=ck_dp, **DP)
@@ -91,6 +112,16 @@ def test_checkpoint_names_and_signatures_pinned_without_gmi(tmp_path):
     for ck in (ck_dp, ck_aw):
         for f in os.listdir(ck):
             assert "gmi" not in np.load(os.path.join(ck, f)).files
+    pinned = [(PINNED_DP_GMI_BMI, lambda ck: sweep.run_dp_sweep(iter=1, num_frames=2, runner=tb._dp_runner([]), checkpoint_dir=ck, gmi=True,
+                                                                 bmi=True, **tb.DP)),
+              (PINNED_CMA_GMI, lambda ck: sweep.run_dp_sweep(loss_type="CMAbatch", iter=1, num_frames=2, runner=tb._dp_runner([]), checkpoint_dir=ck,
+                                                              gmi=True, **tb.DP)),
+              (PINNED_AWGN_BMI, lambda ck: sweep.run_awgn_sweep(mod="16-QAM", runner=tb._aw_runner([]), checkpoint_dir=ck, bmi=True, **tb.AW)),
+              (PINNED_AWGN_CMA, lambda ck: sweep.run_awgn_cma_sweep(mod="16-QAM", runner=tc._runner([]), checkpoint_dir=ck, **tc.LISTS))]
+    for j, (want, run) in enumerate(pinned):
+        ck = str(tmp_path / f"more{j}")
+        run(ck)
+        assert _files(ck) == want, j
 
 
 def test_dp_checkpoints_never_cross_reused(tmp_path):
@@ -201,7 +232,8 @@ def _sharded_all(rank, world, group=None):
     dev = torch.device("cpu")
     kw = dict(flex_step=10, channel="h0", symb_rate=90e9, tau_cd=0.0, tau_pmd=0.0, phiIQ=(0.0, 0.0), N_lrhalf=NF)
     out = [sweep.sweep_vae_dp_sharded(cells, "64-QAM", 2, 25, 100, 1000, NF, device=dev, rank=rank, world=world, group=group, gmi=True),
-           sweep._cma_cells("CMA", cells, ("64-QAM", 2, 25, 100, 1000, NF), kw, dev, rank, world, group, NF, gmi=True),
+           sweep.sweep_cma_dp_sharded(cells, "64-QAM", 2, 25, 100, 1000, NF, kind="CMA", device=dev, rank=rank, world=world, group=group, gmi=True,
+                                      **kw),
            sweep.sweep_vae_awgn_sharded(cells, "16-QAM", 2, 25, 200, 3000, 1200, 2 * NV, 2, "h1", device=dev, rank=rank, world=world,
                                         group=group, gmi=True)]
     from vae_equalizer_b200.parallel import gather_cell_results
@@ -224,7 +256,7 @@ def _gloo_worker(rank, world, port, q):
 
 
 def test_sharded_gmi_gathers_two_ranks_equal_one(monkeypatch):
-    """sweep_vae_dp_sharded, _cma_cells and sweep_vae_awgn_sharded with gmi=True over two ranks: every rank takes part in every gather
+    """sweep_vae_dp_sharded, sweep_cma_dp_sharded and sweep_vae_awgn_sharded with gmi=True over two ranks: every rank takes part in every gather
     (a collective left to rank 0 would pair with another rank's next one), rank 0 gets the one-rank result with its negative and NaN
     GMI entries, the other ranks None."""
     import socket

@@ -2,8 +2,8 @@
 
 * Sweep sharding: the cells of the reference's parameter sweep (Eval_run_DP.py:68-95: nu x batch_len x lr x M x
   theta_diff x symb_rate x flex_step x theta x SNR x iter) are independent `processing()` calls.  `shard_cells`
-  deals them round-robin to the ranks, `gather_cell_results` reassembles the per-cell result tensors on rank 0.
-  No data-path collective.
+  deals them round-robin to the ranks, `gather_cell_results` reassembles the per-cell result tensors on rank 0, NaN entries
+  included.  No data-path collective.
 * Batch-split of ONE long minibatch (VAE-flex with large batch_len): `BatchSplitDP` gives every rank a contiguous
   symbol range of the window and all-reduces (a) the ELBO partial sums (8 + 2(M-1) doubles) before the backward scale
   kappa = (L-Mh)/C is known and (b) the 16*M tap-gradient floats before the replicated Adam step.  Both messages are
@@ -89,13 +89,16 @@ def sweep_cells(**axes):
 
 def gather_cell_results(local, n_cells: int, shape, rank: int, world: int, group=None, device="cpu"):
     """`local` = {global_index: tensor(shape)} computed by this rank.  Returns the (n_cells, *shape) tensor on rank 0
-    (None elsewhere).  One all_gather of a dense, zero-padded block per rank; cells are disjoint so a sum suffices."""
+    (None elsewhere).  One all_reduce of a dense, zero-padded block per rank; cells are disjoint so a sum suffices.  NaN entries
+    (unscored frames) survive it: the block carries the values with NaN as 0 next to a NaN mask, so values of either sign are kept."""
     block = torch.zeros((n_cells,) + tuple(shape), dtype=torch.float32, device=device)
     for i, t in local.items():
         block[i] = t.to(device=device, dtype=torch.float32)
+    nan = torch.isnan(block)
+    block = torch.stack((block.masked_fill(nan, 0.0), nan.to(torch.float32)))
     if world > 1:
         dist.all_reduce(block, op=dist.ReduceOp.SUM, group=group)
-    return block if rank == 0 else None
+    return block[0].masked_fill(block[1] > 0, float("nan")) if rank == 0 else None
 
 
 def allreduce_sum_(t: torch.Tensor, group=None):

@@ -12,6 +12,11 @@ cells are dealt round-robin (parallel.shard_cells), no data-path collective.
 The AWGN single-polarisation VAE-LE (AWGN_channel/func_VAELE_MQAM_shaping.py, driven by Eval_run_shaping_vaele.py) has the same
 structure: `sweep_vae_awgn` steps all cells of a set together (one launch trains every cell's epochs of a validation period,
 one launch runs the validation forward, four score it, no host sync), `run_awgn_sweep` walks the reference's loops.
+
+The engines share their plumbing: `_dp_source` gives sweep_vae_dp and sweep_cma_dp their per-cell constants and frames,
+`_awgn_setup` / `_awgn_periods` give sweep_vae_awgn and sweep_cma_awgn theirs per validation period, `_shard_gather` runs any
+engine on a rank's share of the cells and gathers its results on rank 0, and `_walk_sets` walks the parameter grid of
+run_dp_sweep, run_awgn_sweep and run_awgn_cma_sweep in run sets, with their checkpoints.
 """
 from __future__ import annotations
 
@@ -57,30 +62,6 @@ def sweep_vae_dp(cells, mod, sps, M_est, batch_len, N_frame_max, num_frames, fle
     if kind not in ("VAE", "VAEflex"):
         raise KeyError(kind)
     N_lrhalf = num_frames if N_lrhalf is None else N_lrhalf
-    phiIQ = np.asarray(phiIQ, dtype=np.complex64)
-    init_cache, uniq, which = {}, [], []                                 # cells of a sweep share few (nu, SNR) pairs: sf.init once per pair
-    for c in cells:
-        key = (float(_cell(c, "nu")), float(_cell(c, "SNR")))
-        if key not in init_cache:
-            init_cache[key] = len(uniq)
-            uniq.append(sfun.init(channel, mod, device, key[0], sps, M_est, key[1]))
-        which.append(init_cache[key])
-    consts = [uniq[i] for i in which]
-    h_channel, amp_levels, amps, pol = consts[0][1], consts[0][3], consts[0][4], consts[0][5]
-    num_lev = int(amp_levels.numel())
-    widx = torch.tensor(which, dtype=torch.long)
-    P_all = torch.stack([torch.as_tensor(k[2], dtype=torch.float32) for k in uniq])[widx]
-    var_all = torch.stack([k[7].to(torch.float32).cpu() for k in uniq])[widx]
-    nu_sc_all = torch.tensor([k[6] for k in uniq], dtype=torch.float32)[widx]
-    pow_mean = [k[8] for k in consts]
-    lr0 = torch.tensor([float(_cell(c, "lr_optim")) for c in cells], dtype=torch.float32).to(device)     # on the device: no copy / sync per frame
-    theta = [float(c.get("theta", 0.0)) for c in cells]
-    theta_diff = [float(c.get("theta_diff", 0.0)) for c in cells]
-    seeds = [int(c.get("seed", i)) for i, c in enumerate(cells)]
-    rngs = [np.random.default_rng(s) for s in seeds]
-    eqr = DPEqualizerRuns(R, M_est, sps, amp_levels, P_all, var_all, nu_sc_all, device=device)
-    amp_dev, var_dev, nu_dev = amp_levels.to(device, torch.float32), var_all.to(device), nu_sc_all.to(device)     # evaluation constants: on the device once
-
     if kind == "VAE":
         m_max = N_frame_max // batch_len
         N_frame = m_max * batch_len                                      # VAELE_DP:38-39
@@ -91,56 +72,39 @@ def sweep_vae_dp(cells, mod, sps, M_est, batch_len, N_frame_max, num_frames, fle
         stride, n_steps = flex_step, m_max // flex_step
         keep_lo, keep_hi = (batch_len - flex_step) // 2, (batch_len + flex_step) // 2
         keep_n, N_keep, kd = keep_hi - keep_lo, m_max, False
+    consts, P_all, var_all, nu_sc_all, frames = _dp_source(cells, mod, sps, M_est, channel, N_frame, num_frames, datagen, device, symb_rate,
+                                                           tau_cd, tau_pmd, phiIQ)
+    amp_levels, pol = consts[0][3], consts[0][5]
+    num_lev = int(amp_levels.numel())
+    pow_mean = [k[8] for k in consts]
+    lr0 = torch.tensor([float(_cell(c, "lr_optim")) for c in cells], dtype=torch.float32).to(device)     # on the device: no copy / sync per frame
+    eqr = DPEqualizerRuns(R, M_est, sps, amp_levels, P_all, var_all, nu_sc_all, device=device)
+    amp_dev, var_dev, nu_dev = amp_levels.to(device, torch.float32), var_all.to(device), nu_sc_all.to(device)     # evaluation constants: on the device once
 
     SER_valid = torch.full((R, 4, num_frames), float("nan"), device=device, dtype=torch.float32)
     Var_est = torch.empty(R, pol, num_frames, device=device, dtype=torch.float32)
     rates = {m: torch.full((R, pol, num_frames), float("nan"), device=device, dtype=torch.float32) for m in metrics}
     P_rate = P_all.to(device) if metrics else None
-    rx_all = None if datagen == "gpu_batched" else torch.empty(R, 2, 2, sps * N_frame, device=device, dtype=torch.float32)
     out_train = torch.empty(R, pol, 2 * num_lev, N_keep, device=device, dtype=torch.float32)
     out_const = torch.empty(R, pol, 2, N_keep, device=device, dtype=torch.float32)
     lr_w = lr0
-    for frame in range(num_frames):
+    for frame, (rx_all, tx_all) in enumerate(frames):
         if frame % N_lrhalf == 0 and frame != 0:
             lr_w = lr0 * 0.5                                             # group 0 only, not cumulative (VAELE_DP:45-46)
-        tx_all = []
-        if datagen == "gpu_batched":                                     # all cells' frames in one batched launch sequence
-            if len(h_channel) != 1:
-                raise sfun._lib.VaeqError("datagen='gpu_batched' implements the optical channel 'h0' only")
-            if frame == 0:                                               # per-run parameters live on the device: no copy / sync per frame
-                snr_dev = torch.tensor([float(c["SNR"]) for c in cells], dtype=torch.float32, device=device)
-                theta_dev = torch.tensor(theta, dtype=torch.float64, device=device)
-                theta_diff_dev = torch.tensor(theta_diff, dtype=torch.float64, device=device)
-                P_dev = P_all.to(device)
-            rx_b, tx_b, _ = generate_frames_gpu(N_frame, amps, snr_dev, P_dev, sps, theta_dev.to(torch.float32), device,
-                                                seeds[0] * 100003 + frame, symb_rate=symb_rate, tau_cd=tau_cd, tau_pmd=tau_pmd, phiIQ=phiIQ)
-            rx_all = rx_b
-            if eval_mode != "batched":
-                tx_all = [tx_b[r] if kind == "VAE" else tx_b[r][:, :, batch_len // 2:m_max + batch_len // 2] for r in range(R)]
-            theta_dev = theta_dev + theta_diff_dev                       # VAELE_DP:47 theta drift per frame
-        else:
-            for r in range(R):
-                rx, tx, _ = _make_frame(datagen, N_frame, amps, cells[r]["SNR"], h_channel, consts[r][2], pol, symb_rate, sps, tau_cd,
-                                        tau_pmd, phiIQ, theta[r], device, rngs[r], seeds[r] * 100003 + frame)
-                rx_all[r].copy_(rx)
-                tx_all.append(tx if kind == "VAE" else tx[:, :, batch_len // 2:m_max + batch_len // 2])     # VAEflex_DP:51
-                theta[r] += theta_diff[r]
+        if kind == "VAEflex":
+            tx_all = tx_all[..., batch_len // 2:m_max + batch_len // 2]  # VAEflex_DP:51
         loss_steps, var_steps = eqr.train_frame(rx_all, batch_len, stride, n_steps, lr_w, lr0, out_train, out_const, keep_lo, keep_n,
                                                 keep_lo_in_dst=kd)
         Var_est[:, :, frame] = var_steps.mean(dim=2)
         if frame % eval_every and frame != num_frames - 1:
             continue
         if eval_mode == "batched":
-            if datagen == "gpu_batched":
-                tx_b4 = tx_b if kind == "VAE" else tx_b[:, :, :, batch_len // 2:m_max + batch_len // 2]
-            else:
-                tx_b4 = torch.stack(tx_all)
             seg_len = batch_len if kind == "VAE" else 0
-            ser, al, counts = sfun.frame_eval_runs(out_train, out_const, tx_b4, amp_dev, var_dev, nu_dev, seg_len, n_cut=N_CUT,
+            ser, al, counts = sfun.frame_eval_runs(out_train, out_const, tx_all, amp_dev, var_dev, nu_dev, seg_len, n_cut=N_CUT,
                                                    return_counts=True)
             SER_valid[:, :, frame] = ser
             for m in metrics:                                            # shared_funcs.gmi_runs / bmi_runs
-                rates[m][:, :, frame] = getattr(sfun, f"{m}_runs")(out_train, tx_b4, P_rate, al, counts, seg_len, n_cut=N_CUT)
+                rates[m][:, :, frame] = getattr(sfun, f"{m}_runs")(out_train, tx_all, P_rate, al, counts, seg_len, n_cut=N_CUT)
             if verbose:
                 print(frame, "loss", loss_steps[:, -1].tolist(), "SER", SER_valid[:, :, frame].tolist())
             continue
@@ -169,6 +133,56 @@ def _check_dp_batch_len(mod, M_est, batch_len):
     if int(batch_len) > lim:
         raise sfun._lib.VaeqError(f"batch_len={batch_len} exceeds the largest batch_len the batched DP engine supports at M_est={M_est}, "
                                   f"{mod}: {lim}")
+
+
+def _dp_source(cells, mod, sps, M_est, channel, N, num_frames, datagen, device, symb_rate, tau_cd, tau_pmd, phiIQ):
+    """The per-cell constants and the frames of the DP channel for the cells of sweep_vae_dp / sweep_cma_dp.
+
+    Returns (consts, P, var, nu_sc, frames): consts[r] is sfun.init's tuple for cell r, P (R, n_lev), var (R, 2) and nu_sc (R,) the
+    float32 host stacks of its P, var and nu_sc entries, and frames an iterator over num_frames pairs (rx (R,2,2,sps*N), tx (R,2,2,N)).
+    datagen="gpu_batched": one batched generation for all cells per frame, keyed by the first cell's seed, theta drifting in float64 on
+    the device; otherwise processing._make_frame per cell, cell r keyed by its own seed ("gpu") or drawing from
+    np.random.default_rng(seed) in frame order ("numpy")."""
+    init_cache, uniq, which = {}, [], []                                 # cells of a sweep share few (nu, SNR) pairs: sf.init once per pair
+    for c in cells:
+        key = (float(_cell(c, "nu")), float(_cell(c, "SNR")))
+        if key not in init_cache:
+            init_cache[key] = len(uniq)
+            uniq.append(sfun.init(channel, mod, device, key[0], sps, M_est, key[1]))
+        which.append(init_cache[key])
+    widx = torch.tensor(which, dtype=torch.long)
+    P = torch.stack([torch.as_tensor(k[2], dtype=torch.float32) for k in uniq])[widx]
+    var = torch.stack([k[7].to(torch.float32).cpu() for k in uniq])[widx]
+    nu_sc = torch.tensor([k[6] for k in uniq], dtype=torch.float32)[widx]
+    consts = [uniq[i] for i in which]
+    return consts, P, var, nu_sc, _dp_frames(cells, consts, P, N, num_frames, sps, datagen, device, symb_rate, tau_cd, tau_pmd, phiIQ)
+
+
+def _dp_frames(cells, consts, P, N, num_frames, sps, datagen, device, symb_rate, tau_cd, tau_pmd, phiIQ):
+    h_channel, amps, pol = consts[0][1], consts[0][4], consts[0][5]
+    phiIQ = np.asarray(phiIQ, dtype=np.complex64)
+    theta = [float(c.get("theta", 0.0)) for c in cells]
+    theta_diff = [float(c.get("theta_diff", 0.0)) for c in cells]
+    seeds = [int(c.get("seed", i)) for i, c in enumerate(cells)]
+    if datagen == "gpu_batched":                                         # all cells' frames in one batched launch sequence
+        if len(h_channel) != 1:
+            raise sfun._lib.VaeqError("datagen='gpu_batched' implements the optical channel 'h0' only")
+        snr_dev = torch.tensor([float(c["SNR"]) for c in cells], dtype=torch.float32, device=device)    # per-run parameters live on the
+        theta_dev = torch.tensor(theta, dtype=torch.float64, device=device)                             # device: no copy / sync per frame
+        theta_diff_dev = torch.tensor(theta_diff, dtype=torch.float64, device=device)
+        P_dev = P.to(device)
+        for frame in range(num_frames):
+            rx, tx, _ = generate_frames_gpu(N, amps, snr_dev, P_dev, sps, theta_dev.to(torch.float32), device, seeds[0] * 100003 + frame,
+                                            symb_rate=symb_rate, tau_cd=tau_cd, tau_pmd=tau_pmd, phiIQ=phiIQ)
+            theta_dev = theta_dev + theta_diff_dev                       # VAELE_DP:47 theta drift per frame
+            yield rx, tx
+        return
+    rngs = [np.random.default_rng(s) for s in seeds]
+    for frame in range(num_frames):
+        fr = [_make_frame(datagen, N, amps, c["SNR"], h_channel, k[2], pol, symb_rate, sps, tau_cd, tau_pmd, phiIQ, theta[r], device, rngs[r],
+                          seeds[r] * 100003 + frame) for r, (c, k) in enumerate(zip(cells, consts))]
+        theta = [t + d for t, d in zip(theta, theta_diff)]
+        yield torch.stack([f[0] for f in fr]), torch.stack([f[1] for f in fr])
 
 
 RATE_METRICS = ("gmi", "bmi")          # the engines' optional rate results, appended after their base results in this order
@@ -200,7 +214,6 @@ def sweep_cma_dp(cells, mod, sps, M_est, batch_len, N_train_max, num_frames, fle
     bmi_runs; eval_mode="batched" only).
     Returns (SER_valid (R,4,num_frames), Var_est zeros (R,2,num_frames), var (R,2)), then GMI with gmi=True and BMI with bmi=True, each
     (R,2,num_frames), in that order."""
-    from .processing import _make_frame
     metrics = _metrics(gmi, bmi)
     _rates_batched_only(metrics, eval_mode)
     device = _cuda_device(device)
@@ -209,49 +222,23 @@ def sweep_cma_dp(cells, mod, sps, M_est, batch_len, N_train_max, num_frames, fle
         raise ValueError("no cells")
     mode = {"CMA": 0, "CMAbatch": 1, "CMAflex": 2}[kind]
     N_lrhalf = num_frames if N_lrhalf is None else N_lrhalf
-    phiIQ = np.asarray(phiIQ, dtype=np.complex64)
-    init_cache, consts = {}, []
-    for c in cells:
-        key = (float(_cell(c, "nu")), float(_cell(c, "SNR")))
-        if key not in init_cache:
-            init_cache[key] = sfun.init(channel, mod, device, key[0], sps, M_est, key[1])
-        consts.append(init_cache[key])
-    h_channel, amp_levels, amps, pol = consts[0][1], consts[0][3], consts[0][4], consts[0][5]
+    consts, P_all, var_all, nu_all, frames = _dp_source(cells, mod, sps, M_est, channel, N_train_max, num_frames, datagen, device, symb_rate,
+                                                        tau_cd, tau_pmd, phiIQ)
+    amp_levels, pol = consts[0][3], consts[0][5]
     lrs = [float(_cell(c, "lr_optim")) for c in cells]
     lr_groups = {}
     for r, lr in enumerate(lrs):                                         # vaeq_cma takes one lr per call: one sub-batch per distinct lr
         lr_groups.setdefault(lr, []).append(r)
-    theta = [float(c.get("theta", 0.0)) for c in cells]
-    theta_diff = [float(c.get("theta_diff", 0.0)) for c in cells]
-    seeds = [int(c.get("seed", i)) for i, c in enumerate(cells)]
-    rngs = [np.random.default_rng(s) for s in seeds]
     h_est = consts[0][0].detach().to(device, torch.float32).unsqueeze(0).repeat(R, 1, 1, 1, 1).contiguous()      # Dirac init per cell (sf:583-585)
     SER_valid = torch.empty(R, 4, num_frames, device=device, dtype=torch.float32)
     Var_est = torch.zeros(R, pol, num_frames, device=device, dtype=torch.float32)
-    var_all = torch.stack([k[7].to(device, torch.float32) for k in consts])
-    nu_all = torch.tensor([float(k[6]) for k in consts], dtype=torch.float32, device=device)
+    var_all, nu_all = var_all.to(device), nu_all.to(device)
     rates = {m: torch.full((R, pol, num_frames), float("nan"), device=device, dtype=torch.float32) for m in metrics}
-    P_rate = torch.stack([torch.as_tensor(k[2], dtype=torch.float32) for k in consts]).to(device) if metrics else None
+    P_rate = P_all.to(device) if metrics else None
     lr_scale = 1.0
-    for frame in range(num_frames):
+    for frame, (rx_all, tx_all) in enumerate(frames):
         if frame % N_lrhalf == 0 and frame != 0:
             lr_scale *= 0.5                                              # cumulative (CMA_DP:31-32)
-        if datagen == "gpu_batched":
-            if len(h_channel) != 1:
-                raise sfun._lib.VaeqError("datagen='gpu_batched' implements the optical channel 'h0' only")
-            if frame == 0:                                               # per-run generator parameters live on the device
-                P_dev = torch.stack([torch.as_tensor(k[2], dtype=torch.float32) for k in consts]).to(device)
-                snr_dev = torch.tensor([float(c["SNR"]) for c in cells], dtype=torch.float32, device=device)
-                theta_dev = torch.tensor(theta, dtype=torch.float64, device=device)
-                theta_diff_dev = torch.tensor(theta_diff, dtype=torch.float64, device=device)
-            rx_all, tx_all, _ = generate_frames_gpu(N_train_max, amps, snr_dev, P_dev, sps, theta_dev.to(torch.float32), device,
-                                                    seeds[0] * 100003 + frame, symb_rate=symb_rate, tau_cd=tau_cd, tau_pmd=tau_pmd, phiIQ=phiIQ)
-            theta_dev = theta_dev + theta_diff_dev
-        else:
-            fr = [_make_frame(datagen, N_train_max, amps, cells[r]["SNR"], h_channel, consts[r][2], pol, symb_rate, sps, tau_cd, tau_pmd,
-                              phiIQ, theta[r], device, rngs[r], seeds[r] * 100003 + frame) for r in range(R)]
-            rx_all, tx_all = torch.stack([f[0] for f in fr]), torch.stack([f[1] for f in fr])
-        theta = [t + d for t, d in zip(theta, theta_diff)]
         out_all = torch.empty(R, 2, 2, rx_all.shape[-1] // sps, device=device, dtype=torch.float32)
         for lr, members in lr_groups.items():
             whole = len(members) == R
@@ -322,41 +309,43 @@ def sweep_vae_dp_sharded(cells, *args, rank=0, world=1, group=None, **kw):
     """Round-robin the cells over the ranks (one process per GPU), run each share as one batched run set, and reassemble
     (SER_valid, Var_est, var) -- plus GMI with gmi=True, then BMI with bmi=True -- for ALL cells on rank 0 (None elsewhere).  No data-path
     collective."""
+    nf = _arg(args, kw, 5, "num_frames")
+    shapes = [(4, nf), (2, nf), (2,)] + [(2, nf)] * len(_metrics(**kw))
+    return _shard_gather(sweep_vae_dp, cells, args, kw, shapes, rank, world, group)
+
+
+def sweep_cma_dp_sharded(cells, *args, rank=0, world=1, group=None, **kw):
+    """sweep_cma_dp over a round-robin share of the cells per rank (one process per GPU); (SER_valid, Var_est, var) -- plus GMI with
+    gmi=True, then BMI with bmi=True -- of ALL cells on rank 0 (None elsewhere).  No data-path collective."""
+    nf = _arg(args, kw, 5, "num_frames")
+    shapes = [(4, nf), (2, nf), (2,)] + [(2, nf)] * len(_metrics(**kw))
+    return _shard_gather(sweep_cma_dp, cells, args, kw, shapes, rank, world, group)
+
+
+def _arg(args, kw, i, name):
+    """An engine's argument given at position i (after the cells) or by name."""
+    return args[i] if len(args) > i else kw[name]
+
+
+def _as_tuple(res):
+    """An engine's results as a tuple (the AWGN engines return a bare SER_valid without rate metrics)."""
+    return res if isinstance(res, tuple) else (res,)
+
+
+def _shard_gather(engine, cells, args, kw, shapes, rank, world, group):
+    """Run engine(cells, *args, **kw) on this rank's round-robin share of the cells (parallel.shard_cells) and gather its results for
+    ALL cells on rank 0, result j as a (len(cells), *shapes[j]) tensor (parallel.gather_cell_results: NaN entries survive).  Every rank
+    takes part in every gather, in the same order, a rank without cells too: a collective left out would pair with another rank's next
+    one.  Returns the engine's convention on rank 0 -- a tuple, or the bare tensor when there is one result -- and None elsewhere."""
     from .parallel import gather_cell_results, shard_cells
     mine = shard_cells(cells, rank, world)
-    num_frames = args[5] if len(args) > 5 else kw["num_frames"]
     dev = _cuda_device(kw.get("device"))
-    metrics = _metrics(**kw)
-    if mine:
-        res = sweep_vae_dp([c for _, c in mine], *args, **kw)
-        ser, ve, var = res[:3]
-    loc_ser = {i: ser[k] for k, (i, _) in enumerate(mine)} if mine else {}
-    loc_ve = {i: ve[k] for k, (i, _) in enumerate(mine)} if mine else {}
-    loc_var = {i: var[k] for k, (i, _) in enumerate(mine)} if mine else {}
-    n = len(cells)
-    # NaN marks unscored frames: carry it through the sum-based gather with a mask
-    ser_g = gather_cell_results({i: torch.nan_to_num(t, nan=-1.0) for i, t in loc_ser.items()}, n, (4, num_frames), rank, world, group, dev)
-    ve_g = gather_cell_results(loc_ve, n, (2, num_frames), rank, world, group, dev)
-    var_g = gather_cell_results(loc_var, n, (2,), rank, world, group, dev)
-    rates = []
-    for j, m in enumerate(metrics):                                  # collectives: every rank takes part, before any rank returns
-        loc_m = {i: res[3 + j][k] for k, (i, _) in enumerate(mine)} if mine else {}
-        rates.append(_gather_with_nan(loc_m, n, (2, num_frames), rank, world, group, dev))
+    res = _as_tuple(engine([c for _, c in mine], *args, **kw)) if mine else ()
+    out = tuple(gather_cell_results({i: res[j][k] for k, (i, _) in enumerate(mine)}, len(cells), shape, rank, world, group, dev)
+                for j, shape in enumerate(shapes))
     if rank != 0:
         return None
-    ser_g = torch.where(ser_g < 0, torch.full_like(ser_g, float("nan")), ser_g)
-    return (ser_g, ve_g, var_g) + tuple(rates)
-
-
-def _gather_with_nan(local, n_cells, shape, rank, world, group, dev):
-    """parallel.gather_cell_results for values of any sign with NaN entries (GMI and BMI can be negative, so NaN cannot be carried as a negative
-    sentinel): the values with NaN as 0 and a NaN mask travel in one block.  (n_cells, *shape) on rank 0, None elsewhere."""
-    from .parallel import gather_cell_results
-    packed = {i: torch.stack((torch.where(torch.isnan(t), torch.zeros_like(t), t), torch.isnan(t).to(t.dtype))) for i, t in local.items()}
-    g = gather_cell_results(packed, n_cells, (2,) + tuple(shape), rank, world, group, dev)
-    if g is None:
-        return None
-    return torch.where(g[:, 1] > 0, torch.full_like(g[:, 0], float("nan")), g[:, 0])
+    return out if len(out) > 1 else out[0]
 
 
 # -------------------------------------------------------------------------------------------------
@@ -388,69 +377,38 @@ def run_dp_sweep(mod="64-QAM", sps=2, loss_type="VAE", channel="h0", nu_vec=(0,)
                 _check_dp_batch_len(mod, M, batch_len)
     vecs = dict(SNR=list(SNR_vec), symb_rate=list(symb_rate_vec), nu=list(nu_vec), theta_diff=list(theta_diff_vec), M=list(M_vec),
                 lr_optim=list(lr_optim_vec), batch_len=list(batch_len_vec), flex_step=list(flex_step_vec), theta=list(theta_vec))
-    shape = tuple(len(vecs[a]) for a in AXES) + (iter,)
     dev = torch.device("cpu") if runner is not None and device is None else _cuda_device(device)
-    SER = torch.full((4,) + shape + (num_frames,), float("nan"), dtype=torch.float32, device=dev)
-    Var_est = torch.zeros((2,) + shape + (num_frames,), dtype=torch.float32, device=dev)
-    var_real = torch.zeros((2,) + shape + (1,), dtype=torch.float32, device=dev)
     metrics = _metrics(gmi, bmi)
-    rates = {m: torch.full((2,) + shape + (num_frames,), float("nan"), dtype=torch.float32, device=dev) for m in metrics}
     mkw = {m: True for m in metrics}                                 # a metric off: every call, name and signature exactly as without it
-    groups = {}
-    for idx in np.ndindex(*shape):
-        c = {a: vecs[a][i] for a, i in zip(AXES, idx[:-1])}
-        c["seed"] = int(np.ravel_multi_index(idx, shape))            # one realisation per (cell, iteration), reproducible
-        groups.setdefault((c["M"], c["batch_len"], c["flex_step"], c["symb_rate"]), []).append((idx, c))
-    for (M, batch_len, flex_step, symb_rate), members in groups.items():
-        cells = [c for _, c in members]
-        common = (mod, sps, M, batch_len, N_frame_max, num_frames)
-        ck, sig = None, None
-        if checkpoint_dir is not None:
-            import os
-            os.makedirs(checkpoint_dir, exist_ok=True)
-            # everything the set's results depend on: the file is only reused by a sweep with the same cells and settings
-            sig = _set_signature(loss_type=loss_type, mod=mod, sps=sps, channel=channel, M=M, batch_len=batch_len, flex_step=flex_step,
-                                 symb_rate=symb_rate, N_frame_max=N_frame_max, num_frames=num_frames, N_lrhalf=N_lrhalf, tau_cd=tau_cd,
-                                 tau_pmd=tau_pmd, phiIQ=list(phiIQ), datagen=datagen, eval_every=eval_every,
-                                 cells=[sorted(c.items()) for c in cells], **mkw)
-            ck = os.path.join(checkpoint_dir, f"{loss_type}_{mod}_M{M}_B{batch_len}_F{flex_step}_R{symb_rate:g}_n{len(cells)}_f{num_frames}"
-                                              f"_{sig[:12]}.npz")
-            have = 0
-            if rank == 0 and os.path.exists(ck):
-                z = np.load(ck)
-                if "signature" in z.files and str(z["signature"]) == sig and all(m in z.files for m in metrics):
-                    have = 1
-                    for k, (idx, _) in enumerate(members):
-                        SER[(slice(None),) + idx] = torch.from_numpy(z["ser"][k]).to(dev)
-                        Var_est[(slice(None),) + idx] = torch.from_numpy(z["ve"][k]).to(dev)
-                        var_real[(slice(None),) + idx + (0,)] = torch.from_numpy(z["var"][k]).to(dev)
-                        for m in metrics:
-                            rates[m][(slice(None),) + idx] = torch.from_numpy(z[m][k]).to(dev)
-            if _bcast_flag(have, rank, world, group, dev):           # rank 0 decides (the directory need not be shared); all ranks follow
-                continue
+
+    def signature(key, cells):
+        M, batch_len, flex_step, symb_rate = key
+        return _set_signature(loss_type=loss_type, mod=mod, sps=sps, channel=channel, M=M, batch_len=batch_len, flex_step=flex_step,
+                              symb_rate=symb_rate, N_frame_max=N_frame_max, num_frames=num_frames, N_lrhalf=N_lrhalf, tau_cd=tau_cd,
+                              tau_pmd=tau_pmd, phiIQ=list(phiIQ), datagen=datagen, eval_every=eval_every,
+                              cells=[sorted(c.items()) for c in cells], **mkw)
+
+    def file_name(key, cells, sig):
+        M, batch_len, flex_step, symb_rate = key
+        return f"{loss_type}_{mod}_M{M}_B{batch_len}_F{flex_step}_R{symb_rate:g}_n{len(cells)}_f{num_frames}_{sig[:12]}.npz"
+
+    def run_set(key, cells):
+        M, batch_len, flex_step, symb_rate = key
+        args = (cells, mod, sps, M, batch_len, N_frame_max, num_frames)
         kw = dict(flex_step=flex_step, channel=channel, symb_rate=symb_rate, tau_cd=tau_cd, tau_pmd=tau_pmd, phiIQ=phiIQ, N_lrhalf=N_lrhalf)
         if runner is not None:                                       # test hook: stands for sweep_vae_dp_sharded
-            res = runner(cells, *common, **kw, **mkw)
-        elif loss_type in ("VAE", "VAEflex"):
-            res = sweep_vae_dp_sharded(cells, *common, kind=loss_type, device=dev, datagen=datagen, eval_every=eval_every,
-                                       verbose=verbose, rank=rank, world=world, group=group, **kw, **mkw)
-        else:
-            res = _cma_cells(loss_type, cells, common, kw, dev, rank, world, group, num_frames, datagen=datagen, **mkw)
-        if res is None:
-            continue
-        ser, ve, var = res[:3]
-        if ck is not None and rank == 0:
-            extra = {m: res[3 + j].cpu().numpy() for j, m in enumerate(metrics)}
-            np.savez(ck, ser=ser.cpu().numpy(), ve=ve.cpu().numpy(), var=var.cpu().numpy(), signature=np.array(sig), **extra)
-        for k, (idx, _) in enumerate(members):
-            SER[(slice(None),) + idx] = ser[k].to(dev)
-            Var_est[(slice(None),) + idx] = ve[k].to(dev)
-            var_real[(slice(None),) + idx + (0,)] = var[k].to(dev)
-            for j, m in enumerate(metrics):
-                rates[m][(slice(None),) + idx] = res[3 + j][k].to(dev)
+            return runner(*args, **kw, **mkw)
+        if loss_type in ("VAE", "VAEflex"):
+            return sweep_vae_dp_sharded(*args, kind=loss_type, device=dev, datagen=datagen, eval_every=eval_every, verbose=verbose, rank=rank,
+                                        world=world, group=group, **kw, **mkw)
+        return sweep_cma_dp_sharded(*args, kind=loss_type, device=dev, datagen=datagen, rank=rank, world=world, group=group, **kw, **mkw)
+
+    res = _walk_sets(AXES, vecs, ("M", "batch_len", "flex_step", "symb_rate"), iter, [("ser", (4, num_frames)), ("ve", (2, num_frames)),
+                     ("var", (2,))], metrics, (2, num_frames), dev, checkpoint_dir, rank, world, group, signature, file_name, run_set)
     if rank != 0:
         return None
-    return (SER, Var_est, var_real) + tuple(rates[m] for m in metrics)
+    SER, Var_est, var_real, *rates = (t.movedim(len(AXES) + 1, 0).contiguous() for t in res)      # component axis first (RUN_DP:52,86)
+    return (SER, Var_est, var_real.unsqueeze(-1)) + tuple(rates)
 
 
 def _set_signature(**params):
@@ -480,29 +438,6 @@ def _bcast_flag(flag, rank, world, group, dev):
     return bool(int(t.item()))
 
 
-def _cma_cells(loss_type, cells, common, kw, dev, rank, world, group, num_frames, datagen="gpu", gmi=False, bmi=False):
-    """This rank's share of the cells of a CMA-family run set through the batched engine (sweep_cma_dp), gathered on rank 0."""
-    from .parallel import gather_cell_results, shard_cells
-    mod, sps, M, batch_len, N_frame_max, nf = common
-    mine = shard_cells(cells, rank, world)
-    metrics = _metrics(gmi, bmi)
-    loc_s, loc_v, loc_r, loc_m = {}, {}, {}, {m: {} for m in metrics}
-    if mine:
-        res = sweep_cma_dp([c for _, c in mine], mod, sps, M, batch_len, N_frame_max, nf, kw["flex_step"], kw["channel"], kw["symb_rate"],
-                           kw["tau_cd"], kw["tau_pmd"], kw["phiIQ"], kw["N_lrhalf"], kind=loss_type, device=dev, datagen=datagen,
-                           **{m: True for m in metrics})
-        s, v, r = res[:3]
-        for k, (i, _) in enumerate(mine):
-            loc_s[i], loc_v[i], loc_r[i] = s[k], v[k], r[k]
-            for j, m in enumerate(metrics):
-                loc_m[m][i] = res[3 + j][k]
-    n = len(cells)
-    out = (gather_cell_results(loc_s, n, (4, num_frames), rank, world, group, dev), gather_cell_results(loc_v, n, (2, num_frames), rank, world, group, dev),
-           gather_cell_results(loc_r, n, (2,), rank, world, group, dev))
-    out = out + tuple(_gather_with_nan(loc_m[m], n, (2, num_frames), rank, world, group, dev) for m in metrics)
-    return out if rank == 0 else None
-
-
 def save_mat(path, SER, Var_est, var_real, *, SNR_vec, nu_vec, theta_diff_vec, theta_vec, M_vec, lr_optim_vec, batch_len_vec, symb_rate_vec,
              flex_step_vec, GMI=None, BMI=None):
     """The .mat file of Eval_run_DP.py:99-114: one struct 'dict' with the result arrays and the parameter lists under the same keys.
@@ -526,15 +461,57 @@ def save_mat(path, SER, Var_est, var_real, *, SNR_vec, nu_vec, theta_diff_vec, t
 AWGN_VALID_FRAME0 = 1 << 20          # device generator: frame indices of the validation frames (training frames are the epoch index)
 
 
-def _awgn_check(num_epochs, epe, channel, device):
+def _awgn_check(num_epochs, epe, channel):
     if channel not in ("h1", "h2"):
         raise KeyError(f"AWGN driver knows channels h1/h2, got {channel!r}")       # :239-242
     if epe < 1 or num_epochs % epe != 0:
         raise ValueError(f"num_epochs={num_epochs} must be a multiple of epe={epe} (the single-run driver fails on its last validation)")
+
+
+def _awgn_setup(cells, mod, channel, num_epochs, epe, device, datagen):
+    """The argument checks of sweep_vae_awgn / sweep_cma_awgn (all before any device work) and their per-cell constants: returns
+    (dev, consts, amp_levels, P, lr), consts[r] being awgn_constants of cell r, P (R, n_lev) float32 on the host and lr (R,) float32
+    on the device."""
+    from .constants import awgn_constants
+    _awgn_check(num_epochs, epe, channel)
     dev = _cuda_device(device)
     if dev.type != "cuda":
         raise sfun._lib.VaeqError(f"device {dev}: the AWGN sweep runs on CUDA devices only, there is no CPU path")
-    return dev
+    if datagen not in ("gpu", "numpy"):
+        raise ValueError(f"datagen={datagen!r}: 'gpu' or 'numpy'")
+    if len(cells) == 0:
+        raise ValueError("no cells")
+    consts = [awgn_constants(mod, float(_cell(c, "nu")), float(_cell(c, "SNR"))) for c in cells]
+    amp_levels = torch.tensor(consts[0][0], device=dev, dtype=torch.float32)
+    P = torch.tensor(np.stack([k[1] for k in consts]), dtype=torch.float32)
+    lr = torch.tensor([float(_cell(c, "lr_optim")) for c in cells], dtype=torch.float32, device=dev)     # the fp32 value CMA() passes
+    return dev, consts, amp_levels, P, lr
+
+
+def _awgn_periods(cells, consts, P, sps, channel, N_train, N_valid, n_val, epe, datagen, dev):
+    """The frames of every validation period k of the AWGN drivers, which validate after epoch e when e % epe == 0: yields
+    (rx (R, n_ep, 2, sps*N_train), rx_v (R, 2, sps*N_valid), tx_v (R, 2, N_valid), the period's last epoch), n_ep = 1 for k = 0 and epe
+    after.  datagen="gpu": the device generator keyed by the cell's seed, training frame = epoch index, validation frame
+    AWGN_VALID_FRAME0 + k; "numpy": each cell's frames from np.random.default_rng(seed) in the order the single-run drivers draw them."""
+    from .awgn import generate_frames_awgn_gpu
+    from .constants import upsampled_channel
+    h_channel = upsampled_channel(channel, sps)
+    M = (len(h_channel) - 1) // sps + 1
+    amps = consts[0][0]
+    seeds = [int(c.get("seed", i)) for i, c in enumerate(cells)]
+    rngs = [np.random.default_rng(s) for s in seeds]
+    snr = [float(c["SNR"]) for c in cells]
+    epoch = 0
+    for k in range(n_val):
+        n_ep = 1 if k == 0 else epe                                  # epochs epoch .. epoch + n_ep - 1, then validate (epoch % epe == 0)
+        if datagen == "gpu":
+            rx, _ = generate_frames_awgn_gpu(N_train, amps, snr, P, h_channel, sps, dev, seeds, frame0=epoch, n_frames=n_ep)
+            rx_v, tx_v = generate_frames_awgn_gpu(N_valid, amps, snr, P, h_channel, sps, dev, seeds, frame0=AWGN_VALID_FRAME0 + k)
+        else:
+            rx, _ = _awgn_host_frames(N_train, n_ep, M, amps, snr, h_channel, sps, dev, [c[1] for c in consts], rngs)
+            rx_v, tx_v = _awgn_host_frames(N_valid, 1, M, amps, snr, h_channel, sps, dev, [c[1] for c in consts], rngs)
+        epoch += n_ep
+        yield rx, rx_v[:, 0], tx_v[:, 0], epoch - 1
 
 
 def _awgn_host_frames(N, F, M, amps, snr, h_channel, sps, dev, P, rngs):
@@ -563,77 +540,34 @@ def sweep_vae_awgn(cells, mod, sps, M_est, batch_len, N_valid, N_train, num_epoc
     (awgn.awgn_gmi_runs).  bmi=True: the bit-metric rate of Gray-labelled bits likewise (awgn.awgn_bmi_runs), after GMI when both are on:
     (SER_valid, GMI_valid, BMI_valid)."""
     from . import awgn
-    from .awgn import AWGNEqualizerRuns, awgn_eval_runs, generate_frames_awgn_gpu
-    from .constants import awgn_constants, upsampled_channel
-    dev = _awgn_check(num_epochs, epe, channel, device)
-    if datagen not in ("gpu", "numpy"):
-        raise ValueError(f"datagen={datagen!r}: 'gpu' or 'numpy'")
-    R = len(cells)
-    if R == 0:
-        raise ValueError("no cells")
+    from .awgn import AWGNEqualizerRuns, awgn_eval_runs
+    dev, consts, amp_levels, P, lr = _awgn_setup(cells, mod, channel, num_epochs, epe, device, datagen)
     if N_train // batch_len < 1:
         raise ValueError(f"N_train={N_train} holds no minibatch of batch_len={batch_len}")
-    h_channel = upsampled_channel(channel, sps)
-    M = (len(h_channel) - 1) // sps + 1
-    consts = [awgn_constants(mod, float(_cell(c, "nu")), float(_cell(c, "SNR"))) for c in cells]
-    amps = consts[0][0]
-    amp_levels = torch.tensor(amps, device=dev, dtype=torch.float32)
-    P = torch.tensor(np.stack([k[1] for k in consts]), dtype=torch.float32)
+    R, n_val = len(cells), num_epochs // epe
     eqr = AWGNEqualizerRuns(R, M_est, sps, amp_levels, P, [k[2] for k in consts], [k[3] for k in consts], device=dev)
-    lr = torch.tensor([float(_cell(c, "lr_optim")) for c in cells], dtype=torch.float32, device=dev)
-    seeds = [int(c.get("seed", i)) for i, c in enumerate(cells)]
-    rngs = [np.random.default_rng(s) for s in seeds]
-    snr = [float(c["SNR"]) for c in cells]
-    n_val = num_epochs // epe
     SER_valid = torch.empty(R, n_val, device=dev, dtype=torch.float32)
     metrics = _metrics(gmi, bmi)
     rates = {m: torch.empty(R, n_val, device=dev, dtype=torch.float32) for m in metrics}
     P_rate = P.to(dev) if metrics else None
-
-    def host_frames(N, F):
-        return _awgn_host_frames(N, F, M, amps, snr, h_channel, sps, dev, [k[1] for k in consts], rngs)
-
-    epoch = 0
-    for k in range(n_val):
-        n_ep = 1 if k == 0 else epe                                  # epochs epoch .. epoch + n_ep - 1, then validate (epoch % epe == 0)
-        if datagen == "gpu":
-            rx, _ = generate_frames_awgn_gpu(N_train, amps, snr, P, h_channel, sps, dev, seeds, frame0=epoch, n_frames=n_ep)
-            rx_v, tx_v = generate_frames_awgn_gpu(N_valid, amps, snr, P, h_channel, sps, dev, seeds, frame0=AWGN_VALID_FRAME0 + k)
-        else:
-            rx, _ = host_frames(N_train, n_ep)
-            rx_v, tx_v = host_frames(N_valid, 1)
+    periods = _awgn_periods(cells, consts, P, sps, channel, N_train, N_valid, n_val, epe, datagen, dev)
+    for k, (rx, rx_v, tx_v, epoch) in enumerate(periods):
         loss = eqr.train_frames(rx, lr, batch_len, N_train)
-        epoch += n_ep
-        q_v, _, _ = eqr.forward(rx_v[:, 0])
-        shift, counts, ser = awgn_eval_runs(q_v, tx_v[:, 0], amp_levels)
+        q_v, _, _ = eqr.forward(rx_v)
+        shift, counts, ser = awgn_eval_runs(q_v, tx_v, amp_levels)
         SER_valid[:, k] = ser
         for m in metrics:                                            # awgn.awgn_gmi_runs / awgn_bmi_runs
-            rates[m][:, k] = getattr(awgn, f"awgn_{m}_runs")(q_v, tx_v[:, 0], P_rate, shift, counts)
+            rates[m][:, k] = getattr(awgn, f"awgn_{m}_runs")(q_v, tx_v, P_rate, shift, counts)
         if verbose:
-            print(epoch - 1, "loss", loss[:, -1].tolist(), "shift", shift.tolist(), "SER", ser.tolist())
+            print(epoch, "loss", loss[:, -1].tolist(), "shift", shift.tolist(), "SER", ser.tolist())
     return (SER_valid,) + tuple(rates[m] for m in metrics) if metrics else SER_valid
 
 
 def sweep_vae_awgn_sharded(cells, *args, rank=0, world=1, group=None, **kw):
     """sweep_vae_awgn over a round-robin share of the cells per rank (one process per GPU); SER_valid of ALL cells on rank 0 (None
     elsewhere), with gmi=True / bmi=True the tuple (SER_valid, GMI_valid, BMI_valid) of those switched on.  No data-path collective."""
-    from .parallel import gather_cell_results, shard_cells
-    mine = shard_cells(cells, rank, world)
-    num_epochs, epe = (args[6], args[7]) if len(args) > 7 else (kw["num_epochs"], kw["epe"])
-    dev = _cuda_device(kw.get("device"))
-    metrics = _metrics(**kw)
-    loc, loc_m = {}, {m: {} for m in metrics}
-    if mine:
-        res = sweep_vae_awgn([c for _, c in mine], *args, **kw)
-        ser = res[0] if metrics else res
-        loc = {i: ser[k] for k, (i, _) in enumerate(mine)}
-        for j, m in enumerate(metrics):
-            loc_m[m] = {i: res[1 + j][k] for k, (i, _) in enumerate(mine)}
-    ser_g = gather_cell_results(loc, len(cells), (num_epochs // epe,), rank, world, group, dev)
-    if not metrics:
-        return ser_g
-    rates = tuple(_gather_with_nan(loc_m[m], len(cells), (num_epochs // epe,), rank, world, group, dev) for m in metrics)
-    return None if rank != 0 else (ser_g,) + rates
+    n_val = _arg(args, kw, 6, "num_epochs") // _arg(args, kw, 7, "epe")
+    return _shard_gather(sweep_vae_awgn, cells, args, kw, [(n_val,)] * (1 + len(_metrics(**kw))), rank, world, group)
 
 
 AWGN_AXES = ("batch_len", "lr_optim", "M", "SNR", "nu")           # loop order of Eval_run_shaping_vaele.py (RUN_AWGN:42-58), then iter
@@ -653,10 +587,7 @@ def run_awgn_sweep(mod="64-QAM", sps=2, channel="h1", N_train_vec=(350,), lr_opt
     returns (SER_valid, GMI_valid)).  Its checkpoints hold the GMI and are never mixed up with those of gmi=False.
     bmi=True: likewise the bit-metric rate of Gray-labelled bits (BMI), after GMI when both are on: (SER, epochs, GMI, BMI); the runner
     hook gets bmi=True and returns (SER_valid, [GMI_valid,] BMI_valid)."""
-    if channel not in ("h1", "h2"):
-        raise KeyError(f"AWGN driver knows channels h1/h2, got {channel!r}")
-    if epe < 1 or num_epochs % epe != 0:
-        raise ValueError(f"num_epochs={num_epochs} must be a multiple of epe={epe}")
+    _awgn_check(num_epochs, epe, channel)
     metrics = _metrics(gmi, bmi)
     mkw = {m: True for m in metrics}                                 # a metric off: every call, name and signature exactly as without it
     vecs = dict(batch_len=list(N_train_vec), lr_optim=list(lr_optim_vec), M=list(M_vec), SNR=list(SNR_vec), nu=list(nu_vec))
@@ -678,60 +609,65 @@ def run_awgn_sweep(mod="64-QAM", sps=2, channel="h1", N_train_vec=(350,), lr_opt
             return runner(*args, **mkw)
         return sweep_vae_awgn_sharded(*args, device=dev, datagen=datagen, verbose=verbose, rank=rank, world=world, group=group, **mkw)
 
-    res = _walk_awgn_sets(AWGN_AXES, vecs, ("M", "batch_len"), iter, num_epochs // epe, dev, checkpoint_dir, rank, world, group, signature,
-                          file_name, run_set, metrics=metrics)
+    n_val = num_epochs // epe
+    res = _walk_sets(AWGN_AXES, vecs, ("M", "batch_len"), iter, [("ser", (n_val,))], metrics, (n_val,), dev, checkpoint_dir, rank, world, group,
+                     signature, file_name, run_set, keep=_AWGN_CELL_KEYS)
     if rank != 0:
         return None
-    if metrics:
-        return (res[0], np.arange(0, num_epochs, epe)) + res[1:]
-    return res, np.arange(0, num_epochs, epe)
+    return (res[0], np.arange(0, num_epochs, epe)) + tuple(res[1:])
 
 
-def _walk_awgn_sets(axes, vecs, group_by, iter, n_val, dev, checkpoint_dir, rank, world, group, signature, file_name, run_set, metrics=()):
+_AWGN_CELL_KEYS = ("SNR", "nu", "lr_optim", "seed")                # what an AWGN cell holds (the set's M and batch_len are its key)
+
+
+def _walk_sets(axes, vecs, group_by, iter, base, metrics, rate_shape, dev, checkpoint_dir, rank, world, group, signature, file_name, run_set,
+               keep=None):
     """The cells of vecs[axes[0]] x ... x iter, seeded by their flat index, grouped into one run set per value of the `group_by` axes.
-    Per set: with checkpoint_dir, rank 0 loads the set's file if its stored signature(key, cells) matches (all ranks then skip it);
-    otherwise run_set(key, cells) gives SER_valid (n, n_val) on rank 0 (None elsewhere), which rank 0 stores under
-    file_name(key, cells, sig).  Returns SER (shape of the cells, n_val).  metrics (names of RATE_METRICS, in that order): run_set gives
-    (SER_valid, one array per metric), the files hold them under the metrics' names and (SER, one array per metric) is returned."""
+    A cell holds its value of every axis and its seed, or only the keys in `keep`.
+    base: (name, per-cell shape) of the sweep's base results; metrics (names of RATE_METRICS, in that order) add one result of
+    rate_shape each.  run_set(key, cells) returns these results for the set's cells, (n, *shape) each and in that order (a bare tensor
+    when there is only one), on rank 0 and None elsewhere.
+    Per set: with checkpoint_dir, rank 0 loads the set's file if its stored signature(key, cells) matches and it holds every metric (all
+    ranks then skip the set); otherwise rank 0 stores what run_set gives under file_name(key, cells, sig), each result under its name.
+    Returns one tensor per result, (*shape of the cells, *per-cell shape): the cell at grid index idx is out[idx]."""
     import os
     shape = tuple(len(vecs[a]) for a in axes) + (iter,)
-    SER = torch.full(shape + (n_val,), float("nan"), dtype=torch.float32, device=dev)
-    rates = {m: torch.full(shape + (n_val,), float("nan"), dtype=torch.float32, device=dev) for m in metrics}
+    results = list(base) + [(m, rate_shape) for m in metrics]
+    out = [torch.full(shape + tuple(s), float("nan"), dtype=torch.float32, device=dev) for _, s in results]
     groups = {}
     for idx in np.ndindex(*shape):
         c = {a: vecs[a][i] for a, i in zip(axes, idx[:-1])}
-        c["seed"] = int(np.ravel_multi_index(idx, shape))
+        c["seed"] = int(np.ravel_multi_index(idx, shape))            # one realisation per (cell, iteration), reproducible
         groups.setdefault(tuple(c[a] for a in group_by), []).append((idx, c))
     for key, members in groups.items():
-        cells = [{k: c[k] for k in ("SNR", "nu", "lr_optim", "seed")} for _, c in members]
+        cells = [c if keep is None else {k: c[k] for k in keep} for _, c in members]
         ck, sig = None, None
         if checkpoint_dir is not None:
             os.makedirs(checkpoint_dir, exist_ok=True)
-            sig = signature(key, cells)
-            ck = os.path.join(checkpoint_dir, file_name(key, cells, sig))
+            sig = signature(key, cells)                              # everything the set's results depend on: the file is only reused
+            ck = os.path.join(checkpoint_dir, file_name(key, cells, sig))     # by a sweep with the same cells and settings
             have = 0
             if rank == 0 and os.path.exists(ck):
                 z = np.load(ck)
                 if "signature" in z.files and str(z["signature"]) == sig and all(m in z.files for m in metrics):
                     have = 1
-                    for k, (idx, _) in enumerate(members):
-                        SER[idx] = torch.from_numpy(z["ser"][k]).to(dev)
-                        for m in metrics:
-                            rates[m][idx] = torch.from_numpy(z[m][k]).to(dev)
-            if _bcast_flag(have, rank, world, group, dev):
+                    for o, (name, _) in zip(out, results):
+                        stored = z[name]
+                        for k, (idx, _) in enumerate(members):
+                            o[idx] = torch.from_numpy(stored[k]).to(dev)
+            if _bcast_flag(have, rank, world, group, dev):           # rank 0 decides (the directory need not be shared); all ranks follow
                 continue
         res = run_set(key, cells)
         if res is None:
             continue
-        ser, got = (res[0], res[1:]) if metrics else (res, ())
+        res = _as_tuple(res)
         if ck is not None and rank == 0:
-            extra = {m: t.cpu().numpy() for m, t in zip(metrics, got)}
-            np.savez(ck, ser=ser.cpu().numpy(), signature=np.array(sig), **extra)
-        for k, (idx, _) in enumerate(members):
-            SER[idx] = ser[k].to(dev)
-            for m, t in zip(metrics, got):
-                rates[m][idx] = t[k].to(dev)
-    return (SER,) + tuple(rates[m] for m in metrics) if metrics else SER
+            arrays = {name: t.cpu().numpy() for (name, _), t in zip(results, res)}
+            np.savez(ck, **{name: arrays[name] for name, _ in base}, signature=np.array(sig), **{m: arrays[m] for m in metrics})
+        for o, t in zip(out, res):
+            for k, (idx, _) in enumerate(members):
+                o[idx] = t[k].to(dev)
+    return out
 
 
 # -------------------------------------------------------------------------------------------------
@@ -751,58 +687,25 @@ def sweep_cma_awgn(cells, mod, sps, M_est, N_valid, N_train, num_epochs, epe, ch
     np.random.default_rng(seed) in exactly the order processing_cma_awgn(rng=...) draws them.
     No GMI or BMI: the AWGN CMA driver makes no posteriors (it decides on the nearest level), so there is no q to score."""
     from . import awgn_cma as cm
-    from .awgn import generate_frames_awgn_gpu
-    from .constants import awgn_constants, upsampled_channel
-    dev = _awgn_check(num_epochs, epe, channel, device)
-    if datagen not in ("gpu", "numpy"):
-        raise ValueError(f"datagen={datagen!r}: 'gpu' or 'numpy'")
-    R = len(cells)
-    if R == 0:
-        raise ValueError("no cells")
-    h_channel = upsampled_channel(channel, sps)
-    M = (len(h_channel) - 1) // sps + 1
-    consts = [awgn_constants(mod, float(_cell(c, "nu")), float(_cell(c, "SNR"))) for c in cells]
-    amps = consts[0][0]
-    amp_levels = torch.tensor(amps, device=dev, dtype=torch.float32)
-    P = torch.tensor(np.stack([k[1] for k in consts]), dtype=torch.float32)
-    lr = torch.tensor([float(_cell(c, "lr_optim")) for c in cells], dtype=torch.float32, device=dev)     # the fp32 value CMA() passes
-    seeds = [int(c.get("seed", i)) for i, c in enumerate(cells)]
-    rngs = [np.random.default_rng(s) for s in seeds]
-    snr = [float(c["SNR"]) for c in cells]
+    dev, consts, amp_levels, P, lr = _awgn_setup(cells, mod, channel, num_epochs, epe, device, datagen)
+    R, n_val = len(cells), num_epochs // epe
     h = torch.zeros(R, 2, M_est, device=dev, dtype=torch.float32)         # cm:233-235
     h[:, 0, M_est // 2] = 1.0
-    n_val = num_epochs // epe
     SER_valid = torch.empty(R, n_val, device=dev, dtype=torch.float32)
-    epoch = 0
-    for k in range(n_val):
-        n_ep = 1 if k == 0 else epe                                  # epochs epoch .. epoch + n_ep - 1, then validate (epoch % epe == 0)
-        if datagen == "gpu":
-            rx, _ = generate_frames_awgn_gpu(N_train, amps, snr, P, h_channel, sps, dev, seeds, frame0=epoch, n_frames=n_ep)
-            rx_v, tx_v = generate_frames_awgn_gpu(N_valid, amps, snr, P, h_channel, sps, dev, seeds, frame0=AWGN_VALID_FRAME0 + k)
-        else:
-            rx, _ = _awgn_host_frames(N_train, n_ep, M, amps, snr, h_channel, sps, dev, [c[1] for c in consts], rngs)
-            rx_v, tx_v = _awgn_host_frames(N_valid, 1, M, amps, snr, h_channel, sps, dev, [c[1] for c in consts], rngs)
-        out_v = cm.CMA_runs(rx, rx_v[:, 0], h, lr, sps)
-        epoch += n_ep
-        shift, _, ser = cm.awgn_cma_eval_runs(cm.CPE(out_v), tx_v[:, 0], amp_levels)
+    for k, (rx, rx_v, tx_v, epoch) in enumerate(_awgn_periods(cells, consts, P, sps, channel, N_train, N_valid, n_val, epe, datagen, dev)):
+        out_v = cm.CMA_runs(rx, rx_v, h, lr, sps)
+        shift, _, ser = cm.awgn_cma_eval_runs(cm.CPE(out_v), tx_v, amp_levels)
         SER_valid[:, k] = ser
         if verbose:
-            print(epoch - 1, "shift", shift.tolist(), "SER", ser.tolist())
+            print(epoch, "shift", shift.tolist(), "SER", ser.tolist())
     return SER_valid
 
 
 def sweep_cma_awgn_sharded(cells, *args, rank=0, world=1, group=None, **kw):
     """sweep_cma_awgn over a round-robin share of the cells per rank (one process per GPU); SER_valid of ALL cells on rank 0 (None
     elsewhere).  No data-path collective."""
-    from .parallel import gather_cell_results, shard_cells
-    mine = shard_cells(cells, rank, world)
-    num_epochs, epe = (args[5], args[6]) if len(args) > 6 else (kw["num_epochs"], kw["epe"])
-    dev = _cuda_device(kw.get("device"))
-    loc = {}
-    if mine:
-        ser = sweep_cma_awgn([c for _, c in mine], *args, **kw)
-        loc = {i: ser[k] for k, (i, _) in enumerate(mine)}
-    return gather_cell_results(loc, len(cells), (num_epochs // epe,), rank, world, group, dev)
+    n_val = _arg(args, kw, 5, "num_epochs") // _arg(args, kw, 6, "epe")
+    return _shard_gather(sweep_cma_awgn, cells, args, kw, [(n_val,)], rank, world, group)
 
 
 AWGN_CMA_AXES = ("lr_optim", "M", "SNR", "nu")                     # index order of run_awgn_cma_sweep's SER, then iter
@@ -820,10 +723,7 @@ def run_awgn_cma_sweep(mod="64-QAM", sps=2, channel="h1", lr_optim_vec=(5e-4,), 
     AWGNCMA_..., keyed by the set's full parameters; never mistaken for a VAE-LE set of the same directory); a restarted sweep loads what
     it finds instead of recomputing.  runner: stands for sweep_cma_awgn_sharded (called with its positional arguments).
     No GMI or BMI (unlike run_awgn_sweep): the AWGN CMA driver makes no posteriors to score."""
-    if channel not in ("h1", "h2"):
-        raise KeyError(f"AWGN driver knows channels h1/h2, got {channel!r}")
-    if epe < 1 or num_epochs % epe != 0:
-        raise ValueError(f"num_epochs={num_epochs} must be a multiple of epe={epe}")
+    _awgn_check(num_epochs, epe, channel)
     vecs = dict(lr_optim=list(lr_optim_vec), M=list(M_vec), SNR=list(SNR_vec), nu=list(nu_vec))
     dev = torch.device("cpu") if runner is not None and device is None else _cuda_device(device)
 
@@ -840,8 +740,9 @@ def run_awgn_cma_sweep(mod="64-QAM", sps=2, channel="h1", lr_optim_vec=(5e-4,), 
             return runner(*args)
         return sweep_cma_awgn_sharded(*args, device=dev, datagen=datagen, verbose=verbose, rank=rank, world=world, group=group)
 
-    SER = _walk_awgn_sets(AWGN_CMA_AXES, vecs, ("M",), iter, num_epochs // epe, dev, checkpoint_dir, rank, world, group, signature, file_name,
-                          run_set)
+    n_val = num_epochs // epe
+    SER, = _walk_sets(AWGN_CMA_AXES, vecs, ("M",), iter, [("ser", (n_val,))], (), (n_val,), dev, checkpoint_dir, rank, world, group, signature,
+                      file_name, run_set, keep=_AWGN_CELL_KEYS)
     if rank != 0:
         return None
     return SER, np.arange(0, num_epochs, epe)
