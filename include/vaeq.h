@@ -410,9 +410,9 @@ int vaeq_awgn_cma_eval_runs(const float *y, int64_t ld_y, int64_t rs_y, const ui
                             float *ser_out, void *scratch, void *stream);
 
 /* ------------------------------------------------------------------------------------------------
- * Synthetic test signal on the device, n_runs independent runs per call (generate_data_shaping sf:65-90, channel 'h0'; the
+ * Synthetic test signal on the device, n_runs independent runs per call (generate_data_shaping sf:65-90; the
  * reference's generator is unseeded, parity is statistical).  The host side (vae_equalizer_b200/datagen.py) runs
- *   vaeq_gen_levels -> vaeq_gen_pulse -> FFT -> vaeq_gen_jones -> IFFT -> vaeq_gen_noise
+ *   vaeq_gen_levels -> vaeq_gen_pulse (channel 'h0') or vaeq_gen_pulse_cplx ('h1', 'h2') -> FFT -> vaeq_gen_jones -> IFFT -> vaeq_gen_noise
  * with the two DFTs of the dispersion step (sf:40, 54) on cuFFT.  Random numbers are Philox4x32-10 outputs keyed by
  * (seed, run, row, position): a run's data does not depend on the batch it is generated in.
  * ---------------------------------------------------------------------------------------------- */
@@ -423,6 +423,10 @@ int vaeq_gen_levels(const float *amps, const float *P, int32_t n_lev, int32_t n_
 /* sf:77-80 (simulate_channel sf:56-63 with a one-tap channel): zero insertion by sps = 2 and 'valid' convolution with the pulse h
  * (n_pulse taps, even); shaped (n_runs,2,2*n_conv - n_pulse) complex64, 16-byte aligned */
 int vaeq_gen_pulse(const float *lev, const float *h, int32_t n_pulse, int32_t n_conv, float *shaped, int32_t n_runs, void *stream);
+/* simulate_channel sf:56-63 with an ISI channel ('h1', 'h2'): the two 'valid' convolutions as one, with the composite filter
+ * taps = rrcfir (*) h_channel (K complex taps, re/im interleaved, K even and <= 128); same layout and checks as vaeq_gen_pulse,
+ * shaped (n_runs,2,2*n_conv - K) complex64, 16-byte aligned */
+int vaeq_gen_pulse_cplx(const float *lev, const float *taps, int32_t K, int32_t n_conv, float *shaped, int32_t n_runs, void *stream);
 /* sf:41-53 in the frequency domain, in place: X (n_runs,2,n) complex64 spectra; Pcd = exp_pmd*exp_cd, Picd = exp_cd/exp_pmd (n) complex64;
  * theta (n_runs) rotation angles; phi0, phi1 the IQ phases (exp_phiIQ = exp(-j phi), sf:44) */
 int vaeq_gen_jones(float *X, const float *Pcd, const float *Picd, const float *theta, float phi0, float phi1, int32_t n, int32_t n_runs,

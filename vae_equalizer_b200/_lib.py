@@ -136,6 +136,7 @@ PROTOTYPES = {
     "vaeq_cpe_scratch_bytes": (_sz, [_i32]),
     "vaeq_gen_levels": (C.c_int, [_vp, _vp, _i32, _i32, _i32, _i32, _u64, _vp, _vp, _i32, _vp]),
     "vaeq_gen_pulse": (C.c_int, [_vp, _vp, _i32, _i32, _vp, _i32, _vp]),
+    "vaeq_gen_pulse_cplx": (C.c_int, [_vp, _vp, _i32, _i32, _vp, _i32, _vp]),
     "vaeq_gen_jones": (C.c_int, [_vp, _vp, _vp, _vp, _f, _f, _i32, _i32, _vp]),
     "vaeq_gen_noise": (C.c_int, [_vp, _vp, _u64, _i32, _i32, _vp, _i32, _vp]),
     "vaeq_cpe": (C.c_int, [_vp, _i32, _vp, _vp, _vp]),

@@ -9,7 +9,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from .datagen import PULSE_SPAN, ROLLOFF, rrcfir
+from .datagen import PULSE_SPAN, ROLLOFF, composite_filter, rrcfir
 
 _F32 = torch.float32
 
@@ -252,10 +252,9 @@ _TAPS_CACHE: dict = {}
 
 def _composite_taps(h_channel, sps, dev):
     """rrcfir (*) h_channel as interleaved (re, im) float32 on the device: one 'valid' FIR for the two of generate_data (:52-53)."""
-    h = np.asarray(h_channel, dtype=np.complex64)
-    key = (h.tobytes(), sps, str(dev))
+    key = (np.asarray(h_channel, dtype=np.complex64).tobytes(), sps, str(dev))
     if key not in _TAPS_CACHE:
-        g = np.convolve(rrcfir(PULSE_SPAN, sps, ROLLOFF).astype(np.complex128), h.astype(np.complex128))
+        g = composite_filter(h_channel, sps)
         _TAPS_CACHE[key] = torch.as_tensor(np.stack((g.real, g.imag), -1).astype(np.float32).reshape(-1), device=dev)
     return _TAPS_CACHE[key]
 

@@ -7,6 +7,7 @@
 //
 //   vaeq_gen_levels  sf:75-76   amplitude levels drawn from the run's pmf P (inverse CDF), float rows + the float16 tx slice (sf:89)
 //   vaeq_gen_pulse   sf:77-80   zero insertion (sps = 2) + 'valid' convolution with the RRC pulse = two polyphase FIRs on the symbol grid
+//   vaeq_gen_pulse_cplx  sf:56-63  the same with the complex composite filter rrcfir (*) h_channel of the ISI channels 'h1' / 'h2'
 //   vaeq_gen_jones   sf:41-53   Y = R^T diag(e_pmd, 1/e_pmd) R X * e_cd per frequency bin, R from the run's rotation angle
 //   vaeq_gen_noise   sf:83-88   + sigma_n (N(0,1) + j N(0,1)), cut to sps*N samples, split into the (R,2,2,L) float32 layout
 //
@@ -63,7 +64,8 @@ __global__ void __launch_bounds__(DG_NT) k_gen_levels(const float *amps, const f
 // grid (ceil(n_conv - K/2, DG_NT), nrows / 2 pols, R): thread u produces the even and the odd output sample 2u, 2u+1 (complex) of one pol:
 //   shaped[2u]   = sum_t h[K-1-2t] sym[u+t],   shaped[2u+1] = sum_t h[K-2-2t] sym[u+1+t],   t = 0 .. K/2-1
 // which is np.convolve(zero-stuffed symbols, h, 'valid') for sps = 2 and an even pulse length K (sf:57-61, 77-80).
-// CPLX: h holds K complex taps (re, im interleaved), the composite pulse * channel filter of the AWGN module (:52-53).
+// CPLX: h holds K complex taps (re, im interleaved), the composite pulse * channel filter of the AWGN module (:52-53) and of the DP
+// generator's ISI channels (sf:56-63).
 template <bool CPLX>
 __global__ void __launch_bounds__(DG_NT) k_gen_pulse(const float *lev, const float *h, int K, int n_conv, int nrows, float2 *shaped) {
     __shared__ float2 we[DG_MAXPULSE / 2], wo[DG_MAXPULSE / 2];
@@ -224,7 +226,9 @@ extern "C" int vaeq_gen_levels(const float *amps, const float *P, int32_t n_lev,
     return VAEQ_OK;
 }
 
-extern "C" int vaeq_gen_pulse(const float *lev, const float *h, int32_t n_pulse, int32_t n_conv, float *shaped, int32_t n_runs, void *stream) {
+// vaeq_gen_pulse (real pulse) and vaeq_gen_pulse_cplx (complex composite filter): the 4 level rows of each run, 2 pols per run
+template <bool CPLX>
+static int gen_pulse(const float *lev, const float *h, int32_t n_pulse, int32_t n_conv, float *shaped, int32_t n_runs, void *stream) {
     VAEQ_CHECK_ARG(lev && h && shaped, "NULL pointer");
     VAEQ_CHECK_ARG(n_pulse >= 2 && n_pulse % 2 == 0 && n_pulse <= DG_MAXPULSE && n_conv > n_pulse / 2 && n_runs > 0 && n_runs <= 65535,
                    "bad sizes (n_pulse=%d must be even and <= %d, n_conv=%d, n_runs=%d)", n_pulse, DG_MAXPULSE, n_conv, n_runs);
@@ -232,10 +236,18 @@ extern "C" int vaeq_gen_pulse(const float *lev, const float *h, int32_t n_pulse,
     cudaStream_t st = (cudaStream_t)stream;
     const int nu = n_conv - n_pulse / 2;
     ktime_begin(VAEQ_K_OTHER, st);
-    k_gen_pulse<false><<<dim3((nu + DG_NT - 1) / DG_NT, 2, n_runs), DG_NT, 0, st>>>(lev, h, n_pulse, n_conv, 4, reinterpret_cast<float2 *>(shaped));
+    k_gen_pulse<CPLX><<<dim3((nu + DG_NT - 1) / DG_NT, 2, n_runs), DG_NT, 0, st>>>(lev, h, n_pulse, n_conv, 4, reinterpret_cast<float2 *>(shaped));
     ktime_end(VAEQ_K_OTHER, st);
     VAEQ_LAUNCH_CHECK("k_gen_pulse");
     return VAEQ_OK;
+}
+
+extern "C" int vaeq_gen_pulse(const float *lev, const float *h, int32_t n_pulse, int32_t n_conv, float *shaped, int32_t n_runs, void *stream) {
+    return gen_pulse<false>(lev, h, n_pulse, n_conv, shaped, n_runs, stream);
+}
+
+extern "C" int vaeq_gen_pulse_cplx(const float *lev, const float *taps, int32_t K, int32_t n_conv, float *shaped, int32_t n_runs, void *stream) {
+    return gen_pulse<true>(lev, taps, K, n_conv, shaped, n_runs, stream);
 }
 
 extern "C" int vaeq_gen_jones(float *X, const float *Pcd, const float *Picd, const float *theta, float phi0, float phi1, int32_t n,

@@ -23,7 +23,7 @@ N_CUT = 10     # symbols cut per minibatch/frame edge (VAELE_DP:40, CMA_DP:26)
 
 def _make_frame(datagen, N, amps, SNR, h_channel, P, pol, symb_rate, sps, tau_cd, tau_pmd, phiIQ, theta, device, rng, frame_seed):
     """One frame of test signal.  datagen="numpy": the reference's host-side generator restated (sf:65-90);
-    datagen="gpu": the same signal model generated on the device (statistical, not bitwise, parity; channel 'h0' only);
+    datagen="gpu": the same signal model generated on the device (statistical, not bitwise, parity; channels 'h0', 'h1', 'h2');
     datagen=<iterator of (rx (2,2,sps*N) float32, tx (2,2,N) float16)>: replay recorded frames (parity tests feed the frames the
     reference's processing() was given, tests/golden/make_golden_drivers.py)."""
     if hasattr(datagen, "__next__"):
@@ -33,11 +33,9 @@ def _make_frame(datagen, N, amps, SNR, h_channel, P, pol, symb_rate, sps, tau_cd
             raise sfun._lib.VaeqError(f"replayed frame has {tx.shape[-1]} symbols / {rx.shape[-1]} samples, the driver asked for {N} symbols")
         return rx, tx, 0.0
     if datagen == "gpu":
-        if len(h_channel) != 1:
-            raise sfun._lib.VaeqError("datagen='gpu' implements the optical channel 'h0' only")
         from .datagen import generate_data_gpu
         return generate_data_gpu(N, amps, SNR, P, sps, theta, device, frame_seed, symb_rate=symb_rate, tau_cd=tau_cd,
-                                 tau_pmd=tau_pmd, phiIQ=phiIQ)
+                                 tau_pmd=tau_pmd, phiIQ=phiIQ, h_channel=h_channel)
     return sfun.generate_data_shaping(N, amps, SNR, h_channel, P, pol, symb_rate, sps, tau_cd, tau_pmd, phiIQ, theta, device, rng=rng)
 
 

@@ -165,15 +165,13 @@ def _dp_frames(cells, consts, P, N, num_frames, sps, datagen, device, symb_rate,
     theta_diff = [float(c.get("theta_diff", 0.0)) for c in cells]
     seeds = [int(c.get("seed", i)) for i, c in enumerate(cells)]
     if datagen == "gpu_batched":                                         # all cells' frames in one batched launch sequence
-        if len(h_channel) != 1:
-            raise sfun._lib.VaeqError("datagen='gpu_batched' implements the optical channel 'h0' only")
         snr_dev = torch.tensor([float(c["SNR"]) for c in cells], dtype=torch.float32, device=device)    # per-run parameters live on the
         theta_dev = torch.tensor(theta, dtype=torch.float64, device=device)                             # device: no copy / sync per frame
         theta_diff_dev = torch.tensor(theta_diff, dtype=torch.float64, device=device)
         P_dev = P.to(device)
         for frame in range(num_frames):
             rx, tx, _ = generate_frames_gpu(N, amps, snr_dev, P_dev, sps, theta_dev.to(torch.float32), device, seeds[0] * 100003 + frame,
-                                            symb_rate=symb_rate, tau_cd=tau_cd, tau_pmd=tau_pmd, phiIQ=phiIQ)
+                                            symb_rate=symb_rate, tau_cd=tau_cd, tau_pmd=tau_pmd, phiIQ=phiIQ, h_channel=h_channel)
             theta_dev = theta_dev + theta_diff_dev                       # VAELE_DP:47 theta drift per frame
             yield rx, tx
         return
