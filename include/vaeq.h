@@ -350,6 +350,24 @@ int vaeq_bmi(const float *q, int64_t ld_q, const uint16_t *tx, int64_t ld_tx, co
 int vaeq_bit_llr_runs(const float *q, int64_t ld_q, int64_t rs_q, int32_t n_lev, int32_t N, int32_t n_runs, float *llr, int64_t ld_llr,
                       int64_t rs_llr, void *stream);
 
+/* extension, not in the reference: the data-aided LMMSE reference equalizer of the DP sweeps (DESIGN.md §2).  Per run, the least-squares
+ * taps of the 2x2 complex butterfly FIR of M taps at 2 samples per symbol that map rx onto the run's own transmitted symbols, over the
+ * symbols I = [E, N - E), E = ceil(mh/2) + n_shift/2, at the decision delay in [-n_shift/2, n_shift/2] of least MSE per output pol
+ * (ties to the smaller |delay|, then the negative one), unbiased by beta = rho / S.  Correlations and the Cholesky solve in double.
+ *   rx (n_runs,2,2,L) float, rows ld_rx apart, runs rs_rx apart, L >= 2 N; tx (n_runs,2,2,N) float16 bits, rows ld_tx, runs rs_tx apart
+ *   W (n_runs,2,4,M) float in the layout of twoXtwoFIR.conv_w.weight, var (n_runs,2) float noise variance per real dimension of the
+ *   unbiased output, delay (n_runs,2) int32, ok (n_runs) int32: 0 where R is not positive definite (W and var are then NaN).
+ * M odd <= 63, N - 2E >= 2M; n_shift up to the limits the call reports.  scratch: vaeq_lmmse_taps_scratch_bytes(M, n_shift, n_runs).
+ * A run's result does not depend on the other runs of the call (bitwise). */
+size_t vaeq_lmmse_taps_scratch_bytes(int32_t M, int32_t n_shift, int32_t n_runs);
+int vaeq_lmmse_taps_runs(const float *rx, int64_t ld_rx, int64_t rs_rx, int32_t L, const uint16_t *tx, int64_t ld_tx, int64_t rs_tx, int32_t N,
+                         int32_t M, int32_t n_shift, int32_t n_runs, float *W, float *var, int32_t *delay, int32_t *ok, void *scratch,
+                         size_t scratch_bytes, void *stream);
+/* twoXtwoFIR.forward's FIR (sf:500-518: zero padding M/2, stride 2) for n_runs runs with per-run taps: rx (n_runs,2,2,L) rows ld_rx apart,
+ * runs rs_rx apart (samples >= L read as zero), W (n_runs,2,4,M) contiguous -> out (n_runs,2,2,N) contiguous. */
+int vaeq_fir_runs(const float *rx, int64_t ld_rx, int64_t rs_rx, int32_t L, const float *W, int32_t M, int32_t N, int32_t n_runs, float *out,
+                  void *stream);
+
 /* ------------------------------------------------------------------------------------------------
  * CMA baselines (sf:341-488) and carrier phase estimation (sf:140-186)
  * ---------------------------------------------------------------------------------------------- */

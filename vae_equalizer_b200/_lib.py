@@ -131,6 +131,9 @@ PROTOTYPES = {
     "vaeq_gmi": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _i32, _i32, _vp, _vp, _vp]),
     "vaeq_bmi": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _i32, _i32, _vp, _vp, _vp]),
     "vaeq_bit_llr_runs": (C.c_int, [_vp, _i64, _i64, _i32, _i32, _i32, _vp, _i64, _i64, _vp]),
+    "vaeq_lmmse_taps_scratch_bytes": (_sz, [_i32, _i32, _i32]),
+    "vaeq_lmmse_taps_runs": (C.c_int, [_vp, _i64, _i64, _i32, _vp, _i64, _i64, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "vaeq_fir_runs": (C.c_int, [_vp, _i64, _i64, _i32, _vp, _i32, _i32, _i32, _vp, _vp]),
     "vaeq_cma_scratch_bytes": (_sz, [_i32, _i32, _i32]),
     "vaeq_cma": (C.c_int, [_i32, _vp, _i32, _f, _vp, _i32, _f, _i32, _i32, _i32, _i32, _vp, _vp, _i32, _vp, _vp]),
     "vaeq_cpe_scratch_bytes": (_sz, [_i32]),

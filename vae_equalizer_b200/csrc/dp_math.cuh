@@ -56,6 +56,22 @@ __device__ __forceinline__ void demap_component(float y, float var, const DemapC
     }
 }
 
+// 2x2 butterfly FIR of one symbol (sf:500-518): x0 is the first sample of the symbol's window in row 0 of four staged sample rows
+// (pol 0 I, pol 0 Q, pol 1 I, pol 1 Q) XN floats apart, Ws the taps (2,4,M).  y = (p0 I, p0 Q, p1 I, p1 Q).
+__device__ __forceinline__ void fir_butterfly(const float *x0, int XN, const float *Ws, int M, float (&y)[4]) {
+    y[0] = y[1] = y[2] = y[3] = 0.f;
+    for (int k = 0; k < M; ++k) {
+        float xI0 = x0[k], xQ0 = x0[XN + k], xI1 = x0[2 * XN + k], xQ1 = x0[3 * XN + k];
+#pragma unroll
+        for (int o = 0; o < 2; ++o) {
+            float wr0 = Ws[(o * 4 + 0) * M + k], wr1 = Ws[(o * 4 + 1) * M + k];
+            float wi0 = Ws[(o * 4 + 2) * M + k], wi1 = Ws[(o * 4 + 3) * M + k];
+            y[2 * o] += wr0 * xI0 + wr1 * xI1 - wi0 * xQ0 - wi1 * xQ1;       // sf:505,509
+            y[2 * o + 1] += wr0 * xQ0 + wr1 * xQ1 + wi0 * xI0 + wi1 * xI1;   // sf:507,509
+        }
+    }
+}
+
 // entropy contribution  sum_l -q_l log(q_l/P_l + 1e-12)   (sf:132)
 template <int NL>
 __device__ __forceinline__ float entropy_component(const float (&q)[NL], const DemapConst &c) {

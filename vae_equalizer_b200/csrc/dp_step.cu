@@ -88,18 +88,8 @@ __device__ __forceinline__ void dp_fwd_body(const DpK &p, float *smem, int cta, 
                     p.m1buf4[u] = mom;
                 }
             } else if (u >= 0 && u < p.B) {
-                float y[4] = {0.f, 0.f, 0.f, 0.f};      // (p0 I, p0 Q, p1 I, p1 Q)
-                const float *x0 = xs + 2 * i;
-                for (int k = 0; k < M; ++k) {
-                    float xI0 = x0[k], xQ0 = x0[XN + k], xI1 = x0[2 * XN + k], xQ1 = x0[3 * XN + k];
-#pragma unroll
-                    for (int o = 0; o < 2; ++o) {
-                        float wr0 = Ws[(o * 4 + 0) * M + k], wr1 = Ws[(o * 4 + 1) * M + k];
-                        float wi0 = Ws[(o * 4 + 2) * M + k], wi1 = Ws[(o * 4 + 3) * M + k];
-                        y[2 * o] += wr0 * xI0 + wr1 * xI1 - wi0 * xQ0 - wi1 * xQ1;       // sf:505,509
-                        y[2 * o + 1] += wr0 * xQ0 + wr1 * xQ1 + wi0 * xI0 + wi1 * xI1;   // sf:507,509
-                    }
-                }
+                float y[4];                              // (p0 I, p0 Q, p1 I, p1 Q)
+                fir_butterfly(xs + 2 * i, XN, Ws, M, y);
                 const bool owned = (i >= H) && (i < H + tn);
                 const bool ent_on = owned && (u >= mh) && (u < p.B - mh);                // sf:132 [mh:-mh] in symbols
                 const bool keep = owned && p.qk != nullptr && (u >= p.keep_lo) && (u < p.keep_lo + p.keep_n);

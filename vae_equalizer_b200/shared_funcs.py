@@ -412,6 +412,66 @@ def soft_dec_runs(out, var, amp_levels, nu_sc):
     return q
 
 
+def _runs_rows(t, name, R, rows, dtype):
+    """Check a (R,2,rows,T) tensor with unit time stride and evenly strided rows (views into longer rows allowed) on the current device."""
+    if not t.is_cuda:
+        raise _lib.VaeqError(f"{name} must be a CUDA tensor: vae_equalizer_b200 has no CPU path")
+    _lib.require_current_device(t, name)
+    if t.dtype != dtype:
+        raise _lib.VaeqError(f"{name} must be {dtype}, got {t.dtype}")
+    if t.dim() != 4 or t.shape[0] != R or t.shape[1] != 2 or t.shape[2] != rows or t.stride(3) != 1 or t.stride(1) != rows * t.stride(2):
+        raise _lib.VaeqError(f"{name}: need (R={R},2,{rows},T) with unit time stride and evenly strided rows, got {tuple(t.shape)} {t.stride()}")
+
+
+@_lib.device_guard
+def lmmse_taps_runs(rx, tx, M_est, n_shift=21):
+    """EXTENSION (not in the reference): the data-aided LMMSE taps of R runs (DESIGN.md §2), the reference curve of the blind equalizers.
+    Per run, the least-squares taps of the 2x2 butterfly FIR of M_est taps (the structure of twoXtwoFIR) that map rx onto the run's own
+    transmitted symbols, at the decision delay of least MSE in [-n_shift//2, n_shift//2] per output pol, unbiased.  Correlations and solve in
+    double on the device, one launch pair for all runs, no host sync; a run's result does not depend on the other runs.
+    rx (R,2,2,2N) float32 and tx (R,2,2,N) float16 (views into longer rows allowed).  Returns W (R,2,4,M_est) float32 in the layout of
+    twoXtwoFIR.conv_w.weight, var (R,2) float32 (noise variance per real dimension of the equalized symbols), delay (R,2) int32 and ok (R,)
+    bool: False where the run's correlation matrix is not positive definite (its W and var are then NaN)."""
+    tx = _tx_bits(tx)
+    R, N, M = int(tx.shape[0]), int(tx.shape[-1]), int(M_est)
+    _runs_rows(rx, "rx", R, 2, _F32)
+    _runs_rows(tx, "tx", R, 2, torch.float16)
+    if rx.shape[-1] != 2 * N:
+        raise _lib.VaeqError(f"rx has {rx.shape[-1]} samples per row, tx {N} symbols: need 2 samples per symbol")
+    lib = _lib.load()
+    dev = rx.device
+    W = torch.empty(R, 2, 4, M, dtype=_F32, device=dev)
+    var = torch.empty(R, 2, dtype=_F32, device=dev)
+    delay = torch.empty(R, 2, dtype=torch.int32, device=dev)
+    ok = torch.empty(R, dtype=torch.int32, device=dev)
+    nb = int(lib.vaeq_lmmse_taps_scratch_bytes(M, int(n_shift), R))
+    scr = _scratch(dev, max(nb, 1))
+    _lib.check(lib.vaeq_lmmse_taps_runs(rx.data_ptr(), int(rx.stride(2)), int(rx.stride(0)), 2 * N, tx.data_ptr(), int(tx.stride(2)),
+                                        int(tx.stride(0)), N, M, int(n_shift), R, W.data_ptr(), var.data_ptr(), delay.data_ptr(), ok.data_ptr(),
+                                        scr.data_ptr(), scr.numel(), _lib.current_stream()), "vaeq_lmmse_taps_runs")
+    return W, var, delay, ok.bool()
+
+
+@_lib.device_guard
+def fir_runs(rx, W):
+    """EXTENSION (not in the reference): twoXtwoFIR's butterfly FIR (sf:500-518, zero padding M//2, stride 2) for R runs with per-run taps in
+    one launch: rx (R,2,2,L) float32 (views into longer rows allowed), W (R,2,4,M) float32 -> out (R,2,2,L//2) float32."""
+    _require_cuda(W, "W")
+    R = int(rx.shape[0]) if rx.dim() == 4 else -1
+    _runs_rows(rx, "rx", R, 2, _F32)
+    _lib.require_current_device(W, "W")
+    if W.dim() != 4 or tuple(W.shape[:3]) != (R, 2, 4) or W.dtype != _F32:
+        raise _lib.VaeqError(f"W: need (R={R},2,4,M) float32, got {tuple(W.shape)} {W.dtype}")
+    lib = _lib.load()
+    L, M = int(rx.shape[-1]), int(W.shape[-1])
+    N = L // 2
+    W = W.contiguous()
+    out = torch.empty(R, 2, 2, N, dtype=_F32, device=rx.device)
+    _lib.check(lib.vaeq_fir_runs(rx.data_ptr(), int(rx.stride(2)), int(rx.stride(0)), L, W.data_ptr(), M, N, R, out.data_ptr(),
+                                 _lib.current_stream()), "vaeq_fir_runs")
+    return out
+
+
 @_lib.device_guard
 def cma_align_rescale(out, align, scale, edge=11):
     """CMA_DP:42-48 for R runs: out (R,2,2,N) rolled by (r, -shift) with the evaluated slice rescaled like SER_constell_shaping leaves it

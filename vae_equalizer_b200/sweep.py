@@ -287,6 +287,61 @@ def sweep_cma_dp(cells, mod, sps, M_est, batch_len, N_train_max, num_frames, fle
     return (SER_valid, Var_est, var_all) + tuple(rates[m] for m in metrics)
 
 
+LMMSE_N_SHIFT = 21     # decision delays [-10, 10] of the LMMSE reference: the evaluation's own shift window (DESIGN.md §2)
+
+
+def sweep_lmmse_dp(cells, mod, sps, M_est, batch_len, N_frame_max, num_frames, flex_step=None, channel="h0", symb_rate=90e9,
+                   tau_cd=-26e-24, tau_pmd=0.1e-12 * np.sqrt(1000), phiIQ=(0.0314, 0.0314), N_lrhalf=None, *, device=None, datagen="gpu",
+                   verbose=False, gmi=False, bmi=False):
+    """EXTENSION (not in the reference): the data-aided LMMSE reference equalizer (DESIGN.md §2) of R = len(cells) cells on the frames
+    sweep_vae_dp(kind="VAE") trains on: same positional arguments, frame length (N_frame_max // batch_len) * batch_len, same frame
+    source (_dp_source), so the same cells and seeds give the same frames.  Per frame: the taps of every cell fitted on that frame's own
+    transmitted symbols (shared_funcs.lmmse_taps_runs), the FIR (fir_runs), soft_dec_runs with the fitted noise variance, and the batched
+    evaluation of the VAE-flex drivers (frame_eval_runs, seg_len = 0), then gmi_runs / bmi_runs on request.  No host sync.
+    What the same 2x2 M_est-tap structure reaches with the symbols known: a blind equalizer below it has not converged, a cell whose
+    LMMSE is poor has a channel no such equalizer can undo.  lr_optim, flex_step and N_lrhalf are ignored.
+    Returns (SER_valid (R,4,num_frames), Var_est (R,2,num_frames), var (R,2)), then GMI with gmi=True and BMI with bmi=True, each
+    (R,2,num_frames).  Var_est is the fitted noise variance per real dimension of the unbiased equalizer output in the symbol domain, NOT the
+    VAE's channel-domain estimate var_est.  A cell-frame whose correlation matrix is not positive definite holds NaN in every result."""
+    metrics = _metrics(gmi, bmi)
+    if sps != 2:
+        raise sfun._lib.VaeqError(f"sps={sps}: the LMMSE reference runs at 2 samples per symbol")
+    device = _cuda_device(device)
+    R = len(cells)
+    if R == 0:
+        raise ValueError("no cells")
+    N_frame = (N_frame_max // batch_len) * batch_len                     # VAELE_DP:38-39, the frame sweep_vae_dp(kind="VAE") trains on
+    consts, P_all, var_all, nu_sc_all, frames = _dp_source(cells, mod, sps, M_est, channel, N_frame, num_frames, datagen, device, symb_rate,
+                                                           tau_cd, tau_pmd, phiIQ)
+    amp_dev, nu_dev = consts[0][3].to(device, torch.float32), nu_sc_all.to(device)
+    pol = consts[0][5]
+    SER_valid = torch.empty(R, 4, num_frames, device=device, dtype=torch.float32)
+    Var_est = torch.empty(R, pol, num_frames, device=device, dtype=torch.float32)
+    rates = {m: torch.empty(R, pol, num_frames, device=device, dtype=torch.float32) for m in metrics}
+    P_rate = P_all.to(device) if metrics else None
+    nan = torch.tensor(float("nan"), device=device)
+    for frame, (rx_all, tx_all) in enumerate(frames):
+        W, v, delay, ok = sfun.lmmse_taps_runs(rx_all, tx_all, M_est, LMMSE_N_SHIFT)
+        z = sfun.fir_runs(rx_all, W)
+        q = sfun.soft_dec_runs(z, v, amp_dev, nu_dev)
+        ser, al, counts = sfun.frame_eval_runs(q, z, tx_all, amp_dev, v, nu_dev, 0, return_counts=True)
+        SER_valid[:, :, frame] = torch.where(ok[:, None], ser, nan)
+        Var_est[:, :, frame] = v
+        for m in metrics:                                                # shared_funcs.gmi_runs / bmi_runs
+            rates[m][:, :, frame] = torch.where(ok[:, None], getattr(sfun, f"{m}_runs")(q, tx_all, P_rate, al, counts, 0), nan)
+        if verbose:
+            print(frame, "delay", delay.tolist(), "SER", SER_valid[:, :, frame].tolist())
+    return (SER_valid, Var_est, var_all.to(device)) + tuple(rates[m] for m in metrics)
+
+
+def sweep_lmmse_dp_sharded(cells, *args, rank=0, world=1, group=None, **kw):
+    """sweep_lmmse_dp over a round-robin share of the cells per rank (one process per GPU); (SER_valid, Var_est, var) -- plus GMI with
+    gmi=True, then BMI with bmi=True -- of ALL cells on rank 0 (None elsewhere).  No data-path collective."""
+    nf = _arg(args, kw, 5, "num_frames")
+    shapes = [(4, nf), (2, nf), (2,)] + [(2, nf)] * len(_metrics(**kw))
+    return _shard_gather(sweep_lmmse_dp, cells, args, kw, shapes, rank, world, group)
+
+
 def _score(kind, what, aligned, tx, sh, batch_len, m_max, pol, num_lev, amp_levels, const):
     """Cut the edges like the single-run drivers (VAELE_DP:73-89 / VAEflex_DP:74-84) and run the SER estimator."""
     tail = 11 + max(abs(sh[0]), abs(sh[1]))
@@ -362,7 +417,9 @@ def run_dp_sweep(mod="64-QAM", sps=2, loss_type="VAE", channel="h0", nu_vec=(0,)
     reference's result arrays on rank 0 (None elsewhere):
         SER (4, SNR, symb_rate, nu, theta_diff, M, lr, batch_len, flex_step, theta, iter, num_frames), Var_est (2, ...), var_real (2, ..., 1)
     loss_type 'VAE' / 'VAEflex' use the batched VAE engine (sweep_vae_dp), the CMA variants the batched CMA engine (sweep_cma_dp: a cell's tap
-    recurrence is sequential in the symbols, the cells of a set run side by side).
+    recurrence is sequential in the symbols, the cells of a set run side by side), 'LMMSE' the data-aided LMMSE reference (sweep_lmmse_dp:
+    with the same parameter lists every cell gets the frames it gets under 'VAE', datagen="gpu_batched" included, since the sets are the same;
+    eval_every does not apply, every frame is scored; checkpoints are named LMMSE_...).
     checkpoint_dir: rank 0 writes each finished run set there (one .npz per set, keyed by the set's parameters); a restarted sweep
     loads what it finds instead of recomputing (the reference only saves once, at the very end: RUN_DP:99-114).
     gmi=True: also GMI (2, SNR, ..., iter, num_frames), shaped like Var_est, as a 4th result (sweep_vae_dp / sweep_cma_dp with gmi=True;
@@ -399,6 +456,8 @@ def run_dp_sweep(mod="64-QAM", sps=2, loss_type="VAE", channel="h0", nu_vec=(0,)
         if loss_type in ("VAE", "VAEflex"):
             return sweep_vae_dp_sharded(*args, kind=loss_type, device=dev, datagen=datagen, eval_every=eval_every, verbose=verbose, rank=rank,
                                         world=world, group=group, **kw, **mkw)
+        if loss_type == "LMMSE":
+            return sweep_lmmse_dp_sharded(*args, device=dev, datagen=datagen, verbose=verbose, rank=rank, world=world, group=group, **kw, **mkw)
         return sweep_cma_dp_sharded(*args, kind=loss_type, device=dev, datagen=datagen, rank=rank, world=world, group=group, **kw, **mkw)
 
     res = _walk_sets(AXES, vecs, ("M", "batch_len", "flex_step", "symb_rate"), iter, [("ser", (4, num_frames)), ("ve", (2, num_frames)),
